@@ -2,7 +2,13 @@
 """Benchmark of the velvet-noise decorrelation hot path (BASELINE.json metric:
 "Gsamples/s out (ch x samples) ... + % HBM roofline vs CPU numpy").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--configs 1,2,3,4,5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--configs 1,2,3,4,5] [--dump-outputs DIR]
+
+Every timed loop on the GPU (kernels, end-to-end calls and the copy probe) runs K steps; the CPU figures beside
+them are bounded samples (one pass, or the best of three), and in --impl reference a step is one such sample of
+config 3.  --dump-outputs DIR writes what the timed steps computed in their last step: config 3's
+and config 4's output slabs as fixed seeded samples (sample_slab), configs 1 and 2 whole, config 5's strengths and
+score matrix; the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 The JSON line's headline (`metric`, `value`, `roofline`, `e2e`, `cpu_baseline`) is BASELINE config 3, the one
 the metric is quoted on: 4096 channels x 10 min @ 48 kHz fp32 with one 30 ms / 30-impulse velvet filter per
@@ -147,8 +153,8 @@ _REF = None
 
 
 def reference_modules():
-    """(decorrelation, optimization) of the UNMODIFIED reference from baseline/_ref (a git-ignored copy of its package
-    made by __graft_entry__.build(); it ships to the GPU box with the snapshot), or None."""
+    """(decorrelation, optimization) of the UNMODIFIED reference from baseline/_ref (a git-ignored copy of its
+    package that __graft_entry__.build() makes from the checkout BASELINE.json's `reference_path` names), or None."""
     global _REF
     if _REF is None:
         _REF = False
@@ -311,11 +317,11 @@ def run_reference(args) -> None:
     workers = max(1, cores)
     ch, frames = 4, 960_000  # 20 s @ 48 kHz per worker and step
     sample = f"{workers} processes x {ch} channels x {frames} frames (20 s @ 48 kHz), C-order (frames, channels) fp32, per step"
-    warm = max(0, min(args.warmup, 10))  # a step is a bounded sample (~0.3 s): K and W are honoured up to 100 / 10
+    warm = args.warmup
     for _ in range(warm):
         cpu_fir_rate(workers, ch, frames)
     t_total = 0.0
-    steps = max(1, min(args.steps, 100))
+    steps = args.steps
     for _ in range(steps):
         _, dt = cpu_fir_rate(workers, ch, frames)
         t_total += dt
@@ -431,6 +437,36 @@ def device_slab(env: Env, channels: int, frames: int, seed: int):
     return x
 
 
+def sample_slab(y, window: int = 1 << 15, points: int = 1 << 19) -> dict:
+    """A fixed sample (seed 0) of a device (channels, frames) float32 output, for --dump-outputs: on up to 16 channels
+    (the first and the last among them) the first and the last `window` frames and two windows at seeded positions,
+    as (channels, 4, window); and `points` samples at seeded positions of the whole slab.  ~10 MB."""
+    import torch
+
+    Cy, L = y.shape
+    rng = np.random.default_rng(0)
+    chans = sorted({0, Cy - 1} | set(rng.choice(Cy, size=min(Cy, 14), replace=False).tolist()))
+    W = min(window, L)
+    starts = [0, L - W] + rng.integers(0, L - W + 1, 2).tolist()
+    windows = torch.stack([torch.stack([y[c, s: s + W] for s in starts]) for c in chans])
+    flat = torch.from_numpy(rng.integers(0, Cy * L, min(points, Cy * L))).to(y.device)
+    return {"windows": windows.cpu().numpy(), "points": y.reshape(-1)[flat].cpu().numpy()}
+
+
+def write_outputs(path: str, outputs: dict) -> None:
+    """DIR/<name>.npy for every array, float32 or float64, at most 64 MB in all."""
+    arrays = {}
+    for name, a in outputs.items():
+        a = np.ascontiguousarray(a)
+        arrays[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64_000_000:
+        raise SystemExit(f"bench: --dump-outputs would write {total} bytes, more than 64 MB")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def oracle_windows(x, y, taps, envelope, windows, halo: int) -> bool:
     """GPU output y[ch, a:b] against the oracle on the excerpt x[ch, a : b + halo] for every (ch, a, b) window."""
     from oracle import vnd_oracle as O
@@ -447,7 +483,7 @@ def oracle_windows(x, y, taps, envelope, windows, halo: int) -> bool:
     return ok
 
 
-def copy_probe(env: Env, nbytes: int, steps: int = 3) -> dict:
+def copy_probe(env: Env, nbytes: int, steps: int) -> dict:
     """Ceiling of any host-buffer path on this box: `nbytes` up and `nbytes` down at the same time between page-locked
     host memory and the device, on two streams, all ranks at once (max over ranks)."""
     torch = env.torch
@@ -523,6 +559,7 @@ def run_cfg3(env: Env, args, lib, N, R, VelvetNoise, C):
     launches = int(env.sum_over_ranks(N.launch_count() - launches0))
     clocks = sampler.stop()
     value = env.world * Cg * L * args.steps / (total_ms * 1e-3) / 1e9
+    outputs = {f"cfg3_y_{k}": v for k, v in sample_slab(y).items()} if args.dump_outputs else {}
 
     kernel_ms = float(np.mean(per_step))
     achieved = BYTES_PER_SAMPLE * Cg * L / (kernel_ms * 1e-3) / 1e9
@@ -564,7 +601,7 @@ def run_cfg3(env: Env, args, lib, N, R, VelvetNoise, C):
         tail = O.fir_class_order(np.ascontiguousarray(hx.array[L - n:]), et, O.DEFAULT_ENVELOPE, Ce)
         same = bool(head.tobytes() == np.ascontiguousarray(out[:n]).tobytes() and tail.tobytes() == np.ascontiguousarray(out[L - n:]).tobytes())
         del out
-        e_steps = max(2, min(args.steps, 5))
+        e_steps = args.steps
         holder = []
 
         def e2e_step():
@@ -572,7 +609,7 @@ def run_cfg3(env: Env, args, lib, N, R, VelvetNoise, C):
             holder.append(vne.convolve(hx.array))
 
         dt = env.timed_wall(e2e_step, e_steps)
-        probe = copy_probe(env, Ce * L * 4)
+        probe = copy_probe(env, Ce * L * 4, e_steps)
         ceiling = env.world * Ce * L / probe["seconds"] / 1e9
         e2e = {"value": env.world * Ce * L * e_steps / dt / 1e9, "unit": UNIT, "h2d_bytes_per_step": Ce * L * 4, "d2h_bytes_per_step": Ce * L * 4,
                "steps": e_steps, "channels": Ce, "frames": L,
@@ -596,8 +633,8 @@ def run_cfg3(env: Env, args, lib, N, R, VelvetNoise, C):
                 holder.clear()  # the result block goes back to the pool before the next call takes it
                 holder.append(vnp.convolve(px))
 
-            dtp = env.timed_wall(pageable_step, 2)
-            e2e["pageable_input"] = {"value": env.world * Cp * L * 2 / dtp / 1e9, "unit": UNIT, "channels": Cp,
+            dtp = env.timed_wall(pageable_step, args.steps)
+            e2e["pageable_input"] = {"value": env.world * Cp * L * args.steps / dtp / 1e9, "unit": UNIT, "channels": Cp,
                                      "note": "ordinary numpy input (staged through page-locked memory by a helper thread), pooled page-locked result"}
             del px
         except Exception as exc:
@@ -608,10 +645,11 @@ def run_cfg3(env: Env, args, lib, N, R, VelvetNoise, C):
         e2e = {"value": None, "unit": UNIT, "error": repr(exc)}
     del x, y
     torch.cuda.empty_cache()
-    return dict(value=value, total_ms=total_ms, warm=warm, clocks=clocks, launches=launches, roofline=roofline, e2e=e2e, parity=parity)
+    return dict(value=value, total_ms=total_ms, warm=warm, clocks=clocks, launches=launches, roofline=roofline, e2e=e2e, parity=parity,
+                outputs=outputs)
 
 
-def run_cfg12(env: Env, which: int, lib, N, R, api):
+def run_cfg12(env: Env, args, which: int, lib, N, R, api):
     """Single stereo files: latency-bound, replicas only.  value = device-resident (CUDA tensor in / out), e2e = numpy in / out."""
     torch = env.torch
     if which == 1:
@@ -637,15 +675,20 @@ def run_cfg12(env: Env, which: int, lib, N, R, api):
     for _ in range(5):
         call(xd)
     torch.cuda.synchronize()
-    steps = 50
+    steps = args.steps
+    last = [None]
+
+    def step():
+        last[0] = call(xd)
+
     launches0 = N.launch_count()
-    per_step, _ = env.timed_events(lambda: call(xd), steps)
+    per_step, _ = env.timed_events(step, steps)
     launches = (N.launch_count() - launches0) // steps
     ms = float(np.median(per_step))
     samples_out = got.size
     for _ in range(5):
         call(x)
-    e_ms = sorted(_timed(lambda: call(x)) for _ in range(30))[15] * 1e3
+    e_ms = sorted(_timed(lambda: call(x)) for _ in range(steps))[steps // 2] * 1e3
     peak, _ = measured_peak_gbs()
     bytes_algo = x.size * 4 + samples_out * out_bytes
     return {
@@ -656,6 +699,7 @@ def run_cfg12(env: Env, which: int, lib, N, R, api):
         "e2e": {"value": samples_out / (e_ms * 1e-3) / 1e6, "unit": "Msamples/s", "ms": e_ms, "h2d_bytes_per_step": int(x.nbytes), "d2h_bytes_per_step": int(got.nbytes),
                 "api": "numpy in -> numpy out through the call above (pageable input, page-locked pooled result)"},
         "parity": parity,
+        "outputs": {f"cfg{which}_out": last[0].cpu().numpy()} if args.dump_outputs else {},
     }
 
 
@@ -690,11 +734,12 @@ def run_cfg4(env: Env, args, lib, N, R, VelvetNoise, C):
         if not oracle_windows(x, y, taps, O.DEFAULT_ENVELOPE, windows, prog.halo):
             raise SystemExit("bench cfg4: GPU output differs from the oracle")
         parity = f"bit-exact vs oracle on channels 0 and {Cg - 1}: {n} frames at the start, the middle and the end"
-    steps = max(3, min(args.steps, 5))
+    steps = args.steps
     sampler = ClockSampler(env.local_rank)
     sampler.start()
     per_step, total_ms = env.timed_events(step, steps)
     clocks = sampler.stop()
+    outputs = {f"cfg4_y_{k}": v for k, v in sample_slab(y).items()} if args.dump_outputs else {}
     value = env.world * Cg * L * steps / (total_ms * 1e-3) / 1e9
     kernel_ms = float(np.mean(per_step))
     peak, _ = measured_peak_gbs()
@@ -712,7 +757,7 @@ def run_cfg4(env: Env, args, lib, N, R, VelvetNoise, C):
                                "interleaved per warp, packed FADD2); the last four chunks of every channel through fir_tile_kernel"},
         "lsu_pipe": {"achieved": lsu_bytes / (kernel_ms * 1e-3) / 1e9, "peak": lsu_peak, "unit": "GB/s", "frac": lsu_bytes / (kernel_ms * 1e-3) / 1e9 / lsu_peak,
                      "note": "the binding bound: 300 taps x 4 B per output through the 128 B/clk/SM shared-memory pipe = 31 Gsamples/s per GPU at 1965 MHz"},
-        "parity": parity,
+        "parity": parity, "outputs": outputs,
     }
     # end to end through the Python API on a narrower page-locked slab
     try:
@@ -729,8 +774,8 @@ def run_cfg4(env: Env, args, lib, N, R, VelvetNoise, C):
             holder.clear()
             holder.append(vne.convolve(hx.array))
 
-        dt = env.timed_wall(e2e_step, 3)
-        res["e2e"] = {"value": env.world * Ce * Le * 3 / dt / 1e9, "unit": UNIT, "h2d_bytes_per_step": Ce * Le * 4, "d2h_bytes_per_step": Ce * Le * 4,
+        dt = env.timed_wall(e2e_step, steps)
+        res["e2e"] = {"value": env.world * Ce * Le * steps / dt / 1e9, "unit": UNIT, "h2d_bytes_per_step": Ce * Le * 4, "d2h_bytes_per_step": Ce * Le * 4,
                       "channels": Ce, "frames": Le, "api": "VelvetNoise.convolve(numpy (frames, channels) C-order, page-locked) -> numpy"}
         del hx, holder
         R.trim_pinned_pool(0)
@@ -765,7 +810,7 @@ def run_cfg5(env: Env, args, lib, N, R, OPT):
             return OPT.optimize_velvet_noise_batch(input_signals=inputs, details=True, **kw)
 
     kappa, info = optimise(resident)  # warm-up (NCCL communicator, arenas)
-    steps = max(1, min(args.steps, 2))
+    steps = args.steps
     launches0 = N.launch_count()
     sampler = ClockSampler(env.local_rank)
     env.barrier()
@@ -776,14 +821,16 @@ def run_cfg5(env: Env, args, lib, N, R, OPT):
     torch.cuda.synchronize()
     dt = env.max_over_ranks(time.perf_counter() - t0) / steps
     clocks = sampler.stop()
+    outputs = {"cfg5_kappa": np.asarray(kappa), "cfg5_scores": np.asarray(info["scores"])} if args.dump_outputs else {}
     launches = int(env.sum_over_ranks(N.launch_count() - launches0)) // steps
     evals = int(env.sum_over_ranks(info["evaluations_local"]))
     # end to end: host clips in (the rank uploads its block inside the call)
     env.barrier()
     t0 = time.perf_counter()
-    kappa_h, info_h = optimise(host)
+    for _ in range(steps):
+        kappa_h, info_h = optimise(host)
     torch.cuda.synchronize()
-    dt_e2e = env.max_over_ranks(time.perf_counter() - t0)
+    dt_e2e = env.max_over_ranks(time.perf_counter() - t0) / steps
     same = bool(np.array_equal(kappa, kappa_h) and np.array_equal(info["scores"], info_h["scores"]))
 
     # grid-stage kernel alone (the dominant kernel): one launch over the rank's clips x all strengths
@@ -794,7 +841,7 @@ def run_cfg5(env: Env, args, lib, N, R, OPT):
     OPT.vn_objective_partials(block, prog)
     sampler = ClockSampler(env.local_rank)
     sampler.start()
-    per_step, _ = env.timed_events(lambda: OPT.vn_objective_partials(block, prog), 3)
+    per_step, _ = env.timed_events(lambda: OPT.vn_objective_partials(block, prog), steps)
     k_clocks = sampler.stop()
     k_ms = float(np.mean(per_step))
     k_evals = (hi - lo) * grid
@@ -838,7 +885,7 @@ def run_cfg5(env: Env, args, lib, N, R, OPT):
         "e2e": {"value": evals / dt_e2e, "unit": "objective evaluations/s", "ms": dt_e2e * 1e3, "h2d_bytes_per_step": int((hi - lo) * 2 * frames * 4),
                 "d2h_bytes_per_step": int(evals * 12 * 8 // max(env.world, 1)), "same_result_as_resident": same,
                 "api": "vndecorrelate_b200.optimization.optimize_velvet_noise_batch(input_signals=numpy clips, ...)"},
-        "parity": parity,
+        "parity": parity, "outputs": outputs,
     }
 
 
@@ -856,13 +903,15 @@ def run_b200(args) -> None:
         lib.vnd_debug_fir_plan.restype = C.c_int
     want = _parse_configs(args.configs)
     main = run_cfg3(env, args, lib, N, R, api.VelvetNoise, C)
+    outputs = main.pop("outputs")
     configs = {}
-    for which, fn in ((1, lambda: run_cfg12(env, 1, lib, N, R, api)), (2, lambda: run_cfg12(env, 2, lib, N, R, api)),
+    for which, fn in ((1, lambda: run_cfg12(env, args, 1, lib, N, R, api)), (2, lambda: run_cfg12(env, args, 2, lib, N, R, api)),
                       (4, lambda: run_cfg4(env, args, lib, N, R, api.VelvetNoise, C)), (5, lambda: run_cfg5(env, args, lib, N, R, OPT))):
         if which not in want:
             continue
         try:
             configs[f"cfg{which}"] = fn()
+            outputs.update(configs[f"cfg{which}"].pop("outputs"))
         except SystemExit:
             raise
         except Exception as exc:  # report, do not hide
@@ -890,6 +939,8 @@ def run_b200(args) -> None:
         except Exception as exc:
             configs["cpu_baseline_error"] = repr(exc)
 
+    if env.rank == 0 and args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     if env.rank == 0:
         line = {
             "metric": METRIC, "value": main["value"], "unit": UNIT, "n_gpus": env.world, "steps": args.steps, "warmup": main["warm"],
@@ -918,7 +969,13 @@ def main() -> None:
     ap.add_argument("--cfg5-frames", type=int, default=CFG5_FRAMES)
     ap.add_argument("--cfg5-grid", type=int, default=CFG5_GRID)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed steps computed in their last step (a fixed sample of the "
+                    "large slabs) as DIR/<name>.npy, float32 / float64, at most 64 MB; same arguments, same inputs")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -9,7 +9,6 @@ for t in 36 22 10; do run "smem kernel, tpc=$t" VND_OBJ_TMEM=0 VND_OBJ_TPC=$t; d
 run "tmem kernel, planned chunks" VND_OBJ_TMEM=1
 for t in 48 16 8; do run "tmem kernel, tpc=$t" VND_OBJ_TMEM=1 VND_OBJ_TPC=$t; done
 echo "== gpu tests (objective, optimisers, cfg5, tmem FIR)"; timeout 900 python -m pytest tests -q -m gpu -k "objective or sweeps or optimis or cfg5 or batch or tmem or size_independent or cfg4 or planar" 2>&1 | tail -8
-cat gpurun_out/cfg5_clip0_parity.json; echo
 echo "== same, every tap through shared memory"; VND_OBJ_TMEM=0 timeout 900 python -m pytest tests -q -m gpu -k "objective or sweeps or optimis or cfg5 or batch" 2>&1 | tail -4
 for rep in 1; do
   (cd .r1copy && timeout 200 python bench.py --steps 10 --warmup 3 --no-cpu-baseline --e2e-channels 2 2>&1 | tail -1 | python -c "
