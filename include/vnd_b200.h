@@ -132,6 +132,27 @@ int vnd_vn_decorrelate_workspace(int64_t frames, int32_t channels, const vnd_epi
 int vnd_vn_decorrelate_dev(const vnd_signal* x, const vnd_signal* out, const vnd_tap_program* taps,
                            const vnd_epilogue* ep, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Batched fused decorrelate: vnd_vn_decorrelate_dev on many stereo clips of any lengths in one call, with a fixed number
+ * of launches per batch (1 without rms_normalize, 3 with it) whatever the number of clips.
+ *   x               : packed float32 (rows, 2) C-order input (x_dtype must be VND_F32), 8-byte aligned; clip i is rows
+ *                     [frame_offsets[i], frame_offsets[i + 1]) - a mono clip is packed with its samples in both columns;
+ *   frame_offsets   : n_clips + 1 int64, starting at 0, non-decreasing, ending at rows;
+ *   program_of_clip : n_clips int32; clip i runs channels 2 k and 2 k + 1 of `taps` (k = program_of_clip[i]), a SEGMENTED
+ *                     program with two channels per distinct filter, each pair packed for that clip's length (taps at or
+ *                     beyond the clip's length removed, as vnd_vn_decorrelate_dev expects);
+ *   ep              : shared by all clips;
+ *   out             : F32 or F64 (rows + n_clips * ep->haas_delay, 2) C-order, clip i from row
+ *                     frame_offsets[i] + i * ep->haas_delay, each clip (frames_i + haas_delay) rows.
+ * Every clip's output is byte-identical to vnd_vn_decorrelate_dev on that clip with its channel pair.  The _dev call
+ * cannot read the device-side offsets: it checks everything else and returns VND_EUNSUPPORTED (before any launch)
+ * when the filter's halo does not fit the batched kernel's shared memory, in which case the clips go through
+ * vnd_vn_decorrelate_dev one by one (the _host call does that itself).  Workspace:
+ * vnd_vn_decorrelate_batch_workspace(rows, n_clips, ep) bytes, 16-byte aligned (0 without rms_normalize). */
+int vnd_vn_decorrelate_batch_workspace(int64_t rows, int32_t n_clips, const vnd_epilogue* ep, size_t* bytes);
+int vnd_vn_decorrelate_batch_dev(const void* x, int32_t x_dtype, int64_t rows, const int64_t* frame_offsets, int32_t n_clips,
+                                 const int32_t* program_of_clip, const vnd_tap_program* taps, const vnd_epilogue* ep, void* out,
+                                 int32_t out_dtype, void* workspace, size_t workspace_bytes, void* stream);
+
 /* numpy axis-0 order sum of squares per channel: strict left-to-right float32 running sum of
  * float32-rounded squares (what np.mean(np.square(a), axis=0) does on a C-order array,
  * utils/dsp.py:107-109).  sums: `channels` float32 values on the device. */
@@ -214,6 +235,14 @@ int vnd_host_free(void* ptr);
 int vnd_sparse_fir_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal* y, const vnd_tap_program* taps);
 int vnd_vn_decorrelate_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal* out,
                             const vnd_tap_program* taps, const vnd_epilogue* ep);
+/* vnd_vn_decorrelate_batch_dev with host buffers (offsets, program indices and tap program on the host too).  Checks
+ * that the offsets start at 0, never decrease and end at rows, and that every program index is in range, before any
+ * copy.  Inputs of 8 MB and more flow through the overlapped pipeline in chunks of whole clips (about
+ * VND_PIPE_CHUNK_MB each); filters whose halo does not fit the batched kernel run clip by clip through
+ * vnd_vn_decorrelate_host. */
+int vnd_vn_decorrelate_batch_host(vnd_ctx* ctx, const void* x, int32_t x_dtype, int64_t rows, const int64_t* frame_offsets,
+                                  int32_t n_clips, const int32_t* program_of_clip, const vnd_tap_program* taps, const vnd_epilogue* ep,
+                                  void* out, int32_t out_dtype);
 int vnd_haas_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal* out, int32_t delay,
                   int32_t delayed_channel, int32_t mode_ms, int32_t mono, int32_t use_width, double width);
 int vnd_stereo_op_host(vnd_ctx* ctx, const vnd_signal* a, const vnd_signal* dry, int32_t op, double width);

@@ -76,6 +76,9 @@ SIGNATURES = {
     "vnd_sparse_fir_dev": (C.c_int, [_P(SignalStruct), _P(SignalStruct), _P(TapProgramStruct), C.c_void_p]),
     "vnd_vn_decorrelate_workspace": (C.c_int, [C.c_int64, C.c_int32, _P(EpilogueStruct), _P(C.c_size_t)]),
     "vnd_vn_decorrelate_dev": (C.c_int, [_P(SignalStruct), _P(SignalStruct), _P(TapProgramStruct), _P(EpilogueStruct), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "vnd_vn_decorrelate_batch_workspace": (C.c_int, [C.c_int64, C.c_int32, _P(EpilogueStruct), _P(C.c_size_t)]),
+    "vnd_vn_decorrelate_batch_dev": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, _P(TapProgramStruct),
+                                               _P(EpilogueStruct), C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]),
     "vnd_colsumsq_seq_f32_dev": (C.c_int, [_P(SignalStruct), C.c_void_p, C.c_void_p]),
     "vnd_haas_dev": (C.c_int, [_P(SignalStruct), _P(SignalStruct), C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_void_p]),
     "vnd_stereo_op_dev": (C.c_int, [_P(SignalStruct), _P(SignalStruct), C.c_int32, C.c_double, C.c_void_p, C.c_size_t, C.c_void_p]),
@@ -98,6 +101,8 @@ SIGNATURES = {
     "vnd_host_free": (C.c_int, [C.c_void_p]),
     "vnd_sparse_fir_host": (C.c_int, [C.c_void_p, _P(SignalStruct), _P(SignalStruct), _P(TapProgramStruct)]),
     "vnd_vn_decorrelate_host": (C.c_int, [C.c_void_p, _P(SignalStruct), _P(SignalStruct), _P(TapProgramStruct), _P(EpilogueStruct)]),
+    "vnd_vn_decorrelate_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p,
+                                                _P(TapProgramStruct), _P(EpilogueStruct), C.c_void_p, C.c_int32]),
     "vnd_haas_host": (C.c_int, [C.c_void_p, _P(SignalStruct), _P(SignalStruct), C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double]),
     "vnd_stereo_op_host": (C.c_int, [C.c_void_p, _P(SignalStruct), _P(SignalStruct), C.c_int32, C.c_double]),
     "vnd_vn_objective_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_int64, _P(TapProgramStruct), C.c_void_p]),

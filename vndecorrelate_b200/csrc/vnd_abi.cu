@@ -12,6 +12,7 @@
 #include <thread>
 #include <vector>
 
+#include "vnd_batch.cuh"
 #include "vnd_common.cuh"
 
 namespace vnd {
@@ -203,6 +204,59 @@ extern "C" int vnd_vn_decorrelate_dev(const vnd_signal* x, const vnd_signal* out
     g = gains;
   }
   return place_launch(scratch, C, 1, L, C, out, g, delay, dch, st);
+}
+
+// Arguments of the batched decorrelate that can be checked without reading device memory.
+static int check_batch(const void* x, int32_t x_dtype, int64_t rows, const void* offsets, int32_t n_clips, const void* program_of_clip,
+                       const vnd_tap_program* taps, const vnd_epilogue* ep, const void* out, int32_t out_dtype) {
+  int rc;
+  VND_REQUIRE(rows >= 0 && n_clips >= 0, VND_EINVAL, "negative extent (rows %lld, n_clips %d)", (long long)rows, n_clips);
+  VND_REQUIRE(n_clips > 0 || rows == 0, VND_EINVAL, "%lld rows but no clips", (long long)rows);
+  VND_REQUIRE(x_dtype == VND_F32, VND_EINVAL, "the packed input must be float32 (decorrelate casts first, decorrelation.py:426)");
+  VND_REQUIRE(out_dtype == VND_F32 || out_dtype == VND_F64, VND_EINVAL, "unknown output dtype %d", out_dtype);
+  VND_REQUIRE(ep != nullptr, VND_EINVAL, "epilogue is null");
+  VND_REQUIRE(ep->haas_delay >= 0, VND_EINVAL, "negative Haas delay");
+  if (ep->haas_delay > 0) VND_REQUIRE(ep->haas_channel == 0 || ep->haas_channel == 1, VND_EINVAL, "haas_channel must be 0 or 1");
+  if ((rc = check_taps(taps))) return rc;
+  VND_REQUIRE(taps->order == VND_ORDER_SEGMENTED, VND_EINVAL, "decorrelate needs a SEGMENTED tap program");
+  VND_REQUIRE(taps->channels % 2 == 0, VND_EINVAL, "the tap program has %d channels: it must hold two per filter", taps->channels);
+  VND_REQUIRE(n_clips == 0 || taps->channels >= 2, VND_EINVAL, "the tap program holds no filter");
+  VND_REQUIRE(x != nullptr || rows == 0, VND_EINVAL, "x is null");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(x) % 8 == 0, VND_EINVAL, "x must be 8-byte aligned (one float32 pair per row)");
+  VND_REQUIRE((offsets != nullptr && program_of_clip != nullptr) || n_clips == 0, VND_EINVAL, "frame_offsets or program_of_clip is null");
+  VND_REQUIRE(out != nullptr || rows + (long long)n_clips * ep->haas_delay == 0, VND_EINVAL, "out is null");
+  return VND_OK;
+}
+
+// Does the batched stereo kernel hold tile + halo of this program?
+static bool batch_fits(const vnd_tap_program* taps, int64_t rows) {
+  long long halo = taps->halo > 0 ? taps->halo : 0;
+  if (halo > rows) halo = rows;
+  size_t smem = 0;
+  return vn_batch_smem((int)halo, 2 * taps->max_channel_words, &smem);
+}
+
+extern "C" int vnd_vn_decorrelate_batch_workspace(int64_t rows, int32_t n_clips, const vnd_epilogue* ep, size_t* bytes) {
+  VND_REQUIRE(bytes != nullptr && ep != nullptr, VND_EINVAL, "null argument");
+  VND_REQUIRE(rows >= 0 && n_clips >= 0, VND_EINVAL, "negative extent");
+  *bytes = vn_batch_workspace_bytes(rows, n_clips, ep->rms_normalize);
+  return VND_OK;
+}
+
+extern "C" int vnd_vn_decorrelate_batch_dev(const void* x, int32_t x_dtype, int64_t rows, const int64_t* frame_offsets, int32_t n_clips,
+                                            const int32_t* program_of_clip, const vnd_tap_program* taps, const vnd_epilogue* ep, void* out,
+                                            int32_t out_dtype, void* workspace, size_t workspace_bytes, void* stream) {
+  int rc;
+  if ((rc = check_batch(x, x_dtype, rows, frame_offsets, n_clips, program_of_clip, taps, ep, out, out_dtype))) return rc;
+  if (n_clips == 0) return VND_OK;
+  VND_REQUIRE(batch_fits(taps, rows), VND_EUNSUPPORTED,
+              "a halo of %d frames does not fit the batched kernel; run these clips through vnd_vn_decorrelate_dev", taps->halo);
+  const size_t need = vn_batch_workspace_bytes(rows, n_clips, ep->rms_normalize);
+  VND_REQUIRE(need == 0 || (workspace != nullptr && workspace_bytes >= need), VND_ENOMEM, "workspace too small: need %zu bytes, have %zu",
+              need, workspace_bytes);
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(workspace) % 16 == 0, VND_EINVAL, "workspace must be 16-byte aligned");
+  return vn_batch_launch(reinterpret_cast<const float*>(x), rows, reinterpret_cast<const long long*>(frame_offsets), n_clips,
+                         program_of_clip, taps, ep, out, out_dtype, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int vnd_colsumsq_seq_f32_dev(const vnd_signal* a, float* sums, void* stream) {
@@ -915,6 +969,140 @@ extern "C" int vnd_vn_decorrelate_host(vnd_ctx* ctx, const vnd_signal* x, const 
   od.data = dout;
   if ((rc = vnd_vn_decorrelate_dev(&xd, &od, &dprog, ep, work, wbytes, st))) return rc;
   if (dy.elems) VND_CUDA_OK(cudaMemcpyAsync(out->data, dout, dy.elems * esize(out->dtype), cudaMemcpyDeviceToHost, st));
+  VND_CUDA_OK(cudaStreamSynchronize(st));
+  return VND_OK;
+}
+
+namespace {
+
+// 1 + the largest tap index of channel c of a host SEGMENTED program (0 for an empty block or no taps)
+int channel_halo(const vnd_tap_program* t, int c) {
+  const int32_t* w = t->words + t->offsets[c];
+  if (t->offsets[c + 1] == t->offsets[c]) return 0;
+  const int S = w[0];
+  long long taps = 0;
+  for (int s = 0; s < S; ++s) taps += (long long)w[1 + 3 * s] + w[2 + 3 * s];
+  int halo = 0;
+  for (long long k = 0; k < taps; ++k) halo = w[1 + 3 * S + k] + 1 > halo ? w[1 + 3 * S + k] + 1 : halo;
+  return halo;
+}
+
+// Clip by clip through vnd_vn_decorrelate_host: for filters whose halo does not fit the batched kernel.  Correct, but
+// one upload / launch sequence / download per clip.
+int batch_host_per_clip(vnd_ctx* ctx, const float* x, const int64_t* offs, int32_t n, const int32_t* prog_of, const vnd_tap_program* taps,
+                        const vnd_epilogue* ep, void* out, int32_t out_dtype) {
+  const size_t es = esize(out_dtype);
+  for (int i = 0; i < n; ++i) {
+    const long long L = offs[i + 1] - offs[i];
+    const int p = prog_of[i];
+    vnd_tap_program sub = *taps;
+    sub.offsets = taps->offsets + 2 * p;
+    sub.channels = 2;
+    const int h0 = channel_halo(taps, 2 * p), h1 = channel_halo(taps, 2 * p + 1);
+    sub.halo = h0 > h1 ? h0 : h1;
+    const int b0 = sub.offsets[1] - sub.offsets[0], b1 = sub.offsets[2] - sub.offsets[1];
+    sub.max_channel_words = b0 > b1 ? b0 : b1;
+    vnd_signal xs{const_cast<float*>(x) + 2 * offs[i], L, 2, VND_F32, 2, 1};
+    vnd_signal os{reinterpret_cast<char*>(out) + (size_t)(offs[i] + (long long)i * ep->haas_delay) * 2 * es, L + ep->haas_delay, 2, out_dtype,
+                  2, 1};
+    const int rc = vnd_vn_decorrelate_host(ctx, &xs, &os, &sub, ep);
+    if (rc) return rc;
+  }
+  return VND_OK;
+}
+
+}  // namespace
+
+extern "C" int vnd_vn_decorrelate_batch_host(vnd_ctx* ctx, const void* x, int32_t x_dtype, int64_t rows, const int64_t* frame_offsets,
+                                             int32_t n_clips, const int32_t* program_of_clip, const vnd_tap_program* taps,
+                                             const vnd_epilogue* ep, void* out, int32_t out_dtype) {
+  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  int rc;
+  if ((rc = check_batch(x, x_dtype, rows, frame_offsets, n_clips, program_of_clip, taps, ep, out, out_dtype))) return rc;
+  if (n_clips == 0) return VND_OK;
+  const int64_t* offs = frame_offsets;
+  VND_REQUIRE(offs[0] == 0, VND_EINVAL, "frame_offsets[0] is %lld, not 0", (long long)offs[0]);
+  for (int i = 0; i < n_clips; ++i)
+    VND_REQUIRE(offs[i + 1] >= offs[i], VND_EINVAL, "frame_offsets decrease at clip %d (%lld -> %lld)", i, (long long)offs[i],
+                (long long)offs[i + 1]);
+  VND_REQUIRE(offs[n_clips] == rows, VND_EINVAL, "frame_offsets end at %lld, not at rows = %lld", (long long)offs[n_clips], (long long)rows);
+  const int n_prog = taps->channels / 2;
+  for (int i = 0; i < n_clips; ++i)
+    VND_REQUIRE(program_of_clip[i] >= 0 && program_of_clip[i] < n_prog, VND_EINVAL, "program_of_clip[%d] = %d is outside [0, %d)", i,
+                program_of_clip[i], n_prog);
+  const float* xf = reinterpret_cast<const float*>(x);
+  if (!batch_fits(taps, rows)) return batch_host_per_clip(ctx, xf, offs, n_clips, program_of_clip, taps, ep, out, out_dtype);
+
+  VND_ENTER(ctx);
+  cudaStream_t st = ctx->streams[0];
+  vnd_tap_program dprog;
+  if ((rc = upload_program(ctx, taps, &dprog, st))) return rc;
+  const int delay = ep->haas_delay;
+  const size_t es = esize(out_dtype);
+  const size_t in_bytes = (size_t)rows * 8;
+
+  if (in_bytes >= kPipeMinBytes && getenv("VND_NO_PIPELINE") == nullptr) {
+    // chunks of whole clips of about pipe_chunk_bytes() (at least four chunks when there are four clips), each with its
+    // own offsets rebased to its first row: first[k] .. first[k + 1] are the clips of chunk k
+    size_t target = pipe_chunk_bytes();
+    if (target > in_bytes / 4) target = in_bytes / 4;
+    std::vector<int> first{0};
+    while (first.back() < n_clips) {
+      const int a = first.back();
+      int b = a + 1;
+      while (b < n_clips && (size_t)(offs[b + 1] - offs[a]) * 8 <= target) ++b;
+      first.push_back(b);
+    }
+    const int nchunks = (int)first.size() - 1;
+    std::vector<long long> meta;  // rebased offsets of every chunk (n_k + 1 each), then the program indices
+    meta.reserve((size_t)n_clips + nchunks + n_clips / 2 + 1);
+    long long max_rows = 0, max_out_rows = 0;
+    int max_clips = 0;
+    for (int k = 0; k < nchunks; ++k) {
+      const int a = first[k], b = first[k + 1];
+      for (int i = a; i <= b; ++i) meta.push_back(offs[i] - offs[a]);
+      const long long r = offs[b] - offs[a];
+      max_rows = r > max_rows ? r : max_rows;
+      max_out_rows = r + (long long)(b - a) * delay > max_out_rows ? r + (long long)(b - a) * delay : max_out_rows;
+      max_clips = b - a > max_clips ? b - a : max_clips;
+    }
+    const size_t off_bytes = meta.size() * 8;
+    void* dmeta = nullptr;
+    if ((rc = arena(ctx, S_AUX, off_bytes + (size_t)n_clips * 4, &dmeta))) return rc;
+    VND_CUDA_OK(cudaMemcpyAsync(dmeta, meta.data(), off_bytes, cudaMemcpyHostToDevice, st));
+    VND_CUDA_OK(cudaMemcpyAsync((char*)dmeta + off_bytes, program_of_clip, (size_t)n_clips * 4, cudaMemcpyHostToDevice, st));
+    VND_CUDA_OK(cudaStreamSynchronize(st));  // the program and the offsets are on the device before the other streams read them
+    const long long* doffs = reinterpret_cast<const long long*>(dmeta);
+    const int32_t* dprog_of = reinterpret_cast<const int32_t*>((char*)dmeta + off_bytes);
+    auto chunk_of = [&](int k) {
+      const int a = first[k], b = first[k + 1];
+      const long long r = offs[b] - offs[a];
+      return PipeChunk{reinterpret_cast<const char*>(xf + 2 * offs[a]), (size_t)r * 8,
+                       reinterpret_cast<char*>(out) + (size_t)(offs[a] + (long long)a * delay) * 2 * es, (size_t)(r + (long long)(b - a) * delay) * 2 * es};
+    };
+    auto compute = [&](int k, void* din, void* dout, void* sa, void*, cudaStream_t cs) {
+      const int a = first[k], b = first[k + 1];
+      return vn_batch_launch(reinterpret_cast<const float*>(din), offs[b] - offs[a], doffs + a + k, b - a, dprog_of + a, &dprog, ep, dout,
+                             out_dtype, sa, cs);
+    };
+    return run_pipeline(ctx, nchunks, (size_t)max_rows * 8, (size_t)max_out_rows * 2 * es, vn_batch_workspace_bytes(max_rows, max_clips, ep->rms_normalize),
+                        chunk_of, compute);
+  }
+
+  const size_t out_bytes = (size_t)(rows + (long long)n_clips * delay) * 2 * es;
+  const size_t wbytes = vn_batch_workspace_bytes(rows, n_clips, ep->rms_normalize);
+  const size_t off_bytes = ((size_t)n_clips + 1) * 8;
+  void *din = nullptr, *dout = nullptr, *work = nullptr, *dmeta = nullptr;
+  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) || (rc = arena(ctx, S_WORK, wbytes, &work)) ||
+      (rc = arena(ctx, S_AUX, off_bytes + (size_t)n_clips * 4, &dmeta)))
+    return rc;
+  if (in_bytes) VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
+  VND_CUDA_OK(cudaMemcpyAsync(dmeta, offs, off_bytes, cudaMemcpyHostToDevice, st));
+  VND_CUDA_OK(cudaMemcpyAsync((char*)dmeta + off_bytes, program_of_clip, (size_t)n_clips * 4, cudaMemcpyHostToDevice, st));
+  if ((rc = vnd_vn_decorrelate_batch_dev(din, VND_F32, rows, reinterpret_cast<const int64_t*>(dmeta), n_clips,
+                                         reinterpret_cast<const int32_t*>((char*)dmeta + off_bytes), &dprog, ep, dout, out_dtype, work, wbytes, st)))
+    return rc;
+  if (out_bytes) VND_CUDA_OK(cudaMemcpyAsync(out, dout, out_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
   return VND_OK;
 }

@@ -1,0 +1,97 @@
+// Shared between the batched decorrelate (vnd_batch.cu) and the sum-of-squares scans (vnd_post.cu).
+#pragma once
+
+#include "vnd_common.cuh"
+
+namespace vnd {
+
+// rms_normalize's DUAL_MONO gain of one float32 channel from its two sums of squares (numpy's dtype chain: the mean
+// divides in float64 and stores float32, epsilon is cast to float32); rms_gain_kernel and the batch use it alike.
+__device__ __forceinline__ float rms_gain_f32(float sum_x, float sum_y, long long frames) {
+  const float mx = __double2float_rn((double)sum_x / (double)frames);
+  const float my = __double2float_rn((double)sum_y / (double)frames);
+  return __fdiv_rn(__fsqrt_rn(mx), __fsqrt_rn(fadd(my, 1e-10f)));
+}
+
+// Column 4 i + j of a batch of n clips packed in (rows, 2) float32 arrays: j = 0, 1 are the two channels of clip i's
+// input x, j = 2, 3 those of its FIR / M/S / width result y.  Clip i is rows [offs[i], offs[i + 1]) of both.
+// The sums pass ends with the clip's two gains, so that the placement pass only multiplies (its SASS holds no
+// multiply-add; a correctly rounded division is built from them).
+struct BatchSumCols {
+  const float* x;
+  const float* y;
+  const long long* offs;
+  float* sums;         // 4 n floats
+  float* gains;        // 2 n floats
+  unsigned* arrivals;  // n counters of finished columns, zeroed by the stereo pass that precedes the sums
+  __device__ __forceinline__ void column(int col, const float** base, long long* st, long long* n) const {
+    const int clip = col >> 2, j = col & 3;
+    const long long o = offs[clip];
+    *base = (j < 2 ? x : y) + 2 * o + (j & 1);
+    *st = 2;
+    *n = offs[clip + 1] - o;
+  }
+  __device__ __forceinline__ void store_clip(int clip, float sx0, float sx1, float sy0, float sy1) const {
+    const long long frames = offs[clip + 1] - offs[clip];
+    float* s = sums + 4 * (long long)clip;
+    s[0] = sx0;
+    s[1] = sx1;
+    s[2] = sy0;
+    s[3] = sy1;
+    gains[2 * (long long)clip] = rms_gain_f32(sx0, sy0, frames);
+    gains[2 * (long long)clip + 1] = rms_gain_f32(sx1, sy1, frames);
+  }
+  // one column at a time (the cluster scan): the last of a clip's four columns to finish computes its gains
+  __device__ __forceinline__ void store(int col, float v) const {
+    const int clip = col >> 2;
+    sums[col] = v;
+    __threadfence();
+    if (atomicAdd(&arrivals[clip], 1u) == 3u) {
+      __threadfence();
+      const volatile float* s = sums + 4 * (long long)clip;
+      store_clip(clip, s[0], s[1], s[2], s[3]);
+    }
+  }
+};
+
+// CTA b of a batched kernel with `tile` outputs per CTA takes clip i, the last one with V[i] <= b where
+// V[i] = floor(offs[i] / tile) + i, and that clip's tile b - V[i].  V[i + 1] - V[i] >= max(1, ceil(frames_i / tile)),
+// so floor(rows / tile) + n CTAs - a grid known from host scalars alone - cover every tile of every clip and give an
+// empty clip one CTA (its Haas zero fill); the few CTAs past a clip's last tile exit.
+__device__ __forceinline__ int batch_clip_of(const long long* offs, int n, int tile, long long b) {
+  int lo = 0, hi = n - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (offs[mid] / tile + mid <= b) lo = mid;
+    else hi = mid - 1;
+  }
+  return lo;
+}
+
+// vnd_fir.cu: the batched fused stereo pass (vn_stereo_kernel over (clip, tile) pairs); out is (rows + n delay, 2)
+// C-order, clip i from row offs[i] + i delay.  VND_EUNSUPPORTED (no error text) when tile + halo does not fit.
+// `arrivals` (nullable): n counters the pass zeroes for the sums pass behind it.
+int vn_batch_stereo_launch(const float* x, long long rows, const long long* offs, int n_clips, const int* prog_of,
+                           const vnd_tap_program* taps, const vnd_epilogue* ep, void* out, int out_dtype, int delay, int delay_ch,
+                           unsigned* arrivals, cudaStream_t st);
+
+// vnd_post.cu: the cluster scan of seq_sumsq_cluster_kernel over these columns, and its shape constants
+int batch_sumsq_cluster_launch(const BatchSumCols& cols, int n_cols, cudaStream_t st);
+int seq_sumsq_cluster_width();  // CTAs per column
+int seq_sumsq_scan_round();     // addends per CTA and round
+int seq_sumsq_scan_head();      // addends chained by one thread before the scan starts
+
+// vnd_batch.cu
+#ifndef VND_BATCH_TILE
+#define VND_BATCH_TILE 4096
+#endif
+// Outputs per CTA of the batched stereo and placement kernels.  Measured on a B200 against 1024 (the single-clip kernel's
+// tile): 512 clips of 5-15 s, default VelvetNoise, 12.27 -> 11.58 ms; without normaliser 7.91 -> 7.23 ms - the filter's
+// halo (1324 frames at 44.1 kHz) is staged once per tile.
+constexpr int kBatchTile = VND_BATCH_TILE;
+bool vn_batch_smem(int halo, int prog_words, size_t* smem);
+size_t vn_batch_workspace_bytes(long long rows, int n_clips, int rms);
+int vn_batch_launch(const float* x, long long rows, const long long* offs, int n_clips, const int* prog_of, const vnd_tap_program* taps,
+                    const vnd_epilogue* ep, void* out, int out_dtype, void* workspace, cudaStream_t st);
+
+}  // namespace vnd

@@ -18,6 +18,7 @@
 #include <stdlib.h>
 
 #include "vnd_common.cuh"
+#include "vnd_batch.cuh"
 #include "vnd_fir.cuh"
 
 namespace vnd {
@@ -371,6 +372,93 @@ __global__ void __launch_bounds__(256) vn_stereo_kernel(const StereoParams p) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// Batched fused stereo decorrelate: vn_stereo_kernel's work over the (clip, tile) pairs of many clips packed in one
+// (rows, 2) float32 array (batch_clip_of maps CTAs to pairs).  Each CTA stages its tile plus the halo of both channels
+// and the two program blocks of its clip's filter; staged samples past the clip's end are +0, as in the single-clip
+// kernel, so no tap reads across a clip boundary.  out is (rows + n delay, 2) C-order with clip i from row
+// offs[i] + i delay, and gets the Haas head and tail zero fill of every clip.
+// ------------------------------------------------------------------------------------------------
+struct BatchStereoParams {
+  StereoParams sp;        // x, out (C-order pairs), words, offsets (2 channels per program), tile, halo, epilogue, delay
+  const long long* offs;  // n + 1 clip offsets into x
+  const int* prog_of;     // program of each clip: channels 2 k, 2 k + 1 of sp.offsets
+  unsigned* arrivals;     // nullable: per-clip counters of the sums pass, zeroed here
+  int n_clips;
+};
+
+template <typename TOut, int R>
+__global__ void __launch_bounds__(256) vn_batch_stereo_kernel(const BatchStereoParams bp) {
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  constexpr int NT = 256;
+  const StereoParams& p = bp.sp;
+  const int span = p.tile + p.halo;
+  const int span_al = (span + 3) & ~3;
+  float* s0 = reinterpret_cast<float*>(smem_raw);
+  float* s1 = s0 + span_al;
+  int* prog0 = reinterpret_cast<int*>(s1 + span_al);
+
+  const int clip = batch_clip_of(bp.offs, bp.n_clips, p.tile, blockIdx.x);
+  const long long c0 = bp.offs[clip];
+  const long long L = bp.offs[clip + 1] - c0;
+  const long long k = (long long)blockIdx.x - (c0 / p.tile + clip);
+  const long long ntiles = L > 0 ? ceil_div<long long>(L, p.tile) : 1;
+  if (k < 0 || k >= ntiles) return;
+  if (bp.arrivals && k == 0 && threadIdx.x == 0) bp.arrivals[clip] = 0u;
+  const int pr = bp.prog_of[clip];
+  const int w0 = p.offsets[2 * pr];
+  const int n0 = p.offsets[2 * pr + 1] - w0;
+  const int n1 = p.offsets[2 * pr + 2] - w0 - n0;
+  int* prog1 = prog0 + n0;
+
+  const int tid = threadIdx.x;
+  const long long t0 = k * p.tile;
+  const long long remain = L - t0;
+  const int nvalid = (int)(remain < span ? (remain > 0 ? remain : 0) : span);
+  const float2* __restrict__ x2 = reinterpret_cast<const float2*>(p.x) + c0 + t0;
+  for (int i = tid; i < span; i += NT) {
+    float2 v = make_float2(0.0f, 0.0f);
+    if (i < nvalid) v = x2[i];
+    s0[i] = v.x;
+    s1[i] = v.y;
+  }
+  for (int i = tid; i < n0 + n1; i += NT) prog0[i] = p.words[w0 + i];
+  __syncthreads();
+
+  TOut* __restrict__ out = reinterpret_cast<TOut*>(p.out) + 2 * (c0 + (long long)clip * p.delay);
+  const int sh0 = p.delay_ch == 0 ? p.delay : 0;
+  const int sh1 = p.delay_ch == 1 ? p.delay : 0;
+  const int warp = tid >> 5, lane = tid & 31;
+  constexpr int kSub = 32 * R;
+  const int nsub = p.tile / kSub;
+  for (int sb = warp; sb < nsub; sb += NT / 32) {
+    const int base = sb * kSub;
+    if (base >= remain) break;
+    float y0[R], y1[R];
+    if (n0 > 0) run_program<float, MODE_SEG, R, 32>(s0 + base + lane, prog0, p.apply_gain, y0);
+    if (n1 > 0) run_program<float, MODE_SEG, R, 32>(s1 + base + lane, prog1, p.apply_gain, y1);
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+      const int i = base + lane + 32 * r;
+      const long long t = t0 + i;
+      if (t < L) {
+        const float a = s0[i], b = s1[i];
+        float u = n0 > 0 ? y0[r] : a;  // unfiltered channel: copied through
+        float v = n1 > 0 ? y1[r] : b;
+        stereo_epilogue(a, b, u, v, p, 1.0f, 1.0f);
+        out[(t + sh0) * 2] = (TOut)u;
+        out[(t + sh1) * 2 + 1] = (TOut)v;
+      }
+    }
+  }
+  if (p.delay > 0) {  // Haas zero fill of this clip: head of the delayed channel, tail of the other one
+    if (k == 0)
+      for (int i = tid; i < p.delay; i += NT) out[(long long)i * 2 + p.delay_ch] = (TOut)0;
+    if (k == ntiles - 1)
+      for (int i = tid; i < p.delay; i += NT) out[(L + i) * 2 + (1 - p.delay_ch)] = (TOut)0;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------------
 constexpr int kR = 8;
@@ -606,6 +694,56 @@ int vn_stereo_launch(const vnd_signal* x, void* out, int out_dtype, long long o_
     k<<<blocks, 256, smem, st>>>(p);
   }
   return after_launch("vn_stereo_kernel");
+}
+
+bool vn_batch_smem(int halo, int prog_words, size_t* smem) {
+  const long long h = ((long long)(halo > 0 ? halo : 0) + 3) & ~3LL;
+  const long long bytes = 2 * ((kBatchTile + h + 3) & ~3LL) * 4 + (long long)prog_words * 4 + 16;
+  *smem = (size_t)bytes;
+  return bytes <= kMaxDynSmem;
+}
+
+int vn_batch_stereo_launch(const float* x, long long rows, const long long* offs, int n_clips, const int* prog_of,
+                           const vnd_tap_program* taps, const vnd_epilogue* ep, void* out, int out_dtype, int delay, int delay_ch,
+                           unsigned* arrivals, cudaStream_t st) {
+  if (n_clips == 0) return VND_OK;
+  BatchStereoParams bp{};
+  StereoParams& p = bp.sp;
+  p.x = x;
+  p.out = out;
+  p.words = taps->words;
+  p.offsets = taps->offsets;
+  p.apply_gain = taps->apply_gain;
+  p.ms_encode = ep->ms_encode;
+  p.use_width = ep->use_width;
+  p.w_mid = (float)(1.0 - (double)ep->width);
+  p.w_side = (float)ep->width;
+  p.delay = delay;
+  p.delay_ch = delay_ch;
+  long long halo = taps->halo > 0 ? taps->halo : 0;
+  if (halo > rows) halo = rows;  // no clip is longer than the batch
+  p.halo = (int)((halo + 3) & ~3LL);
+  p.tile = kBatchTile;
+  size_t smem = 0;
+  if (!vn_batch_smem(p.halo, 2 * taps->max_channel_words, &smem)) return VND_EUNSUPPORTED;
+  bp.offs = offs;
+  bp.prog_of = prog_of;
+  bp.arrivals = arrivals;
+  bp.n_clips = n_clips;
+  const long long blocks = rows / kBatchTile + n_clips;
+  VND_REQUIRE(blocks < 0x7fffffffLL, VND_EUNSUPPORTED, "grid too large (%lld CTAs)", blocks);
+  constexpr int R = 4;
+  static_assert(kBatchTile % (32 * R * 8) == 0, "the tile is a whole number of passes of the 8 warps");
+  if (out_dtype == VND_F64) {
+    auto k = vn_batch_stereo_kernel<double, R>;
+    VND_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<(unsigned)blocks, 256, smem, st>>>(bp);
+  } else {
+    auto k = vn_batch_stereo_kernel<float, R>;
+    VND_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<(unsigned)blocks, 256, smem, st>>>(bp);
+  }
+  return after_launch("vn_batch_stereo_kernel");
 }
 
 }  // namespace vnd

@@ -12,6 +12,7 @@
 #include <stdlib.h>
 
 #include "vnd_common.cuh"
+#include "vnd_batch.cuh"
 
 namespace vnd {
 
@@ -30,6 +31,18 @@ struct SeqParams {
   long long frames;
   int channels;
   void* sums;  // T[ncols]
+  // float32 column source of seq_sumsq_cluster_kernel
+  __device__ __forceinline__ void column(int col, const float** base, long long* st, long long* n) const {
+    if (col < channels) {
+      *base = reinterpret_cast<const float*>(a) + (long long)col * a_sc;
+      *st = a_st;
+    } else {
+      *base = reinterpret_cast<const float*>(b) + (long long)(col - channels) * b_sc;
+      *st = b_st;
+    }
+    *n = frames;
+  }
+  __device__ __forceinline__ void store(int col, float s) const { reinterpret_cast<float*>(sums)[col] = s; }
 };
 
 template <typename T>
@@ -303,7 +316,10 @@ constexpr unsigned PS_BK = (unsigned)PS_K * PS_B;  // addends per round
 
 namespace cg = cooperative_groups;
 
-__global__ void __cluster_dims__(PS_K, 1, 1) __launch_bounds__(PS_NT) seq_sumsq_cluster_kernel(const SeqParams p) {
+// The column source is a template parameter so that the batched decorrelate (vnd_batch.cu) runs the same scan over
+// columns that live at device-side clip offsets: Cols::column(col, &base, &stride, &frames) and Cols::store(col, sum).
+template <class Cols>
+__global__ void __cluster_dims__(PS_K, 1, 1) __launch_bounds__(PS_NT) seq_sumsq_cluster_kernel(const Cols p) {
   __shared__ float stage[PS_HEAD];
   __shared__ Tr warp_tot[PS_NT / 32];
   __shared__ Tr cta_tot[PS_K];        // written by every CTA of the cluster (slot = its rank)
@@ -314,16 +330,9 @@ __global__ void __cluster_dims__(PS_K, 1, 1) __launch_bounds__(PS_NT) seq_sumsq_
   const unsigned rank = cluster.block_rank();
   const int col = blockIdx.x / PS_K;
   const float* base;
-  long long st;
-  if (col < p.channels) {
-    base = reinterpret_cast<const float*>(p.a) + (long long)col * p.a_sc;
-    st = p.a_st;
-  } else {
-    base = reinterpret_cast<const float*>(p.b) + (long long)(col - p.channels) * p.b_sc;
-    st = p.b_st;
-  }
+  long long st, N;
+  p.column(col, &base, &st, &N);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const long long N = p.frames;
   float s = 0.0f;
   long long pos = 0;
   {  // head: chained by one thread of every CTA (same result everywhere)
@@ -450,7 +459,7 @@ __global__ void __cluster_dims__(PS_K, 1, 1) __launch_bounds__(PS_NT) seq_sumsq_
     // rewritten only behind the next round's cluster barriers, which every thread reaches after these reads
   }
   cluster.sync();  // nobody leaves while a peer may still write into its shared memory
-  if (rank == 0 && tid == 0) reinterpret_cast<float*>(p.sums)[col] = s;
+  if (rank == 0 && tid == 0) p.store(col, s);
 }
 
 // gains[c] = sqrt(mean_x[c]) / sqrt(mean_y[c] + eps) with numpy's dtype chain: the mean divides in
@@ -461,9 +470,7 @@ __global__ void rms_gain_kernel(const T* __restrict__ sums, T* __restrict__ gain
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= channels) return;
   if constexpr (sizeof(T) == 4) {
-    const float mx = __double2float_rn((double)sums[c] / (double)frames);
-    const float my = __double2float_rn((double)sums[channels + c] / (double)frames);
-    gains[c] = __fdiv_rn(__fsqrt_rn(mx), __fsqrt_rn(fadd(my, 1e-10f)));
+    gains[c] = rms_gain_f32(sums[c], sums[channels + c], frames);
   } else {
     const double mx = __ddiv_rn(sums[c], (double)frames);
     const double my = __ddiv_rn(sums[channels + c], (double)frames);
@@ -699,10 +706,20 @@ int seq_sumsq_launch(const vnd_signal* a, const vnd_signal* b, void* sums, cudaS
   if (a->dtype == VND_F64) seq_sumsq_kernel<double><<<cols, 256, 0, st>>>(p);
   else if (serial_only || a->frames < 4096) seq_sumsq_kernel<float><<<cols, 256, 0, st>>>(p);
   else if (cluster_ok && a->frames >= (long long)PS_HEAD + 2 * PS_B && cols * PS_K <= 2 * sm_count)  // few columns: latency matters, SMs are idle
-    seq_sumsq_cluster_kernel<<<cols * PS_K, PS_NT, 0, st>>>(p);
+    seq_sumsq_cluster_kernel<SeqParams><<<cols * PS_K, PS_NT, 0, st>>>(p);
   else seq_sumsq_par_kernel<<<cols, PS_NT, 0, st>>>(p);
   return after_launch("seq_sumsq_kernel");
 }
+
+// the cluster scan over the 4 columns of every clip of a batch (vnd_batch.cu picks it for few long columns)
+int batch_sumsq_cluster_launch(const BatchSumCols& cols, int n_cols, cudaStream_t st) {
+  if (n_cols == 0) return VND_OK;
+  seq_sumsq_cluster_kernel<BatchSumCols><<<n_cols * PS_K, PS_NT, 0, st>>>(cols);
+  return after_launch("seq_sumsq_cluster_kernel");
+}
+int seq_sumsq_cluster_width() { return PS_K; }
+int seq_sumsq_scan_round() { return PS_B; }
+int seq_sumsq_scan_head() { return PS_HEAD; }
 
 int pairwise_sumsq_launch(const void* col, int dtype, long long n, void* leaf, void* out, cudaStream_t st);
 

@@ -15,6 +15,7 @@ is not provided; ``SignalChain.white_noise`` raises ``NotImplementedError``.
 from __future__ import annotations
 
 import ctypes as C
+import os
 from functools import partial
 from typing import Any, Callable, Sequence
 
@@ -33,7 +34,7 @@ from .taps import (
 )
 from .utils.dsp import LayoutMode, apply_stereo_width, check_equal_length, rms_normalize, to_float32
 
-__all__ = ["Decorrelator", "SignalChain", "HaasEffect", "VelvetNoise", "generate_velvet_noise", "convolve_velvet_noise"]
+__all__ = ["Decorrelator", "SignalChain", "HaasEffect", "VelvetNoise", "decorrelate_batch", "generate_velvet_noise", "convolve_velvet_noise"]
 
 
 class Decorrelator:
@@ -317,6 +318,24 @@ class VelvetNoise(Decorrelator):
         return self._decorrelate(x, haas=None)
 
     def _decorrelate(self, x, haas: "HaasEffect | None"):
+        self._check_input(x)
+        fused_norm = self.normalizer is None or self.normalizer is rms_normalize
+        program = self.tap_program(x.shape[0])
+        kw = dict(num_outs=self.num_outs, ms_encode=_is_mode(self.mode, LayoutMode.MS), width=self.width)
+        if fused_norm:
+            if haas is not None:
+                return _vn_decorrelate(x, program, rms=self.normalizer is not None, haas_delay=haas.delay_len_samples,
+                                       haas_channel=haas.delayed_channel % 2, out_f64=True, **kw)
+            return _vn_decorrelate(x, program, rms=self.normalizer is not None, **kw)
+        # user-supplied normaliser: run everything else fused, then hand (input, output) to it
+        y = _vn_decorrelate(x, program, rms=False, **kw)
+        x2 = x if x.ndim == 2 else (np.column_stack((x, x)) if not R.is_torch_tensor(x) else x[:, None].expand(-1, 2))
+        self.normalizer(x2, y)
+        return y
+
+    def _check_input(self, x) -> int:
+        """The shape checks of ``decorrelate`` on a cast signal (the reference's exceptions); returns the input's
+        channel count, 2 for a mono signal."""
         if x.ndim == 1:
             in_channels = 2  # mono_to_stereo, passed to the kernel as a stride-0 broadcast
         elif x.ndim == 2:
@@ -331,21 +350,9 @@ class VelvetNoise(Decorrelator):
             raise ValueError(f"Input shape invalid: Expected shape (num samples, 2), but got shape {bad}.")
         if self.width is not None and self.num_outs != 2:
             raise ValueError(f"Input shape invalid: Expected shape (num samples, 2), but got shape {(x.shape[0], self.num_outs)}.")
-        fused_norm = self.normalizer is None or self.normalizer is rms_normalize
         if self.normalizer is rms_normalize and in_channels != self.num_outs:
             raise ValueError(f"operands could not be broadcast together with shapes ({x.shape[0]},{self.num_outs}) ({in_channels},)")
-        program = self.tap_program(x.shape[0])
-        kw = dict(num_outs=self.num_outs, ms_encode=ms, width=self.width)
-        if fused_norm:
-            if haas is not None:
-                return _vn_decorrelate(x, program, rms=self.normalizer is not None, haas_delay=haas.delay_len_samples,
-                                       haas_channel=haas.delayed_channel % 2, out_f64=True, **kw)
-            return _vn_decorrelate(x, program, rms=self.normalizer is not None, **kw)
-        # user-supplied normaliser: run everything else fused, then hand (input, output) to it
-        y = _vn_decorrelate(x, program, rms=False, **kw)
-        x2 = x if x.ndim == 2 else (np.column_stack((x, x)) if not R.is_torch_tensor(x) else x[:, None].expand(-1, 2))
-        self.normalizer(x2, y)
-        return y
+        return in_channels
 
 
 def _fusable(vn, haas) -> bool:
@@ -432,6 +439,278 @@ class SignalChain:
                 sig = stages[i](sig)
                 i += 1
         return sig
+
+
+# ------------------------------------------------------------------------------------------------
+# many clips in one call
+# ------------------------------------------------------------------------------------------------
+
+
+def _batch_stages(d) -> "tuple[VelvetNoise, HaasEffect | None]":
+    """The (velvet noise, fused Haas or None) pair a batch decorrelator runs as."""
+    if isinstance(d, VelvetNoise):
+        vn, haas = d, None
+    elif isinstance(d, SignalChain):
+        d._init_decorrelators()  # a lazy chain is instantiated as its first call would
+        stages = d._decorrelators
+        if len(stages) == 1 and isinstance(stages[0], VelvetNoise):
+            vn, haas = stages[0], None
+        elif len(stages) == 2 and _fusable(stages[0], stages[1]):
+            vn, haas = stages
+        else:
+            names = ", ".join(type(st).__name__ for st in stages) or "no stages"
+            raise NotImplementedError("decorrelate_batch runs a SignalChain of one VelvetNoise, or of a VelvetNoise followed by an LR-mode "
+                                      f"HaasEffect without width; this chain has {names}")
+    else:
+        raise NotImplementedError(f"decorrelate_batch takes VelvetNoise or SignalChain decorrelators, not {type(d).__name__}")
+    if vn.normalizer is not None and vn.normalizer is not rms_normalize:
+        raise NotImplementedError("decorrelate_batch fuses rms_normalize or no normaliser; a user-supplied normaliser runs clip by clip")
+    return vn, haas
+
+
+def _batch_settings(vn: VelvetNoise, haas: "HaasEffect | None") -> dict:
+    """What the clips of one batch must share (one epilogue and one apply_gain flag for the whole launch)."""
+    return {
+        "num_outs": vn.num_outs,
+        "mode": "MS" if _is_mode(vn.mode, LayoutMode.MS) else "LR",
+        "width": vn.width,
+        "normalizer": "rms_normalize" if vn.normalizer is rms_normalize else None,
+        "Haas stage": haas is not None,
+        "Haas delay": haas.delay_len_samples if haas is not None else 0,
+        "Haas delayed_channel": haas.delayed_channel % 2 if haas is not None else 0,
+        # multiplying by 1.0 is not payload-safe for NaN, so the identity envelope skips the multiply (decorrelation.py:411)
+        "identity segment_envelope": vn.segment_envelope == IDENTITY_ENVELOPE,
+    }
+
+
+def _check_batch_layout(offsets: np.ndarray, program_of_clip: np.ndarray, n_programs: int, rows: int) -> None:
+    """The packed layout vnd_vn_decorrelate_batch_* reads: offsets from 0 to ``rows``, never decreasing, and a program
+    index in range for every clip (the device entry point cannot check these)."""
+    if len(offsets) != len(program_of_clip) + 1 or len(offsets) == 0 or offsets[0] != 0 or offsets[-1] != rows:
+        raise ValueError(f"frame offsets must run from 0 to {rows} with one entry per clip and one more")
+    if np.any(np.diff(offsets) < 0):
+        raise ValueError("frame offsets must not decrease")
+    if len(program_of_clip) and (program_of_clip.min() < 0 or program_of_clip.max() >= n_programs):
+        raise ValueError(f"program indices must lie in [0, {n_programs})")
+
+
+def _batch_programs(filters: "Sequence[VelvetNoise]", lengths) -> "tuple[list[TapProgram], np.ndarray]":
+    """The distinct tap programs of a batch and the index of each clip's one.  ``tap_program`` caches one program for
+    every length beyond the filter, so all such clips of one filter share it; shorter clips get their truncated one."""
+    index: dict[int, int] = {}
+    progs: list[TapProgram] = []
+    prog_of = np.empty(len(filters), dtype=np.int32)
+    for i, (vn, L) in enumerate(zip(filters, lengths)):
+        prog = vn.tap_program(int(L))
+        if id(prog) not in index:
+            index[id(prog)] = len(progs)
+            progs.append(prog)
+        prog_of[i] = index[id(prog)]
+    return progs, prog_of
+
+
+def _batch_program(progs: "list[TapProgram]") -> TapProgram:
+    """One SEGMENTED program holding the two channels of every distinct filter, pair k = channels 2k, 2k + 1."""
+    words = np.concatenate([p.words for p in progs]).astype(np.int32, copy=False)
+    offsets = np.concatenate([[0]] + [p.offsets[1:].astype(np.int64) + base for p, base in
+                                      zip(progs, np.cumsum([0] + [p.words.size for p in progs[:-1]]))]).astype(np.int32)
+    return TapProgram(np.ascontiguousarray(words), offsets, 2 * len(progs), N.ORDER_SEGMENTED, progs[0].apply_gain, max(p.halo for p in progs),
+                      max(p.max_channel_words for p in progs))
+
+
+def _pack_clips(xp: np.ndarray, clips, offsets: np.ndarray) -> None:
+    """Copy numpy clips into their rows of the packed (rows, 2) array (a mono clip into both columns).  Large batches
+    are copied by several threads: numpy releases the GIL for the copies, and one thread does not reach the host's
+    memory bandwidth."""
+
+    def put(i):
+        x, a, b = clips[i], offsets[i], offsets[i + 1]
+        if x.ndim == 1:
+            xp[a:b, 0] = x
+            xp[a:b, 1] = x
+        else:
+            xp[a:b] = x[:, :2]
+
+    if xp.nbytes < 64 << 20 or len(clips) < 2:
+        for i in range(len(clips)):
+            put(i)
+        return
+    from concurrent.futures import ThreadPoolExecutor
+
+    with ThreadPoolExecutor(max_workers=min(8, os.cpu_count() or 1, len(clips))) as pool:
+        list(pool.map(put, range(len(clips))))
+
+
+def _sums_pairwise(x) -> bool:
+    """True when the single-clip path would sum this signal's squares in numpy's pairwise order (a planar, i.e.
+    column-major, stereo signal); the packed batch is C-order, which numpy sums frame by frame."""
+    if x.ndim != 2 or x.shape[0] <= 1 or x.shape[1] <= 1:
+        return False
+    if R.is_torch_tensor(x):
+        return x.stride(0) == 1 and x.stride(1) >= x.shape[0]
+    xa = R.dense(x)
+    return not xa.flags.c_contiguous
+
+
+def decorrelate_batch(input_signals, decorrelator):
+    """Decorrelate many clips in one call: element ``i`` of the result is byte-identical (dtype, shape, bytes) to
+    ``decorrelator_i(input_signals[i])``, computed with a fixed number of launches for the whole batch.
+
+    ``input_signals``: a sequence of clips - numpy arrays or CUDA tensors, ``(frames_i, 2)`` or mono ``(frames_i,)``,
+    any length including 0, cast per clip with ``to_float32`` - or one equal-length ``(n_clips, frames, 2)`` array or
+    CUDA tensor, returned as one ``(n_clips, frames + haas_delay, 2)`` array.  ``decorrelator``: one ``VelvetNoise``,
+    or a ``SignalChain`` of a ``VelvetNoise`` alone or followed by an LR ``HaasEffect`` without width, shared by all
+    clips, or a sequence of them, one per clip (e.g. the strengths ``optimize_velvet_noise_batch`` found).
+
+    The clips must share ``num_outs == 2``, ``mode``, ``width``, the normaliser (None or ``rms_normalize``), the Haas
+    delay and delayed channel, and whether the envelope is the identity ``(1.0,)``; otherwise ``ValueError`` names the
+    setting, before any device work.  Numpy in gives numpy out (views into one page-locked block); CUDA tensors in give
+    CUDA tensors out, on torch's current stream."""
+    is_array = R.is_torch_tensor(input_signals) or isinstance(input_signals, np.ndarray)
+    if is_array and input_signals.ndim != 3:
+        raise ValueError(f"an array of clips must be (n_clips, frames, 2), got shape {tuple(input_signals.shape)}; pass other clips as a list")
+    if is_array and input_signals.shape[2] != 2:
+        raise ValueError(f"an array of clips must be (n_clips, frames, 2), got shape {tuple(input_signals.shape)}")
+    n = int(input_signals.shape[0]) if is_array else len(input_signals)
+    shared = isinstance(decorrelator, (Decorrelator, SignalChain))  # one for all clips (an unsupported one raises below)
+    decs = [decorrelator] * n if shared else list(decorrelator)
+    if len(decs) != n:
+        raise ValueError(f"{len(decs)} decorrelators for {n} clips: pass one decorrelator, or one per clip")
+
+    # decorrelators and the settings they must share
+    stages: dict[int, tuple] = {}
+    for d in ([decorrelator] if shared else decs):
+        if id(d) not in stages:
+            stages[id(d)] = _batch_stages(d)
+    pairs = [stages[id(d)] for d in decs]
+    settings = None
+    for vn, haas in (stages.values() if n else []):
+        cur = _batch_settings(vn, haas)
+        if settings is None:
+            settings = cur
+            continue
+        for key, value in cur.items():
+            if value != settings[key]:
+                raise ValueError(f"decorrelate_batch needs one {key} for every clip, got {settings[key]!r} and {value!r}")
+    if settings is None and shared:
+        settings = _batch_settings(*stages[id(decorrelator)])
+    if settings is not None and settings["num_outs"] != 2:
+        raise ValueError(f"decorrelate_batch decorrelates stereo clips: num_outs must be 2, got {settings['num_outs']}")
+    delay = settings["Haas delay"] if settings else 0
+    out_f64 = bool(settings and settings["Haas stage"])
+
+    # clips: cast, checked as the single-clip call checks them
+    torch_in = R.is_torch_tensor(input_signals) if is_array else any(R.is_torch_tensor(c) for c in input_signals)
+    if torch_in:
+        import torch
+
+        if is_array:
+            clips_in = [input_signals]
+        else:
+            clips_in = list(input_signals)
+            if not all(R.is_torch_tensor(c) for c in clips_in):
+                raise ValueError("clips must be all numpy arrays or all CUDA tensors")
+        if not all(c.is_cuda for c in clips_in):
+            raise N.VndError(N.VND_EUNSUPPORTED, "decorrelate_batch", "CPU torch tensors are not supported (no CPU fallback); pass CUDA tensors or numpy arrays")
+        device = clips_in[0].device if clips_in else None
+        if any(c.device != device for c in clips_in):
+            raise ValueError("all clips must be on one CUDA device")
+    if is_array:
+        x3 = to_float32(input_signals if torch_in else np.asarray(input_signals))
+        clips = [x3[i] for i in range(n)]
+    else:
+        clips = [to_float32(c if torch_in else np.asarray(c)) for c in input_signals]
+    for (vn, _), x in zip(pairs, clips):
+        vn._check_input(x)
+    if n == 0:
+        dt = np.float64 if out_f64 else np.float32
+        if not is_array:
+            return []
+        if torch_in:
+            return torch.empty((0, int(input_signals.shape[1]) + delay, 2), dtype=torch.float64 if out_f64 else torch.float32, device=input_signals.device)
+        return np.empty((0, int(input_signals.shape[1]) + delay, 2), dtype=dt)
+
+    # programs: one per distinct (filter, truncation), shared by the clips that use it
+    lengths = np.array([int(x.shape[0]) for x in clips], dtype=np.int64)
+    offsets = np.zeros(n + 1, dtype=np.int64)
+    np.cumsum(lengths, out=offsets[1:])
+    rows = int(offsets[-1])
+    progs, prog_of = _batch_programs([vn for vn, _ in pairs], lengths)
+    program = _batch_program(progs)
+    _check_batch_layout(offsets, prog_of, len(progs), rows)
+    vn0 = pairs[0][0]
+    haas_ch = settings["Haas delayed_channel"]
+    ep = N.EpilogueStruct(int(settings["mode"] == "MS"), int(vn0.width is not None), float(vn0.width) if vn0.width is not None else 0.0,
+                          int(settings["normalizer"] is not None), int(delay), int(haas_ch))
+    out_dt = N.VND_F64 if out_f64 else N.VND_F32
+    starts = offsets[:-1] + np.arange(n, dtype=np.int64) * delay
+    lib = N.lib()
+
+    if torch_in:
+        if is_array:
+            xp = x3.contiguous().view(-1, 2)
+        else:
+            xp = torch.cat([x[:, :2] if x.ndim == 2 else x[:, None].expand(-1, 2) for x in clips]) if rows else torch.empty((0, 2), dtype=torch.float32, device=device)
+        if xp.data_ptr() % 8:  # the kernels load one float32 pair per row
+            xp = xp.clone()
+        out = torch.empty((rows + n * delay, 2), dtype=torch.float64 if out_f64 else torch.float32, device=device)
+        stream = R.torch_stream_ptr(xp)
+        with torch.cuda.device(device):
+            d_offs = torch.from_numpy(offsets).to(device)
+            d_prog_of = torch.from_numpy(prog_of).to(device)
+            ps = R.device_program(program, device)
+            nbytes = C.c_size_t()
+            N.check(lib.vnd_vn_decorrelate_batch_workspace(rows, n, C.byref(ep), C.byref(nbytes)), "vnd_vn_decorrelate_batch_workspace")
+            work = torch.empty(max(nbytes.value, 16), dtype=torch.uint8, device=device)
+            rc = lib.vnd_vn_decorrelate_batch_dev(xp.data_ptr(), N.VND_F32, rows, d_offs.data_ptr(), n, d_prog_of.data_ptr(), C.byref(ps), C.byref(ep),
+                                                  out.data_ptr(), out_dt, work.data_ptr(), nbytes.value, stream)
+            if rc == N.VND_EUNSUPPORTED:
+                # the filter's halo does not fit the batched kernel: clip by clip through the single-clip device path
+                for i in range(n):
+                    a, L, o = int(offsets[i]), int(lengths[i]), int(starts[i])
+                    _vn_decorrelate_into(xp[a:a + L], out[o:o + L + delay], progs[prog_of[i]], ep, stream)
+            else:
+                N.check(rc, "vnd_vn_decorrelate_batch_dev")
+        results = out.view(n, -1, 2) if is_array else [out[int(o):int(o) + int(L) + delay] for o, L in zip(starts, lengths)]
+    else:
+        if is_array:
+            xp = np.ascontiguousarray(x3).reshape(-1, 2)  # already packed: a view when the input is C-ordered float32
+        else:
+            xp = R.pinned_empty((rows, 2), np.float32)  # page-locked (within the pool's cap): uploaded by DMA, no staging copy
+            _pack_clips(xp, clips, offsets)
+        if xp.ctypes.data % 8:  # the kernels load one float32 pair per row
+            xp = xp.copy()
+        out = R.pinned_empty((rows + n * delay, 2), np.float64 if out_f64 else np.float32)
+        ps = program.host_struct()
+        N.check(lib.vnd_vn_decorrelate_batch_host(R.HostContext.get().handle, xp.ctypes.data, N.VND_F32, rows, offsets.ctypes.data, n,
+                                                  prog_of.ctypes.data, C.byref(ps), C.byref(ep), out.ctypes.data if out.size else None, out_dt),
+                "vnd_vn_decorrelate_batch_host")
+        results = out.reshape(n, -1, 2) if is_array else [out[o:o + L + delay] for o, L in zip(starts, lengths)]
+
+    if settings["normalizer"] is not None:
+        # numpy sums a column-major clip pairwise, not frame by frame: such clips keep the single-clip path's order
+        for i, ((vn, haas), x) in enumerate(zip(pairs, clips)):
+            if _sums_pairwise(x):
+                y = vn._decorrelate(x, haas)
+                if torch_in:
+                    results[i].copy_(y)
+                else:
+                    results[i][...] = y
+    return results
+
+
+def _vn_decorrelate_into(x32, out, program: TapProgram, ep, stream) -> None:
+    """vnd_vn_decorrelate_dev of one packed (frames, 2) float32 clip into a slice of a batch's output tensor."""
+    import torch
+
+    lib = N.lib()
+    nbytes = C.c_size_t()
+    N.check(lib.vnd_vn_decorrelate_workspace(x32.shape[0], 2, C.byref(ep), C.byref(nbytes)), "vnd_vn_decorrelate_workspace")
+    work = torch.empty(max(nbytes.value, 16), dtype=torch.uint8, device=x32.device)
+    sx, so = R.torch_signal(x32), R.torch_signal(out)
+    ps = R.device_program(program, x32.device)
+    N.check(lib.vnd_vn_decorrelate_dev(C.byref(sx), C.byref(so), C.byref(ps), C.byref(ep), work.data_ptr(), nbytes.value, stream),
+            "vnd_vn_decorrelate_dev")
 
 
 # ------------------------------------------------------------------------------------------------
