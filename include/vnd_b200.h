@@ -213,6 +213,24 @@ int vnd_haas_objective_batch_dev(const void* clips, int32_t clip_dtype, int64_t 
                                  int64_t chan_stride, const int32_t* delays, int32_t n_cand, double* partials,
                                  void* workspace, size_t workspace_bytes, void* stream);
 
+/* The Haas objective above over a flat list of (clip, delay) pairs on ragged clips: one launch, one CTA per pair,
+ * whatever the number of clips and their lengths.
+ *   x             : float32, the clips packed channel-planar: element (t, c) of clip i is
+ *                   x[c * chan_stride + frame_offsets[i] + t], c = 0, 1 (chan_stride >= rows);
+ *   frame_offsets : n_clips + 1 int64, starting at 0, non-decreasing, ending at rows (as for vnd_vn_decorrelate_batch_dev);
+ *   pair_clip, pair_delay : n_pairs int32 each; pair p is clip pair_clip[p] with channel 0 delayed by pair_delay[p] >= 0
+ *                   frames (LR, frames_i + pair_delay[p] output frames).  Any order; listing a clip's delays together keeps
+ *                   the clips that CTAs running at the same time read in L2;
+ *   partials      : n_pairs * 8 float64, the slots of vnd_haas_objective_batch_dev:
+ *                   [sum r, sum r*th, sum r*th^2, sum r*th^3, max|th|, sum L*R, sum L*L, frames].
+ * The 8 partials of pair p equal, bit for bit, those vnd_haas_objective_batch_dev returns for clip pair_clip[p] alone
+ * (float32, planar) with delays = {pair_delay[p]}: both launch the same kernel body (same per-thread striding from frame
+ * 0 of the clip, same accumulation, same warp and block reductions).  The _dev call checks the sizes, the stride and
+ * the pointers; it cannot read the device-side offsets and indices, which must be valid (the _host call checks them).
+ * n_pairs == 0 launches nothing. */
+int vnd_haas_objective_pairs_dev(const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets, int32_t n_clips,
+                                 const int32_t* pair_clip, const int32_t* pair_delay, int32_t n_pairs, double* partials, void* stream);
+
 /* ------------------------------------------------------------------------------ host API */
 typedef struct vnd_ctx vnd_ctx;
 
@@ -257,6 +275,11 @@ int vnd_vn_objective_batch_host(vnd_ctx* ctx, const float* clips, int64_t frames
 int vnd_haas_objective_batch_host(vnd_ctx* ctx, const void* clips, int32_t clip_dtype, int64_t frames, int32_t n_clips,
                                   int64_t clip_stride, int64_t chan_stride, const int32_t* delays,
                                   int32_t n_cand, double* partials);
+/* vnd_haas_objective_pairs_dev with host buffers.  Checks, before any copy, that the offsets start at 0, never decrease
+ * and end at rows, that every pair_clip is in [0, n_clips), that every delay is >= 0, and that no pair puts delay 0 on
+ * an empty clip (an empty signal has no objective: optimization.py:41-43).  Then one upload, one launch, one download. */
+int vnd_haas_objective_pairs_host(vnd_ctx* ctx, const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets,
+                                  int32_t n_clips, const int32_t* pair_clip, const int32_t* pair_delay, int32_t n_pairs, double* partials);
 
 /* The overlapped path of vnd_sparse_fir_host with an explicit stage size: x and y are HOST planar
  * (channels, frames) float32 slabs; channels are cut into groups of `channels_per_chunk`, and

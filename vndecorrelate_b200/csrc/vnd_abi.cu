@@ -38,6 +38,8 @@ int vn_objective_launch(const float* clips, long long frames, int n_clips, long 
                         const vnd_tap_program* cand, double* partials, void* workspace, size_t workspace_bytes, cudaStream_t st);
 int haas_objective_launch(const void* clips, int clip_dtype, long long frames, int n_clips, long long clip_stride, long long chan_stride,
                           const int* delays, int n_cand, double* partials, cudaStream_t st);
+int haas_objective_pairs_launch(const float* x, long long chan_stride, const long long* offs, const int* pair_clip, const int* pair_delay,
+                                int n_pairs, double* partials, cudaStream_t st);
 size_t dsp_workspace_bytes(long long elems);
 int rms_normalize_launch(const vnd_signal* x, const vnd_signal* y, int x_ndim, int y_ndim, int stereo_mode, double eps, void* ws, cudaStream_t st);
 int peak_normalize_launch(const vnd_signal* y, int ndim, int stereo_mode, double eps, void* ws, cudaStream_t st);
@@ -330,6 +332,29 @@ extern "C" int vnd_haas_objective_batch_dev(const void* clips, int32_t clip_dtyp
   VND_REQUIRE((clips != nullptr && partials != nullptr && delays != nullptr) || n_clips == 0 || n_cand == 0, VND_EINVAL, "null buffer");
   VND_REQUIRE(clip_dtype == VND_F32 || clip_dtype == VND_F64, VND_EINVAL, "unknown clip dtype %d", clip_dtype);
   return haas_objective_launch(clips, clip_dtype, frames, n_clips, clip_stride, chan_stride, delays, n_cand, partials, (cudaStream_t)stream);
+}
+
+// Arguments of the pair-list Haas objective that can be checked without reading device memory.
+static int check_haas_pairs(const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets, int32_t n_clips,
+                            const int32_t* pair_clip, const int32_t* pair_delay, int32_t n_pairs, const double* partials) {
+  VND_REQUIRE(rows >= 0 && n_clips >= 0 && n_pairs >= 0, VND_EINVAL, "negative extent (rows %lld, n_clips %d, n_pairs %d)", (long long)rows,
+              n_clips, n_pairs);
+  VND_REQUIRE(chan_stride >= rows, VND_EINVAL, "chan_stride %lld is shorter than rows = %lld: the two channels overlap", (long long)chan_stride,
+              (long long)rows);
+  if (n_pairs == 0) return VND_OK;
+  VND_REQUIRE(n_clips > 0, VND_EINVAL, "%d pairs but no clips", n_pairs);
+  VND_REQUIRE(x != nullptr || rows == 0, VND_EINVAL, "x is null");
+  VND_REQUIRE(frame_offsets != nullptr && pair_clip != nullptr && pair_delay != nullptr && partials != nullptr, VND_EINVAL,
+              "frame_offsets, pair_clip, pair_delay or partials is null");
+  return VND_OK;
+}
+
+extern "C" int vnd_haas_objective_pairs_dev(const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets, int32_t n_clips,
+                                            const int32_t* pair_clip, const int32_t* pair_delay, int32_t n_pairs, double* partials, void* stream) {
+  int rc;
+  if ((rc = check_haas_pairs(x, rows, chan_stride, frame_offsets, n_clips, pair_clip, pair_delay, n_pairs, partials))) return rc;
+  return haas_objective_pairs_launch(x, chan_stride, reinterpret_cast<const long long*>(frame_offsets), pair_clip, pair_delay, n_pairs, partials,
+                                     (cudaStream_t)stream);
 }
 
 static int check_flat(const vnd_signal* s, int ndim, const char* name) {
@@ -1205,6 +1230,51 @@ extern "C" int vnd_haas_objective_batch_host(vnd_ctx* ctx, const void* clips, in
   VND_CUDA_OK(cudaMemcpyAsync(din, clips, in_bytes, cudaMemcpyHostToDevice, st));
   VND_CUDA_OK(cudaMemcpyAsync(dd, delays, (size_t)n_cand * 4, cudaMemcpyHostToDevice, st));
   if ((rc = haas_objective_launch(din, clip_dtype, frames, n_clips, clip_stride, chan_stride, (const int*)dd, n_cand, (double*)dout, st)))
+    return rc;
+  VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
+  VND_CUDA_OK(cudaStreamSynchronize(st));
+  return VND_OK;
+}
+
+extern "C" int vnd_haas_objective_pairs_host(vnd_ctx* ctx, const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets,
+                                             int32_t n_clips, const int32_t* pair_clip, const int32_t* pair_delay, int32_t n_pairs,
+                                             double* partials) {
+  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  int rc;
+  if ((rc = check_haas_pairs(x, rows, chan_stride, frame_offsets, n_clips, pair_clip, pair_delay, n_pairs, partials))) return rc;
+  if (n_pairs == 0) return VND_OK;
+  const int64_t* offs = frame_offsets;
+  VND_REQUIRE(offs[0] == 0, VND_EINVAL, "frame_offsets[0] is %lld, not 0", (long long)offs[0]);
+  for (int i = 0; i < n_clips; ++i)
+    VND_REQUIRE(offs[i + 1] >= offs[i], VND_EINVAL, "frame_offsets decrease at clip %d (%lld -> %lld)", i, (long long)offs[i],
+                (long long)offs[i + 1]);
+  VND_REQUIRE(offs[n_clips] == rows, VND_EINVAL, "frame_offsets end at %lld, not at rows = %lld", (long long)offs[n_clips], (long long)rows);
+  for (int p = 0; p < n_pairs; ++p) {
+    const int c = pair_clip[p], d = pair_delay[p];
+    VND_REQUIRE(c >= 0 && c < n_clips, VND_EINVAL, "pair_clip[%d] = %d is outside [0, %d)", p, c, n_clips);
+    VND_REQUIRE(d >= 0, VND_EINVAL, "pair_delay[%d] = %d is negative", p, d);
+    // the reference takes max(|theta|) of the frames: an empty output is a ValueError there (optimization.py:41-43)
+    VND_REQUIRE(d > 0 || offs[c + 1] > offs[c], VND_EINVAL,
+                "pair %d: objective of an empty signal (clip %d has no frames and delay 0: zero-size array to reduction operation maximum "
+                "which has no identity)", p, c);
+  }
+  VND_ENTER(ctx);
+  cudaStream_t st = ctx->streams[0];
+  const size_t in_bytes = rows > 0 ? ((size_t)chan_stride + rows) * 4 : 0;
+  const size_t out_bytes = (size_t)n_pairs * 8 * 8;
+  const size_t off_bytes = ((size_t)n_clips + 1) * 8, idx_bytes = (size_t)n_pairs * 4;
+  void *din = nullptr, *dout = nullptr, *dmeta = nullptr;
+  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) ||
+      (rc = arena(ctx, S_AUX, off_bytes + 2 * idx_bytes, &dmeta)))
+    return rc;
+  char* meta = reinterpret_cast<char*>(dmeta);
+  if (in_bytes) VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
+  VND_CUDA_OK(cudaMemcpyAsync(meta, offs, off_bytes, cudaMemcpyHostToDevice, st));
+  VND_CUDA_OK(cudaMemcpyAsync(meta + off_bytes, pair_clip, idx_bytes, cudaMemcpyHostToDevice, st));
+  VND_CUDA_OK(cudaMemcpyAsync(meta + off_bytes + idx_bytes, pair_delay, idx_bytes, cudaMemcpyHostToDevice, st));
+  if ((rc = haas_objective_pairs_launch((const float*)din, chan_stride, reinterpret_cast<const long long*>(meta),
+                                        reinterpret_cast<const int*>(meta + off_bytes), reinterpret_cast<const int*>(meta + off_bytes + idx_bytes),
+                                        n_pairs, (double*)dout, st)))
     return rc;
   VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));

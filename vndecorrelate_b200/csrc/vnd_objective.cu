@@ -449,14 +449,60 @@ struct HaasAcc {
   }
 };
 
+// Work-item sources of haas_objective_kernel: each CTA asks its source for one (clip, delay) item - the clip's two
+// planar channels, its frame count, the delay and where its 8 partials go.  The body of the kernel is shared, so an
+// item gives the same bits whichever source hands it out.
 template <typename TIn>
-__global__ void __launch_bounds__(256) haas_objective_kernel(const TIn* __restrict__ clips, long long frames, long long clip_stride,
-                                                             long long chan_stride, const int* __restrict__ delays, int n_cand,
-                                                             double* __restrict__ partials) {
-  const int cand = blockIdx.x, clip = blockIdx.y;
-  const int d = delays[cand];
-  const TIn* __restrict__ x0 = clips + (long long)clip * clip_stride;
-  const TIn* __restrict__ x1 = x0 + chan_stride;
+struct HaasItem {
+  const TIn* x0;  // channel 0 (the delayed one)
+  const TIn* x1;  // channel 1
+  long long frames;
+  int d;
+  double* out;  // HAAS_SLOTS doubles
+};
+
+// grid (cand, clip) over n_clips equal-length planar clips: element (clip, c, t) = clips[clip * clip_stride + c * chan_stride + t]
+template <typename TIn>
+struct HaasGridSrc {
+  using T = TIn;
+  const TIn* clips;
+  long long frames, clip_stride, chan_stride;
+  const int* delays;
+  int n_cand;
+  double* partials;  // (n_clips, n_cand, HAAS_SLOTS)
+  __device__ __forceinline__ HaasItem<TIn> item() const {
+    const int cand = blockIdx.x, clip = blockIdx.y;
+    const TIn* x0 = clips + (long long)clip * clip_stride;
+    return {x0, x0 + chan_stride, frames, delays[cand], partials + ((size_t)clip * n_cand + cand) * HAAS_SLOTS};
+  }
+};
+
+// pair p = blockIdx.x of a flat (clip, delay) list over ragged clips packed channel-planar: element (t, c) of clip i is
+// x[c * chan_stride + offs[i] + t]
+struct HaasPairSrc {
+  using T = float;
+  const float* x;
+  long long chan_stride;
+  const long long* offs;
+  const int* pair_clip;
+  const int* pair_delay;
+  double* partials;  // (n_pairs, HAAS_SLOTS)
+  __device__ __forceinline__ HaasItem<float> item() const {
+    const int p = blockIdx.x;
+    const int clip = pair_clip[p];
+    const long long o = offs[clip];
+    return {x + o, x + chan_stride + o, offs[clip + 1] - o, pair_delay[p], partials + (size_t)p * HAAS_SLOTS};
+  }
+};
+
+template <typename Src>
+__global__ void __launch_bounds__(256) haas_objective_kernel(const Src src) {
+  using TIn = typename Src::T;
+  const HaasItem<TIn> it = src.item();
+  const long long frames = it.frames;
+  const int d = it.d;
+  const TIn* __restrict__ x0 = it.x0;
+  const TIn* __restrict__ x1 = it.x1;
   const long long total = frames + d;
   HaasAcc acc;
   // Three stretches (decorrelation.py:220-222: channel 0 delayed by d, both padded to frames + d): only channel 1 for
@@ -501,9 +547,9 @@ __global__ void __launch_bounds__(256) haas_objective_kernel(const TIn* __restri
     const int k = threadIdx.x;
     double r = red[0][k];
     for (int w = 1; w < 8; ++w) r = (k == 4) ? fmax(r, red[w][k]) : r + red[w][k];
-    partials[((size_t)clip * n_cand + cand) * HAAS_SLOTS + k] = r;
+    it.out[k] = r;
   }
-  if (threadIdx.x == 7) partials[((size_t)clip * n_cand + cand) * HAAS_SLOTS + 7] = (double)total;
+  if (threadIdx.x == 7) it.out[7] = (double)total;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -643,9 +689,16 @@ int haas_objective_launch(const void* clips, int clip_dtype, long long frames, i
   VND_REQUIRE(n_clips <= 65535, VND_EUNSUPPORTED, "too many clips for one launch");
   dim3 grid((unsigned)n_cand, (unsigned)n_clips);
   if (clip_dtype == VND_F64)
-    haas_objective_kernel<double><<<grid, 256, 0, st>>>((const double*)clips, frames, clip_stride, chan_stride, delays, n_cand, partials);
+    haas_objective_kernel<<<grid, 256, 0, st>>>(HaasGridSrc<double>{(const double*)clips, frames, clip_stride, chan_stride, delays, n_cand, partials});
   else
-    haas_objective_kernel<float><<<grid, 256, 0, st>>>((const float*)clips, frames, clip_stride, chan_stride, delays, n_cand, partials);
+    haas_objective_kernel<<<grid, 256, 0, st>>>(HaasGridSrc<float>{(const float*)clips, frames, clip_stride, chan_stride, delays, n_cand, partials});
+  return after_launch("haas_objective_kernel");
+}
+
+int haas_objective_pairs_launch(const float* x, long long chan_stride, const long long* offs, const int* pair_clip, const int* pair_delay,
+                                int n_pairs, double* partials, cudaStream_t st) {
+  if (n_pairs == 0) return VND_OK;
+  haas_objective_kernel<<<(unsigned)n_pairs, 256, 0, st>>>(HaasPairSrc{x, chan_stride, offs, pair_clip, pair_delay, partials});
   return after_launch("haas_objective_kernel");
 }
 

@@ -17,6 +17,9 @@ one kernel launch per Brent iteration over all live minimisers instead of one pe
 ``optimize_velvet_noise_batch`` runs the whole optimisation for MANY clips (BASELINE config 5): clips are
 partitioned over the ranks of ``torch.distributed`` (one process per GPU), the grid scores are all-gathered as one
 float32 matrix (the only collective on the data path), and each rank refines the local minima of its own clips.
+``optimize_haas_delay_batch`` does the same for ``optimize_haas_delay`` on clips of any lengths: one launch of the Haas
+objective over a flat (clip, delay) list for the whole grid, and one per Brent round over every live minimiser of every
+clip of the rank.
 """
 
 from __future__ import annotations
@@ -34,7 +37,8 @@ from .utils.dsp import EPSILON, LayoutMode
 
 __all__ = [
     "symmetry_aware_objective", "grid_scan", "get_local_minima", "optimize_local_minima", "optimize_haas_delay",
-    "optimize_velvet_noise", "optimize_velvet_noise_batch", "vn_objective_partials", "haas_objective_partials", "vn_scores_from_partials", "haas_scores_from_partials",
+    "optimize_velvet_noise", "optimize_velvet_noise_batch", "optimize_haas_delay_batch", "vn_objective_partials", "haas_objective_partials",
+    "haas_objective_pair_partials", "vn_scores_from_partials", "haas_scores_from_partials",
 ]
 
 _F32_HALF_PI = np.float32(np.pi / 2)
@@ -128,6 +132,49 @@ def haas_objective_partials(clips, delays: Sequence[int]):
     return out
 
 
+def haas_objective_pair_partials(x, frame_offsets, pair_clip, pair_delay):
+    """Partial sums of the Haas objective for a flat list of (clip, delay) pairs over ragged clips, in one launch.
+
+    ``x``: float32 ``(2, chan_stride)`` channel-planar clips (numpy array or CUDA tensor); clip ``i`` is columns
+    ``frame_offsets[i]:frame_offsets[i + 1]``.  Pair ``p`` delays channel 0 of clip ``pair_clip[p]`` by ``pair_delay[p]``
+    frames.  Returns float64 ``(n_pairs, 8)``, row ``p`` bit-equal to ``haas_objective_partials(clip, [d])[0, 0]`` of
+    that clip cast to float32.  With a CUDA tensor the offsets and pairs may be numpy or CUDA tensors and the result is
+    a CUDA tensor enqueued on torch's current stream (nothing is checked that would need the device's copy of the
+    offsets); with numpy everything is checked on the host first."""
+    lib = N.lib()
+    if R.is_torch_tensor(x):
+        import torch
+
+        if not x.is_cuda or x.dtype != torch.float32 or x.dim() != 2 or x.shape[0] != 2 or x.stride(1) != 1:
+            raise ValueError("x must be a CUDA float32 tensor of shape (2, chan_stride) with contiguous rows")
+        dev = x.device
+        # rows only bounds the stride check: taken from host offsets, else from x itself (reading a device tensor would wait)
+        rows = x.shape[1] if R.is_torch_tensor(frame_offsets) else int(np.asarray(frame_offsets)[-1])
+        offs = torch.as_tensor(frame_offsets, dtype=torch.int64, device=dev).contiguous()
+        pc = torch.as_tensor(pair_clip, dtype=torch.int32, device=dev).contiguous()
+        pd = torch.as_tensor(pair_delay, dtype=torch.int32, device=dev).contiguous()
+        if pc.shape != pd.shape or pc.dim() != 1 or offs.dim() != 1 or offs.numel() == 0:
+            raise ValueError("frame_offsets must be 1-D with n_clips + 1 entries; pair_clip and pair_delay 1-D and of one length")
+        out = torch.empty((pc.shape[0], N.HAAS_SLOTS), dtype=torch.float64, device=dev)
+        with torch.cuda.device(dev):
+            N.check(lib.vnd_haas_objective_pairs_dev(x.data_ptr(), rows, x.stride(0), offs.data_ptr(), offs.shape[0] - 1, pc.data_ptr(), pd.data_ptr(),
+                                                     pc.shape[0], out.data_ptr(), R.torch_stream_ptr(x)), "vnd_haas_objective_pairs_dev")
+        return out
+    x = np.asarray(x)
+    if x.dtype != np.float32 or x.ndim != 2 or x.shape[0] != 2:
+        raise ValueError("x must be a float32 array of shape (2, chan_stride)")
+    x = np.ascontiguousarray(x)
+    offs = np.ascontiguousarray(frame_offsets, dtype=np.int64)
+    pc = np.ascontiguousarray(pair_clip, dtype=np.int32)
+    pd = np.ascontiguousarray(pair_delay, dtype=np.int32)
+    if pc.shape != pd.shape or pc.ndim != 1 or offs.ndim != 1 or offs.size == 0:
+        raise ValueError("frame_offsets must be 1-D with n_clips + 1 entries; pair_clip and pair_delay 1-D and of one length")
+    out = np.empty((pc.size, N.HAAS_SLOTS), dtype=np.float64)
+    N.check(lib.vnd_haas_objective_pairs_host(R.HostContext.get().handle, x.ctypes.data, int(offs[-1]), x.shape[1], offs.ctypes.data, offs.size - 1,
+                                              pc.ctypes.data, pd.ctypes.data, pc.size, out.ctypes.data), "vnd_haas_objective_pairs_host")
+    return out
+
+
 # ------------------------------------------------------------------------------------------------
 # scalar combination (optimization.py:71-105 and the helpers :11-43)
 # ------------------------------------------------------------------------------------------------
@@ -216,6 +263,29 @@ def _vn_scores_rows(flat: np.ndarray, angle_limit, lambda_mean, lambda_skew, lam
     return -objective
 
 
+def _haas_scores_rows(flat: np.ndarray, angle_limit, lambda_mean, lambda_skew, lambda_correlation, lambda_penalty) -> np.ndarray:
+    """``_haas_score`` for many rows at once, as ``_vn_scores_rows`` does it for ``_vn_score``: the basic operations and
+    ``np.sqrt`` element by element in float64, every ``**`` the scalar call of the one-row chain (Python-float ``** 1.5``
+    and ``** 2``, ``np.float64 ** 2`` for the correlation), and Python's ``max`` as the selection it is.
+    ``tests/test_haas_delay_batch.py`` asserts bit equality with ``_haas_score``."""
+    p = np.asarray(flat, dtype=np.float64)
+    denom = p[:, 0] + EPSILON
+    spread = p[:, 2] / denom
+    cen = p[:, 1] / denom
+    m3 = p[:, 3] / denom
+    floor = np.where(EPSILON > spread, EPSILON, spread)  # max(spread, EPSILON): spread unless EPSILON is greater
+    skew = m3 / np.array([v ** 1.5 for v in floor.tolist()], dtype=np.float64)
+    nl = np.sqrt(p[:, 6]) + EPSILON
+    corr = p[:, 5] / (nl * nl)
+    over = p[:, 4] - angle_limit
+    exceed = np.where(over > 0.0, over, 0.0)  # max(0.0, over): over only if greater
+    sq = lambda v: np.array([t ** 2 for t in v.tolist()], dtype=np.float64)  # noqa: E731  (Python floats)
+    objective = spread - lambda_mean * sq(cen) - lambda_skew * sq(skew)
+    objective = objective - lambda_correlation * np.array([c ** 2 for c in corr], dtype=np.float64)  # np.float64 scalars
+    objective = objective - lambda_penalty * sq(exceed)
+    return -objective
+
+
 def vn_scores_from_partials(partials, **kw) -> np.ndarray:
     p = partials.cpu().numpy() if R.is_torch_tensor(partials) else np.asarray(partials)
     flat = p.reshape(-1, N.OBJ_SLOTS)
@@ -227,7 +297,9 @@ def vn_scores_from_partials(partials, **kw) -> np.ndarray:
 def haas_scores_from_partials(partials, **kw) -> np.ndarray:
     p = partials.cpu().numpy() if R.is_torch_tensor(partials) else np.asarray(partials)
     flat = p.reshape(-1, N.HAAS_SLOTS)
-    return np.array([_haas_score(row, **kw) for row in flat], dtype=np.float64).reshape(p.shape[:-1])
+    if len(flat) == 0:
+        return np.zeros(p.shape[:-1], dtype=np.float64)
+    return _haas_scores_rows(flat, **kw).reshape(p.shape[:-1])
 
 
 # ------------------------------------------------------------------------------------------------
@@ -971,5 +1043,175 @@ def optimize_velvet_noise_batch(*, input_signals=None, sample_rate_hz: int, dura
         info = {"scores": scores, "local_minima": minima, "argmin": [int(np.argmin(r)) for r in scores],
                 "evaluations_local": bank.evaluations if bank is not None else 0, "launches_local": bank.launches if bank is not None else 0,
                 "clips_local": (lo, hi)}
+        return refined, info
+    return refined
+
+
+# ------------------------------------------------------------------------------------------------
+# optimize_haas_delay for many clips of any lengths: one launch for the grid, one per Brent round
+# ------------------------------------------------------------------------------------------------
+
+
+def _haas_batch_clips(signals, first: int = 0) -> list:
+    """The clips of ``signals`` (a list of numpy arrays or CUDA tensors, or one ``(n_clips, frames, 2)`` array or
+    tensor) as a list, after the shape checks ``_as_stereo_f32`` makes, before any device work.  ``first`` is the
+    index of the first clip in the whole batch (for the messages)."""
+    if R.is_torch_tensor(signals) or isinstance(signals, np.ndarray):
+        if signals.ndim != 3 or signals.shape[2] != 2:
+            raise ValueError(f"a batch array must have shape (n_clips, frames, 2), got {tuple(signals.shape)}")
+        clips = [signals[i] for i in range(signals.shape[0])]
+    else:
+        clips = [c if R.is_torch_tensor(c) else np.asarray(c) for c in signals]
+    kinds = {R.is_torch_tensor(c) for c in clips}
+    if len(kinds) > 1:
+        raise ValueError("clips must be all numpy arrays or all CUDA tensors, not a mix")
+    if kinds == {True}:
+        if not all(c.is_cuda for c in clips):
+            raise ValueError("torch clips must be CUDA tensors")
+        if len({c.device for c in clips}) > 1:
+            raise ValueError(f"CUDA clips must be on one device, got {sorted({str(c.device) for c in clips})}")
+    for i, c in enumerate(clips):
+        shape = tuple(c.shape)
+        if len(shape) not in (1, 2) or (len(shape) == 2 and shape[1] < 2):
+            raise ValueError(f"clip {first + i}: Input shape invalid: Expected shape (num samples, 2), but got shape {shape}.")
+        if shape[0] == 0:
+            raise ValueError(f"clip {first + i} is empty: zero-size array to reduction operation maximum which has no identity")
+    return clips
+
+
+class _HaasClipBank:
+    """The rank's clips resident on its GPU, packed once into one channel-planar float32 ``(2, rows)`` tensor (clip ``i``
+    is columns ``offs[i]:offs[i + 1]``, cast and sliced as ``_as_stereo_f32`` does), and the evaluation of flat
+    (clip, delay) lists on them: one launch, one download of the partial sums, one vectorised scoring pass."""
+
+    def __init__(self, clips, kw: dict):
+        import torch
+
+        lengths = [int(c.shape[0]) for c in clips]
+        self.offs = np.zeros(len(clips) + 1, dtype=np.int64)
+        np.cumsum(lengths, out=self.offs[1:])
+        rows = int(self.offs[-1])
+        if clips and R.is_torch_tensor(clips[0]):
+            self.device = clips[0].device
+            x = torch.empty((2, rows), dtype=torch.float32, device=self.device)
+            for c, a, b in zip(clips, self.offs[:-1], self.offs[1:]):
+                t = c.to(torch.float32)  # rounds like numpy's astype
+                x[:, a:b] = (t[:, None].expand(-1, 2) if t.dim() == 1 else t[:, :2]).T
+        else:
+            self.device = torch.device("cuda", R.default_device())
+            host = np.empty((2, rows), dtype=np.float32)
+            for c, a, b in zip(clips, self.offs[:-1], self.offs[1:]):
+                host[:, a:b] = _as_stereo_f32(c).T
+            x = torch.from_numpy(host).to(self.device)
+        self.x = x
+        self.n = len(clips)
+        self.kw = kw
+        self.offs_dev = torch.from_numpy(self.offs).to(self.device)
+        self.evaluations = 0
+        self.launches = 0
+
+    def scores(self, clip_ids, delays) -> np.ndarray:
+        """float64 scores of the pairs (``clip_ids[p]``, ``delays[p]``), in pair order: ONE kernel launch."""
+        import torch
+
+        pc = np.ascontiguousarray(clip_ids, dtype=np.int32)
+        if pc.size == 0:
+            return np.zeros(0, dtype=np.float64)
+        pairs = torch.from_numpy(np.stack((pc, np.ascontiguousarray(delays, dtype=np.int32)))).to(self.device)
+        with torch.cuda.device(self.device):
+            p = haas_objective_pair_partials(self.x, self.offs_dev, pairs[0], pairs[1])
+        self.launches += 1
+        self.evaluations += pc.size
+        return haas_scores_from_partials(p.cpu().numpy(), **self.kw)
+
+
+def optimize_haas_delay_batch(*, input_signals=None, sample_rate_hz: int, max_delay_seconds: float, grid_size: int = 400,
+                              angle_limit: float = np.pi / 4, lambda_mean: float = 5.0, lambda_skew: float = 2.0, lambda_correlation: float = 15.0,
+                              lambda_penalty: float = 1e3, group=None, details: bool = False, local_signals=None, total_clips: int | None = None,
+                              _bank_factory=None):
+    """``optimize_haas_delay`` (optimization.py:158-227) for MANY clips of any lengths: returns the float64 array of
+    optimised ``delay_time_seconds`` values, element ``i`` equal to what ``optimize_haas_delay(input_signal=
+    input_signals[i], ...)`` returns (for a CUDA tensor clip: on ``clip.cpu().numpy()``).
+
+    ``input_signals``: a list of clips - numpy arrays or CUDA tensors (not a mix, one device), mono ``(frames,)``,
+    stereo ``(frames, 2)`` or wider ``(frames, k)`` (the first two channels are used), any dtype, cast to float32 as the
+    single-clip call does - or one ``(n_clips, frames, 2)`` array or tensor.  An empty clip raises ``ValueError`` naming
+    its index before any device work.  With ``torch.distributed`` initialised the clips are partitioned in contiguous
+    blocks over the ranks of ``group`` (``sharding.block_range``), exactly as in ``optimize_velvet_noise_batch``: every
+    rank passes the same ``input_signals``, or its own block as ``local_signals`` with ``total_clips``.
+
+    Per rank: its clips are packed once into one resident channel-planar float32 tensor; the grid stage is ONE launch
+    over every (clip, grid delay) pair; the float64 ``(n_clips, grid_size)`` score matrix is all-gathered once; the
+    local minima of every clip of the rank are refined in lock-step with ONE launch per Brent round over all live
+    minimisers; the refined delays are all-gathered once.  Delays in frames are ``round(t * sample_rate_hz)``, as
+    ``HaasEffect.delay_len_samples`` computes them.  ``details=True`` also returns the score matrix, the local-minima
+    sets, the per-clip argmin, and this rank's evaluation, launch and Brent-round counts and clip range."""
+    from . import sharding as S
+
+    kw = dict(angle_limit=angle_limit, lambda_mean=lambda_mean, lambda_skew=lambda_skew, lambda_correlation=lambda_correlation,
+              lambda_penalty=lambda_penalty)
+    rank, world = S._world(group)
+    if local_signals is not None:
+        if total_clips is None:
+            raise ValueError("local_signals needs total_clips (the number of clips over all ranks)")
+        n_clips = int(total_clips)
+        lo, hi = S.block_range(n_clips, rank, world)
+        local = _haas_batch_clips(local_signals, lo)
+        if len(local) != hi - lo:
+            raise ValueError(f"rank {rank} of {world} owns clips [{lo}, {hi}) but local_signals holds {len(local)}")
+    else:
+        if input_signals is None:
+            raise ValueError("pass input_signals (all clips) or local_signals (this rank's block)")
+        every = _haas_batch_clips(input_signals)  # every rank checks every clip, so that all ranks raise alike
+        n_clips = len(every)
+        lo, hi = S.block_range(n_clips, rank, world)
+        local = every[lo:hi]
+
+    taus = np.linspace(0.0, max_delay_seconds, grid_size)
+    grid_delays = np.array([round(t * sample_rate_hz) for t in taus.tolist()], dtype=np.int64)  # HaasEffect.delay_len_samples
+    n_local = hi - lo
+    if n_local > 0:
+        bank = (_bank_factory or _HaasClipBank)(local, kw)
+        print("Starting Grid Scan")
+        local_scores = bank.scores(np.repeat(np.arange(n_local), grid_size), np.tile(grid_delays, n_local)).reshape(n_local, grid_size)
+    else:
+        bank = None
+        local_scores = np.zeros((0, grid_size), dtype=np.float64)
+
+    counts = [S.block_range(n_clips, r, world)[1] - S.block_range(n_clips, r, world)[0] for r in range(world)]
+    device = bank.device if (bank is not None and getattr(bank, "device", None) is not None) else S.collective_device(group)
+    scores = S.all_gather_rows(np.ascontiguousarray(local_scores, dtype=np.float64), counts, device=device, group=group)
+
+    minima = [get_local_minima(row, grid_size) for row in scores]
+    best = np.zeros(n_local, dtype=np.float64)
+    rounds = 0
+    if n_local > 0:
+        print("Starting Local Minima optimization")
+        lows, highs, owner = [], [], []
+        for ci in range(lo, hi):
+            for i in minima[ci]:
+                lows.append(taus[max(0, i - 1)])
+                highs.append(taus[min(grid_size - 1, i + 1)])
+                owner.append(ci - lo)
+        owner = np.asarray(owner, dtype=np.int64)
+        eng = _BrentBatch(lows, highs, 1e-4)
+        while True:  # one launch per round over every live minimiser of every clip (idx ascends: pairs stay clip-major)
+            idx, xs = eng.pending()
+            if len(idx) == 0:
+                break
+            delays = np.array([round(t * sample_rate_hz) for t in xs.tolist()], dtype=np.int64)
+            eng.feed(idx, bank.scores(owner[idx], delays))
+            rounds += 1
+        xs, funs, _ = eng.results()
+        best_score = [np.inf] * n_local
+        for x, fun, c in zip(xs, funs, owner):  # first strictly best minimum of each clip (optimization.py:150-153)
+            if fun < best_score[c]:
+                best_score[c] = fun
+                best[c] = x
+    refined = S.all_gather_rows(best.reshape(-1, 1), counts, device=device, group=group).reshape(-1)
+    if details:
+        info = {"scores": scores, "local_minima": minima, "argmin": [int(np.argmin(r)) for r in scores],
+                "evaluations_local": bank.evaluations if bank is not None else 0, "launches_local": bank.launches if bank is not None else 0,
+                "rounds_local": rounds, "clips_local": (lo, hi)}
         return refined, info
     return refined
