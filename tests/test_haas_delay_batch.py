@@ -159,18 +159,26 @@ def test_pairs_dev_rejects_bad_arguments_without_cuda():
 class _OracleHaasBank:
     """The clip bank's interface, scoring every (clip, delay) pair with the oracle (the reference's procedure in numpy)."""
 
+    lanes = 1
+
     def __init__(self, clips, kw):
         self.clips = [np.asarray(c) for c in clips]
         self.kw = kw
         self.n, self.device = len(self.clips), None
         self.evaluations = self.launches = 0
 
-    def scores(self, clip_ids, delays):
+    def grid_scores(self, delays):
+        return self.submit(np.repeat(np.arange(self.n), len(delays)), np.tile(delays, self.n)).reshape(self.n, len(delays))
+
+    def submit(self, clip_ids, delays):
         self.launches += 1
         self.evaluations += len(clip_ids)
         # sample_rate_hz=1 makes the oracle's round(t * fs) the delay in frames itself
         return np.array([O.objective(O.haas(self.clips[c], sample_rate_hz=1, delay_time_seconds=int(d)), **self.kw)
                          for c, d in zip(clip_ids, delays)], dtype=np.float64)
+
+    def collect(self, handle):
+        return handle
 
 
 _LENGTHS = (3000, 4500, 1200, 5200, 3700)

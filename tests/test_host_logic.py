@@ -307,50 +307,68 @@ def test_no_gpu_means_loud_failure_not_fallback():
 # ------------------------------------------------------------------ lock-step Brent refinement
 
 
+def _lockstep(lows, highs, f):
+    """optimization._BrentBatch run to the end on the objectives ``f(i, x)`` (minimiser ``i`` at abscissa ``x``): its
+    results, the abscissae each minimiser was evaluated at, and the size of every round."""
+    from vndecorrelate_b200.optimization import _BrentBatch
+
+    eng = _BrentBatch(lows, highs, 1e-4)
+    seen, sizes = [[] for _ in range(len(lows))], []
+    while True:
+        idx, xs = eng.pending()
+        if len(idx) == 0:
+            return eng.results(), seen, sizes
+        sizes.append(len(idx))
+        for i, x in zip(idx, xs.tolist()):
+            seen[i].append(x)
+        eng.feed(idx, np.array([f(i, x) for i, x in zip(idx, xs.tolist())]))
+
+
 def test_lockstep_minimize_equals_scipy_one_at_a_time():
     """The lock-step engine runs scipy's own bounded minimiser per interval, so abscissae, values and
     evaluation counts must equal the sequential loop of the reference (optimization.py:131-155),
-    including on a piecewise-constant objective like the velvet-noise one."""
+    including on a piecewise-constant objective like the velvet-noise one; and the refinement built on it picks, clip
+    by clip and whatever the number of lanes, what optimize_local_minima picks."""
     from scipy.optimize import minimize_scalar
 
-    from vndecorrelate_b200.optimization import lockstep_minimize, optimize_local_minima, optimize_local_minima_batched
+    from vndecorrelate_b200.optimization import _refine_minima, optimize_local_minima
 
     def f(x):
         return np.float32(np.floor(40.0 * np.sin(7.0 * x) ** 2) / 40.0 + 0.3 * (x - 0.55) ** 2)
 
     bounds = [(0.0, 0.1), (0.1, 0.35), (0.3, 0.5), (0.45, 0.7), (0.7, 1.0), (0.2, 0.2000001)]
-    calls = []
-
-    def batch(xs):
-        calls.append(len(xs))
-        return [f(x) for x in xs]
-
-    got = lockstep_minimize(bounds, batch, xatol=1e-4)
-    for (lo, hi), g in zip(bounds, got):
+    (x, fun, nfev, _), _, calls = _lockstep([lo for lo, _ in bounds], [hi for _, hi in bounds], lambda i, x: f(x))
+    for i, (lo, hi) in enumerate(bounds):
         want = minimize_scalar(fun=f, bounds=(lo, hi), method="bounded", options={"xatol": 1e-4})
-        assert g.x == want.x and g.fun == want.fun and g.nfev == want.nfev
-    assert calls[0] == len(bounds) and sum(calls) == sum(g.nfev for g in got)  # every batch holds all live minimisers
-    assert len(calls) == max(g.nfev for g in got)
+        assert x[i] == want.x and fun[i] == want.fun and nfev[i] == want.nfev
+    assert calls[0] == len(bounds) and sum(calls) == nfev.sum()  # every batch holds all live minimisers
+    assert len(calls) == nfev.max()
 
     # selection rule of the reference: bounds from the grid neighbours, first strictly best wins
     grid = np.linspace(0.0, 1.0, 21)
-    scores = np.array([f(x) for x in grid])
-    minima = [i for i in range(1, 20) if scores[i] < scores[i - 1] and scores[i] < scores[i + 1]]
-    assert minima
-    a = optimize_local_minima(minima, grid, 21, f)
-    b = optimize_local_minima_batched(minima, grid, 21, lambda xs: [f(x) for x in xs])
-    assert a == b
-    assert lockstep_minimize([], batch) == []
+    fc = [lambda x, c=c: f(x + 0.07 * c) for c in range(5)]  # one objective per clip
+    minima = []
+    for g in fc:
+        scores = np.array([g(x) for x in grid])
+        minima.append([i for i in range(1, 20) if scores[i] < scores[i - 1] and scores[i] < scores[i + 1]])
+        assert minima[-1]
+    want = [optimize_local_minima(m, grid, 21, g) for m, g in zip(minima, fc)]
+    for lanes in (1, 2, 3):
+        got, rounds = _refine_minima(minima, grid, lambda clip_ids, xs: [fc[c](x) for c, x in zip(clip_ids, xs.tolist())], lanes=lanes)
+        assert got.tolist() == want and rounds >= 1
+    got, rounds = _refine_minima([], grid, lambda clip_ids, xs: [])
+    assert got.shape == (0,) and rounds == 0
 
 
 def test_lockstep_minimize_propagates_errors():
-    from vndecorrelate_b200.optimization import lockstep_minimize
+    from vndecorrelate_b200.optimization import _refine_minima
 
-    def bad(xs):
+    def bad(clip_ids, xs):
         raise ValueError("boom")
 
-    with pytest.raises(ValueError, match="boom"):
-        lockstep_minimize([(0.0, 1.0), (1.0, 2.0)], bad)
+    for lanes in (1, 2):
+        with pytest.raises(ValueError, match="boom"):
+            _refine_minima([[2], [5]], np.linspace(0.0, 1.0, 8), bad, lanes=lanes)
 
 
 def test_pinned_output_pool_falls_back_without_a_device():
@@ -405,14 +423,12 @@ def test_kappa_family_program_equals_table_by_table_packing():
     assert identical >= 10 and declined >= 1  # both branches exercised
 
 
-def test_bounded_brent_coroutine_is_scipys_minimiser():
-    """optimization._bounded_brent (the lock-step refinement) against scipy.optimize.minimize_scalar(method="bounded"),
+def test_bounded_brent_batch_is_scipys_minimiser():
+    """optimization._BrentBatch (the lock-step refinement) against scipy.optimize.minimize_scalar(method="bounded"),
     the routine the reference calls (optimization.py:144-149): same abscissae in the same order, same minimum, same
-    value and dtype, same evaluation count - for float32-valued objectives (what the velvet-noise score is),
-    float64-valued ones (Haas), plateaus with ties, and Python floats."""
+    value and dtype, same evaluation count and status - for float32-valued objectives (what the velvet-noise score is),
+    float64-valued ones (Haas), plateaus with ties, and Python floats; the 25 objectives of a kind in one batch."""
     from scipy.optimize import minimize_scalar
-
-    from vndecorrelate_b200.optimization import lockstep_minimize
 
     def make(kind, seed):
         c = np.random.default_rng(seed).uniform(0, 1, 4)
@@ -428,28 +444,32 @@ def test_bounded_brent_coroutine_is_scipys_minimiser():
 
     rng = np.random.default_rng(1)
     for kind in range(5):
+        fs, lows, highs, wants, seen_ref = [], [], [], [], []
         for seed in range(25):
             f = make(kind, seed)
             lo = np.float64(rng.uniform(0, 0.5))
             hi = lo + np.float64(rng.uniform(1e-3, 0.5))
-            seen_ref, seen = [], []
-            want = minimize_scalar(fun=lambda x: (seen_ref.append(float(x)), f(x))[1], bounds=(lo, hi), method="bounded", options={"xatol": 1e-4})
-            got = lockstep_minimize([(lo, hi)], lambda xs: [(seen.append(x), f(x))[1] for x in xs], xatol=1e-4)[0]
-            assert seen == seen_ref
-            assert got.x == want.x and type(got.x) is type(want.x)
-            assert got.fun == want.fun and type(got.fun) is type(want.fun)
-            assert (got.nfev, got.status, got.success) == (want.nfev, want.status, want.success)
+            seen_ref.append([])
+            wants.append(minimize_scalar(fun=lambda x, f=f, s=seen_ref[-1]: (s.append(float(x)), f(x))[1], bounds=(lo, hi), method="bounded",
+                                         options={"xatol": 1e-4}))
+            fs.append(f)
+            lows.append(lo)
+            highs.append(hi)
+        (x, fun, nfev, status), seen, _ = _lockstep(lows, highs, lambda i, x: fs[i](x))
+        for i, want in enumerate(wants):
+            assert seen[i] == seen_ref[i]
+            assert x[i] == want.x
+            assert fun[i] == want.fun and type(fun[i]) is type(want.fun)
+            assert (nfev[i], status[i], status[i] == 0) == (want.nfev, want.status, want.success)
 
 
 def test_lockstep_minimize_batches_all_minimisers():
-    from vndecorrelate_b200.optimization import lockstep_minimize
-
-    calls = []
     bounds = [(i / 64, (i + 2) / 64) for i in range(0, 62, 3)]
-    res = lockstep_minimize(bounds, lambda xs: (calls.append(len(xs)), [np.float32((x - 0.4) ** 2) for x in xs])[1])
-    assert len(res) == len(bounds) and all(r is not None and r.success for r in res)
+    (x, _, _, status), _, calls = _lockstep([lo for lo, _ in bounds], [hi for _, hi in bounds], lambda i, x: np.float32((x - 0.4) ** 2))
+    assert len(x) == len(bounds) and np.all(status == 0)
     assert calls[0] == len(bounds) and calls == sorted(calls, reverse=True)  # everybody in the first round, finished ones drop out
-    assert lockstep_minimize([], lambda xs: []) == []
+    (x, fun, nfev, status), _, calls = _lockstep([], [], lambda i, x: np.float32(x))
+    assert len(x) == len(fun) == len(nfev) == len(status) == 0 and calls == []
 
 
 def test_vectorised_scores_equal_the_one_row_chain_bit_for_bit():
@@ -578,12 +598,12 @@ def test_interval_grid_family_is_bitwise_the_single_strength_grid():
             assert np.array_equal(w1, w[i]) and np.array_equal(s1, s[i])
 
 
-def test_array_brent_equals_the_coroutine_abscissa_by_abscissa():
-    """optimization._BrentBatch (every minimiser of every clip advanced by array arithmetic) against the coroutine
-    restatement of scipy's bounded minimiser - which the tests above pin to scipy itself - on 2000 float32-valued,
-    piecewise-constant noisy objectives (the shape the rounded-tap objective has) and 300 float64 ones: same abscissae
-    in the same order, same x / fun / nfev, fun in the objective's dtype."""
-    from vndecorrelate_b200 import optimization as OPT
+def test_array_brent_equals_scipy_abscissa_by_abscissa():
+    """optimization._BrentBatch (every minimiser of every clip advanced by array arithmetic) against scipy's bounded
+    minimiser run one objective at a time, on 2000 float32-valued, piecewise-constant noisy objectives (the shape the
+    rounded-tap objective has) and 300 float64 ones: same abscissae in the same order, same x / fun / nfev / status, fun
+    in the objective's dtype."""
+    from scipy.optimize import minimize_scalar
 
     rng = np.random.default_rng(0)
 
@@ -601,24 +621,14 @@ def test_array_brent_equals_the_coroutine_abscissa_by_abscissa():
         fs = [make(dtype) for _ in range(n)]
         lo = rng.uniform(0, 0.9, n)
         hi = lo + rng.uniform(1e-3, 0.2, n)
-        seq_a = [[] for _ in range(n)]
-        seq_b = [[] for _ in range(n)]
-
-        def batch_a(xs, ids):
-            for x, i in zip(xs, ids):
-                seq_a[i].append(x)
-            return [fs[i](x) for x, i in zip(xs, ids)]
-
-        def batch_b(xs, ids):
-            for x, i in zip(xs, ids):
-                seq_b[i].append(float(x))
-            return np.array([fs[i](float(x)) for x, i in zip(xs, ids)], dtype=dtype)
-
-        want = OPT.lockstep_minimize(list(zip(lo, hi)), batch_a, xatol=1e-4, with_ids=True)
-        x, fun, nfev = OPT.lockstep_minimize_arrays(lo, hi, batch_b, xatol=1e-4)
+        (x, fun, nfev, status), seen, _ = _lockstep(lo, hi, lambda i, x: fs[i](x))
         assert fun.dtype == dtype
         for i in range(n):
-            assert seq_a[i] == seq_b[i] and want[i].x == x[i] and want[i].fun == fun[i] and want[i].nfev == nfev[i], i
+            seq = []
+            want = minimize_scalar(fun=lambda v: (seq.append(float(v)), fs[i](v))[1], bounds=(lo[i], hi[i]), method="bounded",
+                                   options={"xatol": 1e-4})
+            assert seq == seen[i], i
+            assert want.x == x[i] and want.fun == fun[i] and type(want.fun) is type(fun[i]) and want.nfev == nfev[i] and want.status == status[i], i
 
 
 def test_fir_kernels_have_no_contracted_multiply_add():

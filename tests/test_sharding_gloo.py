@@ -115,18 +115,29 @@ _FS, _DUR, _NIMP, _GRID, _FRAMES = 48000, 0.03, 30, 24, 4000
 
 
 class _OracleBank:
+    """The clip bank's interface (one batch in flight), scoring with the oracle."""
+
+    lanes = 1
+
     def __init__(self, clips, family, kw):
         self.clips = [np.ascontiguousarray(np.asarray(c)) for c in clips]
         self.n, self.frames, self.device = len(self.clips), self.clips[0].shape[0], None
         self.evaluations = self.launches = 0
 
-    def scores(self, requests):
-        out = []
-        for clip, ks in zip(self.clips, requests):
-            self.evaluations += len(ks)
-            out.append(np.asarray(O.vn_grid_scores(clip, list(ks), sample_rate_hz=_FS, duration_seconds=_DUR, num_impulses=_NIMP, seed=1),
-                                  dtype=np.float32) if len(ks) else np.zeros(0, np.float32))
-        return out
+    def _scores(self, c, ks):
+        self.evaluations += len(ks)
+        return np.asarray(O.vn_grid_scores(self.clips[c], list(ks), sample_rate_hz=_FS, duration_seconds=_DUR, num_impulses=_NIMP, seed=1),
+                          dtype=np.float32)
+
+    def grid_scores(self, kappas):
+        return np.stack([self._scores(c, kappas) for c in range(self.n)])
+
+    def submit(self, clip_ids, kappas):
+        kappas = np.asarray(kappas)
+        return np.concatenate([self._scores(c, kappas[clip_ids == c]) for c in np.unique(clip_ids)])
+
+    def collect(self, handle):
+        return handle
 
 
 def _batch_clips():
@@ -177,20 +188,10 @@ def test_optimize_velvet_noise_batch_world2_gloo(tmp_path):
 
 
 class _OracleBankAsync(_OracleBank):
-    """The same oracle-backed bank with the submit / collect interface of the CUDA bank, so that the refinement takes its
-    two-batches-in-flight path on CPU."""
+    """The same oracle-backed bank with two lanes, as the CUDA bank has, so that the refinement keeps two batches in
+    flight on CPU."""
 
-    def submit(self, requests, clip_ids):
-        out = []
-        for c, ks in zip(clip_ids, requests):
-            self.evaluations += len(ks)
-            if len(ks):
-                out.append(np.asarray(O.vn_grid_scores(self.clips[c], list(ks), sample_rate_hz=_FS, duration_seconds=_DUR, num_impulses=_NIMP, seed=1),
-                                      dtype=np.float32))
-        return np.concatenate(out) if out else np.zeros(0, np.float32)
-
-    def collect(self, handle):
-        return handle
+    lanes = 2
 
 
 def test_refinement_with_two_batches_in_flight_equals_the_single_batch():

@@ -11,15 +11,15 @@ combination below follows the reference's dtype chain (float32 for velvet-noise 
 for Haas candidates; SURVEY.md Appendix A.5).
 
 Refinement is the bounded Brent minimiser scipy runs for the reference (``minimize_scalar(method="bounded")``),
-restated as a coroutine (``_bounded_brent``) so that every local minimum - of every clip - advances in lock-step:
-one kernel launch per Brent iteration over all live minimisers instead of one per evaluation.
+restated in array form (``_BrentBatch``) so that every local minimum - of every clip - advances in lock-step
+(``_refine_minima``): one kernel launch per Brent iteration over all live minimisers instead of one per evaluation.
 
 ``optimize_velvet_noise_batch`` runs the whole optimisation for MANY clips (BASELINE config 5): clips are
 partitioned over the ranks of ``torch.distributed`` (one process per GPU), the grid scores are all-gathered as one
 float32 matrix (the only collective on the data path), and each rank refines the local minima of its own clips.
 ``optimize_haas_delay_batch`` does the same for ``optimize_haas_delay`` on clips of any lengths: one launch of the Haas
 objective over a flat (clip, delay) list for the whole grid, and one per Brent round over every live minimiser of every
-clip of the rank.
+clip of the rank.  Both run the same driver (``_optimize_batch``) over a clip bank of their objective.
 """
 
 from __future__ import annotations
@@ -410,9 +410,9 @@ def optimize_local_minima(local_minima: list[int], scalars, grid_size: int, scal
 
 
 # ------------------------------------------------------------------------------------------------
-# The two functions below (``_bounded_brent`` and, in array form, ``_BrentBatch``) restate
-# ``scipy.optimize._optimize._minimize_scalar_bounded`` statement for statement, which SURVEY.md section 8(f).1 asks for so
-# that every comparison of the refinement comes out as in the reference.  That routine is part of SciPy:
+# ``_BrentBatch`` below restates ``scipy.optimize._optimize._minimize_scalar_bounded`` statement for statement, in array
+# form, which SURVEY.md section 8(f).1 asks for so that every comparison of the refinement comes out as in the reference.
+# That routine is part of SciPy:
 #
 #   Copyright (c) 2001-2002 Enthought, Inc. 2003, SciPy Developers.  All rights reserved.
 #
@@ -435,144 +435,20 @@ def optimize_local_minima(local_minima: list[int], scalars, grid_size: int, scal
 #
 # (BSD 3-Clause; the algorithm is Forsythe, Malcolm and Moler's ``fmin``.)
 # ------------------------------------------------------------------------------------------------
-def _bounded_brent(x1, x2, xatol: float, maxiter: int = 500):
-    """Brent's bounded scalar minimiser as a coroutine: yields the next abscissa, is sent the function value, and
-    returns an ``OptimizeResult`` when it has converged.
-
-    This is the algorithm behind ``scipy.optimize.minimize_scalar(method="bounded")`` - the reference's refinement
-    step (optimization.py:144-149) - restated statement for statement after ``_minimize_scalar_bounded`` of the
-    pinned scipy (1.16 in the reference's lock file, 1.18 here; the routine is Forsythe, Malcolm and Moler's
-    ``fmin``), with the same expressions on the same operand types, so that numpy's promotion rules give every
-    intermediate the dtype it has there (the objective returns ``np.float32``) and every comparison comes out the
-    same.  ``tests/test_host_logic.py`` pins it against scipy itself (abscissae, values, evaluation counts).
-    Written as a coroutine so that hundreds of minimisers advance in lock-step without a thread each."""
-    from math import sqrt
-
-    from scipy.optimize import OptimizeResult
-
-    if not (np.isfinite(x1) and np.isfinite(x2)):
-        raise ValueError("Optimization bounds must be finite scalars.")
-    if x1 > x2:
-        raise ValueError("The lower bound exceeds the upper bound.")
-    flag = 0
-    sqrt_eps = sqrt(2.2e-16)
-    golden_mean = 0.5 * (3.0 - sqrt(5.0))
-    a, b = x1, x2
-    fulc = a + golden_mean * (b - a)
-    nfc, xf = fulc, fulc
-    rat = e = 0.0
-    x = xf
-    fx = yield x
-    num = 1
-    fu = np.inf
-    ffulc = fnfc = fx
-    xm = 0.5 * (a + b)
-    tol1 = sqrt_eps * np.abs(xf) + xatol / 3.0
-    tol2 = 2.0 * tol1
-    while np.abs(xf - xm) > (tol2 - 0.5 * (b - a)):
-        golden = 1
-        if np.abs(e) > tol1:  # try a parabolic step
-            golden = 0
-            r = (xf - nfc) * (fx - ffulc)
-            q = (xf - fulc) * (fx - fnfc)
-            p = (xf - fulc) * q - (xf - nfc) * r
-            q = 2.0 * (q - r)
-            if q > 0.0:
-                p = -p
-            q = np.abs(q)
-            r = e
-            e = rat
-            if (np.abs(p) < np.abs(0.5 * q * r)) and (p > q * (a - xf)) and (p < q * (b - xf)):
-                rat = (p + 0.0) / q
-                x = xf + rat
-                if ((x - a) < tol2) or ((b - x) < tol2):
-                    si = np.sign(xm - xf) + ((xm - xf) == 0)
-                    rat = tol1 * si
-            else:
-                golden = 1
-        if golden:  # golden-section step
-            if xf >= xm:
-                e = a - xf
-            else:
-                e = b - xf
-            rat = golden_mean * e
-        si = np.sign(rat) + (rat == 0)
-        x = xf + si * np.maximum(np.abs(rat), tol1)
-        fu = yield x
-        num += 1
-        if fu <= fx:
-            if x >= xf:
-                a = xf
-            else:
-                b = xf
-            fulc, ffulc = nfc, fnfc
-            nfc, fnfc = xf, fx
-            xf, fx = x, fu
-        else:
-            if x < xf:
-                a = x
-            else:
-                b = x
-            if (fu <= fnfc) or (nfc == xf):
-                fulc, ffulc = nfc, fnfc
-                nfc, fnfc = x, fu
-            elif (fu <= ffulc) or (fulc == xf) or (fulc == nfc):
-                fulc, ffulc = x, fu
-        xm = 0.5 * (a + b)
-        tol1 = sqrt_eps * np.abs(xf) + xatol / 3.0
-        tol2 = 2.0 * tol1
-        if num >= maxiter:
-            flag = 1
-            break
-    if np.isnan(xf) or np.isnan(fx) or np.isnan(fu):
-        flag = 2
-    return OptimizeResult(fun=np.asarray(fx)[()], status=flag, success=(flag == 0), x=xf, nfev=num, nit=num)  # numpy scalar, as minimize_scalar returns it
-
-
-def lockstep_minimize(bounds: Sequence[tuple[float, float]], batch_objective: Callable[..., Sequence[Any]], *, xatol: float = 1e-4,
-                      with_ids: bool = False):
-    """Run the bounded Brent minimiser on many intervals at once, in lock-step.
-
-    Every interval gets its own minimiser (``_bounded_brent``: the reference's refinement step,
-    optimization.py:144-149, comparison for comparison).  In every round the pending abscissae of all live
-    minimisers are evaluated with ONE call of ``batch_objective`` (one kernel launch over all of them) and handed
-    back.  Returns the ``OptimizeResult`` list in input order.  The sequence of abscissae each minimiser sees
-    depends only on its own function values, so the results equal those of the one-at-a-time loop whenever
-    ``batch_objective`` returns the values the scalar objective would.  With ``with_ids`` the callback is called as
-    ``batch_objective(abscissae, ids)`` (``ids`` = positions in ``bounds``), which is how the multi-clip optimiser
-    knows the clip each abscissa belongs to."""
-    n = len(bounds)
-    results: list[Any] = [None] * n
-    live: dict[int, Any] = {}
-    pending: dict[int, Any] = {}
-    for i, (lo, hi) in enumerate(bounds):
-        gen = _bounded_brent(lo, hi, xatol)
-        live[i] = gen
-        pending[i] = next(gen)  # the first abscissa (a minimiser always evaluates at least once)
-    while live:
-        ids = sorted(live)
-        xs = [float(pending[i]) for i in ids]
-        vals = batch_objective(xs, ids) if with_ids else batch_objective(xs)
-        for i, v in zip(ids, vals):
-            try:
-                pending[i] = live[i].send(v)
-            except StopIteration as done:
-                results[i] = done.value
-                del live[i], pending[i]
-    return results
-
-
 class _BrentBatch:
-    """``_bounded_brent`` for MANY intervals at once, as array arithmetic: one state vector per variable of scipy's
-    ``_minimize_scalar_bounded``, every statement of its loop applied under a mask to the minimisers that take it.
+    """Brent's bounded scalar minimiser - ``scipy.optimize.minimize_scalar(method="bounded")``, the reference's
+    refinement step (optimization.py:144-149) - for MANY intervals at once, as array arithmetic: one state vector per
+    variable of ``_minimize_scalar_bounded`` of the pinned scipy (1.16 in the reference's lock file, 1.18 here), every
+    statement of its loop applied under a mask to the minimisers that take it.  ``pending`` hands out the abscissa each
+    live minimiser wants evaluated and ``feed`` takes the values, so that all minimisers advance in lock-step.
 
     The element-wise operations (+, -, *, /, abs, sign, comparisons, maximum) are IEEE basic operations, identical in
     an array and on scalars, and the dtypes are the scalar code's: abscissae and step sizes float64, function values
     the objective's own dtype (float32 for velvet-noise candidates), so that ``(xf - nfc) * (fx - ffulc)`` is a float64
     product of a float64 and an exactly widened float32 difference, as under numpy's scalar promotion.  Every minimiser
-    therefore sees the abscissae, takes the branches and returns the values of the coroutine (and so of scipy);
-    ``tests/test_host_logic.py`` compares them abscissa by abscissa on thousands of float32 objectives.  A Brent round
-    over 20 000 minimisers costs about a millisecond here instead of 0.1 s of Python generator switches."""
+    therefore sees the abscissae, takes the branches and returns the values of scipy's; ``tests/test_host_logic.py``
+    compares them abscissa by abscissa on thousands of float32 and float64 objectives.  A Brent round over 20 000
+    minimisers costs about a millisecond here."""
 
     def __init__(self, lows, highs, xatol: float, maxiter: int = 500):
         from math import sqrt
@@ -598,7 +474,7 @@ class _BrentBatch:
         self.flag = np.zeros(self.n, dtype=np.int64)
         self.live = np.ones(self.n, dtype=bool)
         self.started = False
-        self.fx = self.ffulc = self.fnfc = self.fu = None
+        self.fx = self.ffulc = self.fnfc = self.fu = np.zeros(0)  # set by the first feed (an empty batch is never fed)
 
     def pending(self):
         """Indices of the live minimisers and the abscissa each wants evaluated."""
@@ -699,36 +575,55 @@ class _BrentBatch:
         self._close_or_propose(m & ~over)
 
     def results(self):
-        """(x, fun, nfev) arrays; ``fun`` in the objective's dtype, like ``OptimizeResult.fun``."""
-        return self.xf.copy(), self.fx.copy(), self.num.copy()
+        """(x, fun, nfev, status) arrays, the fields of scipy's ``OptimizeResult``: ``fun`` in the objective's dtype,
+        ``status`` 0 (converged), 1 (``maxiter`` evaluations) or 2 (a NaN)."""
+        status = np.where(np.isnan(self.xf) | np.isnan(self.fx) | np.isnan(self.fu), 2, self.flag)
+        return self.xf.copy(), self.fx.copy(), self.num.copy(), status
 
 
-def lockstep_minimize_arrays(lows, highs, batch_objective: Callable[..., Any], *, xatol: float = 1e-4):
-    """``lockstep_minimize`` on the array engine: ``batch_objective(abscissae, ids)`` (numpy arrays) returns the values
-    as an array in the objective's dtype.  Returns ``(x, fun, nfev)`` arrays in input order."""
-    eng = _BrentBatch(lows, highs, xatol)
-    while True:
-        idx, xs = eng.pending()
-        if len(idx) == 0:
-            break
-        eng.feed(idx, batch_objective(xs, idx))
-    return eng.results()
+def _refine_minima(minima: Sequence[Sequence[int]], grid, submit: Callable[[np.ndarray, np.ndarray], Any],
+                   collect: Callable[[Any], Any] = lambda handle: handle, lanes: int = 1) -> tuple[np.ndarray, int]:
+    """``optimize_local_minima`` for many clips, every minimiser in lock-step: bounded Brent (``xatol=1e-4``) between
+    the grid neighbours of each local minimum (``minima[c]``: the grid indices of clip ``c``'s minima), and per clip
+    the first strictly best result (optimization.py:131-155).  Returns the float64 array of each clip's abscissa and the
+    number of Brent rounds.
 
-
-def optimize_local_minima_batched(local_minima: list[int], scalars, grid_size: int, batch_objective: Callable[[list[float]], Sequence[Any]]):
-    """``optimize_local_minima`` with all minima refined in lock-step (one launch per Brent iteration
-    instead of one per evaluation); same bounds, same ``xatol``, same first-strictly-best rule
-    (optimization.py:131-155).  ``batch_objective(list of abscissae)`` returns their values."""
+    ``submit(clip_ids, abscissae)`` starts the evaluation of a clip-major list of pairs and returns a handle;
+    ``collect(handle)`` returns their values in the objective's dtype.  The clips run in ``lanes`` contiguous blocks,
+    each with its own minimisers and one evaluation in flight, so that the host can advance one lane while the device
+    evaluates another.  A minimiser only ever sees its own values, so the result does not depend on the lanes."""
     print("Starting Local Minima optimization")
-    lows = [scalars[max(0, i - 1)] for i in local_minima]
-    highs = [scalars[min(grid_size - 1, i + 1)] for i in local_minima]
-    xs, funs, _ = lockstep_minimize_arrays(lows, highs, lambda x, ids: np.asarray(batch_objective([float(v) for v in x])), xatol=1e-4)
-    best_scalar, best_score = 0.0, np.inf
-    for x, fun in zip(xs, funs):
-        if fun < best_score:
-            best_score = fun
-            best_scalar = x
-    return best_scalar
+    grid = np.asarray(grid, dtype=np.float64)
+    n = len(minima)
+    at = np.array([i for m in minima for i in m], dtype=np.int64)
+    owner = np.repeat(np.arange(n), [len(m) for m in minima])
+    lows, highs = grid[np.maximum(at - 1, 0)], grid[np.minimum(at + 1, len(grid) - 1)]
+    cuts = np.searchsorted(owner, [h * n // lanes for h in range(lanes + 1)])  # lane h: clips [h n / lanes, (h + 1) n / lanes)
+    members = [np.arange(a, b) for a, b in zip(cuts[:-1], cuts[1:])]
+    engines = [_BrentBatch(lows[m], highs[m], 1e-4) for m in members]
+    rounds = [0] * lanes
+
+    def launch(h):
+        idx, xs = engines[h].pending()
+        if len(idx) == 0:
+            return None
+        rounds[h] += 1
+        return idx, submit(owner[members[h][idx]], xs)
+
+    handles = [launch(h) for h in range(lanes)]
+    while any(handle is not None for handle in handles):
+        for h in range(lanes):
+            if handles[h] is not None:
+                idx, handle = handles[h]
+                engines[h].feed(idx, collect(handle))
+                handles[h] = launch(h)
+    best, best_score = np.zeros(n), [np.inf] * n
+    for eng, m in zip(engines, members):
+        xs, funs = eng.results()[:2]
+        for x, fun, c in zip(xs, funs, owner[m]):  # first strictly best minimum of each clip (optimization.py:150-153)
+            if fun < best_score[c]:
+                best_score[c], best[c] = fun, x
+    return best, max(rounds)
 
 
 def _device_clip(x: np.ndarray):
@@ -761,7 +656,8 @@ def optimize_haas_delay(*, input_signal, sample_rate_hz: int, max_delay_seconds:
         p = p.cpu().numpy() if R.is_torch_tensor(p) else p
         return list(haas_scores_from_partials(p, **kw)[0])
 
-    return optimize_local_minima_batched(local_minima, taus, grid_size, batch)
+    best, _ = _refine_minima([local_minima], taus, lambda _, ts: batch(ts.tolist()))
+    return best[0]
 
 
 def optimize_velvet_noise(*, input_signal, sample_rate_hz: int, duration_seconds: float, num_impulses: int, seed: int = 1, grid_size: int = 400,
@@ -797,7 +693,8 @@ def optimize_velvet_noise(*, input_signal, sample_rate_hz: int, duration_seconds
     scores = np.asarray(batch(kappas))
     local_minima = get_local_minima(scores, grid_size)
 
-    return optimize_local_minima_batched(local_minima, kappas, grid_size, batch)
+    best, _ = _refine_minima([local_minima], kappas, lambda _, ks: batch(ks.tolist()))
+    return best[0]
 
 
 # ------------------------------------------------------------------------------------------------
@@ -806,11 +703,13 @@ def optimize_velvet_noise(*, input_signal, sample_rate_hz: int, duration_seconds
 
 
 class _ClipBank:
-    """The rank's clips resident on its GPU as one planar ``(n, 2, frames)`` float32 tensor, and the evaluation of
-    ragged (clip, strengths) requests on them: ONE tap program for all requested strengths, uploaded once, one
-    launch per clip on a sub-range of its candidates, one download of all partial sums, one vectorised scoring pass."""
+    """The rank's clips resident on its GPU as one planar ``(n, 2, frames)`` float32 tensor, and the velvet-noise
+    objective on them: the grid as one launch over clips x candidates, and flat (clip, strength) lists as ONE tap
+    program for all strengths, uploaded once, one launch per clip on a sub-range of its candidates, one asynchronous
+    download of all partial sums, one vectorised scoring pass.  ``lanes = 2`` from two clips on: the refinement keeps two
+    half-batches of clips in flight, so that scoring and the Brent step of one run under the kernels of the other."""
 
-    def __init__(self, clips, family: Callable[[Sequence[float]], TapProgram], kw: dict):
+    def __init__(self, clips, family: Callable[[Sequence[float], int], TapProgram], kw: dict):
         import torch
 
         if R.is_torch_tensor(clips):
@@ -822,6 +721,7 @@ class _ClipBank:
             self.clips = torch.from_numpy(host).to(f"cuda:{R.default_device()}")
         self.n, _, self.frames = self.clips.shape
         self.device = self.clips.device
+        self.lanes = 2 if self.n >= 2 else 1
         self.family = family
         self.kw = kw
         self.evaluations = 0
@@ -837,78 +737,99 @@ class _ClipBank:
             self._work = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
         return self._work, nbytes.value
 
-    def partials(self, requests: Sequence[Sequence[float]], clip_ids: Sequence[int] | None = None):
-        """``requests[i]`` = strengths to evaluate on clip ``clip_ids[i]`` (default: clip ``i``); returns the float64
-        partial sums ``(total, OBJ_SLOTS)`` in request order (a CUDA tensor) and the per-request counts.  Everything is
-        enqueued on torch's current stream; nothing here waits for the device."""
+    def grid_scores(self, kappas: Sequence[float]) -> np.ndarray:
+        """float32 ``(n, len(kappas))`` scores of every clip at every strength: ONE launch."""
+        partials = vn_objective_partials(self.clips, self.family(kappas, self.frames))
+        self.launches += 1
+        self.evaluations += self.n * len(kappas)
+        return vn_scores_from_partials(partials, **self.kw)
+
+    def submit(self, clip_ids: np.ndarray, kappas: Sequence[float]):
+        """Enqueue the evaluation of the clip-major pairs (``clip_ids[p]``, ``kappas[p]``) and the download of their
+        partial sums into page-locked memory; returns a handle for ``collect``.  Nothing here waits for the device."""
         import torch
 
-        if clip_ids is None:
-            clip_ids = range(len(requests))
-        counts = [len(r) for r in requests]
-        total = sum(counts)
-        out = torch.empty((total, N.OBJ_SLOTS), dtype=torch.float64, device=self.device)
-        if total == 0:
-            return out, counts
-        flat = [float(k) for r in requests for k in r]
-        shared = (len(requests) == self.n and len(set(counts)) == 1 and list(clip_ids) == list(range(self.n))
-                  and all(list(r) == list(requests[0]) for r in requests[1:]))
+        starts = np.flatnonzero(np.r_[True, clip_ids[1:] != clip_ids[:-1]])  # one run of pairs per clip
+        ends = np.r_[starts[1:], len(clip_ids)]
+        prog = self.family(kappas, self.frames)
+        out = torch.empty((len(kappas), N.OBJ_SLOTS), dtype=torch.float64, device=self.device)
         lib = N.lib()
         with torch.cuda.device(self.device):
             stream = torch.cuda.current_stream(self.device).cuda_stream
-            if shared:  # the grid stage: every clip scores the same strengths -> one launch over clips x candidates
-                prog = self.family(flat[: counts[0]])
-                ps = R.device_program(prog, self.device)
-                nbytes = C.c_size_t()
-                N.check(lib.vnd_objective_workspace(self.frames, self.n, prog.channels, C.byref(nbytes)), "vnd_objective_workspace")
-                work = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
-                N.check(lib.vnd_vn_objective_batch_dev(self.clips.data_ptr(), self.frames, self.n, 2 * self.frames, self.frames, C.byref(ps),
-                                                       out.data_ptr(), work.data_ptr(), nbytes.value, stream), "vnd_vn_objective_batch_dev")
+            ps = R.device_program(prog, self.device)
+            work, wbytes = self._workspace(int(np.max(ends - starts)))
+            for a, b in zip(starts.tolist(), ends.tolist()):
+                i = int(clip_ids[a])
+                sub = N.TapProgramStruct(ps.words, ps.offsets + 4 * a, ps.n_words, b - a, ps.order, ps.apply_gain, ps.halo, ps.max_channel_words)
+                N.check(lib.vnd_vn_objective_batch_dev(self.clips.data_ptr() + 4 * i * 2 * self.frames, self.frames, 1, 2 * self.frames, self.frames,
+                                                       C.byref(sub), out.data_ptr() + 8 * N.OBJ_SLOTS * a, work.data_ptr(), wbytes, stream),
+                        "vnd_vn_objective_batch_dev")
                 self.launches += 1
-            else:
-                prog = self.family(flat)
-                ps = R.device_program(prog, self.device)
-                work, wbytes = self._workspace(max(counts))
-                base = 0
-                for i, n_i in zip(clip_ids, counts):
-                    if n_i == 0:
-                        continue
-                    sub = N.TapProgramStruct(ps.words, ps.offsets + 4 * base, ps.n_words, n_i, ps.order, ps.apply_gain, ps.halo, ps.max_channel_words)
-                    N.check(lib.vnd_vn_objective_batch_dev(self.clips.data_ptr() + 4 * i * 2 * self.frames, self.frames, 1, 2 * self.frames, self.frames,
-                                                           C.byref(sub), out.data_ptr() + 8 * N.OBJ_SLOTS * base, work.data_ptr(), wbytes, stream),
-                            "vnd_vn_objective_batch_dev")
-                    self.launches += 1
-                    base += n_i
-        self.evaluations += total
-        return out, counts
-
-    def scores(self, requests: Sequence[Sequence[float]]) -> list[np.ndarray]:
-        p, counts = self.partials(requests)
-        flat = vn_scores_from_partials(p.cpu().numpy(), **self.kw) if p.shape[0] else np.zeros(0, dtype=np.float32)
-        out, base = [], 0
-        for n_i in counts:
-            out.append(flat[base: base + n_i])
-            base += n_i
-        return out
-
-    def submit(self, requests: Sequence[Sequence[float]], clip_ids: Sequence[int]):
-        """Enqueue the evaluation of ``requests`` on the clips ``clip_ids`` and the download of its partial sums into
-        page-locked memory; returns a handle for ``collect``.  The host is free until then: the refinement keeps two such
-        batches in flight, so that scoring and the Brent step of one run under the kernels of the other."""
-        import torch
-
-        p, _ = self.partials(requests, clip_ids)
-        host = torch.empty(p.shape, dtype=p.dtype, pin_memory=True)
-        host.copy_(p, non_blocking=True)
+        self.evaluations += len(kappas)
+        host = torch.empty(out.shape, dtype=out.dtype, pin_memory=True)
+        host.copy_(out, non_blocking=True)
         done = torch.cuda.Event()
         done.record(torch.cuda.current_stream(self.device))
-        return host, done, p  # p is kept alive until the copy has run
+        return host, done, out  # out is kept alive until the copy has run
 
     def collect(self, handle) -> np.ndarray:
-        """Scores (flat float32 array, request order) of a submitted batch."""
+        """Scores (flat float32 array, pair order) of a submitted batch."""
         host, done, _ = handle
         done.synchronize()
-        return vn_scores_from_partials(host.numpy(), **self.kw) if host.shape[0] else np.zeros(0, dtype=np.float32)
+        return vn_scores_from_partials(host.numpy(), **self.kw)
+
+
+def _optimize_batch(*, input_signals, local_signals, total_clips, group, details: bool, split: Callable[[Any, int], Sequence],
+                    make_bank: Callable[[Sequence], Any], grid: np.ndarray, convert: Callable[[np.ndarray], Any], dtype):
+    """The multi-clip optimiser behind ``optimize_velvet_noise_batch`` and ``optimize_haas_delay_batch``: resolve the
+    rank's block of clips, score it on the grid, all-gather the score matrix, refine the local minima of the rank's
+    clips in lock-step and all-gather the results.
+
+    ``split(signals, first)`` checks the clips and returns them as a sequence (``first``: the index of the first clip,
+    for the messages).  ``make_bank(clips)`` holds the rank's clips and scores them: ``grid_scores(args)`` returns the
+    ``(n_local, len(grid))`` score matrix in one launch; ``submit(clip_ids, args)`` and ``collect(handle)`` score flat
+    clip-major pairs; ``lanes``, ``device``, ``evaluations`` and ``launches`` are read.  ``convert`` turns an array of
+    grid values or abscissae into the bank's arguments; ``dtype`` is the objective's."""
+    from . import sharding as S
+
+    rank, world = S._world(group)
+    if local_signals is not None:
+        if total_clips is None:
+            raise ValueError("local_signals needs total_clips (the number of clips over all ranks)")
+        n_clips = int(total_clips)
+        lo, hi = S.block_range(n_clips, rank, world)
+        local = split(local_signals, lo)
+        if len(local) != hi - lo:
+            raise ValueError(f"rank {rank} of {world} owns clips [{lo}, {hi}) but local_signals holds {len(local)}")
+    else:
+        if input_signals is None:
+            raise ValueError("pass input_signals (all clips) or local_signals (this rank's block)")
+        every = split(input_signals, 0)  # every rank checks every clip, so that all ranks raise alike
+        n_clips = len(every)
+        lo, hi = S.block_range(n_clips, rank, world)
+        local = every[lo:hi]
+
+    bank = None
+    local_scores = np.zeros((0, len(grid)), dtype=dtype)
+    if hi > lo:
+        bank = make_bank(local)
+        print("Starting Grid Scan")
+        local_scores = np.ascontiguousarray(bank.grid_scores(convert(grid)), dtype=dtype)
+    counts = [b - a for a, b in (S.block_range(n_clips, r, world) for r in range(world))]
+    device = bank.device if (bank is not None and bank.device is not None) else S.collective_device(group)
+    scores = S.all_gather_rows(local_scores, counts, device=device, group=group)  # every rank: (n_clips, grid)
+
+    minima = [get_local_minima(row, len(grid)) for row in scores]
+    best, rounds = np.zeros(hi - lo), 0
+    if hi > lo:
+        best, rounds = _refine_minima(minima[lo:hi], grid, lambda clip_ids, xs: bank.submit(clip_ids, convert(xs)), bank.collect, bank.lanes)
+    refined = S.all_gather_rows(best.reshape(-1, 1), counts, device=device, group=group).reshape(-1)
+    if details:
+        info = {"scores": scores, "local_minima": minima, "argmin": [int(np.argmin(r)) for r in scores],
+                "evaluations_local": bank.evaluations if bank is not None else 0, "launches_local": bank.launches if bank is not None else 0,
+                "rounds_local": rounds, "clips_local": (lo, hi)}
+        return refined, info
+    return refined
 
 
 def optimize_velvet_noise_batch(*, input_signals=None, sample_rate_hz: int, duration_seconds: float, num_impulses: int, seed: int = 1,
@@ -926,125 +847,25 @@ def optimize_velvet_noise_batch(*, input_signals=None, sample_rate_hz: int, dura
     block as ``local_signals`` (e.g. a resident CUDA tensor) together with ``total_clips``.  Data path per rank: grid scores of its clips (one launch over clips x grid) -> ONE all-gather of the
     float32 score matrix so that every rank holds all rows (``get_local_minima`` needs both neighbours of every grid
     point, optimization.py:120-128) -> lock-step Brent refinement of the local minima of its own clips -> one
-    all-gather of the refined strengths.  ``details=True`` also returns the score matrix, the local-minima sets and
-    evaluation counts."""
-    from . import sharding as S
-
+    all-gather of the refined strengths.  ``details=True`` also returns the score matrix, the local-minima sets, the
+    per-clip argmin, and this rank's evaluation, launch and Brent-round counts and clip range."""
     kw = dict(angle_limit=angle_limit, lambda_mean=lambda_mean, lambda_skew=lambda_skew, lambda_correlation=lambda_correlation,
               lambda_penalty=lambda_penalty)
-    rank, world = S._world(group)
-    if local_signals is not None:
-        if total_clips is None:
-            raise ValueError("local_signals needs total_clips (the number of clips over all ranks)")
-        n_clips = int(total_clips)
-        lo, hi = S.block_range(n_clips, rank, world)
-        local = local_signals
-        n_local = local.shape[0] if (R.is_torch_tensor(local) or (isinstance(local, np.ndarray) and local.ndim == 3)) else len(local)
-        if n_local != hi - lo:
-            raise ValueError(f"rank {rank} of {world} owns clips [{lo}, {hi}) but local_signals holds {n_local}")
-    else:
-        if input_signals is None:
-            raise ValueError("pass input_signals (all clips) or local_signals (this rank's block)")
-        n_clips = input_signals.shape[0] if (R.is_torch_tensor(input_signals) or (isinstance(input_signals, np.ndarray) and input_signals.ndim == 3)) \
-            else len(input_signals)
-        lo, hi = S.block_range(n_clips, rank, world)
-        local = input_signals[lo:hi]
 
     def candidate(kappa):
         return VelvetNoise(sample_rate_hz=sample_rate_hz, duration_seconds=duration_seconds, num_impulses=num_impulses,
                            log_distribution_strength=kappa, normalizer=None, filtered_channels=(0,), mode="LR", seed=seed)
 
     envelope = candidate(0.0).segment_envelope
-    frames_box: list[int] = []
 
-    def family(ks):
-        frames = frames_box[0]
+    def family(ks, frames):
         prog = kappa_family_program(ks, sample_rate_hz=sample_rate_hz, duration_seconds=duration_seconds, num_impulses=num_impulses,
                                     envelope=envelope, seed=seed, frames=frames) if seed is not None else None
         return prog if prog is not None else _vn_family_program([candidate(k) for k in ks], frames)
 
-    kappas = np.linspace(0.0, 1.0, grid_size)
-    if hi > lo:
-        bank = (_bank_factory or _ClipBank)(local, family, kw)
-        frames_box.append(bank.frames)
-        print("Starting Grid Scan")
-        local_scores = np.stack(bank.scores([kappas] * (hi - lo))).astype(np.float32)
-    else:
-        bank = None
-        local_scores = np.zeros((0, grid_size), dtype=np.float32)
-
-    counts = [S.block_range(n_clips, r, world)[1] - S.block_range(n_clips, r, world)[0] for r in range(world)]
-    device = bank.device if (bank is not None and getattr(bank, "device", None) is not None) else S.collective_device(group)
-    scores = S.all_gather_rows(local_scores, counts, device=device, group=group)  # every rank: (n_clips, grid)
-
-    minima = [get_local_minima(row, grid_size) for row in scores]
-    best = np.zeros(hi - lo, dtype=np.float64)
-    if hi > lo:
-        print("Starting Local Minima optimization")
-        lows, highs, owner = [], [], []
-        for ci in range(lo, hi):
-            for i in minima[ci]:
-                lows.append(kappas[max(0, i - 1)])
-                highs.append(kappas[min(grid_size - 1, i + 1)])
-                owner.append(ci - lo)
-        owner = np.asarray(owner, dtype=np.int64)
-
-        def requests_of(xs, ids, clips_of_lane):  # ids ascend and the minimisers are listed clip by clip: a clip's requests are one contiguous run
-            own = owner[ids]
-            cuts = np.searchsorted(own, np.asarray(list(clips_of_lane) + [clips_of_lane[-1] + 1]))
-            return [xs[cuts[j]: cuts[j + 1]] for j in range(len(clips_of_lane))]
-
-        n_local = hi - lo
-        if hasattr(bank, "submit") and n_local >= 2:
-            # Two half-batches of clips in flight: while the kernels of one half run, the host scores the other half,
-            # advances its minimisers and packs their next programs.  A minimiser only ever sees its own values, so
-            # the results do not depend on the split.
-            halves = [list(range(0, n_local // 2)), list(range(n_local // 2, n_local))]
-            lows, highs = np.asarray(lows, dtype=np.float64), np.asarray(highs, dtype=np.float64)
-            members = [np.nonzero(np.isin(owner, h))[0] for h in halves]
-            engines = [_BrentBatch(lows[m], highs[m], 1e-4) for m in members]
-            handles: list[Any] = [None, None]
-
-            def launch(h):
-                idx, xs_h = engines[h].pending()
-                if len(idx) == 0:
-                    handles[h] = None
-                    return
-                handles[h] = (idx, bank.submit(requests_of(xs_h, members[h][idx], halves[h]), halves[h]))
-
-            for h in (0, 1):
-                launch(h)
-            while handles[0] is not None or handles[1] is not None:
-                for h in (0, 1):
-                    if handles[h] is None:
-                        continue
-                    idx, handle = handles[h]
-                    engines[h].feed(idx, bank.collect(handle))
-                    launch(h)
-            xs = np.empty(len(owner), dtype=np.float64)
-            funs = np.empty(len(owner), dtype=np.float32)
-            for h in (0, 1):
-                x_h, f_h, _ = engines[h].results()
-                xs[members[h]] = x_h
-                funs[members[h]] = f_h
-        else:
-            def batch(xs, ids):
-                vals = bank.scores(requests_of(xs, ids, list(range(n_local))))
-                return np.concatenate(vals) if len(vals) else np.zeros(0, dtype=np.float32)
-
-            xs, funs, _ = lockstep_minimize_arrays(lows, highs, batch, xatol=1e-4)
-        best_score = [np.inf] * (hi - lo)
-        for x, fun, c in zip(xs, funs, owner):  # first strictly best minimum of each clip (optimization.py:150-153)
-            if fun < best_score[c]:
-                best_score[c] = fun
-                best[c] = x
-    refined = S.all_gather_rows(best.reshape(-1, 1), counts, device=device, group=group).reshape(-1)
-    if details:
-        info = {"scores": scores, "local_minima": minima, "argmin": [int(np.argmin(r)) for r in scores],
-                "evaluations_local": bank.evaluations if bank is not None else 0, "launches_local": bank.launches if bank is not None else 0,
-                "clips_local": (lo, hi)}
-        return refined, info
-    return refined
+    return _optimize_batch(input_signals=input_signals, local_signals=local_signals, total_clips=total_clips, group=group, details=details,
+                           split=lambda signals, first: signals, make_bank=lambda clips: (_bank_factory or _ClipBank)(clips, family, kw),
+                           grid=np.linspace(0.0, 1.0, grid_size), convert=np.ndarray.tolist, dtype=np.float32)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -1082,7 +903,8 @@ def _haas_batch_clips(signals, first: int = 0) -> list:
 class _HaasClipBank:
     """The rank's clips resident on its GPU, packed once into one channel-planar float32 ``(2, rows)`` tensor (clip ``i``
     is columns ``offs[i]:offs[i + 1]``, cast and sliced as ``_as_stereo_f32`` does), and the evaluation of flat
-    (clip, delay) lists on them: one launch, one download of the partial sums, one vectorised scoring pass."""
+    (clip, delay) lists on them: one launch, one synchronous download of the partial sums, one vectorised scoring pass.
+    ``lanes = 1``: one batch in flight, so that the launches are one for the grid and one per Brent round."""
 
     def __init__(self, clips, kw: dict):
         import torch
@@ -1107,22 +929,29 @@ class _HaasClipBank:
         self.n = len(clips)
         self.kw = kw
         self.offs_dev = torch.from_numpy(self.offs).to(self.device)
+        self.lanes = 1
         self.evaluations = 0
         self.launches = 0
 
-    def scores(self, clip_ids, delays) -> np.ndarray:
-        """float64 scores of the pairs (``clip_ids[p]``, ``delays[p]``), in pair order: ONE kernel launch."""
+    def grid_scores(self, delays) -> np.ndarray:
+        """float64 ``(n, len(delays))`` scores of every clip at every delay: ONE launch."""
+        return self.collect(self.submit(np.repeat(np.arange(self.n), len(delays)), np.tile(delays, self.n))).reshape(self.n, len(delays))
+
+    def submit(self, clip_ids, delays) -> np.ndarray:
+        """float64 scores of the pairs (``clip_ids[p]``, ``delays[p]``), in pair order: ONE kernel launch; the scores
+        are the handle."""
         import torch
 
         pc = np.ascontiguousarray(clip_ids, dtype=np.int32)
-        if pc.size == 0:
-            return np.zeros(0, dtype=np.float64)
         pairs = torch.from_numpy(np.stack((pc, np.ascontiguousarray(delays, dtype=np.int32)))).to(self.device)
         with torch.cuda.device(self.device):
             p = haas_objective_pair_partials(self.x, self.offs_dev, pairs[0], pairs[1])
         self.launches += 1
         self.evaluations += pc.size
         return haas_scores_from_partials(p.cpu().numpy(), **self.kw)
+
+    def collect(self, handle) -> np.ndarray:
+        return handle
 
 
 def optimize_haas_delay_batch(*, input_signals=None, sample_rate_hz: int, max_delay_seconds: float, grid_size: int = 400,
@@ -1146,72 +975,12 @@ def optimize_haas_delay_batch(*, input_signals=None, sample_rate_hz: int, max_de
     minimisers; the refined delays are all-gathered once.  Delays in frames are ``round(t * sample_rate_hz)``, as
     ``HaasEffect.delay_len_samples`` computes them.  ``details=True`` also returns the score matrix, the local-minima
     sets, the per-clip argmin, and this rank's evaluation, launch and Brent-round counts and clip range."""
-    from . import sharding as S
-
     kw = dict(angle_limit=angle_limit, lambda_mean=lambda_mean, lambda_skew=lambda_skew, lambda_correlation=lambda_correlation,
               lambda_penalty=lambda_penalty)
-    rank, world = S._world(group)
-    if local_signals is not None:
-        if total_clips is None:
-            raise ValueError("local_signals needs total_clips (the number of clips over all ranks)")
-        n_clips = int(total_clips)
-        lo, hi = S.block_range(n_clips, rank, world)
-        local = _haas_batch_clips(local_signals, lo)
-        if len(local) != hi - lo:
-            raise ValueError(f"rank {rank} of {world} owns clips [{lo}, {hi}) but local_signals holds {len(local)}")
-    else:
-        if input_signals is None:
-            raise ValueError("pass input_signals (all clips) or local_signals (this rank's block)")
-        every = _haas_batch_clips(input_signals)  # every rank checks every clip, so that all ranks raise alike
-        n_clips = len(every)
-        lo, hi = S.block_range(n_clips, rank, world)
-        local = every[lo:hi]
 
-    taus = np.linspace(0.0, max_delay_seconds, grid_size)
-    grid_delays = np.array([round(t * sample_rate_hz) for t in taus.tolist()], dtype=np.int64)  # HaasEffect.delay_len_samples
-    n_local = hi - lo
-    if n_local > 0:
-        bank = (_bank_factory or _HaasClipBank)(local, kw)
-        print("Starting Grid Scan")
-        local_scores = bank.scores(np.repeat(np.arange(n_local), grid_size), np.tile(grid_delays, n_local)).reshape(n_local, grid_size)
-    else:
-        bank = None
-        local_scores = np.zeros((0, grid_size), dtype=np.float64)
+    def delays(ts):  # HaasEffect.delay_len_samples
+        return np.array([round(t * sample_rate_hz) for t in ts.tolist()], dtype=np.int64)
 
-    counts = [S.block_range(n_clips, r, world)[1] - S.block_range(n_clips, r, world)[0] for r in range(world)]
-    device = bank.device if (bank is not None and getattr(bank, "device", None) is not None) else S.collective_device(group)
-    scores = S.all_gather_rows(np.ascontiguousarray(local_scores, dtype=np.float64), counts, device=device, group=group)
-
-    minima = [get_local_minima(row, grid_size) for row in scores]
-    best = np.zeros(n_local, dtype=np.float64)
-    rounds = 0
-    if n_local > 0:
-        print("Starting Local Minima optimization")
-        lows, highs, owner = [], [], []
-        for ci in range(lo, hi):
-            for i in minima[ci]:
-                lows.append(taus[max(0, i - 1)])
-                highs.append(taus[min(grid_size - 1, i + 1)])
-                owner.append(ci - lo)
-        owner = np.asarray(owner, dtype=np.int64)
-        eng = _BrentBatch(lows, highs, 1e-4)
-        while True:  # one launch per round over every live minimiser of every clip (idx ascends: pairs stay clip-major)
-            idx, xs = eng.pending()
-            if len(idx) == 0:
-                break
-            delays = np.array([round(t * sample_rate_hz) for t in xs.tolist()], dtype=np.int64)
-            eng.feed(idx, bank.scores(owner[idx], delays))
-            rounds += 1
-        xs, funs, _ = eng.results()
-        best_score = [np.inf] * n_local
-        for x, fun, c in zip(xs, funs, owner):  # first strictly best minimum of each clip (optimization.py:150-153)
-            if fun < best_score[c]:
-                best_score[c] = fun
-                best[c] = x
-    refined = S.all_gather_rows(best.reshape(-1, 1), counts, device=device, group=group).reshape(-1)
-    if details:
-        info = {"scores": scores, "local_minima": minima, "argmin": [int(np.argmin(r)) for r in scores],
-                "evaluations_local": bank.evaluations if bank is not None else 0, "launches_local": bank.launches if bank is not None else 0,
-                "rounds_local": rounds, "clips_local": (lo, hi)}
-        return refined, info
-    return refined
+    return _optimize_batch(input_signals=input_signals, local_signals=local_signals, total_clips=total_clips, group=group, details=details,
+                           split=_haas_batch_clips, make_bank=lambda clips: (_bank_factory or _HaasClipBank)(clips, kw),
+                           grid=np.linspace(0.0, max_delay_seconds, grid_size), convert=delays, dtype=np.float64)
