@@ -231,6 +231,35 @@ int vnd_haas_objective_batch_dev(const void* clips, int32_t clip_dtype, int64_t 
 int vnd_haas_objective_pairs_dev(const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets, int32_t n_clips,
                                  const int32_t* pair_clip, const int32_t* pair_delay, int32_t n_pairs, double* partials, void* stream);
 
+/* The velvet-noise objective above over a list of RUNS on ragged clips: one objective launch and one combine launch,
+ * whatever the number of clips, runs and their lengths.
+ *   x             : float32, the clips packed channel-planar: element (t, c) of clip i is
+ *                   x[c * chan_stride + frame_offsets[i] + t], c = 0, 1 (chan_stride >= rows);
+ *   frame_offsets : n_clips + 1 int64, starting at 0, non-decreasing, ending at rows;
+ *   cand          : SEGMENTED tap program (device words and offsets), one channel per candidate;
+ *   run r         : clip run_clip[r] scored on the run_count[r] >= 0 consecutive channels of `cand` that start at
+ *                   run_cand[r]; candidate j's 12 partials go to row run_out[r] + j of `partials` (n_partial_rows x 12
+ *                   float64 on the device, the slots of vnd_vn_objective_batch_dev).  Rows no run names are not written.
+ *                   The channels a run uses must be packed for its clip's length (taps at or beyond it removed).
+ * Unlike the other _dev calls, frame_offsets and the four run arrays (n_runs int32 each) are HOST arrays: the launch
+ * geometry depends on every clip's length and every run's size.  The call checks them (offsets as above, chan_stride
+ * >= rows, every run's clip in range and not empty - VND_EINVAL "objective of an empty signal" -, its channels inside
+ * the program and its rows inside n_partial_rows) before it touches the device, plans the launch, and writes the
+ * derived work-item table into the front of the workspace with one cudaMemcpyAsync on `stream` (the host table may be
+ * freed on return).  Workspace: vnd_vn_objective_runs_workspace bytes for the same offsets and runs, 256-byte aligned.
+ * A filter whose halo (clamped to the longest clip of the runs) does not fit in shared memory returns VND_EUNSUPPORTED
+ * before any launch.  n_runs == 0 launches nothing.
+ * Bit contract: the 12 partials of (run r, candidate j) equal, bit for bit, row j of what vnd_vn_objective_batch_dev
+ * returns for clip run_clip[r] alone (planar) with the one channel run_cand[r] + j as its program (shared-memory kernel,
+ * VND_OBJ_TMEM unset): tiles are counted from frame 0 of each clip, staging reads nothing past the clip's last frame,
+ * and the chunk partials are added in tile order. */
+int vnd_vn_objective_runs_workspace(const int64_t* frame_offsets, int32_t n_clips, const int32_t* run_clip, const int32_t* run_count,
+                                    int32_t n_runs, size_t* bytes);
+int vnd_vn_objective_runs_dev(const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets, int32_t n_clips,
+                              const vnd_tap_program* cand, const int32_t* run_clip, const int32_t* run_cand, const int32_t* run_count,
+                              const int32_t* run_out, int32_t n_runs, double* partials, int64_t n_partial_rows, void* workspace,
+                              size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------ host API */
 typedef struct vnd_ctx vnd_ctx;
 
@@ -280,6 +309,12 @@ int vnd_haas_objective_batch_host(vnd_ctx* ctx, const void* clips, int32_t clip_
  * an empty clip (an empty signal has no objective: optimization.py:41-43).  Then one upload, one launch, one download. */
 int vnd_haas_objective_pairs_host(vnd_ctx* ctx, const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets,
                                   int32_t n_clips, const int32_t* pair_clip, const int32_t* pair_delay, int32_t n_pairs, double* partials);
+
+/* vnd_vn_objective_runs_dev with host buffers (x, program, tables and partials): the same checks before any copy, then
+ * one upload, one launch of each kernel, one download.  Rows no run names come back as zeros. */
+int vnd_vn_objective_runs_host(vnd_ctx* ctx, const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets, int32_t n_clips,
+                               const vnd_tap_program* cand, const int32_t* run_clip, const int32_t* run_cand, const int32_t* run_count,
+                               const int32_t* run_out, int32_t n_runs, double* partials, int64_t n_partial_rows);
 
 /* The overlapped path of vnd_sparse_fir_host with an explicit stage size: x and y are HOST planar
  * (channels, frames) float32 slabs; channels are cut into groups of `channels_per_chunk`, and

@@ -38,6 +38,10 @@ int vn_objective_launch(const float* clips, long long frames, int n_clips, long 
                         const vnd_tap_program* cand, double* partials, void* workspace, size_t workspace_bytes, cudaStream_t st);
 int haas_objective_launch(const void* clips, int clip_dtype, long long frames, int n_clips, long long clip_stride, long long chan_stride,
                           const int* delays, int n_cand, double* partials, cudaStream_t st);
+int objective_runs_workspace_bytes(const long long* offs, const int* run_clip, const int* run_count, int n_runs, size_t* bytes);
+int vn_objective_runs_launch(const float* x, long long chan_stride, const long long* offs, const int* run_clip, const int* run_cand,
+                             const int* run_count, const int* run_out, int n_runs, const vnd_tap_program* cand, double* partials,
+                             void* workspace, size_t workspace_bytes, cudaStream_t st);
 int haas_objective_pairs_launch(const float* x, long long chan_stride, const long long* offs, const int* pair_clip, const int* pair_delay,
                                 int n_pairs, double* partials, cudaStream_t st);
 size_t dsp_workspace_bytes(long long elems);
@@ -355,6 +359,82 @@ extern "C" int vnd_haas_objective_pairs_dev(const float* x, int64_t rows, int64_
   if ((rc = check_haas_pairs(x, rows, chan_stride, frame_offsets, n_clips, pair_clip, pair_delay, n_pairs, partials))) return rc;
   return haas_objective_pairs_launch(x, chan_stride, reinterpret_cast<const long long*>(frame_offsets), pair_clip, pair_delay, n_pairs, partials,
                                      (cudaStream_t)stream);
+}
+
+// Host tables of the run-list objective: offsets (n_clips + 1, from 0, non-decreasing, ending at rows) and every run's
+// clip.  Runs of at least one candidate need a clip with frames.
+static int check_run_clips(int64_t rows, const int64_t* offs, int32_t n_clips, const int32_t* run_clip, const int32_t* run_count, int32_t n_runs) {
+  VND_REQUIRE(rows >= 0 && n_clips >= 0 && n_runs >= 0, VND_EINVAL, "negative extent (rows %lld, n_clips %d, n_runs %d)", (long long)rows,
+              n_clips, n_runs);
+  VND_REQUIRE(offs != nullptr, VND_EINVAL, "frame_offsets is null");
+  VND_REQUIRE(offs[0] == 0, VND_EINVAL, "frame_offsets[0] is %lld, not 0", (long long)offs[0]);
+  for (int i = 0; i < n_clips; ++i)
+    VND_REQUIRE(offs[i + 1] >= offs[i], VND_EINVAL, "frame_offsets decrease at clip %d (%lld -> %lld)", i, (long long)offs[i],
+                (long long)offs[i + 1]);
+  VND_REQUIRE(offs[n_clips] == rows, VND_EINVAL, "frame_offsets end at %lld, not at rows = %lld", (long long)offs[n_clips], (long long)rows);
+  if (n_runs == 0) return VND_OK;
+  VND_REQUIRE(run_clip != nullptr && run_count != nullptr, VND_EINVAL, "run_clip or run_count is null");
+  for (int r = 0; r < n_runs; ++r) {
+    const int c = run_clip[r];
+    VND_REQUIRE(c >= 0 && c < n_clips, VND_EINVAL, "run_clip[%d] = %d is outside [0, %d)", r, c, n_clips);
+    VND_REQUIRE(run_count[r] >= 0, VND_EINVAL, "run_count[%d] = %d is negative", r, run_count[r]);
+    // the reference takes max(|theta|) of the frames: an empty signal is a ValueError there (optimization.py:41-43)
+    VND_REQUIRE(run_count[r] == 0 || offs[c + 1] > offs[c], VND_EINVAL,
+                "run %d: objective of an empty signal (clip %d has no frames: zero-size array to reduction operation maximum which has no identity)",
+                r, c);
+  }
+  return VND_OK;
+}
+
+// Everything vnd_vn_objective_runs_dev can check on the host before it touches the device.
+static int check_runs(const float* x, int64_t rows, int64_t chan_stride, const int64_t* offs, int32_t n_clips, const vnd_tap_program* cand,
+                      const int32_t* run_clip, const int32_t* run_cand, const int32_t* run_count, const int32_t* run_out, int32_t n_runs,
+                      const double* partials, int64_t n_partial_rows) {
+  int rc;
+  if ((rc = check_taps(cand))) return rc;
+  VND_REQUIRE(cand->order == VND_ORDER_SEGMENTED, VND_EINVAL, "objective candidates need SEGMENTED tap programs");
+  VND_REQUIRE(chan_stride >= rows, VND_EINVAL, "chan_stride %lld is shorter than rows = %lld: the two channels overlap", (long long)chan_stride,
+              (long long)rows);
+  VND_REQUIRE(n_partial_rows >= 0, VND_EINVAL, "negative n_partial_rows %lld", (long long)n_partial_rows);
+  if ((rc = check_run_clips(rows, offs, n_clips, run_clip, run_count, n_runs))) return rc;
+  if (n_runs == 0) return VND_OK;
+  VND_REQUIRE(run_cand != nullptr && run_out != nullptr, VND_EINVAL, "run_cand or run_out is null");
+  for (int r = 0; r < n_runs; ++r) {
+    VND_REQUIRE(run_cand[r] >= 0 && (long long)run_cand[r] + run_count[r] <= cand->channels, VND_EINVAL,
+                "run %d: channels [%d, %lld) are outside the program's %d", r, run_cand[r], (long long)run_cand[r] + run_count[r], cand->channels);
+    VND_REQUIRE(run_out[r] >= 0 && (long long)run_out[r] + run_count[r] <= n_partial_rows, VND_EINVAL,
+                "run %d: output rows [%d, %lld) are outside the %lld partial rows", r, run_out[r], (long long)run_out[r] + run_count[r],
+                (long long)n_partial_rows);
+  }
+  VND_REQUIRE(x != nullptr || rows == 0, VND_EINVAL, "x is null");
+  VND_REQUIRE(partials != nullptr || n_partial_rows == 0, VND_EINVAL, "partials is null");
+  return VND_OK;
+}
+
+extern "C" int vnd_vn_objective_runs_workspace(const int64_t* frame_offsets, int32_t n_clips, const int32_t* run_clip, const int32_t* run_count,
+                                               int32_t n_runs, size_t* bytes) {
+  VND_REQUIRE(bytes != nullptr, VND_EINVAL, "bytes is null");
+  VND_REQUIRE(frame_offsets != nullptr && n_clips >= 0, VND_EINVAL, "frame_offsets is null or n_clips negative");
+  int rc;
+  if ((rc = check_run_clips(frame_offsets[n_clips], frame_offsets, n_clips, run_clip, run_count, n_runs))) return rc;
+  if (n_runs == 0) {
+    *bytes = 0;
+    return VND_OK;
+  }
+  return objective_runs_workspace_bytes(reinterpret_cast<const long long*>(frame_offsets), run_clip, run_count, n_runs, bytes);
+}
+
+extern "C" int vnd_vn_objective_runs_dev(const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets, int32_t n_clips,
+                                         const vnd_tap_program* cand, const int32_t* run_clip, const int32_t* run_cand, const int32_t* run_count,
+                                         const int32_t* run_out, int32_t n_runs, double* partials, int64_t n_partial_rows, void* workspace,
+                                         size_t workspace_bytes, void* stream) {
+  int rc;
+  if ((rc = check_runs(x, rows, chan_stride, frame_offsets, n_clips, cand, run_clip, run_cand, run_count, run_out, n_runs, partials,
+                       n_partial_rows)))
+    return rc;
+  if (n_runs == 0) return VND_OK;
+  return vn_objective_runs_launch(x, chan_stride, reinterpret_cast<const long long*>(frame_offsets), run_clip, run_cand, run_count, run_out, n_runs,
+                                  cand, partials, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 static int check_flat(const vnd_signal* s, int ndim, const char* name) {
@@ -1275,6 +1355,38 @@ extern "C" int vnd_haas_objective_pairs_host(vnd_ctx* ctx, const float* x, int64
   if ((rc = haas_objective_pairs_launch((const float*)din, chan_stride, reinterpret_cast<const long long*>(meta),
                                         reinterpret_cast<const int*>(meta + off_bytes), reinterpret_cast<const int*>(meta + off_bytes + idx_bytes),
                                         n_pairs, (double*)dout, st)))
+    return rc;
+  VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
+  VND_CUDA_OK(cudaStreamSynchronize(st));
+  return VND_OK;
+}
+
+extern "C" int vnd_vn_objective_runs_host(vnd_ctx* ctx, const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets,
+                                          int32_t n_clips, const vnd_tap_program* cand, const int32_t* run_clip, const int32_t* run_cand,
+                                          const int32_t* run_count, const int32_t* run_out, int32_t n_runs, double* partials,
+                                          int64_t n_partial_rows) {
+  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  int rc;
+  if ((rc = check_runs(x, rows, chan_stride, frame_offsets, n_clips, cand, run_clip, run_cand, run_count, run_out, n_runs, partials,
+                       n_partial_rows)))
+    return rc;
+  if (n_partial_rows == 0) return VND_OK;
+  VND_ENTER(ctx);
+  cudaStream_t st = ctx->streams[0];
+  size_t wbytes = 0;
+  if (n_runs > 0 &&
+      (rc = objective_runs_workspace_bytes(reinterpret_cast<const long long*>(frame_offsets), run_clip, run_count, n_runs, &wbytes)))
+    return rc;
+  const size_t in_bytes = rows > 0 ? ((size_t)chan_stride + rows) * 4 : 0;
+  const size_t out_bytes = (size_t)n_partial_rows * 12 * 8;
+  vnd_tap_program dprog;
+  void *din = nullptr, *dout = nullptr, *work = nullptr;
+  if ((rc = upload_program(ctx, cand, &dprog, st))) return rc;
+  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) || (rc = arena(ctx, S_WORK, wbytes, &work))) return rc;
+  if (in_bytes) VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
+  VND_CUDA_OK(cudaMemsetAsync(dout, 0, out_bytes, st));  // rows no run names come back as zeros
+  if (n_runs > 0 && (rc = vn_objective_runs_launch((const float*)din, chan_stride, reinterpret_cast<const long long*>(frame_offsets), run_clip,
+                                                   run_cand, run_count, run_out, n_runs, &dprog, (double*)dout, work, wbytes, st)))
     return rc;
   VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));

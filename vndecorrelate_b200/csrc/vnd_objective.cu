@@ -23,6 +23,9 @@
 // candidate loop), reduces with warp shuffles and accumulates float64 partials in shared memory.
 
 #include <stdlib.h>
+#include <string.h>
+
+#include <vector>
 
 #include "vnd_objective.cuh"
 
@@ -216,7 +219,43 @@ __device__ __forceinline__ void run_candidate_v4(const float* __restrict__ px, c
 #ifndef VND_OBJ_MINB
 #define VND_OBJ_MINB 1  // CTAs per SM the register and shared-memory budgets are planned for (measured: 16 frames per lane in one CTA beats 8 in two)
 #endif
-__global__ void __launch_bounds__(OBJ_NT, VND_OBJ_MINB) vn_objective_kernel(const ObjParams p, int max_prog_words) {
+// Work-item sources of vn_objective_kernel.  A CTA scores the tiles [tile_first, tile_first + n_tiles) of one clip (the
+// loop stops at the clip's end) on the candidates [cand0, cand0 + ncand) of the program, and writes ncand x OBJ_SLOTS
+// chunk partials to out.  Tiles are counted from frame 0 of the clip and staging reads nothing past the clip's last
+// frame, so a (clip, candidate) pair gives the same bits whichever source hands it out.  Each field is asked for
+// where the kernel needs it.
+//
+// grid (chunk, clip, group) over n_clips equal-length planar clips sharing one candidate list
+struct ObjGridSrc {
+  ObjParams p;
+  __device__ __forceinline__ int cand0() const { return blockIdx.z * p.cand_per_group; }
+  __device__ __forceinline__ int ncand(int cand0) const { return min(p.cand_per_group, p.n_cand - cand0); }
+  __device__ __forceinline__ const float* x0() const { return p.clips + (long long)blockIdx.y * p.clip_stride; }
+  __device__ __forceinline__ long long frames() const { return p.frames; }
+  __device__ __forceinline__ long long tile_first() const { return (long long)blockIdx.x * p.tiles_per_chunk; }
+  __device__ __forceinline__ int n_tiles() const { return p.tiles_per_chunk; }
+  __device__ __forceinline__ double* out(int cand0) const {
+    return p.chunk_partials + (((size_t)blockIdx.y * p.n_chunks + blockIdx.x) * p.n_cand + cand0) * OBJ_SLOTS;
+  }
+};
+
+// CTA blockIdx.x runs work item items[blockIdx.x] (built on the host by plan_runs) over ragged clips packed
+// channel-planar: element (t, c) of a clip is p.clips[c * chan_stride + base + t]
+struct ObjRunSrc {
+  ObjParams p;
+  const ObjRunItem* items;
+  __device__ __forceinline__ int cand0() const { return items[blockIdx.x].cand0; }
+  __device__ __forceinline__ int ncand(int) const { return items[blockIdx.x].ncand; }
+  __device__ __forceinline__ const float* x0() const { return p.clips + items[blockIdx.x].base; }
+  __device__ __forceinline__ long long frames() const { return items[blockIdx.x].frames; }
+  __device__ __forceinline__ long long tile_first() const { return items[blockIdx.x].tile_first; }
+  __device__ __forceinline__ int n_tiles() const { return items[blockIdx.x].n_tiles; }
+  __device__ __forceinline__ double* out(int) const { return p.chunk_partials + (size_t)items[blockIdx.x].part * OBJ_SLOTS; }
+};
+
+template <typename Src>
+__global__ void __launch_bounds__(OBJ_NT, VND_OBJ_MINB) vn_objective_kernel(const Src src, int max_prog_words) {
+  const ObjParams& p = src.p;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int span = OBJ_TILE + p.halo;
   const int span4 = (span + 7) & ~3;  // words per shifted copy (a multiple of 4, room for the shift)
@@ -227,10 +266,9 @@ __global__ void __launch_bounds__(OBJ_NT, VND_OBJ_MINB) vn_objective_kernel(cons
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   constexpr int kWarps = OBJ_NT / 32;
-  const int chunk = blockIdx.x, clip = blockIdx.y, group = blockIdx.z;
-  const int cand0 = group * p.cand_per_group;
-  const int ncand = min(p.cand_per_group, p.n_cand - cand0);
-  const float* __restrict__ x0 = p.clips + (long long)clip * p.clip_stride;
+  const int cand0 = src.cand0();
+  const int ncand = src.ncand(cand0);
+  const float* __restrict__ x0 = src.x0();
   const float* __restrict__ x1 = x0 + p.chan_stride;
   int* myprog = progs + warp * max_prog_words;
   int* mydec = progs + (kWarps + warp) * max_prog_words;
@@ -240,11 +278,11 @@ __global__ void __launch_bounds__(OBJ_NT, VND_OBJ_MINB) vn_objective_kernel(cons
     acc[i] = (slot == 7 || slot == 9) ? 1.0 : 0.0;  // ratio trackers start at 0 / 1
   }
 
-  const long long tile_first = (long long)chunk * p.tiles_per_chunk;
-  for (int ti = 0; ti < p.tiles_per_chunk; ++ti) {
+  const long long tile_first = src.tile_first();
+  for (int ti = 0; ti < src.n_tiles(); ++ti) {
     const long long t0 = (tile_first + ti) * OBJ_TILE;
-    if (t0 >= p.frames) break;
-    const long long remain = p.frames - t0;
+    if (t0 >= src.frames()) break;
+    const long long remain = src.frames() - t0;
     __syncthreads();  // previous tile fully consumed (also orders the acc init)
     for (int i = tid; i < span + 3; i += OBJ_NT) {  // copy c holds x0[t0 + c + j] at j
       const float v = i < remain ? x0[t0 + i] : 0.0f;
@@ -329,30 +367,49 @@ __global__ void __launch_bounds__(OBJ_NT, VND_OBJ_MINB) vn_objective_kernel(cons
     }
   }
   __syncthreads();
-  double* out = p.chunk_partials + (((size_t)clip * p.n_chunks + chunk) * p.n_cand + cand0) * OBJ_SLOTS;
+  double* out = src.out(cand0);
   for (int i = tid; i < ncand * OBJ_SLOTS; i += OBJ_NT) out[i] = acc[i];
 }
 
 // Fixed-order combine of the chunk partials: sums added chunk by chunk, ratio trackers by exact
-// cross multiplication (earlier chunk wins ties, like np.max keeps the value either way).
-__global__ void obj_combine_kernel(const double* __restrict__ chunk_partials, double* __restrict__ partials, int n_clips,
-                                   int n_chunks, int n_cand) {
-  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= (long long)n_clips * n_cand) return;
-  const int clip = (int)(idx / n_cand), cand = (int)(idx % n_cand);
+// cross multiplication (earlier chunk wins ties, like np.max keeps the value either way).  Chunk ch of the row is
+// q[ch * stride].
+__device__ __forceinline__ void obj_combine_row(const double* __restrict__ q, size_t stride, int n_chunks, double* __restrict__ o) {
   double r[OBJ_SLOTS];
   for (int k = 0; k < OBJ_SLOTS; ++k) r[k] = 0.0;
   r[7] = 1.0;
   r[9] = 1.0;
-  for (int ch = 0; ch < n_chunks; ++ch) {
-    const double* q = chunk_partials + (((size_t)clip * n_chunks + ch) * n_cand + cand) * OBJ_SLOTS;
+  for (int ch = 0; ch < n_chunks; ++ch, q += stride) {
     for (int k = 0; k < 6; ++k) r[k] += q[k];
     if (q[6] * r[7] > r[6] * q[7]) { r[6] = q[6]; r[7] = q[7]; }
     if (q[8] * r[9] > r[8] * q[9]) { r[8] = q[8]; r[9] = q[9]; }
     r[10] += q[10];
   }
-  double* o = partials + (size_t)idx * OBJ_SLOTS;
   for (int k = 0; k < OBJ_SLOTS; ++k) o[k] = r[k];
+}
+
+__global__ void obj_combine_kernel(const double* __restrict__ chunk_partials, double* __restrict__ partials, int n_clips,
+                                   int n_chunks, int n_cand) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (long long)n_clips * n_cand) return;
+  const int clip = (int)(idx / n_cand), cand = (int)(idx % n_cand);
+  obj_combine_row(chunk_partials + ((size_t)clip * n_chunks * n_cand + cand) * OBJ_SLOTS, (size_t)n_cand * OBJ_SLOTS, n_chunks,
+                  partials + (size_t)idx * OBJ_SLOTS);
+}
+
+// The combine of the run-list objective: CTA r combines run r's rows.  Its chunk partials are [chunk][candidate] from
+// row `part`, chunks in tile order.
+struct ObjRunCombine {
+  long long part, out;
+  int n_chunks, count;
+};
+
+__global__ void obj_combine_runs_kernel(const double* __restrict__ chunk_partials, double* __restrict__ partials,
+                                        const ObjRunCombine* __restrict__ runs) {
+  const ObjRunCombine r = runs[blockIdx.x];
+  for (int j = threadIdx.x; j < r.count; j += blockDim.x)
+    obj_combine_row(chunk_partials + (size_t)(r.part + j) * OBJ_SLOTS, (size_t)r.count * OBJ_SLOTS, r.n_chunks,
+                    partials + (size_t)(r.out + j) * OBJ_SLOTS);
 }
 
 int obj_combine_launch(const double* chunk_partials, double* partials, int n_clips, int n_chunks, int n_cand, cudaStream_t st) {
@@ -566,6 +623,8 @@ static bool obj_tmem_disabled() {
 }
 #define g_obj_disable_tmem obj_tmem_disabled()
 
+static size_t align_up_sz(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
 struct ObjPlan {
   int cand_per_group, n_groups, tiles_per_chunk, n_chunks;
   size_t smem;
@@ -578,10 +637,9 @@ static long long max_chunks(long long tiles, int n_clips, int sm_count) {
   return c < 1 ? 1 : c;
 }
 
-static int plan_objective(long long frames, int n_clips, int n_cand, int halo, int max_prog_words, ObjPlan* pl) {
-  DeviceInfo di;
-  int rc = device_info(&di);
-  if (rc) return rc;
+// Shared memory of vn_objective_kernel for a launch halo: the bytes that do not depend on the group size, and the most
+// candidates a group can hold.  VND_EUNSUPPORTED when not even 16 fit.
+static int obj_group_budget(int halo, int max_prog_words, size_t* fixed_out, int* cpg_out) {
   const size_t span4 = (size_t)((OBJ_TILE + halo + 7) & ~3);
   const size_t fixed = (4 * span4 + OBJ_TILE) * 4 + (size_t)(OBJ_NT / 32) * 2 * max_prog_words * 4 + 64;
   // VND_OBJ_MINB CTAs share the SM's 228 KB (1 KB of each is reserved by the system); a single CTA may take it all
@@ -589,7 +647,18 @@ static int plan_objective(long long frames, int n_clips, int n_cand, int halo, i
   if (budget > (size_t)kMaxDynSmem) budget = (size_t)kMaxDynSmem;
   if (fixed + OBJ_SLOTS * 8 * 16 > budget) budget = (size_t)kMaxDynSmem;  // long filters: one CTA per SM
   if (fixed + OBJ_SLOTS * 8 * 16 > budget) return VND_EUNSUPPORTED;
-  int cpg = (int)((budget - fixed) / (OBJ_SLOTS * 8));
+  *fixed_out = fixed;
+  *cpg_out = (int)((budget - fixed) / (OBJ_SLOTS * 8));
+  return VND_OK;
+}
+
+static int plan_objective(long long frames, int n_clips, int n_cand, int halo, int max_prog_words, ObjPlan* pl) {
+  DeviceInfo di;
+  int rc = device_info(&di);
+  if (rc) return rc;
+  size_t fixed;
+  int cpg;
+  if ((rc = obj_group_budget(halo, max_prog_words, &fixed, &cpg))) return rc;
   if (cpg > n_cand) cpg = n_cand;
   if (cpg > 1024) cpg = 1024;
   const long long tiles = ceil_div<long long>(frames, OBJ_TILE);
@@ -675,12 +744,185 @@ int vn_objective_launch(const float* clips, long long frames, int n_clips, long 
   p.tiles_per_chunk = pl.tiles_per_chunk;
   p.n_chunks = pl.n_chunks;
   p.chunk_partials = reinterpret_cast<double*>(workspace);
-  VND_CUDA_OK(cudaFuncSetAttribute(vn_objective_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+  VND_CUDA_OK(cudaFuncSetAttribute(vn_objective_kernel<ObjGridSrc>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
   dim3 grid((unsigned)pl.n_chunks, (unsigned)n_clips, (unsigned)pl.n_groups);
-  vn_objective_kernel<<<grid, OBJ_NT, pl.smem, st>>>(p, mpw);
+  vn_objective_kernel<ObjGridSrc><<<grid, OBJ_NT, pl.smem, st>>>(ObjGridSrc{p}, mpw);
   rc = after_launch("vn_objective_kernel");
   if (rc) return rc;
   return obj_combine_launch(p.chunk_partials, partials, n_clips, pl.n_chunks, cand->channels, st);
+}
+
+// ------------------------------------------------------------------------------------------------
+// run-list objective over ragged clips (vnd_vn_objective_runs_dev)
+// ------------------------------------------------------------------------------------------------
+static long long run_tiles(const long long* offs, int clip) { return ceil_div<long long>(offs[clip + 1] - offs[clip], OBJ_TILE); }
+
+// Chunk-partial rows (and so work items) the plan below can ask for at most: each run is cut into at most
+// max_chunks(longest clip, runs) chunks, and no more than its tiles.
+static long long runs_partial_rows_bound(const long long* offs, const int* run_clip, const int* run_count, int n_runs, int sm_count) {
+  long long tmax = 0, active = 0, rows = 0;
+  for (int r = 0; r < n_runs; ++r)
+    if (run_count[r] > 0) {
+      const long long t = run_tiles(offs, run_clip[r]);
+      tmax = t > tmax ? t : tmax;
+      ++active;
+    }
+  if (active == 0) return 0;
+  const long long cap = max_chunks(tmax, (int)(active < 0x7fffffff ? active : 0x7fffffff), sm_count);
+  for (int r = 0; r < n_runs; ++r)
+    if (run_count[r] > 0) {
+      const long long t = run_tiles(offs, run_clip[r]);
+      rows += (t < cap ? t : cap) * run_count[r];
+    }
+  return rows;
+}
+
+static size_t runs_table_bytes(long long items, long long runs) {
+  return align_up_sz((size_t)items * sizeof(ObjRunItem) + (size_t)runs * sizeof(ObjRunCombine), 256);
+}
+
+int objective_runs_workspace_bytes(const long long* offs, const int* run_clip, const int* run_count, int n_runs, size_t* bytes) {
+  DeviceInfo di;
+  int rc = device_info(&di);
+  if (rc) return rc;
+  const long long rows = runs_partial_rows_bound(offs, run_clip, run_count, n_runs, di.sm_count);
+  *bytes = runs_table_bytes(rows, n_runs) + (size_t)rows * OBJ_SLOTS * 8 + 256;
+  return VND_OK;
+}
+
+// plan_objective for a run list: the same group size and the same choice of chunks, with the tiles of each run's clip
+// in place of the common clip length.  Groups are as large as shared memory allows, halved while the launch would not
+// fill about four waves; then the tiles per chunk (one value for every run, chunks counted from frame 0 of each clip)
+// that minimise waves x tiles per chunk, ties to fewer chunks of the longest clip.  With equal clips and equal runs
+// this is plan_objective's choice and CTA order.
+struct ObjRunPlan {
+  int cand_per_group = 0;
+  size_t smem = 0;
+  std::vector<ObjRunItem> items;
+  std::vector<ObjRunCombine> comb;
+  long long partial_rows = 0;
+};
+
+static int plan_runs(const long long* offs, const int* run_clip, const int* run_cand, const int* run_count, const int* run_out, int n_runs,
+                     int halo, int max_prog_words, ObjRunPlan* pl) {
+  DeviceInfo di;
+  int rc = device_info(&di);
+  if (rc) return rc;
+  size_t fixed;
+  int cpg;
+  if ((rc = obj_group_budget(halo, max_prog_words, &fixed, &cpg))) return rc;
+  int max_count = 0, active = 0;
+  long long tmax = 0;
+  for (int r = 0; r < n_runs; ++r)
+    if (run_count[r] > 0) {
+      max_count = run_count[r] > max_count ? run_count[r] : max_count;
+      const long long t = run_tiles(offs, run_clip[r]);
+      tmax = t > tmax ? t : tmax;
+      ++active;
+    }
+  if (active == 0) return VND_OK;
+  if (cpg > max_count) cpg = max_count;
+  if (cpg > 1024) cpg = 1024;
+  const long long want = (long long)di.sm_count * 4;
+  auto tile_groups = [&](int g) {
+    long long w = 0;
+    for (int r = 0; r < n_runs; ++r)
+      if (run_count[r] > 0) w += run_tiles(offs, run_clip[r]) * ceil_div(run_count[r], g);
+    return w;
+  };
+  while (tile_groups(cpg) < want && cpg > 16) cpg = (cpg + 1) / 2;
+  const long long cap = max_chunks(tmax, active, di.sm_count);
+  long long n_chunks = 1, best = -1;
+  for (long long c = 1; c <= cap; ++c) {
+    const long long tpc_c = ceil_div<long long>(tmax, c);
+    long long ctas = 0;
+    for (int r = 0; r < n_runs; ++r)
+      if (run_count[r] > 0) ctas += ceil_div<long long>(run_tiles(offs, run_clip[r]), tpc_c) * ceil_div(run_count[r], cpg);
+    const long long real_c = ceil_div<long long>(tmax, tpc_c);
+    const long long cost = ceil_div<long long>(ctas, di.sm_count) * tpc_c * 4096 + real_c;
+    if (best < 0 || cost < best) {
+      best = cost;
+      n_chunks = real_c;
+    }
+  }
+  const long long tpc = ceil_div<long long>(tmax, n_chunks);
+  // partial rows: run r owns [chunk][candidate] from part_r; CTAs ordered (group, run, chunk) like plan_objective's grid
+  std::vector<long long> part(n_runs, 0);
+  int max_groups = 0;
+  long long rows = 0;
+  for (int r = 0; r < n_runs; ++r) {
+    if (run_count[r] <= 0) continue;
+    const long long chunks = ceil_div<long long>(run_tiles(offs, run_clip[r]), tpc);
+    part[r] = rows;
+    rows += chunks * run_count[r];
+    pl->comb.push_back({part[r], run_out[r], (int)chunks, run_count[r]});
+    const int g = ceil_div(run_count[r], cpg);
+    max_groups = g > max_groups ? g : max_groups;
+  }
+  for (int g = 0; g < max_groups; ++g)
+    for (int r = 0; r < n_runs; ++r) {
+      if (run_count[r] <= 0 || g * cpg >= run_count[r]) continue;
+      const int clip = run_clip[r];
+      const long long tiles = run_tiles(offs, clip);
+      const int ncand = run_count[r] - g * cpg < cpg ? run_count[r] - g * cpg : cpg;
+      for (long long k = 0; k * tpc < tiles; ++k) {
+        const long long nt = tiles - k * tpc < tpc ? tiles - k * tpc : tpc;
+        pl->items.push_back({offs[clip], offs[clip + 1] - offs[clip], part[r] + k * run_count[r] + (long long)g * cpg, (int)(k * tpc), (int)nt,
+                             run_cand[r] + g * cpg, ncand});
+      }
+    }
+  pl->cand_per_group = cpg;
+  pl->smem = fixed + (size_t)cpg * OBJ_SLOTS * 8;
+  pl->partial_rows = rows;
+  return VND_OK;
+}
+
+int vn_objective_runs_launch(const float* x, long long chan_stride, const long long* offs, const int* run_clip, const int* run_cand,
+                             const int* run_count, const int* run_out, int n_runs, const vnd_tap_program* cand, double* partials,
+                             void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  long long max_frames = 0;
+  for (int r = 0; r < n_runs; ++r)
+    if (run_count[r] > 0) {
+      const long long f = offs[run_clip[r] + 1] - offs[run_clip[r]];
+      max_frames = f > max_frames ? f : max_frames;
+    }
+  if (max_frames == 0) return VND_OK;
+  int halo = cand->halo > 0 ? cand->halo : 0;  // the program's halo, clamped to the longest clip as for one clip
+  if (halo > max_frames) halo = (int)max_frames;
+  halo = (halo + 3) & ~3;
+  const int mpw = cand->max_channel_words > 0 ? cand->max_channel_words : 1;
+  ObjRunPlan pl;
+  int rc = plan_runs(offs, run_clip, run_cand, run_count, run_out, n_runs, halo, mpw, &pl);
+  if (rc == VND_EUNSUPPORTED) set_error("objective kernel: filter halo %d does not fit in shared memory", halo);
+  if (rc) return rc;
+  VND_REQUIRE(pl.items.size() <= 0x7fffffffu, VND_EUNSUPPORTED, "too many work items for one launch");
+  const size_t table = runs_table_bytes((long long)pl.items.size(), (long long)pl.comb.size());
+  const size_t need = table + (size_t)pl.partial_rows * OBJ_SLOTS * 8;
+  VND_REQUIRE(workspace && workspace_bytes >= need, VND_ENOMEM, "objective workspace too small: need %zu bytes, have %zu", need, workspace_bytes);
+  // the tables, one copy: work items, then the combine table
+  std::vector<unsigned char> host(table);
+  const size_t item_bytes = pl.items.size() * sizeof(ObjRunItem);
+  memcpy(host.data(), pl.items.data(), item_bytes);
+  memcpy(host.data() + item_bytes, pl.comb.data(), pl.comb.size() * sizeof(ObjRunCombine));
+  unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
+  VND_CUDA_OK(cudaMemcpyAsync(ws, host.data(), item_bytes + pl.comb.size() * sizeof(ObjRunCombine), cudaMemcpyHostToDevice, st));
+  ObjRunSrc src{};
+  src.p.clips = x;
+  src.p.chan_stride = chan_stride;
+  src.p.words = cand->words;
+  src.p.offsets = cand->offsets;
+  src.p.n_cand = cand->channels;
+  src.p.apply_gain = cand->apply_gain;
+  src.p.halo = halo;
+  src.p.cand_per_group = pl.cand_per_group;
+  src.p.chunk_partials = reinterpret_cast<double*>(ws + table);
+  src.items = reinterpret_cast<const ObjRunItem*>(ws);
+  VND_CUDA_OK(cudaFuncSetAttribute(vn_objective_kernel<ObjRunSrc>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+  vn_objective_kernel<ObjRunSrc><<<(unsigned)pl.items.size(), OBJ_NT, pl.smem, st>>>(src, mpw);
+  if ((rc = after_launch("vn_objective_kernel"))) return rc;
+  obj_combine_runs_kernel<<<(unsigned)pl.comb.size(), 128, 0, st>>>(src.p.chunk_partials, partials,
+                                                                    reinterpret_cast<const ObjRunCombine*>(ws + item_bytes));
+  return after_launch("obj_combine_runs_kernel");
 }
 
 int haas_objective_launch(const void* clips, int clip_dtype, long long frames, int n_clips, long long clip_stride, long long chan_stride,

@@ -33,6 +33,15 @@ struct ObjParams {
   double* chunk_partials;  // [clip][chunk][cand][OBJ_SLOTS]
 };
 
+// One CTA of the run-list objective (vnd_vn_objective_runs_dev): a chunk of one clip's tiles on one group of one run's
+// candidates.  Built on the host, read by the CTA from the front of the workspace.
+struct ObjRunItem {
+  long long base;    // packed column of the clip's frame 0
+  long long frames;  // the clip's length
+  long long part;    // first chunk-partial row (OBJ_SLOTS doubles) of the item
+  int tile_first, n_tiles, cand0, ncand;
+};
+
 // atan(t) for t in [0, 1]: t * P(t^2), |error| <= 1e-7 (degree-8 minimax fit, float32 Horner).
 __device__ __forceinline__ float atan01(float t) {
   const float z = t * t;

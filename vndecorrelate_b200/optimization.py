@@ -14,9 +14,10 @@ Refinement is the bounded Brent minimiser scipy runs for the reference (``minimi
 restated in array form (``_BrentBatch``) so that every local minimum - of every clip - advances in lock-step
 (``_refine_minima``): one kernel launch per Brent iteration over all live minimisers instead of one per evaluation.
 
-``optimize_velvet_noise_batch`` runs the whole optimisation for MANY clips (BASELINE config 5): clips are
-partitioned over the ranks of ``torch.distributed`` (one process per GPU), the grid scores are all-gathered as one
-float32 matrix (the only collective on the data path), and each rank refines the local minima of its own clips.
+``optimize_velvet_noise_batch`` runs the whole optimisation for MANY clips of any lengths (BASELINE config 5): clips
+are partitioned over the ranks of ``torch.distributed`` (one process per GPU), the grid scores are all-gathered as one
+float32 matrix (the only collective on the data path), and each rank refines the local minima of its own clips, with
+one call of the run-list objective (``vn_objective_run_partials``) for the grid and one per batch of Brent steps.
 ``optimize_haas_delay_batch`` does the same for ``optimize_haas_delay`` on clips of any lengths: one launch of the Haas
 objective over a flat (clip, delay) list for the whole grid, and one per Brent round over every live minimiser of every
 clip of the rank.  Both run the same driver (``_optimize_batch``) over a clip bank of their objective.
@@ -38,7 +39,7 @@ from .utils.dsp import EPSILON, LayoutMode
 __all__ = [
     "symmetry_aware_objective", "grid_scan", "get_local_minima", "optimize_local_minima", "optimize_haas_delay",
     "optimize_velvet_noise", "optimize_velvet_noise_batch", "optimize_haas_delay_batch", "vn_objective_partials", "haas_objective_partials",
-    "haas_objective_pair_partials", "vn_scores_from_partials", "haas_scores_from_partials",
+    "haas_objective_pair_partials", "vn_objective_run_partials", "vn_scores_from_partials", "haas_scores_from_partials",
 ]
 
 _F32_HALF_PI = np.float32(np.pi / 2)
@@ -172,6 +173,59 @@ def haas_objective_pair_partials(x, frame_offsets, pair_clip, pair_delay):
     out = np.empty((pc.size, N.HAAS_SLOTS), dtype=np.float64)
     N.check(lib.vnd_haas_objective_pairs_host(R.HostContext.get().handle, x.ctypes.data, int(offs[-1]), x.shape[1], offs.ctypes.data, offs.size - 1,
                                               pc.ctypes.data, pd.ctypes.data, pc.size, out.ctypes.data), "vnd_haas_objective_pairs_host")
+    return out
+
+
+def vn_objective_run_partials(x, frame_offsets, program: TapProgram, runs):
+    """Partial sums of the velvet-noise objective for a list of runs over ragged clips: one objective launch and one
+    combine launch.
+
+    ``x``: float32 ``(2, chan_stride)`` channel-planar clips (numpy array or CUDA tensor with contiguous rows); clip ``i``
+    is columns ``frame_offsets[i]:frame_offsets[i + 1]``.  ``runs``: a ``(4, n_runs)`` integer array (or four sequences)
+    of ``(clip, first channel, count, first output row)``: run ``r`` scores clip ``runs[0][r]`` on the ``runs[2][r]``
+    consecutive channels of ``program`` that start at ``runs[1][r]``, into rows ``runs[3][r]`` on.  The channels a run
+    uses must be packed for its clip's length.  Returns float64 ``(n_rows, 12)``, ``n_rows`` the end of the last output
+    row; rows no run names are zero.  Each row is bit-equal to ``vn_objective_partials`` on that clip alone with that
+    channel.  The offsets and runs are read on the host (they size the launch); with a CUDA tensor the result is a CUDA
+    tensor enqueued on torch's current stream, with numpy everything is uploaded and downloaded inside the call."""
+    lib = N.lib()
+    offs = np.ascontiguousarray(frame_offsets.cpu().numpy() if R.is_torch_tensor(frame_offsets) else frame_offsets, dtype=np.int64)
+    table = np.asarray(runs, dtype=np.int64)
+    if table.size == 0:
+        table = table.reshape(4, 0)
+    if table.ndim != 2 or table.shape[0] != 4 or offs.ndim != 1 or offs.size == 0:
+        raise ValueError("frame_offsets must be 1-D with n_clips + 1 entries and runs a (4, n_runs) integer array")
+    if table.size and (table.min() < -2**31 or table.max() >= 2**31):
+        raise ValueError("run entries must fit in int32")
+    run_clip, run_cand, run_count, run_out = (np.ascontiguousarray(r, dtype=np.int32) for r in table)
+    n_runs = table.shape[1]
+    n_rows = max(0, int((table[3] + table[2]).max())) if n_runs else 0
+    tables = (run_clip.ctypes.data, run_cand.ctypes.data, run_count.ctypes.data, run_out.ctypes.data, n_runs)
+    if R.is_torch_tensor(x):
+        import torch
+
+        if not x.is_cuda or x.dtype != torch.float32 or x.dim() != 2 or x.shape[0] != 2 or x.stride(1) != 1:
+            raise ValueError("x must be a CUDA float32 tensor of shape (2, chan_stride) with contiguous rows")
+        dev = x.device
+        out = torch.zeros((n_rows, N.OBJ_SLOTS), dtype=torch.float64, device=dev)
+        nbytes = C.c_size_t()
+        N.check(lib.vnd_vn_objective_runs_workspace(offs.ctypes.data, offs.size - 1, run_clip.ctypes.data, run_count.ctypes.data, n_runs,
+                                                    C.byref(nbytes)), "vnd_vn_objective_runs_workspace")
+        with torch.cuda.device(dev):
+            work = torch.empty(max(nbytes.value, 1), dtype=torch.uint8, device=dev)
+            ps = R.device_program(program, dev)
+            N.check(lib.vnd_vn_objective_runs_dev(x.data_ptr(), int(offs[-1]), x.stride(0), offs.ctypes.data, offs.size - 1, C.byref(ps), *tables,
+                                                  out.data_ptr(), n_rows, work.data_ptr(), nbytes.value, R.torch_stream_ptr(x)),
+                    "vnd_vn_objective_runs_dev")
+        return out
+    x = np.asarray(x)
+    if x.dtype != np.float32 or x.ndim != 2 or x.shape[0] != 2:
+        raise ValueError("x must be a float32 array of shape (2, chan_stride)")
+    x = np.ascontiguousarray(x)
+    out = np.zeros((n_rows, N.OBJ_SLOTS), dtype=np.float64)
+    ps = program.host_struct()
+    N.check(lib.vnd_vn_objective_runs_host(R.HostContext.get().handle, x.ctypes.data, int(offs[-1]), x.shape[1], offs.ctypes.data, offs.size - 1,
+                                           C.byref(ps), *tables, out.ctypes.data, n_rows), "vnd_vn_objective_runs_host")
     return out
 
 
@@ -702,69 +756,129 @@ def optimize_velvet_noise(*, input_signal, sample_rate_hz: int, duration_seconds
 # ------------------------------------------------------------------------------------------------
 
 
+_NO_FRAME_LIMIT = 2**31 - 1  # a clip length no tap reaches: family(kappas, _NO_FRAME_LIMIT) keeps every tap
+
+
+def _concat_programs(progs: Sequence[TapProgram]) -> TapProgram:
+    """The channels of several SEGMENTED programs of one envelope, in order, as one program."""
+    if len(progs) == 1:
+        return progs[0]
+    base = np.cumsum([0] + [p.words.size for p in progs])
+    offsets = np.concatenate([p.offsets[:-1].astype(np.int64) + b for p, b in zip(progs, base[:-1])] + [base[-1:]])
+    if offsets[-1] >= 2**31:
+        raise ValueError("tap program too large")
+    return TapProgram(np.ascontiguousarray(np.concatenate([p.words for p in progs]), dtype=np.int32), offsets.astype(np.int32),
+                      sum(p.channels for p in progs), N.ORDER_SEGMENTED, progs[0].apply_gain, max(p.halo for p in progs),
+                      max(p.max_channel_words for p in progs))
+
+
+def _run_program(family: Callable[[Sequence[float], int], TapProgram], lengths, groups, base: list) -> tuple[TapProgram, np.ndarray]:
+    """One tap program and the ``(4, n_runs)`` run table of ``vn_objective_run_partials`` for ``groups``: run ``r`` is
+    ``(clip, kappas, position of kappas[0] in base, first output row)``.
+
+    A program drops the taps at or beyond the clip's length, so a channel is valid for every clip longer than its
+    largest tap.  Channels ``[0, len(base))`` are ``family(base, ...)`` with every tap kept: the runs of clips longer
+    than the largest tap of ``base`` point into it.  Each shorter length is a class of its own, packed exactly as
+    ``family(kappas, frames)`` packs it for one clip of that length, and appended; runs of one class that share a kappa
+    list (the grid) share its channels."""
+    full = family(base, _NO_FRAME_LIMIT)
+    last_tap = full.halo - 1
+    classes: dict[int, tuple[list, dict]] = {}
+    where = []
+    for clip, ks, pos, _ in groups:
+        f = int(lengths[clip])
+        if f > last_tap:
+            where.append((None, pos))
+            continue
+        kappas, seen = classes.setdefault(f, ([], {}))
+        if id(ks) not in seen:
+            seen[id(ks)] = len(kappas)
+            kappas.extend(ks)
+        where.append((f, seen[id(ks)]))
+    progs, first = [full], {}
+    at = full.channels
+    for f, (kappas, _) in classes.items():
+        progs.append(family(kappas, f))
+        first[f] = at
+        at += progs[-1].channels
+    runs = np.array([[g[0] for g in groups], [pos if f is None else first[f] + pos for f, pos in where], [len(g[1]) for g in groups],
+                     [g[3] for g in groups]], dtype=np.int64).reshape(4, len(groups))
+    return _concat_programs(progs), runs
+
+
+def _pack_clips(clips):
+    """The clips as one channel-planar float32 ``(2, rows)`` tensor on their GPU (clip ``i`` is columns
+    ``offs[i]:offs[i + 1]``, cast and sliced as ``_as_stereo_f32`` does), the int64 offsets and the device.  ``clips``:
+    a list of numpy arrays or of CUDA tensors, or a planar ``(n, 2, frames)`` array or CUDA tensor (one copy)."""
+    import torch
+
+    planar = R.is_torch_tensor(clips) or isinstance(clips, np.ndarray)
+    lengths = [int(clips.shape[2])] * int(clips.shape[0]) if planar else [int(c.shape[0]) for c in clips]
+    offs = np.zeros(len(lengths) + 1, dtype=np.int64)
+    np.cumsum(lengths, out=offs[1:])
+    rows = int(offs[-1])
+    if planar:
+        if R.is_torch_tensor(clips):
+            return clips.to(torch.float32).permute(1, 0, 2).contiguous().reshape(2, rows), offs, clips.device  # one copy, whatever the strides
+        device = torch.device("cuda", R.default_device())
+        host = np.ascontiguousarray(np.asarray(clips).astype(np.float32, copy=False).transpose(1, 0, 2)).reshape(2, rows)
+        return torch.from_numpy(host).to(device), offs, device
+    if clips and R.is_torch_tensor(clips[0]):
+        device = clips[0].device
+        x = torch.empty((2, rows), dtype=torch.float32, device=device)
+        for c, a, b in zip(clips, offs[:-1], offs[1:]):
+            t = c.to(torch.float32)  # rounds like numpy's astype
+            x[:, a:b] = (t[:, None].expand(-1, 2) if t.dim() == 1 else t[:, :2]).T
+        return x, offs, device
+    device = torch.device("cuda", R.default_device())
+    host = np.empty((2, rows), dtype=np.float32)
+    for c, a, b in zip(clips, offs[:-1], offs[1:]):
+        host[:, a:b] = _as_stereo_f32(c).T
+    return torch.from_numpy(host).to(device), offs, device
+
+
 class _ClipBank:
-    """The rank's clips resident on its GPU as one planar ``(n, 2, frames)`` float32 tensor, and the velvet-noise
-    objective on them: the grid as one launch over clips x candidates, and flat (clip, strength) lists as ONE tap
-    program for all strengths, uploaded once, one launch per clip on a sub-range of its candidates, one asynchronous
-    download of all partial sums, one vectorised scoring pass.  ``lanes = 2`` from two clips on: the refinement keeps two
-    half-batches of clips in flight, so that scoring and the Brent step of one run under the kernels of the other."""
+    """The rank's clips resident on its GPU, packed once into one channel-planar float32 ``(2, rows)`` tensor
+    (``_pack_clips``), and the velvet-noise objective on them: the grid and every flat (clip, strength) list are ONE
+    ``vn_objective_run_partials`` call each (one run per clip, one tap program per call with a class of channels per
+    clip length that drops taps, ``_run_program``), then one asynchronous download of the partial sums and one
+    vectorised scoring pass.  ``lanes = 2`` from two clips on: the refinement keeps two half-batches of clips in flight,
+    so that scoring and the Brent step of one run under the kernels of the other."""
 
     def __init__(self, clips, family: Callable[[Sequence[float], int], TapProgram], kw: dict):
-        import torch
-
-        if R.is_torch_tensor(clips):
-            if not clips.is_cuda or clips.dtype != torch.float32 or clips.dim() != 3 or clips.shape[1] != 2:
-                raise ValueError("clips must be a CUDA float32 tensor of shape (n_clips, 2, frames)")
-            self.clips = clips.contiguous()
-        else:
-            host = _planar_clips(clips)
-            self.clips = torch.from_numpy(host).to(f"cuda:{R.default_device()}")
-        self.n, _, self.frames = self.clips.shape
-        self.device = self.clips.device
+        self.x, self.offs, self.device = _pack_clips(clips)
+        self.lengths = np.diff(self.offs)
+        self.n = len(self.lengths)
         self.lanes = 2 if self.n >= 2 else 1
         self.family = family
         self.kw = kw
         self.evaluations = 0
         self.launches = 0
-        self._work = None
 
-    def _workspace(self, n_cand: int):
+    def _partials(self, groups, base):
+        prog, runs = _run_program(self.family, self.lengths, groups, base)
         import torch
 
-        nbytes = C.c_size_t()
-        N.check(N.lib().vnd_objective_workspace(self.frames, 1, n_cand, C.byref(nbytes)), "vnd_objective_workspace")
-        if self._work is None or self._work.numel() < nbytes.value:
-            self._work = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
-        return self._work, nbytes.value
+        with torch.cuda.device(self.device):
+            out = vn_objective_run_partials(self.x, self.offs, prog, runs)
+        self.launches += 1
+        return out
 
     def grid_scores(self, kappas: Sequence[float]) -> np.ndarray:
-        """float32 ``(n, len(kappas))`` scores of every clip at every strength: ONE launch."""
-        partials = vn_objective_partials(self.clips, self.family(kappas, self.frames))
-        self.launches += 1
-        self.evaluations += self.n * len(kappas)
-        return vn_scores_from_partials(partials, **self.kw)
+        """float32 ``(n, len(kappas))`` scores of every clip at every strength: ONE call."""
+        k = len(kappas)
+        partials = self._partials([(i, kappas, 0, i * k) for i in range(self.n)], kappas)
+        self.evaluations += self.n * k
+        return vn_scores_from_partials(partials.cpu().numpy().reshape(self.n, k, N.OBJ_SLOTS), **self.kw)
 
     def submit(self, clip_ids: np.ndarray, kappas: Sequence[float]):
-        """Enqueue the evaluation of the clip-major pairs (``clip_ids[p]``, ``kappas[p]``) and the download of their
-        partial sums into page-locked memory; returns a handle for ``collect``.  Nothing here waits for the device."""
+        """Enqueue the evaluation of the clip-major pairs (``clip_ids[p]``, ``kappas[p]``) - ONE call, one run per
+        clip - and the download of their partial sums into page-locked memory; returns a handle for ``collect``."""
         import torch
 
         starts = np.flatnonzero(np.r_[True, clip_ids[1:] != clip_ids[:-1]])  # one run of pairs per clip
         ends = np.r_[starts[1:], len(clip_ids)]
-        prog = self.family(kappas, self.frames)
-        out = torch.empty((len(kappas), N.OBJ_SLOTS), dtype=torch.float64, device=self.device)
-        lib = N.lib()
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-            ps = R.device_program(prog, self.device)
-            work, wbytes = self._workspace(int(np.max(ends - starts)))
-            for a, b in zip(starts.tolist(), ends.tolist()):
-                i = int(clip_ids[a])
-                sub = N.TapProgramStruct(ps.words, ps.offsets + 4 * a, ps.n_words, b - a, ps.order, ps.apply_gain, ps.halo, ps.max_channel_words)
-                N.check(lib.vnd_vn_objective_batch_dev(self.clips.data_ptr() + 4 * i * 2 * self.frames, self.frames, 1, 2 * self.frames, self.frames,
-                                                       C.byref(sub), out.data_ptr() + 8 * N.OBJ_SLOTS * a, work.data_ptr(), wbytes, stream),
-                        "vnd_vn_objective_batch_dev")
-                self.launches += 1
+        out = self._partials([(int(clip_ids[a]), kappas[a:b], a, a) for a, b in zip(starts.tolist(), ends.tolist())], kappas)
         self.evaluations += len(kappas)
         host = torch.empty(out.shape, dtype=out.dtype, pin_memory=True)
         host.copy_(out, non_blocking=True)
@@ -832,25 +946,9 @@ def _optimize_batch(*, input_signals, local_signals, total_clips, group, details
     return refined
 
 
-def optimize_velvet_noise_batch(*, input_signals=None, sample_rate_hz: int, duration_seconds: float, num_impulses: int, seed: int = 1,
-                                grid_size: int = 400, angle_limit: float = np.pi / 4, lambda_mean: float = 5.0, lambda_skew: float = 2.0,
-                                lambda_correlation: float = 15.0, lambda_penalty: float = 1e3, group=None, details: bool = False,
-                                local_signals=None, total_clips: int | None = None, _bank_factory=None):
-    """``optimize_velvet_noise`` (optimization.py:230-310) for MANY clips of equal length: returns the float64 array of
-    optimised ``log_distribution_strength`` values, element ``i`` equal to what ``optimize_velvet_noise(input_signal=
-    input_signals[i], ...)`` returns.
-
-    ``input_signals``: a sequence of ``(frames, 2)`` arrays, a planar ``(n_clips, 2, frames)`` float32 array, or a CUDA
-    tensor of that shape.  With ``torch.distributed`` initialised (one process per GPU) the clips are partitioned in
-    contiguous blocks over the ranks of ``group`` (``sharding.block_range``); every rank passes the SAME
-    ``input_signals`` (only its block is read and uploaded) - or, when the clips already live on the ranks, its own
-    block as ``local_signals`` (e.g. a resident CUDA tensor) together with ``total_clips``.  Data path per rank: grid scores of its clips (one launch over clips x grid) -> ONE all-gather of the
-    float32 score matrix so that every rank holds all rows (``get_local_minima`` needs both neighbours of every grid
-    point, optimization.py:120-128) -> lock-step Brent refinement of the local minima of its own clips -> one
-    all-gather of the refined strengths.  ``details=True`` also returns the score matrix, the local-minima sets, the
-    per-clip argmin, and this rank's evaluation, launch and Brent-round counts and clip range."""
-    kw = dict(angle_limit=angle_limit, lambda_mean=lambda_mean, lambda_skew=lambda_skew, lambda_correlation=lambda_correlation,
-              lambda_penalty=lambda_penalty)
+def _vn_family(*, sample_rate_hz: int, duration_seconds: float, num_impulses: int, seed) -> Callable[[Sequence[float], int], TapProgram]:
+    """``family(kappas, frames)``: the tap program of the candidates ``optimize_velvet_noise`` scores for a clip of
+    ``frames`` samples, packed as it packs them (``kappa_family_program``, table by table when that does not apply)."""
 
     def candidate(kappa):
         return VelvetNoise(sample_rate_hz=sample_rate_hz, duration_seconds=duration_seconds, num_impulses=num_impulses,
@@ -863,8 +961,40 @@ def optimize_velvet_noise_batch(*, input_signals=None, sample_rate_hz: int, dura
                                     envelope=envelope, seed=seed, frames=frames) if seed is not None else None
         return prog if prog is not None else _vn_family_program([candidate(k) for k in ks], frames)
 
+    return family
+
+
+def optimize_velvet_noise_batch(*, input_signals=None, sample_rate_hz: int, duration_seconds: float, num_impulses: int, seed: int = 1,
+                                grid_size: int = 400, angle_limit: float = np.pi / 4, lambda_mean: float = 5.0, lambda_skew: float = 2.0,
+                                lambda_correlation: float = 15.0, lambda_penalty: float = 1e3, group=None, details: bool = False,
+                                local_signals=None, total_clips: int | None = None, _bank_factory=None):
+    """``optimize_velvet_noise`` (optimization.py:230-310) for MANY clips of any lengths: returns the float64 array of
+    optimised ``log_distribution_strength`` values, element ``i`` equal to what ``optimize_velvet_noise(input_signal=
+    input_signals[i], ...)`` returns (for a CUDA tensor clip: on ``clip.cpu().numpy()``).  All clips share the
+    optimiser's settings.
+
+    ``input_signals``: a list of clips - numpy arrays or CUDA tensors (not a mix, one device), mono ``(frames,)``,
+    stereo ``(frames, 2)`` or wider ``(frames, k)`` (the first two channels are used), any dtype, cast to float32 as the
+    single-clip call does - or one PLANAR ``(n_clips, 2, frames)`` array or CUDA tensor (unlike
+    ``optimize_haas_delay_batch``, whose batch array is ``(n_clips, frames, 2)``).  An empty clip raises ``ValueError``
+    naming its index before any device work, and so do bad shapes and mixed numpy and CUDA clips.  With
+    ``torch.distributed`` initialised (one process per GPU) the clips are partitioned in contiguous blocks over the ranks
+    of ``group`` (``sharding.block_range``); every rank passes the SAME ``input_signals`` (only its block is read and
+    uploaded) - or, when the clips already live on the ranks, its own block as ``local_signals`` (e.g. a resident CUDA
+    tensor) together with ``total_clips``.
+
+    Data path per rank: its clips are packed once into one resident channel-planar float32 tensor; the grid scores are
+    ONE run-list objective call over every clip (``vn_objective_run_partials``) -> ONE all-gather of the float32 score
+    matrix so that every rank holds all rows (``get_local_minima`` needs both neighbours of every grid point,
+    optimization.py:120-128) -> lock-step Brent refinement of the local minima of its own clips, ONE call per batch of
+    live minimisers -> one all-gather of the refined strengths.  ``details=True`` also returns the score matrix, the
+    local-minima sets, the per-clip argmin, and this rank's evaluation, launch (objective calls) and Brent-round counts
+    and clip range."""
+    kw = dict(angle_limit=angle_limit, lambda_mean=lambda_mean, lambda_skew=lambda_skew, lambda_correlation=lambda_correlation,
+              lambda_penalty=lambda_penalty)
+    family = _vn_family(sample_rate_hz=sample_rate_hz, duration_seconds=duration_seconds, num_impulses=num_impulses, seed=seed)
     return _optimize_batch(input_signals=input_signals, local_signals=local_signals, total_clips=total_clips, group=group, details=details,
-                           split=lambda signals, first: signals, make_bank=lambda clips: (_bank_factory or _ClipBank)(clips, family, kw),
+                           split=_vn_batch_clips, make_bank=lambda clips: (_bank_factory or _ClipBank)(clips, family, kw),
                            grid=np.linspace(0.0, 1.0, grid_size), convert=np.ndarray.tolist, dtype=np.float32)
 
 
@@ -873,16 +1003,11 @@ def optimize_velvet_noise_batch(*, input_signals=None, sample_rate_hz: int, dura
 # ------------------------------------------------------------------------------------------------
 
 
-def _haas_batch_clips(signals, first: int = 0) -> list:
-    """The clips of ``signals`` (a list of numpy arrays or CUDA tensors, or one ``(n_clips, frames, 2)`` array or
-    tensor) as a list, after the shape checks ``_as_stereo_f32`` makes, before any device work.  ``first`` is the
-    index of the first clip in the whole batch (for the messages)."""
-    if R.is_torch_tensor(signals) or isinstance(signals, np.ndarray):
-        if signals.ndim != 3 or signals.shape[2] != 2:
-            raise ValueError(f"a batch array must have shape (n_clips, frames, 2), got {tuple(signals.shape)}")
-        clips = [signals[i] for i in range(signals.shape[0])]
-    else:
-        clips = [c if R.is_torch_tensor(c) else np.asarray(c) for c in signals]
+def _check_clip_list(clips, first: int) -> list:
+    """The per-clip checks both multi-clip optimisers make before any device work: all numpy arrays or all CUDA tensors
+    on one device, each mono ``(frames,)`` or ``(frames, k >= 2)`` (the shapes ``_as_stereo_f32`` accepts) and not
+    empty.  ``first`` is the index of the first clip in the whole batch (for the messages)."""
+    clips = [c if R.is_torch_tensor(c) else np.asarray(c) for c in clips]
     kinds = {R.is_torch_tensor(c) for c in clips}
     if len(kinds) > 1:
         raise ValueError("clips must be all numpy arrays or all CUDA tensors, not a mix")
@@ -900,6 +1025,30 @@ def _haas_batch_clips(signals, first: int = 0) -> list:
     return clips
 
 
+def _haas_batch_clips(signals, first: int = 0) -> list:
+    """The clips of ``signals`` (a list of numpy arrays or CUDA tensors, or one ``(n_clips, frames, 2)`` array or
+    tensor) as a list, after ``_check_clip_list``."""
+    if R.is_torch_tensor(signals) or isinstance(signals, np.ndarray):
+        if signals.ndim != 3 or signals.shape[2] != 2:
+            raise ValueError(f"a batch array must have shape (n_clips, frames, 2), got {tuple(signals.shape)}")
+        return _check_clip_list([signals[i] for i in range(signals.shape[0])], first)
+    return _check_clip_list(signals, first)
+
+
+def _vn_batch_clips(signals, first: int = 0):
+    """The clips of ``signals`` for ``optimize_velvet_noise_batch``: a list after ``_check_clip_list``, or a planar
+    ``(n_clips, 2, frames)`` numpy array or CUDA tensor, kept whole (it packs with one copy)."""
+    if R.is_torch_tensor(signals) or isinstance(signals, np.ndarray):
+        if signals.ndim != 3 or signals.shape[1] != 2:
+            raise ValueError(f"a batch array must be planar with shape (n_clips, 2, frames), got {tuple(signals.shape)}")
+        if R.is_torch_tensor(signals) and not signals.is_cuda:
+            raise ValueError("torch clips must be CUDA tensors")
+        if signals.shape[0] and signals.shape[2] == 0:
+            raise ValueError(f"clip {first} is empty: zero-size array to reduction operation maximum which has no identity")
+        return signals
+    return _check_clip_list(signals, first)
+
+
 class _HaasClipBank:
     """The rank's clips resident on its GPU, packed once into one channel-planar float32 ``(2, rows)`` tensor (clip ``i``
     is columns ``offs[i]:offs[i + 1]``, cast and sliced as ``_as_stereo_f32`` does), and the evaluation of flat
@@ -909,23 +1058,7 @@ class _HaasClipBank:
     def __init__(self, clips, kw: dict):
         import torch
 
-        lengths = [int(c.shape[0]) for c in clips]
-        self.offs = np.zeros(len(clips) + 1, dtype=np.int64)
-        np.cumsum(lengths, out=self.offs[1:])
-        rows = int(self.offs[-1])
-        if clips and R.is_torch_tensor(clips[0]):
-            self.device = clips[0].device
-            x = torch.empty((2, rows), dtype=torch.float32, device=self.device)
-            for c, a, b in zip(clips, self.offs[:-1], self.offs[1:]):
-                t = c.to(torch.float32)  # rounds like numpy's astype
-                x[:, a:b] = (t[:, None].expand(-1, 2) if t.dim() == 1 else t[:, :2]).T
-        else:
-            self.device = torch.device("cuda", R.default_device())
-            host = np.empty((2, rows), dtype=np.float32)
-            for c, a, b in zip(clips, self.offs[:-1], self.offs[1:]):
-                host[:, a:b] = _as_stereo_f32(c).T
-            x = torch.from_numpy(host).to(self.device)
-        self.x = x
+        self.x, self.offs, self.device = _pack_clips(clips)
         self.n = len(clips)
         self.kw = kw
         self.offs_dev = torch.from_numpy(self.offs).to(self.device)
