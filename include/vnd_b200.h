@@ -163,6 +163,29 @@ int vnd_colsumsq_seq_f32_dev(const vnd_signal* a, float* sums, void* stream);
 int vnd_haas_dev(const vnd_signal* x, const vnd_signal* out, int32_t delay, int32_t delayed_channel,
                  int32_t mode_ms, int32_t mono, int32_t use_width, double width, void* stream);
 
+/* The Haas settings of one clip of vnd_haas_batch_dev: those of vnd_haas_dev.  32 bytes. */
+typedef struct vnd_haas_clip {
+  int32_t delay;           /* >= 0 frames                                                   */
+  int32_t delayed_channel; /* 0 or 1                                                        */
+  int32_t mode_ms, mono, use_width, reserved;
+  double width;
+} vnd_haas_clip;
+
+/* Batched HaasEffect.decorrelate: vnd_haas_dev on many clips of any lengths, each with its own settings, in ONE launch
+ * whatever the number of clips (none when out_rows == 0).
+ *   x             : packed float32 (rows, 2) C-order input, 8-byte aligned; clip i is rows [frame_offsets[i],
+ *                   frame_offsets[i + 1]) - a mono clip is packed with its samples in both columns and mono = 1;
+ *   frame_offsets : n_clips + 1 int64, starting at 0, non-decreasing, ending at rows;
+ *   clips         : n_clips settings records;
+ *   out_offsets   : n_clips int64, out_offsets[i] = frame_offsets[i] + sum_{j < i} clips[j].delay;
+ *   out           : float64 (out_rows, 2) C-order, 16-byte aligned, out_rows = rows + sum of the delays; clip i is rows
+ *                   [out_offsets[i], out_offsets[i] + frames_i + delay_i).
+ * Every clip's output is byte-identical to vnd_haas_dev on that clip with its settings.  The _dev call checks the
+ * pointers and sizes it sees; it cannot read the device-side offsets and settings, which must be valid (the _host call
+ * checks them). */
+int vnd_haas_batch_dev(const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_clips, const vnd_haas_clip* clips,
+                       const int64_t* out_offsets, int64_t out_rows, double* out, void* stream);
+
 /* In-place stereo helpers on a (frames, 2) signal, F32 or F64 (utils/dsp.py:21-63, :124-167).
  * op: 0 LR_to_MS, 1 MS_to_LR, 2 apply_stereo_width(width), 3 encode_signal_to_side_channel(x, y)
  * (x = `dry`, y = `a`), 4 rms_normalize(dry, a) DUAL_MONO.  Op 4 sums each signal in the order numpy uses for its
@@ -292,6 +315,12 @@ int vnd_vn_decorrelate_batch_host(vnd_ctx* ctx, const void* x, int32_t x_dtype, 
                                   void* out, int32_t out_dtype);
 int vnd_haas_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal* out, int32_t delay,
                   int32_t delayed_channel, int32_t mode_ms, int32_t mono, int32_t use_width, double width);
+/* vnd_haas_batch_dev with host buffers (x, offsets, settings and out on the host).  Checks, before any copy, that the
+ * offsets start at 0, never decrease and end at rows, and that every clip's delay is >= 0 and its delayed_channel 0 or 1;
+ * derives the out offsets itself (out holds rows + sum of the delays rows).  Inputs of 8 MB and more flow through the
+ * overlapped pipeline in chunks of whole clips (about VND_PIPE_CHUNK_MB each). */
+int vnd_haas_batch_host(vnd_ctx* ctx, const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_clips,
+                        const vnd_haas_clip* clips, double* out);
 int vnd_stereo_op_host(vnd_ctx* ctx, const vnd_signal* a, const vnd_signal* dry, int32_t op, double width);
 int vnd_rms_normalize_host(vnd_ctx* ctx, const vnd_signal* x, int32_t x_ndim, const vnd_signal* y, int32_t y_ndim, int32_t stereo_mode,
                            double epsilon);

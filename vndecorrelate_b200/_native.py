@@ -12,6 +12,8 @@ import os
 import subprocess
 import threading
 
+import numpy as np
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("VND_B200_LIB") or os.path.join(_HERE, "_lib", "libvnd_b200.so")  # the override is for A/B builds of the kernels
 BUILD_SCRIPT = os.path.join(_HERE, "csrc", "build.sh")
@@ -65,6 +67,12 @@ class EpilogueStruct(C.Structure):
     ]
 
 
+# vnd_haas_clip, one record per clip of vnd_haas_batch_dev (32 bytes)
+HAAS_CLIP_DTYPE = np.dtype([("delay", "<i4"), ("delayed_channel", "<i4"), ("mode_ms", "<i4"), ("mono", "<i4"), ("use_width", "<i4"),
+                            ("reserved", "<i4"), ("width", "<f8")])
+assert HAAS_CLIP_DTYPE.itemsize == 32
+
+
 # name -> (restype, argtypes); every symbol include/vnd_b200.h declares
 _P = C.POINTER
 SIGNATURES = {
@@ -81,6 +89,7 @@ SIGNATURES = {
                                                _P(EpilogueStruct), C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]),
     "vnd_colsumsq_seq_f32_dev": (C.c_int, [_P(SignalStruct), C.c_void_p, C.c_void_p]),
     "vnd_haas_dev": (C.c_int, [_P(SignalStruct), _P(SignalStruct), C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_void_p]),
+    "vnd_haas_batch_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "vnd_stereo_op_dev": (C.c_int, [_P(SignalStruct), _P(SignalStruct), C.c_int32, C.c_double, C.c_void_p, C.c_size_t, C.c_void_p]),
     "vnd_dsp_workspace": (C.c_int, [C.c_int64, _P(C.c_size_t)]),
     "vnd_rms_normalize_dev": (C.c_int, [_P(SignalStruct), C.c_int32, _P(SignalStruct), C.c_int32, C.c_int32, C.c_double, C.c_void_p, C.c_size_t, C.c_void_p]),
@@ -109,6 +118,7 @@ SIGNATURES = {
     "vnd_vn_decorrelate_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p,
                                                 _P(TapProgramStruct), _P(EpilogueStruct), C.c_void_p, C.c_int32]),
     "vnd_haas_host": (C.c_int, [C.c_void_p, _P(SignalStruct), _P(SignalStruct), C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double]),
+    "vnd_haas_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "vnd_stereo_op_host": (C.c_int, [C.c_void_p, _P(SignalStruct), _P(SignalStruct), C.c_int32, C.c_double]),
     "vnd_vn_objective_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_int64, _P(TapProgramStruct), C.c_void_p]),
     "vnd_haas_objective_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p]),

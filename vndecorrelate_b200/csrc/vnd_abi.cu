@@ -284,6 +284,29 @@ extern "C" int vnd_haas_dev(const vnd_signal* x, const vnd_signal* out, int32_t 
   return haas_launch(x, out, delay, delayed_channel, mode_ms, mono, use_width, width, (cudaStream_t)stream);
 }
 
+// Arguments of the batched Haas effect that can be checked without reading the tables.
+static int check_haas_batch(const float* x, int64_t rows, const void* frame_offsets, int32_t n_clips, const vnd_haas_clip* clips) {
+  VND_REQUIRE(rows >= 0 && n_clips >= 0, VND_EINVAL, "negative extent (rows %lld, n_clips %d)", (long long)rows, n_clips);
+  VND_REQUIRE(n_clips > 0 || rows == 0, VND_EINVAL, "%lld rows but no clips", (long long)rows);
+  VND_REQUIRE(x != nullptr || rows == 0, VND_EINVAL, "x is null");
+  VND_REQUIRE((frame_offsets != nullptr && clips != nullptr) || n_clips == 0, VND_EINVAL, "frame_offsets or clips is null");
+  return VND_OK;
+}
+
+extern "C" int vnd_haas_batch_dev(const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_clips, const vnd_haas_clip* clips,
+                                  const int64_t* out_offsets, int64_t out_rows, double* out, void* stream) {
+  int rc;
+  if ((rc = check_haas_batch(x, rows, frame_offsets, n_clips, clips))) return rc;
+  VND_REQUIRE(out_rows >= rows, VND_EINVAL, "out_rows = %lld is less than rows = %lld", (long long)out_rows, (long long)rows);
+  VND_REQUIRE(out_offsets != nullptr || n_clips == 0, VND_EINVAL, "out_offsets is null");
+  VND_REQUIRE(out != nullptr || out_rows == 0, VND_EINVAL, "out is null");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(x) % 8 == 0, VND_EINVAL, "x must be 8-byte aligned (one float32 pair per row)");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(clips) % 16 == 0, VND_EINVAL, "clips must be 16-byte aligned");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(out) % 16 == 0, VND_EINVAL, "out must be 16-byte aligned (one float64 pair per row)");
+  return haas_batch_launch(x, reinterpret_cast<const long long*>(frame_offsets), n_clips, clips, reinterpret_cast<const long long*>(out_offsets),
+                           out_rows, out, (cudaStream_t)stream);
+}
+
 extern "C" int vnd_stereo_op_dev(const vnd_signal* a, const vnd_signal* dry, int32_t op, double width, void* workspace,
                                  size_t workspace_bytes, void* stream) {
   int rc;
@@ -1229,6 +1252,101 @@ extern "C" int vnd_haas_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal
   od.data = dout;
   if ((rc = vnd_haas_dev(&xd, &od, delay, delayed_channel, mode_ms, mono, use_width, width, st))) return rc;
   if (dy.elems) VND_CUDA_OK(cudaMemcpyAsync(out->data, dout, dy.elems * esize(out->dtype), cudaMemcpyDeviceToHost, st));
+  VND_CUDA_OK(cudaStreamSynchronize(st));
+  return VND_OK;
+}
+
+extern "C" int vnd_haas_batch_host(vnd_ctx* ctx, const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_clips,
+                                   const vnd_haas_clip* clips, double* out) {
+  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  int rc;
+  if ((rc = check_haas_batch(x, rows, frame_offsets, n_clips, clips))) return rc;
+  if (n_clips == 0) return VND_OK;
+  const int64_t* offs = frame_offsets;
+  VND_REQUIRE(offs[0] == 0, VND_EINVAL, "frame_offsets[0] is %lld, not 0", (long long)offs[0]);
+  for (int i = 0; i < n_clips; ++i)
+    VND_REQUIRE(offs[i + 1] >= offs[i], VND_EINVAL, "frame_offsets decrease at clip %d (%lld -> %lld)", i, (long long)offs[i],
+                (long long)offs[i + 1]);
+  VND_REQUIRE(offs[n_clips] == rows, VND_EINVAL, "frame_offsets end at %lld, not at rows = %lld", (long long)offs[n_clips], (long long)rows);
+  // out offsets of every clip and one more (the total)
+  std::vector<long long> oo((size_t)n_clips + 1);
+  long long shift = 0;
+  for (int i = 0; i < n_clips; ++i) {
+    VND_REQUIRE(clips[i].delay >= 0, VND_EINVAL, "clip %d has a negative delay (%d)", i, clips[i].delay);
+    VND_REQUIRE(clips[i].delayed_channel == 0 || clips[i].delayed_channel == 1, VND_EINVAL, "clip %d: delayed_channel must be 0 or 1, is %d", i,
+                clips[i].delayed_channel);
+    oo[i] = offs[i] + shift;
+    shift += clips[i].delay;
+  }
+  oo[n_clips] = rows + shift;
+  const long long out_rows = oo[n_clips];
+  VND_REQUIRE(out != nullptr || out_rows == 0, VND_EINVAL, "out is null");
+
+  VND_ENTER(ctx);
+  cudaStream_t st = ctx->streams[0];
+  const size_t in_bytes = (size_t)rows * 8, clip_bytes = (size_t)n_clips * sizeof(vnd_haas_clip);
+
+  if (in_bytes >= kPipeMinBytes && getenv("VND_NO_PIPELINE") == nullptr) {
+    // chunks of whole clips of about pipe_chunk_bytes() (at least four chunks when there are four clips), each with its
+    // own offsets rebased to its first row: first[k] .. first[k + 1] are the clips of chunk k, meta[at[k]..] their frame
+    // offsets (n_k + 1) and then their out offsets (n_k)
+    size_t target = pipe_chunk_bytes();
+    if (target > in_bytes / 4) target = in_bytes / 4;
+    std::vector<int> first{0};
+    while (first.back() < n_clips) {
+      const int a = first.back();
+      int b = a + 1;
+      while (b < n_clips && (size_t)(offs[b + 1] - offs[a]) * 8 <= target) ++b;
+      first.push_back(b);
+    }
+    const int nchunks = (int)first.size() - 1;
+    std::vector<long long> meta;
+    std::vector<size_t> at;
+    meta.reserve(2 * (size_t)n_clips + nchunks);
+    long long max_rows = 0, max_out_rows = 0;
+    for (int k = 0; k < nchunks; ++k) {
+      const int a = first[k], b = first[k + 1];
+      at.push_back(meta.size());
+      for (int i = a; i <= b; ++i) meta.push_back(offs[i] - offs[a]);
+      for (int i = a; i < b; ++i) meta.push_back(oo[i] - oo[a]);
+      max_rows = offs[b] - offs[a] > max_rows ? offs[b] - offs[a] : max_rows;
+      max_out_rows = oo[b] - oo[a] > max_out_rows ? oo[b] - oo[a] : max_out_rows;
+    }
+    void* dmeta = nullptr;
+    if ((rc = arena(ctx, S_AUX, clip_bytes + meta.size() * 8, &dmeta))) return rc;
+    VND_CUDA_OK(cudaMemcpyAsync(dmeta, clips, clip_bytes, cudaMemcpyHostToDevice, st));
+    VND_CUDA_OK(cudaMemcpyAsync((char*)dmeta + clip_bytes, meta.data(), meta.size() * 8, cudaMemcpyHostToDevice, st));
+    VND_CUDA_OK(cudaStreamSynchronize(st));  // the tables are on the device before the other streams read them
+    const vnd_haas_clip* dclips = reinterpret_cast<const vnd_haas_clip*>(dmeta);
+    const long long* dtab = reinterpret_cast<const long long*>((char*)dmeta + clip_bytes);
+    auto chunk_of = [&](int k) {
+      const int a = first[k], b = first[k + 1];
+      return PipeChunk{reinterpret_cast<const char*>(x + 2 * offs[a]), (size_t)(offs[b] - offs[a]) * 8, reinterpret_cast<char*>(out + 2 * oo[a]),
+                       (size_t)(oo[b] - oo[a]) * 16};
+    };
+    auto compute = [&](int k, void* din, void* dout, void*, void*, cudaStream_t cs) {
+      const int a = first[k], b = first[k + 1];
+      return haas_batch_launch(reinterpret_cast<const float*>(din), dtab + at[k], b - a, dclips + a, dtab + at[k] + (b - a + 1), oo[b] - oo[a],
+                               reinterpret_cast<double*>(dout), cs);
+    };
+    return run_pipeline(ctx, nchunks, (size_t)max_rows * 8, (size_t)max_out_rows * 16, 0, chunk_of, compute);
+  }
+
+  const size_t out_bytes = (size_t)out_rows * 16;
+  void *din = nullptr, *dout = nullptr, *dmeta = nullptr;
+  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) ||
+      (rc = arena(ctx, S_AUX, clip_bytes + (2 * (size_t)n_clips + 1) * 8, &dmeta)))
+    return rc;
+  if (in_bytes) VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
+  char* dm = reinterpret_cast<char*>(dmeta);
+  VND_CUDA_OK(cudaMemcpyAsync(dm, clips, clip_bytes, cudaMemcpyHostToDevice, st));
+  VND_CUDA_OK(cudaMemcpyAsync(dm + clip_bytes, offs, ((size_t)n_clips + 1) * 8, cudaMemcpyHostToDevice, st));
+  VND_CUDA_OK(cudaMemcpyAsync(dm + clip_bytes + ((size_t)n_clips + 1) * 8, oo.data(), (size_t)n_clips * 8, cudaMemcpyHostToDevice, st));
+  if ((rc = vnd_haas_batch_dev(reinterpret_cast<const float*>(din), rows, reinterpret_cast<const int64_t*>(dm + clip_bytes), n_clips,
+                               reinterpret_cast<const vnd_haas_clip*>(dm), reinterpret_cast<const int64_t*>(dm + clip_bytes + ((size_t)n_clips + 1) * 8),
+                               out_rows, reinterpret_cast<double*>(dout), st)))
+    return rc;
+  if (out_bytes) VND_CUDA_OK(cudaMemcpyAsync(out, dout, out_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
   return VND_OK;
 }

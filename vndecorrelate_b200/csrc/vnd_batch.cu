@@ -121,6 +121,61 @@ __global__ void __launch_bounds__(256) batch_place_kernel(const BatchPlaceParams
 }
 
 // ------------------------------------------------------------------------------------------------
+// Batched HaasEffect.decorrelate (vnd_haas_batch_dev): each CTA takes one (clip, output tile) pair (batch_clip_of over
+// the out offsets) and writes every output frame of its tile, the clip's head and tail zeros included, as one double2;
+// the two input frames it reads (undelayed and delayed) are float2 loads that coalesce across the warp.  The second
+// read of each input frame comes `delay` frames later, from L1 or L2.
+// ------------------------------------------------------------------------------------------------
+static_assert(sizeof(vnd_haas_clip) == 32, "vnd_haas_clip is two 16-byte words");
+
+struct HaasBatchParams {
+  const float* x;               // packed (rows, 2)
+  const long long* offs;        // n + 1
+  const long long* out_offs;    // n
+  const vnd_haas_clip* clips;   // n, 16-byte aligned
+  double* out;                  // (out_rows, 2)
+  int n_clips;
+};
+
+__global__ void __launch_bounds__(256) haas_batch_kernel(const HaasBatchParams p) {
+  constexpr int NT = 256;
+  const int clip = batch_clip_of(p.out_offs, p.n_clips, kHaasTile, blockIdx.x);
+  const long long o0 = p.out_offs[clip];
+  const long long k = (long long)blockIdx.x - (o0 / kHaasTile + clip);
+  const int4* rec = reinterpret_cast<const int4*>(p.clips + clip);
+  const int4 w0 = __ldg(rec), w1 = __ldg(rec + 1);
+  const int delay = w0.x, dch = w0.y, mode_ms = w0.z, mono = w0.w, use_width = w1.x;
+  const double width = __hiloint2double(w1.w, w1.z);
+  const long long x0 = p.offs[clip];
+  const long long L = p.offs[clip + 1] - x0;
+  const long long t0 = k * kHaasTile;
+  const long long t1 = t0 + kHaasTile < L + delay ? t0 + kHaasTile : L + delay;
+  if (k < 0 || t0 >= t1) return;
+  const float2* __restrict__ x2 = reinterpret_cast<const float2*>(p.x) + x0;
+  double2* __restrict__ o2 = reinterpret_cast<double2*>(p.out) + o0;
+  const int sh0 = dch == 0 ? delay : 0, sh1 = dch == 1 ? delay : 0;
+#pragma unroll 4
+  for (long long m = t0 + threadIdx.x; m < t1; m += NT) {
+    const long long q0 = m - sh0, q1 = m - sh1;
+    const bool v0 = q0 >= 0 && q0 < L, v1 = q1 >= 0 && q1 < L;
+    float2 s0 = make_float2(0.0f, 0.0f), s1 = make_float2(0.0f, 0.0f);
+    if (v0) s0 = __ldg(x2 + q0);
+    if (v1) s1 = __ldg(x2 + q1);
+    o2[m] = haas_frame(s0.x, s0.y, v0, s1.x, s1.y, v1, mode_ms, mono, use_width, width);
+  }
+}
+
+int haas_batch_launch(const float* x, const long long* offs, int n_clips, const vnd_haas_clip* clips, const long long* out_offs,
+                      long long out_rows, double* out, cudaStream_t st) {
+  if (n_clips == 0 || out_rows == 0) return VND_OK;
+  const long long blocks = out_rows / kHaasTile + n_clips;
+  VND_REQUIRE(blocks < 0x7fffffffLL, VND_EUNSUPPORTED, "grid too large (%lld CTAs)", blocks);
+  const HaasBatchParams p{x, offs, out_offs, clips, out, n_clips};
+  haas_batch_kernel<<<(unsigned)blocks, 256, 0, st>>>(p);
+  return after_launch("haas_batch_kernel");
+}
+
+// ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
 size_t vn_batch_workspace_bytes(long long rows, int n_clips, int rms) {

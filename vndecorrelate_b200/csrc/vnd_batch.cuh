@@ -54,6 +54,41 @@ struct BatchSumCols {
   }
 };
 
+// HaasEffect.decorrelate at one output frame (float64 throughout, SURVEY.md A.6): channel 0 comes from input frame
+// (a0, b0) and channel 1 from (a1, b1) - one of them the delayed frame -, each 0 where its frame lies outside the
+// signal (v0, v1 false).  A mono signal has a == b.  haas_kernel and haas_batch_kernel both call it, so the batch
+// gives every clip the single call's bits.
+__device__ __forceinline__ double2 haas_frame(float a0, float b0, bool v0, float a1, float b1, bool v1, int mode_ms, int mono,
+                                              int use_width, double width) {
+  // the channel pair as the reference stores it after the optional LR->MS, at one frame
+  auto chan = [&](float af, float bf, bool v, int c) -> double {
+    if (!v) return 0.0;
+    const double a = (double)af, b = (double)bf;
+    if (mode_ms && !mono) return c == 0 ? dmul(dadd(a, b), 0.5) : dmul(dsub(a, b), 0.5);
+    return c == 0 ? a : b;
+  };
+  double c0 = chan(a0, b0, v0, 0);
+  double c1 = chan(a1, b1, v1, 1);
+  if (mode_ms) {
+    const double l = dadd(c0, c1), r = dsub(c0, c1);
+    c0 = l;
+    c1 = r;
+    if (mono) {
+      c0 = dmul(c0, 0.5);
+      c1 = dmul(c1, 0.5);
+    }
+  }
+  if (use_width) {
+    double M = dmul(dadd(c0, c1), 0.5);
+    double S = dmul(dsub(c0, c1), 0.5);
+    M = dmul(M, dsub(1.0, width));
+    S = dmul(S, width);
+    c0 = dadd(M, S);
+    c1 = dsub(M, S);
+  }
+  return make_double2(c0, c1);
+}
+
 // CTA b of a batched kernel with `tile` outputs per CTA takes clip i, the last one with V[i] <= b where
 // V[i] = floor(offs[i] / tile) + i, and that clip's tile b - V[i].  V[i + 1] - V[i] >= max(1, ceil(frames_i / tile)),
 // so floor(rows / tile) + n CTAs - a grid known from host scalars alone - cover every tile of every clip and give an
@@ -93,5 +128,12 @@ bool vn_batch_smem(int halo, int prog_words, size_t* smem);
 size_t vn_batch_workspace_bytes(long long rows, int n_clips, int rms);
 int vn_batch_launch(const float* x, long long rows, const long long* offs, int n_clips, const int* prog_of, const vnd_tap_program* taps,
                     const vnd_epilogue* ep, void* out, int out_dtype, void* workspace, cudaStream_t st);
+
+// Output frames per CTA of haas_batch_kernel (16 per thread).
+constexpr int kHaasTile = 4096;
+// vnd_haas_batch_dev's launch: one haas_batch_kernel over floor(out_rows / kHaasTile) + n_clips CTAs, none when
+// out_rows == 0.  offs (n + 1), out_offs (n) and clips (n, 16-byte aligned) are device arrays.
+int haas_batch_launch(const float* x, const long long* offs, int n_clips, const vnd_haas_clip* clips, const long long* out_offs,
+                      long long out_rows, double* out, cudaStream_t st);
 
 }  // namespace vnd

@@ -522,35 +522,20 @@ struct HaasParams {
 __global__ void __launch_bounds__(256) haas_kernel(const HaasParams p) {
   const long long total = p.frames + p.delay;
   for (long long m = (long long)blockIdx.x * blockDim.x + threadIdx.x; m < total; m += (long long)gridDim.x * blockDim.x) {
-    // channel pair (as the reference stores it after the optional LR->MS) at frame q, 0 outside
-    auto chan = [&](long long q, int c) -> double {
-      if (q < 0 || q >= p.frames) return 0.0;
-      const double a = (double)p.x[q * p.x_st];
-      const double b = (double)p.x[q * p.x_st + p.x_sc];
-      if (p.mode_ms && !p.mono) return c == 0 ? dmul(dadd(a, b), 0.5) : dmul(dsub(a, b), 0.5);
-      return c == 0 ? a : b;
-    };
-    double c0 = chan(m - (p.delay_ch == 0 ? p.delay : 0), 0);
-    double c1 = chan(m - (p.delay_ch == 1 ? p.delay : 0), 1);
-    if (p.mode_ms) {
-      const double l = dadd(c0, c1), r = dsub(c0, c1);
-      c0 = l;
-      c1 = r;
-      if (p.mono) {
-        c0 = dmul(c0, 0.5);
-        c1 = dmul(c1, 0.5);
-      }
+    const long long q0 = m - (p.delay_ch == 0 ? p.delay : 0), q1 = m - (p.delay_ch == 1 ? p.delay : 0);
+    const bool v0 = q0 >= 0 && q0 < p.frames, v1 = q1 >= 0 && q1 < p.frames;
+    float a0 = 0.0f, b0 = 0.0f, a1 = 0.0f, b1 = 0.0f;
+    if (v0) {
+      a0 = p.x[q0 * p.x_st];
+      b0 = p.x[q0 * p.x_st + p.x_sc];
     }
-    if (p.use_width) {
-      double M = dmul(dadd(c0, c1), 0.5);
-      double S = dmul(dsub(c0, c1), 0.5);
-      M = dmul(M, dsub(1.0, p.width));
-      S = dmul(S, p.width);
-      c0 = dadd(M, S);
-      c1 = dsub(M, S);
+    if (v1) {
+      a1 = p.x[q1 * p.x_st];
+      b1 = p.x[q1 * p.x_st + p.x_sc];
     }
-    p.out[m * p.o_st] = c0;
-    p.out[m * p.o_st + p.o_sc] = c1;
+    const double2 c = haas_frame(a0, b0, v0, a1, b1, v1, p.mode_ms, p.mono, p.use_width, p.width);
+    p.out[m * p.o_st] = c.x;
+    p.out[m * p.o_st + p.o_sc] = c.y;
   }
 }
 

@@ -34,7 +34,8 @@ from .taps import (
 )
 from .utils.dsp import LayoutMode, apply_stereo_width, check_equal_length, rms_normalize, to_float32
 
-__all__ = ["Decorrelator", "SignalChain", "HaasEffect", "VelvetNoise", "decorrelate_batch", "generate_velvet_noise", "convolve_velvet_noise"]
+__all__ = ["Decorrelator", "SignalChain", "HaasEffect", "VelvetNoise", "decorrelate_batch", "haas_effect_batch", "generate_velvet_noise",
+           "convolve_velvet_noise"]
 
 
 class Decorrelator:
@@ -483,13 +484,19 @@ def _batch_settings(vn: VelvetNoise, haas: "HaasEffect | None") -> dict:
     }
 
 
-def _check_batch_layout(offsets: np.ndarray, program_of_clip: np.ndarray, n_programs: int, rows: int) -> None:
-    """The packed layout vnd_vn_decorrelate_batch_* reads: offsets from 0 to ``rows``, never decreasing, and a program
-    index in range for every clip (the device entry point cannot check these)."""
-    if len(offsets) != len(program_of_clip) + 1 or len(offsets) == 0 or offsets[0] != 0 or offsets[-1] != rows:
+def _check_offsets(offsets: np.ndarray, n: int, rows: int) -> None:
+    """The frame offsets of a packed batch of ``n`` clips: from 0 to ``rows``, never decreasing (the device entry points
+    cannot check them)."""
+    if len(offsets) != n + 1 or offsets[0] != 0 or offsets[-1] != rows:
         raise ValueError(f"frame offsets must run from 0 to {rows} with one entry per clip and one more")
     if np.any(np.diff(offsets) < 0):
         raise ValueError("frame offsets must not decrease")
+
+
+def _check_batch_layout(offsets: np.ndarray, program_of_clip: np.ndarray, n_programs: int, rows: int) -> None:
+    """The packed layout vnd_vn_decorrelate_batch_* reads: offsets from 0 to ``rows``, never decreasing, and a program
+    index in range for every clip (the device entry point cannot check these)."""
+    _check_offsets(offsets, len(program_of_clip), rows)
     if len(program_of_clip) and (program_of_clip.min() < 0 or program_of_clip.max() >= n_programs):
         raise ValueError(f"program indices must lie in [0, {n_programs})")
 
@@ -539,6 +546,44 @@ def _pack_clips(xp: np.ndarray, clips, offsets: np.ndarray) -> None:
 
     with ThreadPoolExecutor(max_workers=min(8, os.cpu_count() or 1, len(clips))) as pool:
         list(pool.map(put, range(len(clips))))
+
+
+def _pack_tensors(clips, rows: int, device):
+    """The CUDA clips packed into one (rows, 2) float32 tensor (a mono clip into both columns)."""
+    import torch
+
+    if not rows:
+        return torch.empty((0, 2), dtype=torch.float32, device=device)
+    return torch.cat([x[:, :2] if x.ndim == 2 else x[:, None].expand(-1, 2) for x in clips])
+
+
+def _batch_device(input_signals, is_array: bool, where: str):
+    """``(torch_in, device)`` of a batch's clips: all CUDA tensors on one device, or all numpy (device None).  Mixed
+    clips and clips on several devices raise ``ValueError``, CPU tensors ``VndError(VND_EUNSUPPORTED)``."""
+    torch_in = R.is_torch_tensor(input_signals) if is_array else any(R.is_torch_tensor(c) for c in input_signals)
+    if not torch_in:
+        return False, None
+    if is_array:
+        clips_in = [input_signals]
+    else:
+        clips_in = list(input_signals)
+        if not all(R.is_torch_tensor(c) for c in clips_in):
+            raise ValueError("clips must be all numpy arrays or all CUDA tensors")
+    if not all(c.is_cuda for c in clips_in):
+        raise N.VndError(N.VND_EUNSUPPORTED, where, "CPU torch tensors are not supported (no CPU fallback); pass CUDA tensors or numpy arrays")
+    device = clips_in[0].device if clips_in else None
+    if any(c.device != device for c in clips_in):
+        raise ValueError("all clips must be on one CUDA device")
+    return True, device
+
+
+def _cast_clips(input_signals, is_array: bool, torch_in: bool):
+    """``(x3, clips)``: the clips cast with ``to_float32`` as the single-clip calls cast them, and for an array of clips
+    the cast array itself (None for a list)."""
+    if is_array:
+        x3 = to_float32(input_signals if torch_in else np.asarray(input_signals))
+        return x3, [x3[i] for i in range(int(x3.shape[0]))]
+    return None, [to_float32(c if torch_in else np.asarray(c)) for c in input_signals]
 
 
 def _sums_pairwise(x) -> bool:
@@ -600,26 +645,10 @@ def decorrelate_batch(input_signals, decorrelator):
     out_f64 = bool(settings and settings["Haas stage"])
 
     # clips: cast, checked as the single-clip call checks them
-    torch_in = R.is_torch_tensor(input_signals) if is_array else any(R.is_torch_tensor(c) for c in input_signals)
+    torch_in, device = _batch_device(input_signals, is_array, "decorrelate_batch")
     if torch_in:
         import torch
-
-        if is_array:
-            clips_in = [input_signals]
-        else:
-            clips_in = list(input_signals)
-            if not all(R.is_torch_tensor(c) for c in clips_in):
-                raise ValueError("clips must be all numpy arrays or all CUDA tensors")
-        if not all(c.is_cuda for c in clips_in):
-            raise N.VndError(N.VND_EUNSUPPORTED, "decorrelate_batch", "CPU torch tensors are not supported (no CPU fallback); pass CUDA tensors or numpy arrays")
-        device = clips_in[0].device if clips_in else None
-        if any(c.device != device for c in clips_in):
-            raise ValueError("all clips must be on one CUDA device")
-    if is_array:
-        x3 = to_float32(input_signals if torch_in else np.asarray(input_signals))
-        clips = [x3[i] for i in range(n)]
-    else:
-        clips = [to_float32(c if torch_in else np.asarray(c)) for c in input_signals]
+    x3, clips = _cast_clips(input_signals, is_array, torch_in)
     for (vn, _), x in zip(pairs, clips):
         vn._check_input(x)
     if n == 0:
@@ -647,10 +676,7 @@ def decorrelate_batch(input_signals, decorrelator):
     lib = N.lib()
 
     if torch_in:
-        if is_array:
-            xp = x3.contiguous().view(-1, 2)
-        else:
-            xp = torch.cat([x[:, :2] if x.ndim == 2 else x[:, None].expand(-1, 2) for x in clips]) if rows else torch.empty((0, 2), dtype=torch.float32, device=device)
+        xp = x3.contiguous().view(-1, 2) if is_array else _pack_tensors(clips, rows, device)
         if xp.data_ptr() % 8:  # the kernels load one float32 pair per row
             xp = xp.clone()
         out = torch.empty((rows + n * delay, 2), dtype=torch.float64 if out_f64 else torch.float32, device=device)
@@ -711,6 +737,160 @@ def _vn_decorrelate_into(x32, out, program: TapProgram, ep, stream) -> None:
     ps = R.device_program(program, x32.device)
     N.check(lib.vnd_vn_decorrelate_dev(C.byref(sx), C.byref(so), C.byref(ps), C.byref(ep), work.data_ptr(), nbytes.value, stream),
             "vnd_vn_decorrelate_dev")
+
+
+def _haas_table(haases: "Sequence[HaasEffect]", clips, shared: bool) -> np.ndarray:
+    """The ``vnd_haas_clip`` record of every clip (``N.HAAS_CLIP_DTYPE``), checked as ``HaasEffect.decorrelate`` checks
+    its clip: the first clip the single call would reject raises that call's exception, with the clip's index.  The
+    attributes of the effects and the shapes of the clips are read once each; the rest is vectorised."""
+    n = len(clips)
+    src = haases[:1] if shared else haases
+    delays = np.array([h.delay_len_samples for h in src], dtype=object)
+    channels = np.array([h.delayed_channel for h in src], dtype=object)
+    mode_ms = np.array([h.mode for h in src], dtype=object) == LayoutMode.MS
+    widths = np.array([h.width for h in src], dtype=object)
+    use_width = widths != None  # noqa: E711 - elementwise
+    ndim = np.fromiter((x.ndim for x in clips), dtype=np.int64, count=n)
+    cols = np.fromiter((x.shape[1] if x.ndim == 2 else 2 for x in clips), dtype=np.int64, count=n)
+    bad_shape = ((ndim != 1) & (ndim != 2)) | (cols != 2)
+    bad_channel = np.broadcast_to(~np.isin(channels, (0, 1, -1, -2)), (n,))
+    bad_delay = np.broadcast_to((delays < 0) | (delays >= 2**31), (n,))
+    bad = np.flatnonzero(bad_shape | bad_channel | bad_delay)
+    if bad.size:
+        i = int(bad[0])
+        try:
+            haases[i]._check(clips[i])
+        except (ValueError, IndexError) as e:
+            raise type(e)(f"clip {i}: {e}") from None
+        raise ValueError(f"clip {i}: the Haas delay of {haases[i].delay_len_samples} frames must lie in [0, 2**31)")
+    table = np.zeros(n, dtype=N.HAAS_CLIP_DTYPE)
+    table["delay"] = delays.astype(np.int64)
+    table["delayed_channel"] = channels.astype(np.int64) % 2
+    table["mode_ms"] = mode_ms
+    table["mono"] = ndim == 1
+    table["use_width"] = use_width
+    table["width"] = np.where(use_width, widths, 0.0).astype(np.float64)
+    return table
+
+
+def _haas_offsets(lengths: np.ndarray, delays: np.ndarray) -> "tuple[np.ndarray, np.ndarray]":
+    """``(frame_offsets, out_offsets)`` of a packed Haas batch: clip ``i`` is input rows ``[frame_offsets[i],
+    frame_offsets[i + 1])`` and output rows from ``out_offsets[i] = frame_offsets[i] + sum_{j < i} delays[j]``."""
+    n = len(lengths)
+    offsets = np.zeros(n + 1, dtype=np.int64)
+    np.cumsum(lengths, out=offsets[1:])
+    _check_offsets(offsets, n, int(offsets[-1]))
+    out_offsets = offsets[:-1].copy()
+    out_offsets[1:] += np.cumsum(delays[:-1], dtype=np.int64)
+    return offsets, out_offsets
+
+
+def _packed_base(clips, offsets: np.ndarray, torch_in: bool) -> "int | None":
+    """The address of row 0 when the clips are already consecutive row ranges of one C-order (rows, 2) float32 buffer
+    (e.g. the views ``decorrelate_batch`` returns without a Haas stage), else None.  Only the clips' own rows are read
+    from it, so the clips may come from separate allocations as long as their addresses line up."""
+    n = len(clips)
+    if torch_in:
+        import torch
+
+        if not all(x.dtype == torch.float32 and x.ndim == 2 and x.shape[1] == 2 and x.stride(1) == 1 and (x.shape[0] <= 1 or x.stride(0) == 2)
+                   for x in clips):
+            return None
+        ptrs = np.fromiter((x.data_ptr() for x in clips), dtype=np.int64, count=n)
+    else:
+        if not all(x.dtype == np.float32 and x.ndim == 2 and x.shape[1] == 2 and x.strides[1] == 4 and (x.shape[0] <= 1 or x.strides[0] == 8)
+                   for x in clips):
+            return None
+        ptrs = np.fromiter((x.ctypes.data for x in clips), dtype=np.int64, count=n)
+    used = np.diff(offsets) > 0
+    if not used.any():
+        return None
+    starts = offsets[:-1][used]
+    base = int(ptrs[used][0] - 8 * starts[0])
+    if base % 8 or not np.array_equal(ptrs[used], base + 8 * starts):
+        return None
+    return base
+
+
+def haas_effect_batch(input_signals, haas_effect):
+    """Apply the Haas effect to many clips in one call: element ``i`` of the result is byte-identical (dtype float64,
+    shape, bytes) to ``haas_effect_i.decorrelate(input_signals[i])``, computed with one launch for the whole batch.
+
+    ``input_signals``: a sequence of clips - numpy arrays or CUDA tensors, ``(frames_i, 2)`` or mono ``(frames_i,)``,
+    any length including 0, cast per clip with ``to_float32`` - or one ``(n_clips, frames, 2)`` array or CUDA tensor,
+    returned as one ``(n_clips, frames + delay, 2)`` array (its clips must then share one delay).  ``haas_effect``: one
+    ``HaasEffect`` shared by all clips, or a sequence with one per clip (e.g. with the delays
+    ``optimize_haas_delay_batch`` found); each clip's delay, delayed channel, mode and width are its own.
+
+    Every error is raised before any device work, with the index of the clip it concerns.  Numpy in gives numpy out
+    (views into one page-locked block); CUDA tensors in give CUDA tensors out (views into one tensor), on torch's
+    current stream.  Clips that already are consecutive rows of one (rows, 2) float32 buffer, such as the output of
+    ``decorrelate_batch`` without a Haas stage, are read in place."""
+    is_array = R.is_torch_tensor(input_signals) or isinstance(input_signals, np.ndarray)
+    if is_array and (input_signals.ndim != 3 or input_signals.shape[2] != 2):
+        raise ValueError(f"an array of clips must be (n_clips, frames, 2), got shape {tuple(input_signals.shape)}; pass other clips as a list")
+    n = int(input_signals.shape[0]) if is_array else len(input_signals)
+    shared = isinstance(haas_effect, HaasEffect)
+    haases = [haas_effect] * n if shared else list(haas_effect)
+    if len(haases) != n:
+        raise ValueError(f"{len(haases)} Haas effects for {n} clips: pass one HaasEffect, or one per clip")
+    if not all(isinstance(h, HaasEffect) for h in (haases[:1] if shared else haases)):
+        raise TypeError("haas_effect_batch takes a HaasEffect or a sequence of them")
+    torch_in, device = _batch_device(input_signals, is_array, "haas_effect_batch")
+    if torch_in:
+        import torch
+    raw = input_signals if is_array or torch_in else [np.asarray(c) for c in input_signals]
+    table = _haas_table(haases, [raw[i] for i in range(n)], shared)
+    delays = table["delay"].astype(np.int64)
+    if is_array and n and np.any(delays != delays[0]):
+        raise ValueError("the clips of an (n_clips, frames, 2) array need one Haas delay; pass clips with different delays as a list")
+    if n == 0:
+        if not is_array:
+            return []
+        shape = (0, int(input_signals.shape[1]) + (haas_effect.delay_len_samples if shared else 0), 2)
+        return torch.empty(shape, dtype=torch.float64, device=input_signals.device) if torch_in else np.empty(shape, dtype=np.float64)
+
+    x3, clips = _cast_clips(raw, is_array, torch_in)
+    lengths = np.fromiter((x.shape[0] for x in clips), dtype=np.int64, count=n)
+    offsets, out_offsets = _haas_offsets(lengths, delays)
+    rows, out_rows = int(offsets[-1]), int(offsets[-1] + delays.sum())
+    lib = N.lib()
+
+    keep = None  # the packed input, when the clips are packed here
+    if torch_in:
+        if is_array:
+            keep = x3.contiguous().view(-1, 2)
+            base = keep.data_ptr()
+        else:
+            base = _packed_base(clips, offsets, True)
+            if base is None:
+                keep = _pack_tensors(clips, rows, device)
+                base = keep.data_ptr()
+        if base % 8:  # the kernel loads one float32 pair per row
+            keep = keep.clone()
+            base = keep.data_ptr()
+        out = torch.empty((out_rows, 2), dtype=torch.float64, device=device)
+        with torch.cuda.device(device):
+            meta = torch.from_numpy(np.concatenate([table.view(np.int64), offsets, out_offsets])).to(device)
+            m = meta.data_ptr()
+            N.check(lib.vnd_haas_batch_dev(base if rows else None, rows, m + 32 * n, n, m, m + 32 * n + 8 * (n + 1), out_rows,
+                                           out.data_ptr() if out_rows else None, R.torch_stream_ptr(out)), "vnd_haas_batch_dev")
+        results = out.view(n, -1, 2) if is_array else [out[int(o):int(o) + int(L) + int(d)] for o, L, d in zip(out_offsets, lengths, delays)]
+    else:
+        if is_array:
+            keep = np.ascontiguousarray(x3).reshape(-1, 2)  # already packed: a view when the input is C-ordered float32
+            base = keep.ctypes.data
+        else:
+            base = _packed_base(clips, offsets, False)
+            if base is None:
+                keep = R.pinned_empty((rows, 2), np.float32)  # page-locked (within the pool's cap): uploaded by DMA, no staging copy
+                _pack_clips(keep, clips, offsets)
+                base = keep.ctypes.data
+        out = R.pinned_empty((out_rows, 2), np.float64)
+        N.check(lib.vnd_haas_batch_host(R.HostContext.get().handle, base if rows else None, rows, offsets.ctypes.data, n, table.ctypes.data,
+                                        out.ctypes.data if out_rows else None), "vnd_haas_batch_host")
+        results = out.reshape(n, -1, 2) if is_array else [out[o:o + L + d] for o, L, d in zip(out_offsets, lengths, delays)]
+    return results
 
 
 # ------------------------------------------------------------------------------------------------
