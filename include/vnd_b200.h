@@ -186,6 +186,45 @@ typedef struct vnd_haas_clip {
 int vnd_haas_batch_dev(const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_clips, const vnd_haas_clip* clips,
                        const int64_t* out_offsets, int64_t out_rows, double* out, void* stream);
 
+/* One step of many live signals that arrive block by block: ONE launch for all signals (none when rows == 0 and
+ * out_rows == 0; history_out is then not written and history_in stays the current history).
+ *   x              : packed float32 (rows, 2) C-order blocks, 8-byte aligned; signal i's block is rows [frame_offsets[i],
+ *                    frame_offsets[i + 1]) - a mono block is packed with its samples in both columns;
+ *   frame_offsets  : n_signals + 1 int64, starting at 0, non-decreasing, ending at rows;
+ *   received       : n_signals int64, the frames signal i received before this step (T0; T1 = T0 + its block's rows);
+ *   history_in/out : two float32 (n_signals, history_frames, 2) C-order buffers, 8-byte aligned.  Rows [i H, i H + H) of
+ *                    history_in must hold signal i's frames [T0 - H, T0) as the previous step wrote them; the step writes
+ *                    its frames [T1 - H, T1) to history_out (those before frame 0 as +0).  The caller swaps the two after
+ *                    every step that launched.  A frame the kernel reads before T0 - H or before 0 is +0;
+ *   out_offsets    : n_signals + 1 int64, starting at 0, non-decreasing, ending at out_rows: signal i writes out rows
+ *                    [out_offsets[i], out_offsets[i + 1]).
+ * A final step is the caller's matter: frames at or past T1 read as +0, as past the end of a one-shot signal of T1
+ * frames, and the next step of a signal that starts over passes received = 0 (its old history is never read).
+ * Neither _dev call can read the device-side tables, which must be valid; both check the pointers and sizes they see.
+ *
+ * vnd_vn_block_step_dev: VelvetNoise.decorrelate without normaliser.  taps, program_of_signal and ep are those of
+ * vnd_vn_decorrelate_batch_dev with every program packed for an unbounded length (all taps kept); ep->rms_normalize
+ * and ep->haas_delay must be 0.  emitted[i] = E0 is the number of frames signal i has emitted before; it writes its
+ * output frames [E0, E0 + out_offsets[i + 1] - out_offsets[i]) to float32 (out_rows, 2) `out`.  history_frames must be at
+ * least taps->halo - 1.  Bit contract: output frame t is byte-identical to frame t of vnd_vn_decorrelate_dev on the
+ * signal's first T frames with its channel pair, for any T > t with t + taps->halo - 1 < T1 or T = T1: the frames it reads
+ * are the same, and a tap past the end reads +0, which adds nothing, as the one-shot call drops it.  VND_EUNSUPPORTED,
+ * checked before anything else after the program and the epilogue, when the filter's halo does not fit the kernel's
+ * shared memory (the rule of vnd_vn_decorrelate_batch_dev): a call with n_signals = 0 asks it without a launch.
+ *
+ * vnd_haas_block_step_dev: HaasEffect.decorrelate with the settings record signals[i] (vnd_haas_batch_dev's; mono as
+ * the block is packed), history_frames >= every delay.  Signal i writes its output frames [T0, T0 + out_offsets[i + 1] -
+ * out_offsets[i]) to float64 (out_rows, 2) `out`, 16-byte aligned.  Bit contract: output frame m < T1 is byte-identical
+ * to frame m of vnd_haas_dev on the signal's first T1 frames (it reads input frames m and m - delay only), and frames
+ * [T1, T1 + delay) - a final step's tail - to those of vnd_haas_dev on exactly T1 frames. */
+int vnd_vn_block_step_dev(const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_signals, const int64_t* received,
+                          const int64_t* emitted, const int32_t* program_of_signal, const vnd_tap_program* taps, const vnd_epilogue* ep,
+                          const float* history_in, float* history_out, int32_t history_frames, const int64_t* out_offsets,
+                          int64_t out_rows, float* out, void* stream);
+int vnd_haas_block_step_dev(const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_signals, const int64_t* received,
+                            const vnd_haas_clip* signals, const float* history_in, float* history_out, int32_t history_frames,
+                            const int64_t* out_offsets, int64_t out_rows, double* out, void* stream);
+
 /* In-place stereo helpers on a (frames, 2) signal, F32 or F64 (utils/dsp.py:21-63, :124-167).
  * op: 0 LR_to_MS, 1 MS_to_LR, 2 apply_stereo_width(width), 3 encode_signal_to_side_channel(x, y)
  * (x = `dry`, y = `a`), 4 rms_normalize(dry, a) DUAL_MONO.  Op 4 sums each signal in the order numpy uses for its

@@ -307,6 +307,80 @@ extern "C" int vnd_haas_batch_dev(const float* x, int64_t rows, const int64_t* f
                            out_rows, out, (cudaStream_t)stream);
 }
 
+// Arguments of a block step that can be checked without reading device memory; fills the step's tables.
+static int check_block_step(const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_signals, const int64_t* received,
+                            const float* history_in, float* history_out, int32_t history_frames, const int64_t* out_offsets,
+                            int64_t out_rows, const void* out, BlockStepParams* b) {
+  VND_REQUIRE(rows >= 0 && n_signals >= 0 && out_rows >= 0 && history_frames >= 0, VND_EINVAL,
+              "negative extent (rows %lld, n_signals %d, out_rows %lld, history_frames %d)", (long long)rows, n_signals, (long long)out_rows,
+              history_frames);
+  VND_REQUIRE(n_signals > 0 || rows + out_rows == 0, VND_EINVAL, "%lld rows and %lld out rows but no signals", (long long)rows,
+              (long long)out_rows);
+  VND_REQUIRE(x != nullptr || rows == 0, VND_EINVAL, "x is null");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(x) % 8 == 0, VND_EINVAL, "x must be 8-byte aligned (one float32 pair per row)");
+  VND_REQUIRE((frame_offsets != nullptr && received != nullptr && out_offsets != nullptr) || n_signals == 0, VND_EINVAL,
+              "frame_offsets, received or out_offsets is null");
+  VND_REQUIRE(out != nullptr || out_rows == 0, VND_EINVAL, "out is null");
+  const bool hist = history_frames > 0 && n_signals > 0;
+  VND_REQUIRE(!hist || (history_in != nullptr && history_out != nullptr), VND_EINVAL, "a history buffer is null");
+  VND_REQUIRE(!hist || history_in != history_out, VND_EINVAL, "history_in and history_out must be two buffers");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(history_in) % 8 == 0 && reinterpret_cast<uintptr_t>(history_out) % 8 == 0, VND_EINVAL,
+              "the history buffers must be 8-byte aligned");
+  *b = BlockStepParams{};
+  b->x = x;
+  b->offs = reinterpret_cast<const long long*>(frame_offsets);
+  b->received = reinterpret_cast<const long long*>(received);
+  b->out_offs = reinterpret_cast<const long long*>(out_offsets);
+  b->hist_in = history_in;
+  b->hist_out = history_out;
+  b->n = n_signals;
+  b->H = history_frames;
+  return VND_OK;
+}
+
+extern "C" int vnd_vn_block_step_dev(const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_signals, const int64_t* received,
+                                     const int64_t* emitted, const int32_t* program_of_signal, const vnd_tap_program* taps,
+                                     const vnd_epilogue* ep, const float* history_in, float* history_out, int32_t history_frames,
+                                     const int64_t* out_offsets, int64_t out_rows, float* out, void* stream) {
+  int rc;
+  if ((rc = check_taps(taps))) return rc;
+  VND_REQUIRE(taps->order == VND_ORDER_SEGMENTED, VND_EINVAL, "decorrelate needs a SEGMENTED tap program");
+  VND_REQUIRE(taps->channels % 2 == 0, VND_EINVAL, "the tap program has %d channels: it must hold two per filter", taps->channels);
+  VND_REQUIRE(ep != nullptr, VND_EINVAL, "epilogue is null");
+  VND_REQUIRE(!ep->rms_normalize, VND_EINVAL, "rms_normalize depends on the whole signal and cannot run block by block");
+  VND_REQUIRE(ep->haas_delay == 0, VND_EINVAL, "the Haas stage of a block step is vnd_haas_block_step_dev");
+  size_t smem = 0;
+  VND_REQUIRE(vn_batch_smem(((taps->halo > 0 ? taps->halo : 0) + 3) & ~3, 2 * taps->max_channel_words, &smem), VND_EUNSUPPORTED,
+              "a halo of %d frames does not fit the block-step kernel's shared memory", taps->halo);
+  VND_REQUIRE(history_frames >= taps->halo - 1, VND_EINVAL, "%d history frames cannot hold the %d frames the filter reads ahead",
+              history_frames, taps->halo - 1);
+  BlockStepParams b;
+  if ((rc = check_block_step(x, rows, frame_offsets, n_signals, received, history_in, history_out, history_frames, out_offsets, out_rows, out,
+                             &b)))
+    return rc;
+  VND_REQUIRE(n_signals == 0 || taps->channels >= 2, VND_EINVAL, "the tap program holds no filter");
+  VND_REQUIRE((emitted != nullptr && program_of_signal != nullptr) || n_signals == 0, VND_EINVAL, "emitted or program_of_signal is null");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(out) % 8 == 0, VND_EINVAL, "out must be 8-byte aligned (one float32 pair per row)");
+  if (n_signals == 0 || rows + out_rows == 0) return VND_OK;
+  b.emitted = reinterpret_cast<const long long*>(emitted);
+  return vn_block_step_launch(b, out_rows, program_of_signal, taps, ep, out, (cudaStream_t)stream);
+}
+
+extern "C" int vnd_haas_block_step_dev(const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_signals, const int64_t* received,
+                                       const vnd_haas_clip* signals, const float* history_in, float* history_out, int32_t history_frames,
+                                       const int64_t* out_offsets, int64_t out_rows, double* out, void* stream) {
+  int rc;
+  BlockStepParams b;
+  if ((rc = check_block_step(x, rows, frame_offsets, n_signals, received, history_in, history_out, history_frames, out_offsets, out_rows, out,
+                             &b)))
+    return rc;
+  VND_REQUIRE(signals != nullptr || n_signals == 0, VND_EINVAL, "signals is null");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(signals) % 16 == 0, VND_EINVAL, "signals must be 16-byte aligned");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(out) % 16 == 0, VND_EINVAL, "out must be 16-byte aligned (one float64 pair per row)");
+  if (n_signals == 0 || rows + out_rows == 0) return VND_OK;
+  return haas_block_step_launch(b, out_rows, signals, out, (cudaStream_t)stream);
+}
+
 extern "C" int vnd_stereo_op_dev(const vnd_signal* a, const vnd_signal* dry, int32_t op, double width, void* workspace,
                                  size_t workspace_bytes, void* stream) {
   int rc;

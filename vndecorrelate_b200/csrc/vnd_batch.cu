@@ -176,6 +176,55 @@ int haas_batch_launch(const float* x, const long long* offs, int n_clips, const 
 }
 
 // ------------------------------------------------------------------------------------------------
+// One Haas step of many live signals (vnd_haas_block_step_dev): signal i's output frames [T0, T0 + count) are those of
+// HaasEffect.decorrelate on its whole input, because output frame m reads input frames m - sh0, m - sh1 <= m only.
+// A frame at or past T1 is +0 and not valid, as past the end of a one-shot signal of T1 frames: a final step's tail.
+// ------------------------------------------------------------------------------------------------
+bool block_step_grid(BlockStepParams* b, long long out_rows, int tile, long long* blocks) {
+  b->out_blocks = out_rows / tile + b->n;
+  b->hchunks = (b->H + kHistTile - 1) / kHistTile;
+  *blocks = b->out_blocks + (long long)b->n * b->hchunks;
+  return *blocks < 0x7fffffffLL;
+}
+
+__global__ void __launch_bounds__(256) haas_block_step_kernel(const BlockStepParams b, const vnd_haas_clip* clips, double* out) {
+  constexpr int NT = 256;
+  if (blockIdx.x >= b.out_blocks) {
+    block_step_history(b, (long long)blockIdx.x - b.out_blocks);
+    return;
+  }
+  const int sig = batch_clip_of(b.out_offs, b.n, kHaasTile, blockIdx.x);
+  const long long o0 = b.out_offs[sig];
+  const long long cnt = b.out_offs[sig + 1] - o0;
+  const long long k = (long long)blockIdx.x - (o0 / kHaasTile + sig);
+  const long long j0 = k * kHaasTile;
+  if (k < 0 || j0 >= cnt) return;
+  const long long j1 = j0 + kHaasTile < cnt ? j0 + kHaasTile : cnt;
+  const int4* rec = reinterpret_cast<const int4*>(clips + sig);
+  const int4 w0 = __ldg(rec), w1 = __ldg(rec + 1);
+  const int delay = w0.x, dch = w0.y, mode_ms = w0.z, mono = w0.w, use_width = w1.x;
+  const double width = __hiloint2double(w1.w, w1.z);
+  const long long T0 = b.received[sig], x0 = b.offs[sig];
+  const long long T1 = T0 + (b.offs[sig + 1] - x0);
+  double2* __restrict__ o2 = reinterpret_cast<double2*>(out) + o0;
+  const int sh0 = dch == 0 ? delay : 0, sh1 = dch == 1 ? delay : 0;
+  for (long long j = j0 + threadIdx.x; j < j1; j += NT) {
+    const long long q0 = T0 + j - sh0, q1 = T0 + j - sh1;
+    const bool v0 = q0 >= 0 && q0 < T1, v1 = q1 >= 0 && q1 < T1;
+    const float2 s0 = block_step_frame(b, sig, q0, T0, T1, x0);
+    const float2 s1 = block_step_frame(b, sig, q1, T0, T1, x0);
+    o2[j] = haas_frame(s0.x, s0.y, v0, s1.x, s1.y, v1, mode_ms, mono, use_width, width);
+  }
+}
+
+int haas_block_step_launch(BlockStepParams b, long long out_rows, const vnd_haas_clip* clips, double* out, cudaStream_t st) {
+  long long blocks = 0;
+  VND_REQUIRE(block_step_grid(&b, out_rows, kHaasTile, &blocks), VND_EUNSUPPORTED, "grid too large (%lld CTAs)", blocks);
+  haas_block_step_kernel<<<(unsigned)blocks, 256, 0, st>>>(b, clips, out);
+  return after_launch("haas_block_step_kernel");
+}
+
+// ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
 size_t vn_batch_workspace_bytes(long long rows, int n_clips, int rms) {

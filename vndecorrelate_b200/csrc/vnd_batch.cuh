@@ -136,4 +136,56 @@ constexpr int kHaasTile = 4096;
 int haas_batch_launch(const float* x, const long long* offs, int n_clips, const vnd_haas_clip* clips, const long long* out_offs,
                       long long out_rows, double* out, cudaStream_t st);
 
+// ------------------------------------------------------------------------------------------------
+// One step of many live signals (vnd_vn_block_step_dev, vnd_haas_block_step_dev).  Signal i has received
+// received[i] = T0 frames before the step and gets rows [offs[i], offs[i + 1]) of the packed (rows, 2) blocks, so it
+// has T1 = T0 + those rows after it.  Its history holds its frames [T0 - H, T0) as rows [i H, i H + H) of hist_in;
+// the step writes frames [T1 - H, T1) to hist_out (frames before 0 as +0).  Together they are the signal's virtual
+// input: a frame before T0 - H, before 0 or from T1 on reads as +0.  The first out_blocks CTAs write the outputs, one
+// (signal, output tile) pair each through batch_clip_of over out_offs; the n * hchunks CTAs after them write the history.
+// ------------------------------------------------------------------------------------------------
+struct BlockStepParams {
+  const float* x;               // packed (rows, 2) blocks
+  const long long* offs;        // n + 1
+  const long long* received;    // n
+  const long long* emitted;     // n, output frames written before the step (the velvet-noise step only)
+  const long long* out_offs;    // n + 1: signal i writes out rows [out_offs[i], out_offs[i + 1])
+  const float* hist_in;         // (n, H, 2)
+  float* hist_out;              // (n, H, 2)
+  long long out_blocks;
+  int n, H, hchunks;
+};
+
+// History frames per CTA of the history pass.
+constexpr int kHistTile = 4096;
+
+// Frame f of signal `sig`'s virtual input, (+0, +0) where it has no frame.
+__device__ __forceinline__ float2 block_step_frame(const BlockStepParams& b, int sig, long long f, long long T0, long long T1, long long x0) {
+  if (f >= T0) return f < T1 ? __ldg(reinterpret_cast<const float2*>(b.x) + x0 + (f - T0)) : make_float2(0.0f, 0.0f);
+  if (f < 0 || f < T0 - b.H) return make_float2(0.0f, 0.0f);
+  return __ldg(reinterpret_cast<const float2*>(b.hist_in) + (long long)sig * b.H + (f - (T0 - b.H)));
+}
+
+// History CTA j: chunk j % hchunks of signal j / hchunks's new history.
+__device__ __forceinline__ void block_step_history(const BlockStepParams& b, long long j) {
+  const int sig = (int)(j / b.hchunks);
+  const int lo = (int)(j % b.hchunks) * kHistTile;
+  const int hi = lo + kHistTile < b.H ? lo + kHistTile : b.H;
+  const long long T0 = b.received[sig], x0 = b.offs[sig];
+  const long long T1 = T0 + (b.offs[sig + 1] - x0);
+  float2* __restrict__ h2 = reinterpret_cast<float2*>(b.hist_out) + (long long)sig * b.H;
+  for (int i = lo + (int)threadIdx.x; i < hi; i += (int)blockDim.x) h2[i] = block_step_frame(b, sig, T1 - b.H + i, T0, T1, x0);
+}
+
+// Grid of a block step: output CTAs (tile outputs each) then history CTAs; false when it exceeds the grid limit.
+bool block_step_grid(BlockStepParams* b, long long out_rows, int tile, long long* blocks);
+
+// vnd_fir.cu: the velvet-noise step (vn_block_step_kernel); float32 (out_rows, 2) out.  VND_EUNSUPPORTED (no error
+// text) when tile + halo does not fit (the vn_batch_smem rule).
+int vn_block_step_launch(BlockStepParams b, long long out_rows, const int* prog_of, const vnd_tap_program* taps, const vnd_epilogue* ep,
+                         float* out, cudaStream_t st);
+// vnd_batch.cu: the Haas step (haas_block_step_kernel); float64 (out_rows, 2) out, signal i's first row is its output
+// frame T0.
+int haas_block_step_launch(BlockStepParams b, long long out_rows, const vnd_haas_clip* clips, double* out, cudaStream_t st);
+
 }  // namespace vnd

@@ -459,6 +459,71 @@ __global__ void __launch_bounds__(256) vn_batch_stereo_kernel(const BatchStereoP
 }
 
 // ------------------------------------------------------------------------------------------------
+// One velvet-noise step of many live signals (vnd_vn_block_step_dev): vn_batch_stereo_kernel's work on each signal's
+// ready frames [E0, E0 + count), E0 = emitted[sig].  The CTA stages its tile plus the halo of the signal's virtual
+// input (history, then block, then +0: block_step_frame), so every output frame reads exactly the samples the one-shot
+// call reads, and +0 where the one-shot call drops a tap past the end.  Same tap loop and epilogue, float32 out.
+// ------------------------------------------------------------------------------------------------
+template <int R>
+__global__ void __launch_bounds__(256) vn_block_step_kernel(const StereoParams p, const BlockStepParams b, const int* prog_of) {
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  constexpr int NT = 256;
+  constexpr int kSub = 32 * R;
+  if (blockIdx.x >= b.out_blocks) {
+    block_step_history(b, (long long)blockIdx.x - b.out_blocks);
+    return;
+  }
+  const int span_al = (p.tile + p.halo + 3) & ~3;
+  float* s0 = reinterpret_cast<float*>(smem_raw);
+  float* s1 = s0 + span_al;
+  int* prog0 = reinterpret_cast<int*>(s1 + span_al);
+
+  const int sig = batch_clip_of(b.out_offs, b.n, p.tile, blockIdx.x);
+  const long long o0 = b.out_offs[sig];
+  const long long cnt = b.out_offs[sig + 1] - o0;
+  const long long k = (long long)blockIdx.x - (o0 / p.tile + sig);
+  if (k < 0 || k * p.tile >= cnt) return;
+  const int nout = (int)(cnt - k * p.tile < p.tile ? cnt - k * p.tile : p.tile);
+  const int pr = prog_of[sig];
+  const int w0 = p.offsets[2 * pr];
+  const int n0 = p.offsets[2 * pr + 1] - w0;
+  const int n1 = p.offsets[2 * pr + 2] - w0 - n0;
+  int* prog1 = prog0 + n0;
+
+  const int tid = threadIdx.x;
+  const long long T0 = b.received[sig], x0 = b.offs[sig];
+  const long long T1 = T0 + (b.offs[sig + 1] - x0);
+  const long long t0 = b.emitted[sig] + k * p.tile;  // first output frame of the tile
+  const int nstage = (nout + kSub - 1) / kSub * kSub + p.halo;  // what the warps below read
+  for (int i = tid; i < nstage; i += NT) {
+    const float2 v = block_step_frame(b, sig, t0 + i, T0, T1, x0);
+    s0[i] = v.x;
+    s1[i] = v.y;
+  }
+  for (int i = tid; i < n0 + n1; i += NT) prog0[i] = p.words[w0 + i];
+  __syncthreads();
+
+  float2* __restrict__ out = reinterpret_cast<float2*>(p.out) + o0 + k * p.tile;
+  const int warp = tid >> 5, lane = tid & 31;
+  for (int base = warp * kSub; base < nout; base += NT / 32 * kSub) {
+    float y0[R], y1[R];
+    if (n0 > 0) run_program<float, MODE_SEG, R, 32>(s0 + base + lane, prog0, p.apply_gain, y0);
+    if (n1 > 0) run_program<float, MODE_SEG, R, 32>(s1 + base + lane, prog1, p.apply_gain, y1);
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+      const int i = base + lane + 32 * r;
+      if (i < nout) {
+        const float a = s0[i], c = s1[i];
+        float u = n0 > 0 ? y0[r] : a;  // unfiltered channel: copied through
+        float v = n1 > 0 ? y1[r] : c;
+        stereo_epilogue(a, c, u, v, p, 1.0f, 1.0f);
+        out[i] = make_float2(u, v);
+      }
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------------
 constexpr int kR = 8;
@@ -744,6 +809,30 @@ int vn_batch_stereo_launch(const float* x, long long rows, const long long* offs
     k<<<(unsigned)blocks, 256, smem, st>>>(bp);
   }
   return after_launch("vn_batch_stereo_kernel");
+}
+
+int vn_block_step_launch(BlockStepParams b, long long out_rows, const int* prog_of, const vnd_tap_program* taps, const vnd_epilogue* ep,
+                         float* out, cudaStream_t st) {
+  StereoParams p{};
+  p.out = out;
+  p.words = taps->words;
+  p.offsets = taps->offsets;
+  p.apply_gain = taps->apply_gain;
+  p.ms_encode = ep->ms_encode;
+  p.use_width = ep->use_width;
+  p.w_mid = (float)(1.0 - (double)ep->width);
+  p.w_side = (float)ep->width;
+  p.halo = ((taps->halo > 0 ? taps->halo : 0) + 3) & ~3;
+  p.tile = kBatchTile;
+  size_t smem = 0;
+  if (!vn_batch_smem(p.halo, 2 * taps->max_channel_words, &smem)) return VND_EUNSUPPORTED;
+  long long blocks = 0;
+  VND_REQUIRE(block_step_grid(&b, out_rows, kBatchTile, &blocks), VND_EUNSUPPORTED, "grid too large (%lld CTAs)", blocks);
+  constexpr int R = 4;
+  auto k = vn_block_step_kernel<R>;
+  VND_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k<<<(unsigned)blocks, 256, smem, st>>>(p, b, prog_of);
+  return after_launch("vn_block_step_kernel");
 }
 
 }  // namespace vnd

@@ -34,7 +34,7 @@ from .taps import (
 )
 from .utils.dsp import LayoutMode, apply_stereo_width, check_equal_length, rms_normalize, to_float32
 
-__all__ = ["Decorrelator", "SignalChain", "HaasEffect", "VelvetNoise", "decorrelate_batch", "haas_effect_batch", "generate_velvet_noise",
+__all__ = ["Decorrelator", "SignalChain", "HaasEffect", "VelvetNoise", "BlockDecorrelator", "decorrelate_batch", "haas_effect_batch", "generate_velvet_noise",
            "convolve_velvet_noise"]
 
 
@@ -891,6 +891,313 @@ def haas_effect_batch(input_signals, haas_effect):
                                         out.ctypes.data if out_rows else None), "vnd_haas_batch_host")
         results = out.reshape(n, -1, 2) if is_array else [out[o:o + L + d] for o, L, d in zip(out_offsets, lengths, delays)]
     return results
+
+
+# ------------------------------------------------------------------------------------------------
+# live signals, block by block
+# ------------------------------------------------------------------------------------------------
+
+
+class BlockStepPlan:
+    """What one step of live signals does (``plan_block_step``), per signal: ``total`` frames received after the step,
+    ``ready`` frames emitted after it, ``out_offsets`` (n + 1) of the step's outputs - signal ``i`` emits its frames
+    ``[emitted[i], ready[i])`` -, ``history_start``, the first frame of the history the step leaves (``total - H``), and
+    the ``(received, emitted)`` state the next step starts from: zero for a signal whose step was final."""
+
+    __slots__ = ("total", "ready", "out_offsets", "history_start", "next_received", "next_emitted")
+
+    def __init__(self, total, ready, out_offsets, history_start, next_received, next_emitted):
+        self.total, self.ready, self.out_offsets = total, ready, out_offsets
+        self.history_start, self.next_received, self.next_emitted = history_start, next_received, next_emitted
+
+
+def plan_block_step(received, emitted, lengths, final, latency, tail, history: int) -> BlockStepPlan:
+    """The step planner of ``BlockDecorrelator``, vectorised over signals (int64 arrays, ``final`` bool).  A signal that
+    has received ``T`` frames has emitted ``max(0, T - latency)`` of them after a non-final step, and ``T + tail`` after
+    its final step; ``latency`` is the filter's look-ahead ``A`` (0 for the Haas effect alone) and ``tail`` the Haas
+    delay ``d`` (0 for velvet noise alone)."""
+    total = received + lengths
+    ready = np.where(final, total + tail, np.maximum(total - latency, 0))
+    out_offsets = np.zeros(len(total) + 1, dtype=np.int64)
+    np.cumsum(ready - emitted, out=out_offsets[1:])
+    zero = np.zeros_like(total)
+    return BlockStepPlan(total, ready, out_offsets, total - history, np.where(final, zero, total), np.where(final, zero, ready))
+
+
+def _block_stages(d) -> "tuple[VelvetNoise | None, HaasEffect | None]":
+    """The (velvet noise, Haas) stages a live decorrelator runs as, either of them None."""
+    if isinstance(d, VelvetNoise):
+        vn, haas = d, None
+    elif isinstance(d, HaasEffect):
+        vn, haas = None, d
+    elif isinstance(d, SignalChain):
+        d._init_decorrelators()
+        stages = d._decorrelators
+        kinds = tuple(type(st) for st in stages)
+        if kinds == (VelvetNoise,):
+            vn, haas = stages[0], None
+        elif kinds == (HaasEffect,):
+            vn, haas = None, stages[0]
+        elif kinds == (VelvetNoise, HaasEffect):
+            vn, haas = stages
+        else:
+            names = ", ".join(getattr(st, "__name__", type(st).__name__) for st in stages) or "no stages"
+            raise NotImplementedError(f"BlockDecorrelator runs a SignalChain of [VelvetNoise], [HaasEffect] or [VelvetNoise, HaasEffect]; "
+                                      f"this chain has {names}")
+    else:
+        raise NotImplementedError(f"BlockDecorrelator takes VelvetNoise, HaasEffect or SignalChain decorrelators, not {type(d).__name__}")
+    if vn is not None and vn.normalizer is not None:
+        raise NotImplementedError("rms_normalize and other normalisers scale by statistics of the whole signal, which a block cannot know; "
+                                  "pass normalizer=None to the VelvetNoise")
+    return vn, haas
+
+
+_STEREO0 = np.empty((0, 2), np.float32)
+
+
+class BlockDecorrelator:
+    """Decorrelates ``n_signals`` live signals that arrive block by block, one launch per step for all of them (two for a
+    velvet-noise + Haas chain).
+
+    ``decorrelator``: one ``VelvetNoise`` with ``normalizer=None``, ``HaasEffect``, or ``SignalChain`` of
+    ``[VelvetNoise]``, ``[HaasEffect]`` or ``[VelvetNoise, HaasEffect]``, shared by all signals, or a sequence with one
+    per signal.  Velvet-noise filters of different signals must share what ``decorrelate_batch`` needs them to share
+    (``ValueError`` otherwise); Haas settings are each signal's own.
+
+    ``process(blocks, final=False)`` takes one block per signal - a numpy array or CUDA tensor, ``(frames, 2)`` or mono
+    ``(frames,)``, any dtype ``to_float32`` accepts, or None / empty for a signal that received nothing - and returns one
+    output per signal.  Concatenating signal ``i``'s outputs up to and including its final step gives the bytes (dtype,
+    shape and values) of ``decorrelator_i(np.concatenate(its blocks))``, however the input was cut.  After its final step
+    a signal starts over.
+
+    Latency: with ``A_i = latency_frames[i]`` (the filter's largest tap index; 0 for the Haas effect alone), ``d_i`` the
+    Haas delay and ``T_i`` the frames received, a signal has emitted ``max(0, T_i - A_i)`` frames after a non-final step
+    (``T_i`` for the Haas effect alone), and ``T_i`` (velvet noise) or ``T_i + d_i`` (Haas, chain) after its final step.
+    Outputs are float32 for velvet noise and float64 with a Haas stage, as the one-shot call returns them.  Numpy blocks
+    give numpy outputs (views of one page-locked block); CUDA tensors give CUDA tensors, on torch's current stream.
+    Every error is raised before any device work and names the signal."""
+
+    def __init__(self, decorrelator, n_signals: int = 1, device=None):
+        n = int(n_signals)
+        if n < 1:
+            raise ValueError(f"n_signals must be at least 1, got {n_signals}")
+        shared = isinstance(decorrelator, (Decorrelator, SignalChain)) or not hasattr(decorrelator, "__iter__")  # else one per signal
+        decs = [decorrelator] * n if shared else list(decorrelator)
+        if len(decs) != n:
+            raise ValueError(f"{len(decs)} decorrelators for {n} signals: pass one decorrelator, or one per signal")
+        stages: dict[int, tuple] = {}
+        for d in ([decorrelator] if shared else decs):
+            if id(d) not in stages:
+                stages[id(d)] = _block_stages(d)
+        pairs = [stages[id(d)] for d in decs]
+        kind = (pairs[0][0] is not None, pairs[0][1] is not None)
+        for i, (vn, haas) in enumerate(pairs):
+            if (vn is not None, haas is not None) != kind:
+                raise ValueError(f"signal {i}: every signal needs the same stages (velvet noise, Haas effect or both)")
+        self.n_signals = n
+        self.device = device
+        self._vn_stage, self._haas_stage = kind
+        self.latency_frames = np.zeros(n, dtype=np.int64)
+        self._H_vn = self._H_haas = 0
+        if self._vn_stage:
+            settings = None
+            for i, (vn, _) in enumerate(pairs):
+                cur = _batch_settings(vn, None)
+                if settings is None:
+                    settings = cur
+                for key, value in cur.items():
+                    if value != settings[key]:
+                        raise ValueError(f"signal {i}: BlockDecorrelator needs one {key} for every signal, got {settings[key]!r} and {value!r}")
+            if settings["num_outs"] != 2:
+                raise ValueError(f"BlockDecorrelator decorrelates stereo signals: num_outs must be 2, got {settings['num_outs']}")
+            vns = [vn for vn, _ in pairs]
+            progs, self._prog_of = _batch_programs(vns, np.full(n, np.iinfo(np.int64).max))
+            self._program = _batch_program(progs)
+            self.latency_frames = np.array([max(p.halo - 1, 0) for p in progs], dtype=np.int64)[self._prog_of]
+            self._H_vn = int(self.latency_frames.max())
+            vn0 = vns[0]
+            self._ep = N.EpilogueStruct(int(settings["mode"] == "MS"), int(vn0.width is not None), float(vn0.width) if vn0.width is not None else 0.0,
+                                        0, 0, 0)
+            ps = self._program.host_struct()
+            rc = N.lib().vnd_vn_block_step_dev(None, 0, None, 0, None, None, None, C.byref(ps), C.byref(self._ep), None, None, self._H_vn, None, 0,
+                                               None, None)  # no signals: checks the filter, launches nothing
+            if rc == N.VND_EUNSUPPORTED:
+                raise NotImplementedError(f"a filter reading {self._H_vn} frames ahead does not fit the block-step kernel's shared memory; "
+                                          "decorrelate such signals whole")
+            N.check(rc, "vnd_vn_block_step_dev")
+        self._tail = np.zeros(n, dtype=np.int64)
+        if self._haas_stage:
+            haases = [h for _, h in pairs]
+            self._table = _haas_table(haases, [_STEREO0] * n, shared)
+            self._tail = self._table["delay"].astype(np.int64)
+            self._H_haas = int(self._tail.max())
+        self._received = np.zeros(n, dtype=np.int64)
+        self._emitted = np.zeros(n, dtype=np.int64)
+        self._mono = np.full(n, -1, dtype=np.int8)  # -1: not known yet (no frame since the signal started)
+        self._dev = None  # device state, made at the first launch
+
+    # ---- host side ------------------------------------------------------------------------------
+    def _blocks(self, blocks, final):
+        """``(torch_in, clips, lengths, final, mono)`` of one step, every check done; no device work."""
+        n = self.n_signals
+        blocks = list(blocks)
+        if len(blocks) != n:
+            raise ValueError(f"{len(blocks)} blocks for {n} signals: pass one block (or None) per signal")
+        if isinstance(final, (bool, np.bool_)):
+            fin = np.full(n, bool(final))
+        else:
+            fin = np.array([bool(f) for f in final], dtype=bool)
+            if fin.size != n:
+                raise ValueError(f"{fin.size} final flags for {n} signals: pass one bool, or one per signal")
+        is_t = [R.is_torch_tensor(b) for b in blocks]
+        given = [i for i, b in enumerate(blocks) if b is not None]
+        torch_in = bool(given) and is_t[given[0]]
+        for i in given:
+            if is_t[i] != torch_in:
+                raise ValueError(f"signal {i}: the blocks of one step must be all numpy arrays or all CUDA tensors")
+        if torch_in:
+            for i in given:
+                if not blocks[i].is_cuda:
+                    raise N.VndError(N.VND_EUNSUPPORTED, "BlockDecorrelator",
+                                     f"signal {i}: CPU torch tensors are not supported (no CPU fallback); pass CUDA tensors or numpy arrays")
+            device = self.device if self.device is not None else blocks[given[0]].device
+            import torch
+
+            device = torch.device(device)
+            for i in given:
+                if blocks[i].device != device:
+                    raise ValueError(f"signal {i}: the block is on {blocks[i].device}, this BlockDecorrelator on {device}")
+        clips = [_STEREO0 if b is None else to_float32(b if t else np.asarray(b)) for b, t in zip(blocks, is_t)]
+        for i in given:
+            x = clips[i]
+            if x.ndim not in (1, 2) or (x.ndim == 2 and x.shape[1] != 2):
+                raise ValueError(f"signal {i}: a block must be (frames, 2) or mono (frames,), got shape {tuple(x.shape)}")
+        lengths = np.fromiter((x.shape[0] for x in clips), dtype=np.int64, count=n)
+        mono = np.fromiter((x.ndim == 1 for x in clips), dtype=np.int8, count=n)
+        clash = (lengths > 0) & (self._mono >= 0) & (mono != self._mono)
+        if clash.any():
+            i = int(np.flatnonzero(clash)[0])
+            was = "mono" if self._mono[i] else "stereo"
+            raise ValueError(f"signal {i}: a {'mono' if mono[i] else 'stereo'} block for a {was} signal; a signal keeps its layout until its final step")
+        mono = np.where(lengths > 0, mono, self._mono)
+        return torch_in, clips, lengths, fin, mono
+
+    def _device_state(self, device):
+        import torch
+
+        if self._dev is None:
+            self.device = device
+            n = self.n_signals
+            st = {"vn": None, "haas": None}
+            if self._vn_stage:
+                st["vn"] = [torch.zeros((n, self._H_vn, 2), dtype=torch.float32, device=device) for _ in range(2)]
+                st["program"] = R.device_program(self._program, device)
+                st["prog_of"] = torch.from_numpy(self._prog_of).to(device)
+            if self._haas_stage:
+                st["haas"] = [torch.zeros((n, self._H_haas, 2), dtype=torch.float32, device=device) for _ in range(2)]
+                st["table"] = None
+                st["mono"] = None
+            self._dev = st
+        return self._dev
+
+    # ---- one step -------------------------------------------------------------------------------
+    def process(self, blocks, final=False):
+        """One step: ``blocks`` has one block (or None) per signal, ``final`` is a bool or one bool per signal.  Returns
+        each signal's output frames that became ready in this step (see the class documentation)."""
+        torch_in, clips, lengths, fin, mono = self._blocks(blocks, final)
+        import torch
+
+        if torch_in:
+            device = next(x.device for x in clips if R.is_torch_tensor(x))
+        else:
+            device = torch.device(self.device if self.device is not None else f"cuda:{torch.cuda.current_device()}")
+        n = self.n_signals
+        offsets = np.zeros(n + 1, dtype=np.int64)
+        np.cumsum(lengths, out=offsets[1:])
+        plan = plan_block_step(self._received, self._emitted, lengths, fin, self.latency_frames, self._tail,
+                               self._H_vn if self._vn_stage else self._H_haas)
+        # a chain's Haas stage reads the velvet-noise output: its block is what the velvet-noise stage emits in this step
+        vn_oo = plan_block_step(self._received, self._emitted, lengths, fin, self.latency_frames, 0, 0).out_offsets if self._vn_stage else None
+        rows, out_rows = int(offsets[-1]), int(plan.out_offsets[-1])
+        vn_rows = int(vn_oo[-1]) if self._vn_stage else 0
+        launch_vn = self._vn_stage and rows + vn_rows > 0
+        haas_rows = vn_rows if self._vn_stage else rows
+        launch_haas = self._haas_stage and haas_rows + out_rows > 0
+        out_dtype = torch.float64 if self._haas_stage else torch.float32
+
+        with torch.cuda.device(device):
+            stream = torch.cuda.current_stream(device)
+            out = torch.empty((0, 2), dtype=out_dtype, device=device)
+            if launch_vn or launch_haas:
+                st = self._device_state(device)
+                tables = [offsets, self._received, self._emitted, plan.out_offsets] + ([vn_oo] if self._vn_stage else [])
+                meta = torch.from_numpy(np.concatenate(tables)).to(device)
+                m = meta.data_ptr()
+                d_offs, d_recv, d_emit, d_oo, d_vn_oo = (m + 8 * k for k in (0, n + 1, 2 * n + 1, 3 * n + 1, 4 * n + 2))
+                keep, x_ptr = self._pack(clips, offsets, rows, torch_in, device)
+                lib = N.lib()
+                y = None
+                if launch_vn:
+                    y = torch.empty((vn_rows, 2), dtype=torch.float32, device=device)
+                    h_in, h_out = st["vn"]
+                    N.check(lib.vnd_vn_block_step_dev(x_ptr, rows, d_offs, n, d_recv, d_emit, st["prog_of"].data_ptr(), C.byref(st["program"]),
+                                                      C.byref(self._ep), h_in.data_ptr(), h_out.data_ptr(), self._H_vn, d_vn_oo, vn_rows,
+                                                      y.data_ptr() if vn_rows else None, stream.cuda_stream), "vnd_vn_block_step_dev")
+                    st["vn"] = [h_out, h_in]
+                    out = y
+                if launch_haas:
+                    h_mono = np.zeros(n, np.int32) if self._vn_stage else np.maximum(mono, 0).astype(np.int32)
+                    if st["mono"] is None or not np.array_equal(st["mono"], h_mono):  # the records change only with a layout
+                        table = self._table.copy()
+                        table["mono"] = h_mono
+                        st["table"], st["mono"] = torch.from_numpy(table.view(np.uint8)).to(device), h_mono
+                    if self._vn_stage:
+                        hx, h_offs, h_recv = (y.data_ptr() if vn_rows else None), d_vn_oo, d_emit
+                    else:
+                        hx, h_offs, h_recv = x_ptr, d_offs, d_recv
+                    out = torch.empty((out_rows, 2), dtype=torch.float64, device=device)
+                    h_in, h_out = st["haas"]
+                    N.check(lib.vnd_haas_block_step_dev(hx, haas_rows, h_offs, n, h_recv, st["table"].data_ptr(), h_in.data_ptr(), h_out.data_ptr(),
+                                                        self._H_haas, d_oo, out_rows, out.data_ptr() if out_rows else None, stream.cuda_stream),
+                            "vnd_haas_block_step_dev")
+                    st["haas"] = [h_out, h_in]
+            bounds = zip(plan.out_offsets[:-1].tolist(), plan.out_offsets[1:].tolist())
+            if torch_in:
+                results = [out[a:b] for a, b in bounds]
+            else:
+                host = R.pinned_empty((out_rows, 2), np.float64 if self._haas_stage else np.float32)
+                if out_rows:
+                    torch.from_numpy(host).copy_(out, non_blocking=True)
+                if launch_vn or launch_haas:
+                    stream.synchronize()  # the output is read, and the page-locked input may be reused, from here on
+                results = [host[a:b] for a, b in bounds]
+        self._received, self._emitted = plan.next_received, plan.next_emitted
+        self._mono = np.where(fin, -1, mono).astype(np.int8)
+        return results
+
+    @staticmethod
+    def _pack(clips, offsets, rows: int, torch_in: bool, device):
+        """``(keep, address)`` of the step's blocks as one float32 (rows, 2) buffer on the device (a mono block in both
+        columns); ``keep`` holds what the address points into.  CUDA blocks that already are consecutive rows of one
+        buffer are read in place."""
+        import torch
+
+        if not rows:
+            return None, None
+        if torch_in:
+            empty = torch.empty((0, 2), dtype=torch.float32, device=device)
+            ts = [x if R.is_torch_tensor(x) else empty for x in clips]
+            base = _packed_base(ts, offsets, True)
+            if base is not None:
+                return ts, base
+            xp = _pack_tensors(ts, rows, device)
+            if xp.data_ptr() % 8:  # the kernels load one float32 pair per row
+                xp = xp.clone()
+            return xp, xp.data_ptr()
+        xh = R.pinned_empty((rows, 2), np.float32)  # page-locked: uploaded by DMA
+        _pack_clips(xh, clips, offsets)
+        xp = torch.from_numpy(xh).to(device, non_blocking=True)
+        return (xh, xp), xp.data_ptr()
 
 
 # ------------------------------------------------------------------------------------------------
