@@ -225,6 +225,28 @@ int vnd_haas_block_step_dev(const float* x, int64_t rows, const int64_t* frame_o
                             const vnd_haas_clip* signals, const float* history_in, float* history_out, int32_t history_frames,
                             const int64_t* out_offsets, int64_t out_rows, double* out, void* stream);
 
+/* One VelvetNoise.convolve step of many live multichannel signals: ONE launch for all signals and channels (none when
+ * rows == 0 and out_rows == 0).  The step model is vnd_vn_block_step_dev's, with `channels` = C values per row:
+ *   x              : packed (rows, C) C-order blocks of `dtype` (VND_F32, or VND_F64 for the float64 arithmetic convolve uses
+ *                    on float64 and 32-bit integer input), aligned to the value size;
+ *   frame_offsets, received, emitted, out_offsets : as vnd_vn_block_step_dev (n_signals + 1, n, n, n + 1 int64);
+ *   taps           : a SEGMENTED program with C channels per filter, filter k = channels [k C, (k + 1) C), each packed for an
+ *                    unbounded length (all taps kept); program_of_signal[i] (int32) is signal i's filter;
+ *   history_in/out : two (n_signals, history_frames, C) C-order buffers of `dtype`, history_frames >= taps->halo - 1, with
+ *                    vnd_vn_block_step_dev's roles (the caller swaps them after every step that launched);
+ *   out            : float32 (out_rows, C) C-order, 4-byte aligned; signal i writes its output frames [E0, E0 + out_offsets[i
+ *                    + 1] - out_offsets[i]), E0 = emitted[i], to rows [out_offsets[i], out_offsets[i + 1]).
+ * Bit contract: output frame t is byte-identical to frame t of vnd_sparse_fir_dev on the signal's first T frames (same
+ * dtype), for any T > t with t + taps->halo - 1 < T1 or T = T1.  A tap the one-shot call drops reads +0 here, which in
+ * SEGMENTED order cannot change the bits (vnd_fir.cu states why).  Filters of any halo are served: those whose halo does
+ * not fit shared memory read their taps from global memory.  Checked before any launch: null or misaligned pointers, one
+ * buffer passed as both histories, history_frames < taps->halo - 1, taps->channels not a multiple of channels, a dtype
+ * other than VND_F32 / VND_F64, a non-SEGMENTED program, n_signals == 0 with rows. */
+int vnd_fir_block_step_dev(const void* x, int32_t dtype, int64_t rows, int32_t channels, const int64_t* frame_offsets, int32_t n_signals,
+                           const int64_t* received, const int64_t* emitted, const int32_t* program_of_signal, const vnd_tap_program* taps,
+                           const void* history_in, void* history_out, int32_t history_frames, const int64_t* out_offsets, int64_t out_rows,
+                           float* out, void* stream);
+
 /* In-place stereo helpers on a (frames, 2) signal, F32 or F64 (utils/dsp.py:21-63, :124-167).
  * op: 0 LR_to_MS, 1 MS_to_LR, 2 apply_stereo_width(width), 3 encode_signal_to_side_channel(x, y)
  * (x = `dry`, y = `a`), 4 rms_normalize(dry, a) DUAL_MONO.  Op 4 sums each signal in the order numpy uses for its

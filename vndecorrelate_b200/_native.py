@@ -94,6 +94,8 @@ SIGNATURES = {
                                         _P(EpilogueStruct), C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "vnd_haas_block_step_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                           C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
+    "vnd_fir_block_step_dev": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         _P(TapProgramStruct), C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "vnd_stereo_op_dev": (C.c_int, [_P(SignalStruct), _P(SignalStruct), C.c_int32, C.c_double, C.c_void_p, C.c_size_t, C.c_void_p]),
     "vnd_dsp_workspace": (C.c_int, [C.c_int64, _P(C.c_size_t)]),
     "vnd_rms_normalize_dev": (C.c_int, [_P(SignalStruct), C.c_int32, _P(SignalStruct), C.c_int32, C.c_int32, C.c_double, C.c_void_p, C.c_size_t, C.c_void_p]),

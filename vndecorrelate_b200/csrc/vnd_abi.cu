@@ -307,25 +307,26 @@ extern "C" int vnd_haas_batch_dev(const float* x, int64_t rows, const int64_t* f
                            out_rows, out, (cudaStream_t)stream);
 }
 
-// Arguments of a block step that can be checked without reading device memory; fills the step's tables.
-static int check_block_step(const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_signals, const int64_t* received,
-                            const float* history_in, float* history_out, int32_t history_frames, const int64_t* out_offsets,
-                            int64_t out_rows, const void* out, BlockStepParams* b) {
+// Arguments of a block step that can be checked without reading device memory; fills the step's tables.  x and the
+// history buffers hold `align`-byte values (a float32 pair per row for the stereo steps).
+static int check_block_step(const void* x, int64_t rows, const int64_t* frame_offsets, int32_t n_signals, const int64_t* received,
+                            const void* history_in, void* history_out, int32_t history_frames, const int64_t* out_offsets,
+                            int64_t out_rows, const void* out, int align, BlockStepParams* b) {
   VND_REQUIRE(rows >= 0 && n_signals >= 0 && out_rows >= 0 && history_frames >= 0, VND_EINVAL,
               "negative extent (rows %lld, n_signals %d, out_rows %lld, history_frames %d)", (long long)rows, n_signals, (long long)out_rows,
               history_frames);
   VND_REQUIRE(n_signals > 0 || rows + out_rows == 0, VND_EINVAL, "%lld rows and %lld out rows but no signals", (long long)rows,
               (long long)out_rows);
   VND_REQUIRE(x != nullptr || rows == 0, VND_EINVAL, "x is null");
-  VND_REQUIRE(reinterpret_cast<uintptr_t>(x) % 8 == 0, VND_EINVAL, "x must be 8-byte aligned (one float32 pair per row)");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(x) % align == 0, VND_EINVAL, "x must be %d-byte aligned", align);
   VND_REQUIRE((frame_offsets != nullptr && received != nullptr && out_offsets != nullptr) || n_signals == 0, VND_EINVAL,
               "frame_offsets, received or out_offsets is null");
   VND_REQUIRE(out != nullptr || out_rows == 0, VND_EINVAL, "out is null");
   const bool hist = history_frames > 0 && n_signals > 0;
   VND_REQUIRE(!hist || (history_in != nullptr && history_out != nullptr), VND_EINVAL, "a history buffer is null");
   VND_REQUIRE(!hist || history_in != history_out, VND_EINVAL, "history_in and history_out must be two buffers");
-  VND_REQUIRE(reinterpret_cast<uintptr_t>(history_in) % 8 == 0 && reinterpret_cast<uintptr_t>(history_out) % 8 == 0, VND_EINVAL,
-              "the history buffers must be 8-byte aligned");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(history_in) % align == 0 && reinterpret_cast<uintptr_t>(history_out) % align == 0, VND_EINVAL,
+              "the history buffers must be %d-byte aligned", align);
   *b = BlockStepParams{};
   b->x = x;
   b->offs = reinterpret_cast<const long long*>(frame_offsets);
@@ -335,6 +336,7 @@ static int check_block_step(const float* x, int64_t rows, const int64_t* frame_o
   b->hist_out = history_out;
   b->n = n_signals;
   b->H = history_frames;
+  b->C = 2;
   return VND_OK;
 }
 
@@ -356,7 +358,7 @@ extern "C" int vnd_vn_block_step_dev(const float* x, int64_t rows, const int64_t
               history_frames, taps->halo - 1);
   BlockStepParams b;
   if ((rc = check_block_step(x, rows, frame_offsets, n_signals, received, history_in, history_out, history_frames, out_offsets, out_rows, out,
-                             &b)))
+                             8, &b)))
     return rc;
   VND_REQUIRE(n_signals == 0 || taps->channels >= 2, VND_EINVAL, "the tap program holds no filter");
   VND_REQUIRE((emitted != nullptr && program_of_signal != nullptr) || n_signals == 0, VND_EINVAL, "emitted or program_of_signal is null");
@@ -372,13 +374,40 @@ extern "C" int vnd_haas_block_step_dev(const float* x, int64_t rows, const int64
   int rc;
   BlockStepParams b;
   if ((rc = check_block_step(x, rows, frame_offsets, n_signals, received, history_in, history_out, history_frames, out_offsets, out_rows, out,
-                             &b)))
+                             8, &b)))
     return rc;
   VND_REQUIRE(signals != nullptr || n_signals == 0, VND_EINVAL, "signals is null");
   VND_REQUIRE(reinterpret_cast<uintptr_t>(signals) % 16 == 0, VND_EINVAL, "signals must be 16-byte aligned");
   VND_REQUIRE(reinterpret_cast<uintptr_t>(out) % 16 == 0, VND_EINVAL, "out must be 16-byte aligned (one float64 pair per row)");
   if (n_signals == 0 || rows + out_rows == 0) return VND_OK;
   return haas_block_step_launch(b, out_rows, signals, out, (cudaStream_t)stream);
+}
+
+extern "C" int vnd_fir_block_step_dev(const void* x, int32_t dtype, int64_t rows, int32_t channels, const int64_t* frame_offsets,
+                                      int32_t n_signals, const int64_t* received, const int64_t* emitted, const int32_t* program_of_signal,
+                                      const vnd_tap_program* taps, const void* history_in, void* history_out, int32_t history_frames,
+                                      const int64_t* out_offsets, int64_t out_rows, float* out, void* stream) {
+  int rc;
+  if ((rc = check_taps(taps))) return rc;
+  VND_REQUIRE(taps->order == VND_ORDER_SEGMENTED, VND_EINVAL, "convolve needs a SEGMENTED tap program");
+  VND_REQUIRE(dtype == VND_F32 || dtype == VND_F64, VND_EINVAL, "unknown dtype %d", dtype);
+  VND_REQUIRE(channels > 0, VND_EINVAL, "channels must be positive, got %d", channels);
+  VND_REQUIRE(taps->channels % channels == 0, VND_EINVAL, "the tap program has %d channels: it must hold %d per filter", taps->channels,
+              channels);
+  VND_REQUIRE(history_frames >= taps->halo - 1, VND_EINVAL, "%d history frames cannot hold the %d frames the filter reads ahead",
+              history_frames, taps->halo - 1);
+  BlockStepParams b;
+  const int elem = dtype == VND_F64 ? 8 : 4;
+  if ((rc = check_block_step(x, rows, frame_offsets, n_signals, received, history_in, history_out, history_frames, out_offsets, out_rows, out,
+                             elem, &b)))
+    return rc;
+  VND_REQUIRE(n_signals == 0 || taps->channels >= channels, VND_EINVAL, "the tap program holds no filter");
+  VND_REQUIRE((emitted != nullptr && program_of_signal != nullptr) || n_signals == 0, VND_EINVAL, "emitted or program_of_signal is null");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(out) % 4 == 0, VND_EINVAL, "out must be 4-byte aligned");
+  if (n_signals == 0 || rows + out_rows == 0) return VND_OK;
+  b.emitted = reinterpret_cast<const long long*>(emitted);
+  b.C = channels;
+  return fir_block_step_launch(b, out_rows, dtype, program_of_signal, taps, out, (cudaStream_t)stream);
 }
 
 extern "C" int vnd_stereo_op_dev(const vnd_signal* a, const vnd_signal* dry, int32_t op, double width, void* workspace,

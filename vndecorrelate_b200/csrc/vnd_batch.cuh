@@ -137,23 +137,26 @@ int haas_batch_launch(const float* x, const long long* offs, int n_clips, const 
                       long long out_rows, double* out, cudaStream_t st);
 
 // ------------------------------------------------------------------------------------------------
-// One step of many live signals (vnd_vn_block_step_dev, vnd_haas_block_step_dev).  Signal i has received
-// received[i] = T0 frames before the step and gets rows [offs[i], offs[i + 1]) of the packed (rows, 2) blocks, so it
-// has T1 = T0 + those rows after it.  Its history holds its frames [T0 - H, T0) as rows [i H, i H + H) of hist_in;
-// the step writes frames [T1 - H, T1) to hist_out (frames before 0 as +0).  Together they are the signal's virtual
-// input: a frame before T0 - H, before 0 or from T1 on reads as +0.  The first out_blocks CTAs write the outputs, one
-// (signal, output tile) pair each through batch_clip_of over out_offs; the n * hchunks CTAs after them write the history.
+// One step of many live signals (vnd_vn_block_step_dev, vnd_haas_block_step_dev, vnd_fir_block_step_dev).  Signal i
+// has received received[i] = T0 frames before the step and gets rows [offs[i], offs[i + 1]) of the packed (rows, C)
+// blocks, so it has T1 = T0 + those rows after it.  Its history holds its frames [T0 - H, T0) as rows [i H, i H + H) of
+// hist_in; the step writes frames [T1 - H, T1) to hist_out (frames before 0 as +0).  Together they are the signal's
+// virtual input: a frame before T0 - H, before 0 or from T1 on reads as +0.  The first out_blocks CTAs write the
+// outputs, one (signal, output tile) pair each (times a channel group for the convolve step) through batch_clip_of over
+// out_offs; the n * hchunks CTAs after them write the history.  The stereo steps are float32 with C = 2; the convolve
+// step's rows hold C values of its compute dtype.
 // ------------------------------------------------------------------------------------------------
 struct BlockStepParams {
-  const float* x;               // packed (rows, 2) blocks
+  const void* x;                // packed (rows, C) blocks
   const long long* offs;        // n + 1
   const long long* received;    // n
-  const long long* emitted;     // n, output frames written before the step (the velvet-noise step only)
+  const long long* emitted;     // n, output frames written before the step (the velvet-noise and convolve steps)
   const long long* out_offs;    // n + 1: signal i writes out rows [out_offs[i], out_offs[i + 1])
-  const float* hist_in;         // (n, H, 2)
-  float* hist_out;              // (n, H, 2)
+  const void* hist_in;          // (n, H, C)
+  void* hist_out;               // (n, H, C)
   long long out_blocks;
   int n, H, hchunks;
+  int C;                        // values per row (the convolve step)
 };
 
 // History frames per CTA of the history pass.
@@ -187,5 +190,9 @@ int vn_block_step_launch(BlockStepParams b, long long out_rows, const int* prog_
 // vnd_batch.cu: the Haas step (haas_block_step_kernel); float64 (out_rows, 2) out, signal i's first row is its output
 // frame T0.
 int haas_block_step_launch(BlockStepParams b, long long out_rows, const vnd_haas_clip* clips, double* out, cudaStream_t st);
+// vnd_fir.cu: the convolve step (fir_block_step_kernel) on (rows, b.C) blocks of `dtype` (VND_F32 or VND_F64); float32
+// (out_rows, b.C) out.  Program k of `taps` is channels [k C, (k + 1) C).
+int fir_block_step_launch(BlockStepParams b, long long out_rows, int dtype, const int* prog_of, const vnd_tap_program* taps, float* out,
+                          cudaStream_t st);
 
 }  // namespace vnd

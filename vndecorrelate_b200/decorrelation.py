@@ -34,7 +34,7 @@ from .taps import (
 )
 from .utils.dsp import LayoutMode, apply_stereo_width, check_equal_length, rms_normalize, to_float32
 
-__all__ = ["Decorrelator", "SignalChain", "HaasEffect", "VelvetNoise", "BlockDecorrelator", "decorrelate_batch", "haas_effect_batch", "generate_velvet_noise",
+__all__ = ["Decorrelator", "SignalChain", "HaasEffect", "VelvetNoise", "BlockDecorrelator", "BlockConvolver", "decorrelate_batch", "haas_effect_batch", "generate_velvet_noise",
            "convolve_velvet_noise"]
 
 
@@ -62,17 +62,34 @@ def _is_mode(mode, which: LayoutMode) -> bool:
     return mode == which  # StrEnum compares equal to plain 'LR' / 'MS' strings (decorrelation.py:217,433)
 
 
-def _fir_compute_array(x: np.ndarray) -> np.ndarray:
-    """The array numpy would effectively feed ``f32_buffer -= x[i:]`` with: float32 stays float32,
+def _fir_compute_dtype(dtype) -> np.dtype:
+    """The dtype numpy would effectively feed ``f32_buffer -= x[i:]`` with: float32 stays float32,
     float64 stays float64, small integers behave like float32 and 32/64-bit integers like float64
     (numpy type promotion with a float32 accumulator)."""
-    if x.dtype in (np.float32, np.float64):
-        return x
-    if x.dtype == np.float16 or (x.dtype.kind in "iub" and x.dtype.itemsize <= 2):
-        return x.astype(np.float32)
-    if x.dtype.kind in "iuf":
-        return x.astype(np.float64)
-    raise TypeError(f"unsupported input dtype {x.dtype}")
+    dtype = np.dtype(dtype)
+    if dtype in (np.float32, np.float64):
+        return dtype
+    if dtype == np.float16 or (dtype.kind in "iub" and dtype.itemsize <= 2):
+        return np.dtype(np.float32)
+    if dtype.kind in "iuf":
+        return np.dtype(np.float64)
+    raise TypeError(f"unsupported input dtype {dtype}")
+
+
+def _fir_compute_array(x: np.ndarray) -> np.ndarray:
+    """``x`` in ``_fir_compute_dtype``: the array itself when it already has that dtype."""
+    dt = _fir_compute_dtype(x.dtype)
+    return x if x.dtype == dt else x.astype(dt)
+
+
+def _fir_tensor_dtype(x):
+    """The torch dtype ``_sparse_fir`` computes a tensor in: float32 and float64 as they are, half precision and
+    integers of up to 2 bytes in float32, anything wider in float64."""
+    import torch
+
+    if x.dtype in (torch.float32, torch.float64):
+        return x.dtype
+    return torch.float32 if (x.dtype == torch.float16 or x.element_size() <= 2) else torch.float64
 
 
 def _sparse_fir(x, program: TapProgram, num_outs: int):
@@ -83,8 +100,7 @@ def _sparse_fir(x, program: TapProgram, num_outs: int):
 
         if not x.is_cuda:
             raise N.VndError(N.VND_EUNSUPPORTED, "sparse FIR", "CPU torch tensors are not supported (no CPU fallback); pass a CUDA tensor or a numpy array")
-        if x.dtype not in (torch.float32, torch.float64):
-            x = x.to(torch.float32 if (x.dtype == torch.float16 or x.element_size() <= 2) else torch.float64)
+        x = x.to(_fir_tensor_dtype(x))
         frames = x.shape[0]
         # planar inputs (a transposed (C, n) tensor) get a planar output, so loads and stores coalesce
         planar = x.dim() == 2 and x.shape[1] > 1 and x.stride(0) == 1
@@ -517,16 +533,21 @@ def _batch_programs(filters: "Sequence[VelvetNoise]", lengths) -> "tuple[list[Ta
 
 
 def _batch_program(progs: "list[TapProgram]") -> TapProgram:
-    """One SEGMENTED program holding the two channels of every distinct filter, pair k = channels 2k, 2k + 1."""
+    """One SEGMENTED program holding the k channels of every distinct filter (k = their common channel count, 2 for the
+    stereo calls): filter j = channels [j k, (j + 1) k)."""
+    k = progs[0].channels
+    if any(p.channels != k for p in progs):
+        raise ValueError(f"the filters of one batch need one channel count, got {sorted({p.channels for p in progs})}")
     words = np.concatenate([p.words for p in progs]).astype(np.int32, copy=False)
     offsets = np.concatenate([[0]] + [p.offsets[1:].astype(np.int64) + base for p, base in
                                       zip(progs, np.cumsum([0] + [p.words.size for p in progs[:-1]]))]).astype(np.int32)
-    return TapProgram(np.ascontiguousarray(words), offsets, 2 * len(progs), N.ORDER_SEGMENTED, progs[0].apply_gain, max(p.halo for p in progs),
+    return TapProgram(np.ascontiguousarray(words), offsets, k * len(progs), N.ORDER_SEGMENTED, progs[0].apply_gain, max(p.halo for p in progs),
                       max(p.max_channel_words for p in progs))
 
 
 def _pack_clips(xp: np.ndarray, clips, offsets: np.ndarray) -> None:
-    """Copy numpy clips into their rows of the packed (rows, 2) array (a mono clip into both columns).  Large batches
+    """Copy numpy clips into their rows of the packed (rows, k) array: the first k columns, cast to its dtype (a mono
+    clip into both columns of a stereo array).  Large batches
     are copied by several threads: numpy releases the GIL for the copies, and one thread does not reach the host's
     memory bandwidth."""
 
@@ -536,7 +557,7 @@ def _pack_clips(xp: np.ndarray, clips, offsets: np.ndarray) -> None:
             xp[a:b, 0] = x
             xp[a:b, 1] = x
         else:
-            xp[a:b] = x[:, :2]
+            xp[a:b] = x[:, :xp.shape[1]]
 
     if xp.nbytes < 64 << 20 or len(clips) < 2:
         for i in range(len(clips)):
@@ -548,13 +569,15 @@ def _pack_clips(xp: np.ndarray, clips, offsets: np.ndarray) -> None:
         list(pool.map(put, range(len(clips))))
 
 
-def _pack_tensors(clips, rows: int, device):
-    """The CUDA clips packed into one (rows, 2) float32 tensor (a mono clip into both columns)."""
+def _pack_tensors(clips, rows: int, device, cols: int = 2, dtype=None):
+    """The CUDA clips packed into one (rows, cols) tensor of ``dtype``, float32 by default: the first ``cols`` columns of
+    each clip (a mono clip into both columns of a stereo tensor)."""
     import torch
 
+    dtype = torch.float32 if dtype is None else dtype
     if not rows:
-        return torch.empty((0, 2), dtype=torch.float32, device=device)
-    return torch.cat([x[:, :2] if x.ndim == 2 else x[:, None].expand(-1, 2) for x in clips])
+        return torch.empty((0, cols), dtype=dtype, device=device)
+    return torch.cat([(x[:, :cols] if x.ndim == 2 else x[:, None].expand(-1, cols)).to(dtype) for x in clips])
 
 
 def _batch_device(input_signals, is_array: bool, where: str):
@@ -898,6 +921,65 @@ def haas_effect_batch(input_signals, haas_effect):
 # ------------------------------------------------------------------------------------------------
 
 
+def _live_step(blocks, final, n: int, device, who: str):
+    """``(blocks, fin, is_t, given, torch_in)`` of one step of ``n`` live signals: one block or None per signal (``given``:
+    the signals with a block), all numpy or all CUDA tensors on ``device`` when it is set, and ``final`` as one bool
+    per signal (``fin``).  Raises, naming the signal, before any device work."""
+    blocks = list(blocks)
+    if len(blocks) != n:
+        raise ValueError(f"{len(blocks)} blocks for {n} signals: pass one block (or None) per signal")
+    if isinstance(final, (bool, np.bool_)):
+        fin = np.full(n, bool(final))
+    else:
+        fin = np.array([bool(f) for f in final], dtype=bool)
+        if fin.size != n:
+            raise ValueError(f"{fin.size} final flags for {n} signals: pass one bool, or one per signal")
+    is_t = [R.is_torch_tensor(b) for b in blocks]
+    given = [i for i, b in enumerate(blocks) if b is not None]
+    torch_in = bool(given) and is_t[given[0]]
+    for i in given:
+        if is_t[i] != torch_in:
+            raise ValueError(f"signal {i}: the blocks of one step must be all numpy arrays or all CUDA tensors")
+    if torch_in:
+        for i in given:
+            if not blocks[i].is_cuda:
+                raise N.VndError(N.VND_EUNSUPPORTED, who,
+                                 f"signal {i}: CPU torch tensors are not supported (no CPU fallback); pass CUDA tensors or numpy arrays")
+        device = device if device is not None else blocks[given[0]].device
+        import torch
+
+        device = torch.device(device)
+        for i in given:
+            if blocks[i].device != device:
+                raise ValueError(f"signal {i}: the block is on {blocks[i].device}, this {who} on {device}")
+    return blocks, fin, is_t, given, torch_in
+
+
+def _live_device(clips, torch_in: bool, device):
+    """The torch device a step runs on: its tensors', else the object's, else torch's current one."""
+    import torch
+
+    if torch_in:
+        return next(x.device for x in clips if R.is_torch_tensor(x))
+    return torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+
+
+def _live_results(out, out_offsets: np.ndarray, torch_in: bool, launched: bool, stream):
+    """Each signal's rows of a step's output ``out``: views of it for tensor input, else views of one page-locked copy,
+    complete when this returns."""
+    import torch
+
+    bounds = zip(out_offsets[:-1].tolist(), out_offsets[1:].tolist())
+    if torch_in:
+        return [out[a:b] for a, b in bounds]
+    host = R.pinned_empty(tuple(out.shape), np.float64 if out.dtype == torch.float64 else np.float32)
+    if out.shape[0]:
+        torch.from_numpy(host).copy_(out, non_blocking=True)
+    if launched:
+        stream.synchronize()  # the output is read, and the page-locked input may be reused, from here on
+    return [host[a:b] for a, b in bounds]
+
+
 class BlockStepPlan:
     """What one step of live signals does (``plan_block_step``), per signal: ``total`` frames received after the step,
     ``ready`` frames emitted after it, ``out_offsets`` (n + 1) of the step's outputs - signal ``i`` emits its frames
@@ -1040,33 +1122,7 @@ class BlockDecorrelator:
     def _blocks(self, blocks, final):
         """``(torch_in, clips, lengths, final, mono)`` of one step, every check done; no device work."""
         n = self.n_signals
-        blocks = list(blocks)
-        if len(blocks) != n:
-            raise ValueError(f"{len(blocks)} blocks for {n} signals: pass one block (or None) per signal")
-        if isinstance(final, (bool, np.bool_)):
-            fin = np.full(n, bool(final))
-        else:
-            fin = np.array([bool(f) for f in final], dtype=bool)
-            if fin.size != n:
-                raise ValueError(f"{fin.size} final flags for {n} signals: pass one bool, or one per signal")
-        is_t = [R.is_torch_tensor(b) for b in blocks]
-        given = [i for i, b in enumerate(blocks) if b is not None]
-        torch_in = bool(given) and is_t[given[0]]
-        for i in given:
-            if is_t[i] != torch_in:
-                raise ValueError(f"signal {i}: the blocks of one step must be all numpy arrays or all CUDA tensors")
-        if torch_in:
-            for i in given:
-                if not blocks[i].is_cuda:
-                    raise N.VndError(N.VND_EUNSUPPORTED, "BlockDecorrelator",
-                                     f"signal {i}: CPU torch tensors are not supported (no CPU fallback); pass CUDA tensors or numpy arrays")
-            device = self.device if self.device is not None else blocks[given[0]].device
-            import torch
-
-            device = torch.device(device)
-            for i in given:
-                if blocks[i].device != device:
-                    raise ValueError(f"signal {i}: the block is on {blocks[i].device}, this BlockDecorrelator on {device}")
+        blocks, fin, is_t, given, torch_in = _live_step(blocks, final, n, self.device, "BlockDecorrelator")
         clips = [_STEREO0 if b is None else to_float32(b if t else np.asarray(b)) for b, t in zip(blocks, is_t)]
         for i in given:
             x = clips[i]
@@ -1107,10 +1163,7 @@ class BlockDecorrelator:
         torch_in, clips, lengths, fin, mono = self._blocks(blocks, final)
         import torch
 
-        if torch_in:
-            device = next(x.device for x in clips if R.is_torch_tensor(x))
-        else:
-            device = torch.device(self.device if self.device is not None else f"cuda:{torch.cuda.current_device()}")
+        device = _live_device(clips, torch_in, self.device)
         n = self.n_signals
         offsets = np.zeros(n + 1, dtype=np.int64)
         np.cumsum(lengths, out=offsets[1:])
@@ -1161,16 +1214,7 @@ class BlockDecorrelator:
                                                         self._H_haas, d_oo, out_rows, out.data_ptr() if out_rows else None, stream.cuda_stream),
                             "vnd_haas_block_step_dev")
                     st["haas"] = [h_out, h_in]
-            bounds = zip(plan.out_offsets[:-1].tolist(), plan.out_offsets[1:].tolist())
-            if torch_in:
-                results = [out[a:b] for a, b in bounds]
-            else:
-                host = R.pinned_empty((out_rows, 2), np.float64 if self._haas_stage else np.float32)
-                if out_rows:
-                    torch.from_numpy(host).copy_(out, non_blocking=True)
-                if launch_vn or launch_haas:
-                    stream.synchronize()  # the output is read, and the page-locked input may be reused, from here on
-                results = [host[a:b] for a, b in bounds]
+            results = _live_results(out, plan.out_offsets, torch_in, launch_vn or launch_haas, stream)
         self._received, self._emitted = plan.next_received, plan.next_emitted
         self._mono = np.where(fin, -1, mono).astype(np.int8)
         return results
@@ -1196,6 +1240,161 @@ class BlockDecorrelator:
             return xp, xp.data_ptr()
         xh = R.pinned_empty((rows, 2), np.float32)  # page-locked: uploaded by DMA
         _pack_clips(xh, clips, offsets)
+        xp = torch.from_numpy(xh).to(device, non_blocking=True)
+        return (xh, xp), xp.data_ptr()
+
+
+class BlockConvolver:
+    """Convolves ``n_signals`` live multichannel signals that arrive block by block with their velvet-noise filters, one
+    launch per step for all signals and channels: the streaming form of ``VelvetNoise.convolve``.
+
+    ``filters``: one ``VelvetNoise`` shared by all signals, or a sequence with one per signal.  They must share
+    ``num_outs`` and whether the envelope is the identity ``(1.0,)`` (``ValueError`` naming the signal otherwise);
+    ``mode``, ``width`` and ``normalizer`` are ignored, as ``convolve`` ignores them.
+
+    ``process(blocks, final=False)`` takes one block per signal - a 2-D numpy array or CUDA tensor ``(frames, >=
+    num_outs)`` of any dtype ``convolve`` accepts, or None for a signal that received nothing - and returns one float32
+    ``(frames, num_outs)`` output per signal.  Concatenating signal ``i``'s outputs up to and including its final step
+    gives the bytes (dtype, shape and values) of ``filters_i.convolve(np.concatenate(its blocks))``, however the input
+    was cut.  After its final step a signal starts over.  Only the first ``num_outs`` columns are read; a signal keeps
+    its column count until its final step, as ``np.concatenate`` requires.
+
+    Latency: with ``A_i = latency_frames[i]`` (the filter's largest tap index) and ``T_i`` the frames received, a signal
+    has emitted ``max(0, T_i - A_i)`` frames after a non-final step and ``T_i`` after its final step.
+
+    Arithmetic: the compute dtype of ``convolve`` - float32 for float32, float16 and integers of up to 2 bytes, float64
+    for float64 and wider integers.  The first non-empty block fixes it for the object, and a block of the other compute
+    dtype raises ``ValueError``: the concatenation of both would run in float64, which the steps already emitted did not.
+    Numpy blocks give numpy outputs (views of one page-locked block); CUDA tensors give CUDA tensors, on torch's current
+    stream.  Every error is raised before any device work and names the signal."""
+
+    def __init__(self, filters, n_signals: int = 1, device=None):
+        n = int(n_signals)
+        if n < 1:
+            raise ValueError(f"n_signals must be at least 1, got {n_signals}")
+        shared = isinstance(filters, VelvetNoise) or not hasattr(filters, "__iter__")
+        if shared and not isinstance(filters, VelvetNoise):
+            raise TypeError(f"BlockConvolver takes a VelvetNoise, or one per signal, not {type(filters).__name__}")
+        vns = [filters] * n if shared else list(filters)
+        if len(vns) != n:
+            raise ValueError(f"{len(vns)} filters for {n} signals: pass one VelvetNoise, or one per signal")
+        for i, vn in enumerate(vns):
+            if not isinstance(vn, VelvetNoise):
+                raise TypeError(f"signal {i}: BlockConvolver takes VelvetNoise filters, not {type(vn).__name__}")
+        settings = [(vn.num_outs, vn.segment_envelope == IDENTITY_ENVELOPE) for vn in (vns[:1] if shared else vns)]
+        for i, cur in enumerate(settings):
+            for key, a, b in zip(("num_outs", "identity segment_envelope"), settings[0], cur):
+                if a != b:
+                    raise ValueError(f"signal {i}: BlockConvolver needs one {key} for every signal, got {a!r} and {b!r}")
+        self.n_signals = n
+        self.device = device
+        self.num_outs = int(settings[0][0])
+        progs, self._prog_of = _batch_programs(vns, np.full(n, np.iinfo(np.int64).max))
+        self._program = _batch_program(progs)
+        self.latency_frames = np.array([max(p.halo - 1, 0) for p in progs], dtype=np.int64)[self._prog_of]
+        self._H = int(self.latency_frames.max())
+        ps = self._program.host_struct()
+        N.check(N.lib().vnd_fir_block_step_dev(None, N.VND_F32, 0, self.num_outs, None, 0, None, None, None, C.byref(ps), None, None, self._H,
+                                               None, 0, None, None), "vnd_fir_block_step_dev")  # no signals: checks the filter only
+        self._received = np.zeros(n, dtype=np.int64)
+        self._emitted = np.zeros(n, dtype=np.int64)
+        self._cols = np.full(n, -1, dtype=np.int64)  # -1: not known yet (no block since the signal started)
+        self._dtype = None  # the compute dtype, numpy's; fixed by the first non-empty block
+        self._dev = None  # device state, made at the first launch
+
+    def _blocks(self, blocks, final):
+        """``(torch_in, blocks, lengths, final, cols, dtype)`` of one step, every check done; no device work."""
+        n, k = self.n_signals, self.num_outs
+        blocks, fin, is_t, given, torch_in = _live_step(blocks, final, n, self.device, "BlockConvolver")
+        if not torch_in:
+            blocks = [None if b is None else np.asarray(b) for b in blocks]
+        cols = self._cols.copy()
+        dtype = self._dtype
+        for i in given:
+            x = blocks[i]
+            if x.ndim != 2:  # convolve's exceptions (decorrelation.py:393-415)
+                raise IndexError(f"signal {i}: too many indices for array: array is {x.ndim}-dimensional, but 2 were indexed")
+            if x.shape[1] < k:
+                raise IndexError(f"signal {i}: index {x.shape[1]} is out of bounds for axis 1 with size {x.shape[1]}")
+            if cols[i] >= 0 and x.shape[1] != cols[i]:
+                raise ValueError(f"signal {i}: a block of {x.shape[1]} columns for a signal of {cols[i]}; a signal keeps its column count "
+                                 "until its final step")
+            cols[i] = x.shape[1]
+            dt = np.dtype(str(_fir_tensor_dtype(x)).replace("torch.", "")) if torch_in else _fir_compute_dtype(x.dtype)
+            if dtype is None and x.shape[0]:
+                dtype = dt
+            if dtype is not None and dt != dtype:
+                raise ValueError(f"signal {i}: a block computed in {dt} for a BlockConvolver computing in {dtype}; convolve the "
+                                 f"concatenation of both in one dtype, or use a BlockConvolver for each")
+        lengths = np.array([0 if b is None else int(b.shape[0]) for b in blocks], dtype=np.int64)
+        return torch_in, blocks, lengths, fin, cols, dtype
+
+    def process(self, blocks, final=False):
+        """One step: ``blocks`` has one block (or None) per signal, ``final`` is a bool or one bool per signal.  Returns
+        each signal's output frames that became ready in this step (see the class documentation)."""
+        torch_in, blocks, lengths, fin, cols, dtype = self._blocks(blocks, final)
+        import torch
+
+        device = _live_device(blocks, torch_in, self.device)
+        n, k = self.n_signals, self.num_outs
+        offsets = np.zeros(n + 1, dtype=np.int64)
+        np.cumsum(lengths, out=offsets[1:])
+        plan = plan_block_step(self._received, self._emitted, lengths, fin, self.latency_frames, 0, self._H)
+        rows, out_rows = int(offsets[-1]), int(plan.out_offsets[-1])
+        launch = rows + out_rows > 0
+        with torch.cuda.device(device):
+            stream = torch.cuda.current_stream(device)
+            out = torch.empty((out_rows, k), dtype=torch.float32, device=device)
+            if launch:
+                st = self._device_state(device, dtype)
+                meta = torch.from_numpy(np.concatenate([offsets, self._received, self._emitted, plan.out_offsets])).to(device)
+                m = meta.data_ptr()
+                keep, x_ptr = self._pack(blocks, offsets, rows, torch_in, device, dtype)
+                h_in, h_out = st["history"]
+                N.check(N.lib().vnd_fir_block_step_dev(x_ptr, N.VND_F64 if dtype == np.float64 else N.VND_F32, rows, k, m, n, m + 8 * (n + 1),
+                                                       m + 8 * (2 * n + 1), st["prog_of"].data_ptr(), C.byref(st["program"]),
+                                                       h_in.data_ptr() if self._H else None, h_out.data_ptr() if self._H else None, self._H,
+                                                       m + 8 * (3 * n + 1), out_rows, out.data_ptr() if out_rows else None, stream.cuda_stream),
+                        "vnd_fir_block_step_dev")
+                st["history"] = [h_out, h_in]
+            results = _live_results(out, plan.out_offsets, torch_in, launch, stream)
+        self._received, self._emitted = plan.next_received, plan.next_emitted
+        self._cols = np.where(fin, -1, cols)
+        self._dtype = dtype
+        return results
+
+    def _device_state(self, device, dtype):
+        import torch
+
+        if self._dev is None:
+            self.device = device
+            tdt = torch.float64 if dtype == np.float64 else torch.float32
+            self._dev = {"history": [torch.zeros((self.n_signals, self._H, self.num_outs), dtype=tdt, device=device) for _ in range(2)],
+                         "program": R.device_program(self._program, device), "prog_of": torch.from_numpy(self._prog_of).to(device)}
+        return self._dev
+
+    def _pack(self, blocks, offsets, rows: int, torch_in: bool, device, dtype):
+        """``(keep, address)`` of the step's blocks as one C-order (rows, num_outs) buffer of the compute dtype on the
+        device; ``keep`` holds what the address points into.  The only non-empty block of a step is read in place when it
+        already is such a buffer."""
+        import torch
+
+        if not rows:
+            return None, None
+        k = self.num_outs
+        full = [b for b in blocks if b is not None and b.shape[0]]
+        one = full[0] if len(full) == 1 else None
+        if torch_in:
+            tdt = torch.float64 if dtype == np.float64 else torch.float32
+            if one is not None and one.dtype == tdt and one.shape[1] == k and one.is_contiguous():
+                return one, one.data_ptr()
+            xp = _pack_tensors(full, rows, device, cols=k, dtype=tdt)
+            return xp, xp.data_ptr()
+        if one is not None and one.dtype == dtype and one.shape[1] == k and one.flags.c_contiguous:
+            xp = torch.from_numpy(one).to(device, non_blocking=True)
+            return xp, xp.data_ptr()
+        xh = R.pinned_empty((rows, k), dtype)  # page-locked: uploaded by DMA
+        _pack_clips(xh, [b if b is not None else np.empty((0, k), dtype) for b in blocks], offsets)
         xp = torch.from_numpy(xh).to(device, non_blocking=True)
         return (xh, xp), xp.data_ptr()
 
