@@ -344,6 +344,47 @@ int vnd_vn_objective_runs_dev(const float* x, int64_t rows, int64_t chan_stride,
                               const int32_t* run_out, int32_t n_runs, double* partials, int64_t n_partial_rows, void* workspace,
                               size_t workspace_bytes, void* stream);
 
+/* Settings of one candidate of vnd_vn_stereo_objective_dev: the epilogue of vnd_vn_decorrelate_dev without normaliser
+ * or Haas stage.  16 bytes. */
+typedef struct vnd_vn_stereo_cand {
+  int32_t ms_encode;  /* 1: M/S side-channel encode (mode 'MS')                                      */
+  int32_t use_width;  /* 1: apply the stereo width                                                   */
+  float w_mid;        /* float32(1 - width), the rounding vnd_vn_decorrelate_dev applies to ep->width */
+  float w_side;       /* float32(width)                                                              */
+} vnd_vn_stereo_cand;
+
+/* The objective of many VelvetNoise candidates with two outputs and no normaliser - any filtered channels, LR or MS,
+ * any width - on one clip, in one objective launch and one combine launch.
+ *   x        : float32 channel-planar clip, element (t, c) = x[c * chan_stride + t], c = 0, 1 (chan_stride >= frames >= 1);
+ *   taps     : SEGMENTED program (device words and offsets) with 2 n_cand channels: candidate j's filter is channels
+ *              2 j (left) and 2 j + 1 (right), each packed for `frames` (vnd_vn_decorrelate_dev's program for that
+ *              candidate; an unfiltered channel has no words and is copied through).  One apply_gain for all;
+ *   cands    : n_cand settings records (device);
+ *   partials : n_cand * 12 float64 on the device, the slots of vnd_vn_objective_batch_dev.
+ * Bit contract: candidate j's 12 partials equal, bit for bit, those of vnd_vn_objective_batch_dev on the float32 output
+ * of vnd_vn_decorrelate_dev for that candidate (planar, with the one-tap identity program; shared-memory kernel).  The
+ * output is never stored: the kernel builds it in registers with the same tap loop and epilogue and feeds the moments
+ * with the same frame-to-lane mapping, tiles and chunks.  Checked before any launch: the program (SEGMENTED, 2 n_cand
+ * channels), the sizes and the pointers.  VND_EUNSUPPORTED (no launch) when the program's halo does not fit shared
+ * memory or VND_OBJ_TMEM selects the tensor-memory objective: the caller then scores candidate by candidate.
+ * Workspace: vnd_vn_stereo_objective_workspace bytes, 256-byte aligned. */
+int vnd_vn_stereo_objective_workspace(int64_t frames, int32_t n_cand, size_t* bytes);
+int vnd_vn_stereo_objective_dev(const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,
+                                int32_t n_cand, double* partials, void* workspace, size_t workspace_bytes, void* stream);
+
+/* The objective of many HaasEffect candidates - any delayed channel, LR or MS, any width - on one clip: one launch, one
+ * CTA per candidate.
+ *   x        : float32 channel-planar clip as above (a mono clip with its samples in both channels and mono = 1 in every
+ *              record);
+ *   cands    : n_cand vnd_haas_clip records (device, 16-byte aligned): delay >= 0, delayed_channel 0 or 1;
+ *   partials : n_cand * 8 float64 on the device, the slots of vnd_haas_objective_batch_dev.
+ * Bit contract: candidate j's 8 partials equal, bit for bit, those of vnd_haas_objective_batch_dev with delays = {0} on
+ * the float64 output of vnd_haas_dev for that candidate: every output frame comes from the same per-frame function and
+ * enters the sums in the same thread and order.  The _dev call checks the sizes and pointers; it cannot read the
+ * device-side records, which must be valid (the _host call checks them). */
+int vnd_haas_effect_objective_dev(const float* x, int64_t frames, int64_t chan_stride, const vnd_haas_clip* cands, int32_t n_cand,
+                                  double* partials, void* stream);
+
 /* ------------------------------------------------------------------------------ host API */
 typedef struct vnd_ctx vnd_ctx;
 
@@ -399,6 +440,14 @@ int vnd_haas_objective_batch_host(vnd_ctx* ctx, const void* clips, int32_t clip_
  * an empty clip (an empty signal has no objective: optimization.py:41-43).  Then one upload, one launch, one download. */
 int vnd_haas_objective_pairs_host(vnd_ctx* ctx, const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets,
                                   int32_t n_clips, const int32_t* pair_clip, const int32_t* pair_delay, int32_t n_pairs, double* partials);
+
+/* vnd_vn_stereo_objective_dev and vnd_haas_effect_objective_dev with host buffers (x, program, records and partials):
+ * the same checks before any copy - for the Haas records also every delay >= 0 and every delayed_channel 0 or 1 -,
+ * then one upload, one launch of each kernel, one download. */
+int vnd_vn_stereo_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps,
+                                 const vnd_vn_stereo_cand* cands, int32_t n_cand, double* partials);
+int vnd_haas_effect_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, int64_t chan_stride, const vnd_haas_clip* cands, int32_t n_cand,
+                                   double* partials);
 
 /* vnd_vn_objective_runs_dev with host buffers (x, program, tables and partials): the same checks before any copy, then
  * one upload, one launch of each kernel, one download.  Rows no run names come back as zeros. */

@@ -72,6 +72,10 @@ HAAS_CLIP_DTYPE = np.dtype([("delay", "<i4"), ("delayed_channel", "<i4"), ("mode
                             ("reserved", "<i4"), ("width", "<f8")])
 assert HAAS_CLIP_DTYPE.itemsize == 32
 
+# vnd_vn_stereo_cand, one record per candidate of vnd_vn_stereo_objective_dev (16 bytes)
+VN_STEREO_CAND_DTYPE = np.dtype([("ms_encode", "<i4"), ("use_width", "<i4"), ("w_mid", "<f4"), ("w_side", "<f4")])
+assert VN_STEREO_CAND_DTYPE.itemsize == 16
+
 
 # name -> (restype, argtypes); every symbol include/vnd_b200.h declares
 _P = C.POINTER
@@ -114,6 +118,10 @@ SIGNATURES = {
     "vnd_vn_objective_runs_workspace": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, _P(C.c_size_t)]),
     "vnd_vn_objective_runs_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, _P(TapProgramStruct), C.c_void_p, C.c_void_p,
                                             C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "vnd_vn_stereo_objective_workspace": (C.c_int, [C.c_int64, C.c_int32, _P(C.c_size_t)]),
+    "vnd_vn_stereo_objective_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, _P(TapProgramStruct), C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                              C.c_size_t, C.c_void_p]),
+    "vnd_haas_effect_objective_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "vnd_ctx_create": (C.c_int, [C.c_int, _P(C.c_void_p)]),
     "vnd_ctx_destroy": (C.c_int, [C.c_void_p]),
     "vnd_host_alloc": (C.c_int, [C.c_size_t, _P(C.c_void_p)]),
@@ -132,6 +140,8 @@ SIGNATURES = {
                                                 C.c_void_p]),
     "vnd_vn_objective_runs_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, _P(TapProgramStruct), C.c_void_p,
                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64]),
+    "vnd_vn_stereo_objective_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, _P(TapProgramStruct), C.c_void_p, C.c_int32, C.c_void_p]),
+    "vnd_haas_effect_objective_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p]),
     "vnd_sparse_fir_stream_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, _P(TapProgramStruct), C.c_int32]),
     "vnd_launch_count": (C.c_int64, []),
 }

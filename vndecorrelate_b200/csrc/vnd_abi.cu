@@ -44,6 +44,11 @@ int vn_objective_runs_launch(const float* x, long long chan_stride, const long l
                              void* workspace, size_t workspace_bytes, cudaStream_t st);
 int haas_objective_pairs_launch(const float* x, long long chan_stride, const long long* offs, const int* pair_clip, const int* pair_delay,
                                 int n_pairs, double* partials, cudaStream_t st);
+int haas_effect_objective_launch(const float* x, long long frames, long long chan_stride, const vnd_haas_clip* cands, int n_cand, double* partials,
+                                 cudaStream_t st);
+int vn_stereo_objective_workspace_bytes(long long frames, int n_cand, size_t* bytes);
+int vn_stereo_objective_launch(const float* x, long long frames, long long chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,
+                               int n_cand, double* partials, void* workspace, size_t workspace_bytes, cudaStream_t st);
 size_t dsp_workspace_bytes(long long elems);
 int rms_normalize_launch(const vnd_signal* x, const vnd_signal* y, int x_ndim, int y_ndim, int stereo_mode, double eps, void* ws, cudaStream_t st);
 int peak_normalize_launch(const vnd_signal* y, int ndim, int stereo_mode, double eps, void* ws, cudaStream_t st);
@@ -485,6 +490,52 @@ extern "C" int vnd_haas_objective_pairs_dev(const float* x, int64_t rows, int64_
   if ((rc = check_haas_pairs(x, rows, chan_stride, frame_offsets, n_clips, pair_clip, pair_delay, n_pairs, partials))) return rc;
   return haas_objective_pairs_launch(x, chan_stride, reinterpret_cast<const long long*>(frame_offsets), pair_clip, pair_delay, n_pairs, partials,
                                      (cudaStream_t)stream);
+}
+
+// The clip of the one-clip family objectives: float32 channel-planar, at least one frame.
+static int check_family_clip(const float* x, int64_t frames, int64_t chan_stride, int32_t n_cand, const double* partials) {
+  VND_REQUIRE(n_cand >= 0, VND_EINVAL, "negative n_cand %d", n_cand);
+  // the reference takes max(|theta|) of the frames: an empty signal is a ValueError there (optimization.py:41-43)
+  VND_REQUIRE(frames > 0, VND_EINVAL, "objective of an empty signal (zero-size array to reduction operation maximum which has no identity)");
+  VND_REQUIRE(chan_stride >= frames, VND_EINVAL, "chan_stride %lld is shorter than frames = %lld: the two channels overlap", (long long)chan_stride,
+              (long long)frames);
+  VND_REQUIRE((x != nullptr && partials != nullptr) || n_cand == 0, VND_EINVAL, "x or partials is null");
+  return VND_OK;
+}
+
+static int check_vn_stereo(const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,
+                           int32_t n_cand, const double* partials) {
+  int rc;
+  if ((rc = check_family_clip(x, frames, chan_stride, n_cand, partials))) return rc;
+  if ((rc = check_taps(taps))) return rc;
+  VND_REQUIRE(taps->order == VND_ORDER_SEGMENTED, VND_EINVAL, "objective candidates need SEGMENTED tap programs");
+  VND_REQUIRE((long long)taps->channels == 2LL * n_cand, VND_EINVAL, "the tap program has %d channels, %d candidates need %lld", taps->channels,
+              n_cand, 2LL * n_cand);
+  VND_REQUIRE(cands != nullptr || n_cand == 0, VND_EINVAL, "cands is null");
+  return VND_OK;
+}
+
+extern "C" int vnd_vn_stereo_objective_workspace(int64_t frames, int32_t n_cand, size_t* bytes) {
+  VND_REQUIRE(bytes != nullptr, VND_EINVAL, "bytes is null");
+  VND_REQUIRE(frames >= 0 && n_cand >= 0, VND_EINVAL, "negative extent");
+  return vn_stereo_objective_workspace_bytes(frames, n_cand, bytes);
+}
+
+extern "C" int vnd_vn_stereo_objective_dev(const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps,
+                                           const vnd_vn_stereo_cand* cands, int32_t n_cand, double* partials, void* workspace,
+                                           size_t workspace_bytes, void* stream) {
+  int rc;
+  if ((rc = check_vn_stereo(x, frames, chan_stride, taps, cands, n_cand, partials))) return rc;
+  return vn_stereo_objective_launch(x, frames, chan_stride, taps, cands, n_cand, partials, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int vnd_haas_effect_objective_dev(const float* x, int64_t frames, int64_t chan_stride, const vnd_haas_clip* cands, int32_t n_cand,
+                                             double* partials, void* stream) {
+  int rc;
+  if ((rc = check_family_clip(x, frames, chan_stride, n_cand, partials))) return rc;
+  VND_REQUIRE(cands != nullptr || n_cand == 0, VND_EINVAL, "cands is null");
+  VND_REQUIRE(reinterpret_cast<uintptr_t>(cands) % 16 == 0, VND_EINVAL, "cands must be 16-byte aligned");
+  return haas_effect_objective_launch(x, frames, chan_stride, cands, n_cand, partials, (cudaStream_t)stream);
 }
 
 // Host tables of the run-list objective: offsets (n_clips + 1, from 0, non-decreasing, ending at rows) and every run's
@@ -1577,6 +1628,60 @@ extern "C" int vnd_haas_objective_pairs_host(vnd_ctx* ctx, const float* x, int64
                                         reinterpret_cast<const int*>(meta + off_bytes), reinterpret_cast<const int*>(meta + off_bytes + idx_bytes),
                                         n_pairs, (double*)dout, st)))
     return rc;
+  VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
+  VND_CUDA_OK(cudaStreamSynchronize(st));
+  return VND_OK;
+}
+
+extern "C" int vnd_vn_stereo_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps,
+                                            const vnd_vn_stereo_cand* cands, int32_t n_cand, double* partials) {
+  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  int rc;
+  if ((rc = check_vn_stereo(x, frames, chan_stride, taps, cands, n_cand, partials))) return rc;
+  if (n_cand == 0) return VND_OK;
+  VND_ENTER(ctx);
+  cudaStream_t st = ctx->streams[0];
+  size_t wbytes = 0;
+  if ((rc = vn_stereo_objective_workspace_bytes(frames, n_cand, &wbytes))) return rc;
+  const size_t in_bytes = ((size_t)chan_stride + frames) * 4;
+  const size_t out_bytes = (size_t)n_cand * 12 * 8, cand_bytes = (size_t)n_cand * sizeof(vnd_vn_stereo_cand);
+  vnd_tap_program dprog;
+  void *din = nullptr, *dout = nullptr, *work = nullptr, *dc = nullptr;
+  if ((rc = upload_program(ctx, taps, &dprog, st))) return rc;
+  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) || (rc = arena(ctx, S_WORK, wbytes, &work)) ||
+      (rc = arena(ctx, S_AUX, cand_bytes, &dc)))
+    return rc;
+  VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
+  VND_CUDA_OK(cudaMemcpyAsync(dc, cands, cand_bytes, cudaMemcpyHostToDevice, st));
+  if ((rc = vn_stereo_objective_launch((const float*)din, frames, chan_stride, &dprog, (const vnd_vn_stereo_cand*)dc, n_cand, (double*)dout, work,
+                                       wbytes, st)))
+    return rc;
+  VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
+  VND_CUDA_OK(cudaStreamSynchronize(st));
+  return VND_OK;
+}
+
+extern "C" int vnd_haas_effect_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, int64_t chan_stride, const vnd_haas_clip* cands,
+                                              int32_t n_cand, double* partials) {
+  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  int rc;
+  if ((rc = check_family_clip(x, frames, chan_stride, n_cand, partials))) return rc;
+  VND_REQUIRE(cands != nullptr || n_cand == 0, VND_EINVAL, "cands is null");
+  for (int i = 0; i < n_cand; ++i) {
+    VND_REQUIRE(cands[i].delay >= 0, VND_EINVAL, "candidate %d: negative delay %d", i, cands[i].delay);
+    VND_REQUIRE(cands[i].delayed_channel == 0 || cands[i].delayed_channel == 1, VND_EINVAL, "candidate %d: delayed_channel %d is not 0 or 1", i,
+                cands[i].delayed_channel);
+  }
+  if (n_cand == 0) return VND_OK;
+  VND_ENTER(ctx);
+  cudaStream_t st = ctx->streams[0];
+  const size_t in_bytes = ((size_t)chan_stride + frames) * 4;
+  const size_t out_bytes = (size_t)n_cand * 8 * 8, cand_bytes = (size_t)n_cand * sizeof(vnd_haas_clip);
+  void *din = nullptr, *dout = nullptr, *dc = nullptr;
+  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) || (rc = arena(ctx, S_AUX, cand_bytes, &dc))) return rc;
+  VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
+  VND_CUDA_OK(cudaMemcpyAsync(dc, cands, cand_bytes, cudaMemcpyHostToDevice, st));
+  if ((rc = haas_effect_objective_launch((const float*)din, frames, chan_stride, (const vnd_haas_clip*)dc, n_cand, (double*)dout, st))) return rc;
   VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
   return VND_OK;

@@ -53,6 +53,28 @@ __device__ __forceinline__ double dadd(double a, double b) { return __dadd_rn(a,
 __device__ __forceinline__ double dsub(double a, double b) { return __dsub_rn(a, b); }
 __device__ __forceinline__ double dmul(double a, double b) { return __dmul_rn(a, b); }
 
+// VelvetNoise.decorrelate after the FIR, at one frame: the optional M/S side-channel encode of the filtered pair (y0, y1)
+// against the input pair (x0, x1) (utils/dsp.py:59-63), then the optional width (utils/dsp.py:34-37 with LR_to_MS /
+// MS_to_LR, utils/dsp.py:140-166), w_mid = float32(1 - width), w_side = float32(width).  The fused decorrelate kernels
+// (vnd_fir.cu) and the stereo objective (vnd_objective.cu) both call it, so a scored candidate sees decorrelate's bits.
+__device__ __forceinline__ void ms_width_epilogue(float x0, float x1, float& y0, float& y1, int ms_encode, int use_width, float w_mid,
+                                                  float w_side) {
+  if (ms_encode) {
+    const float M = fadd(x0, x1);
+    const float S = fmul(fsub(y0, y1), 0.5f);
+    y0 = fmul(fadd(M, S), 0.5f);
+    y1 = fmul(fsub(M, S), 0.5f);
+  }
+  if (use_width) {
+    float M = fmul(fadd(y0, y1), 0.5f);
+    float S = fmul(fsub(y0, y1), 0.5f);
+    M = fmul(M, w_mid);
+    S = fmul(S, w_side);
+    y0 = fadd(M, S);
+    y1 = fsub(M, S);
+  }
+}
+
 // ---- shared-memory / TMA bulk-copy primitives (sm_90+ PTX, UBLKCP in SASS) -------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 

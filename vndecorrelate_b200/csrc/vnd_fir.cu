@@ -279,20 +279,7 @@ struct StereoParams {
 };
 
 __device__ __forceinline__ void stereo_epilogue(float x0, float x1, float& y0, float& y1, const StereoParams& p, float g0, float g1) {
-  if (p.ms_encode) {  // utils/dsp.py:59-63
-    const float M = fadd(x0, x1);
-    const float S = fmul(fsub(y0, y1), 0.5f);
-    y0 = fmul(fadd(M, S), 0.5f);
-    y1 = fmul(fsub(M, S), 0.5f);
-  }
-  if (p.use_width) {  // utils/dsp.py:34-37 with LR_to_MS / MS_to_LR (utils/dsp.py:140-166)
-    float M = fmul(fadd(y0, y1), 0.5f);
-    float S = fmul(fsub(y0, y1), 0.5f);
-    M = fmul(M, p.w_mid);
-    S = fmul(S, p.w_side);
-    y0 = fadd(M, S);
-    y1 = fsub(M, S);
-  }
+  ms_width_epilogue(x0, x1, y0, y1, p.ms_encode, p.use_width, p.w_mid, p.w_side);
   if (p.gains) {
     y0 = fmul(y0, g0);
     y1 = fmul(y1, g1);

@@ -27,6 +27,7 @@
 
 #include <vector>
 
+#include "vnd_batch.cuh"
 #include "vnd_objective.cuh"
 
 namespace vnd {
@@ -419,6 +420,170 @@ int obj_combine_launch(const double* chunk_partials, double* partials, int n_cli
 }
 
 // ------------------------------------------------------------------------------------------------
+// Velvet-noise stereo candidates (vnd_vn_stereo_objective_dev): VelvetNoise with two outputs and no normaliser, any
+// filtered channels, LR or MS, any width.  The score of such a candidate is today's two-step one: decorrelate (the
+// fused vn_stereo_kernel: FIR of both channels, unfiltered ones copied, then ms_width_epilogue) and the objective of
+// its float32 output with the one-tap identity program.  This kernel computes each candidate's output in registers and
+// feeds the moments exactly as vn_objective_kernel sees the materialised output: the left value through the identity
+// program's two adds (0 + (0 + y0), which turns -0 into +0), the right value as it is, whole tiles with lane l owning
+// the four consecutive frames 128 j + 4 l + e and lane_acc_pair, the last partial tile with frames base + lane + 32 r
+// and lane_acc_frame, and the chunks of the one-candidate plan (plan_objective for the identity program) combined by
+// obj_combine_kernel.  The per-tile float32 lane sums and the float64 chunk sums therefore see the same values in the
+// same order.
+//
+// The output is computed in the conflict-free layout (lane owns frames base + lane + 32 r, plain LDS per tap, as
+// vn_stereo_kernel reads) and passed through a per-warp scratch row into the four-consecutive-frames layout.
+// Shared memory: float x0[span] | float x1[span] | float scratch[warps][2][32 OBJ_R] | double acc[cand_per_group][OBJ_SLOTS]
+//                | int prog[warps][2 max_prog_words]
+// ------------------------------------------------------------------------------------------------
+#ifndef VND_OBJ_STEREO_NT
+#define VND_OBJ_STEREO_NT 512  // 16 warps: 128 registers a thread (the two channels' taps and outputs of a pass)
+#endif
+struct VnStereoObjParams {
+  const float* x;  // channel 0; channel 1 at x + chan_stride
+  long long frames, chan_stride;
+  const int* words;
+  const int* offsets;  // candidate j: channels 2 j and 2 j + 1
+  const vnd_vn_stereo_cand* cands;
+  int n_cand, apply_gain, halo, cand_per_group, tiles_per_chunk;
+  double* chunk_partials;  // [chunk][cand][OBJ_SLOTS]
+};
+
+// One pass of one candidate: its output (l, r) at frames i0 + 32 rr of the staged tile.
+__device__ __forceinline__ void stereo_candidate_pass(const float* __restrict__ s0, const float* __restrict__ s1, int i0, const int* __restrict__ prog,
+                                                      int n0, int n1, const vnd_vn_stereo_cand& cd, int apply_gain, float (&l)[OBJ_R],
+                                                      float (&r)[OBJ_R]) {
+  if (n0 > 0) run_candidate<OBJ_R>(s0 + i0, prog, apply_gain, l);
+  if (n1 > 0) run_candidate<OBJ_R>(s1 + i0, prog + n0, apply_gain, r);
+#pragma unroll
+  for (int k = 0; k < OBJ_R; ++k) {
+    const float a = s0[i0 + 32 * k], b = s1[i0 + 32 * k];
+    float u = n0 > 0 ? l[k] : a;  // unfiltered channel: copied through
+    float v = n1 > 0 ? r[k] : b;
+    ms_width_epilogue(a, b, u, v, cd.ms_encode, cd.use_width, cd.w_mid, cd.w_side);
+    l[k] = fadd(0.0f, fadd(0.0f, u));  // the identity program's segment sum and running output
+    r[k] = v;
+  }
+}
+
+__global__ void __launch_bounds__(VND_OBJ_STEREO_NT, 1) vn_stereo_objective_kernel(const VnStereoObjParams p, int max_prog_words) {
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  constexpr int kWarps = VND_OBJ_STEREO_NT / 32;
+  constexpr int kPass = 32 * OBJ_R;
+  const int span = OBJ_TILE + p.halo;
+  const int span_al = (span + 3) & ~3;
+  float* s0 = reinterpret_cast<float*>(smem_raw);
+  float* s1 = s0 + span_al;
+  float* scratch = s1 + span_al;
+  double* acc = reinterpret_cast<double*>(scratch + kWarps * 2 * kPass);
+  int* progs = reinterpret_cast<int*>(acc + (size_t)p.cand_per_group * OBJ_SLOTS);
+
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int cand0 = blockIdx.y * p.cand_per_group;
+  const int ncand = min(p.cand_per_group, p.n_cand - cand0);
+  const float* __restrict__ x0 = p.x;
+  const float* __restrict__ x1 = p.x + p.chan_stride;
+  float* my0 = scratch + warp * 2 * kPass;
+  float* my1 = my0 + kPass;
+  int* myprog = progs + warp * 2 * max_prog_words;
+
+  for (int i = tid; i < ncand * OBJ_SLOTS; i += VND_OBJ_STEREO_NT) {
+    const int slot = i % OBJ_SLOTS;
+    acc[i] = (slot == 7 || slot == 9) ? 1.0 : 0.0;  // ratio trackers start at 0 / 1
+  }
+
+  for (int ti = 0; ti < p.tiles_per_chunk; ++ti) {
+    const long long t0 = ((long long)blockIdx.x * p.tiles_per_chunk + ti) * OBJ_TILE;
+    if (t0 >= p.frames) break;
+    const long long remain = p.frames - t0;
+    __syncthreads();  // previous tile fully consumed (also orders the acc init)
+    for (int i = tid; i < span; i += VND_OBJ_STEREO_NT) {
+      s0[i] = i < remain ? x0[t0 + i] : 0.0f;
+      s1[i] = i < remain ? x1[t0 + i] : 0.0f;
+    }
+    __syncthreads();
+    const int nvalid = (int)(remain < OBJ_TILE ? remain : OBJ_TILE);
+
+    for (int ci = warp; ci < ncand; ci += kWarps) {
+      const int c = cand0 + ci;
+      const int w0 = p.offsets[2 * c];
+      const int n0 = p.offsets[2 * c + 1] - w0;
+      const int n1 = p.offsets[2 * c + 2] - w0 - n0;
+      __syncwarp();
+      for (int i = lane; i < n0 + n1; i += 32) myprog[i] = p.words[w0 + i];
+      __syncwarp();
+      const vnd_vn_stereo_cand cd = p.cands[c];
+      LaneAcc a{0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 1.f, 0.f, 1.f};
+      if (nvalid == OBJ_TILE) {  // whole tile: lane owns frames base + 128 j + 4 lane + e, in packed pairs
+        LaneAcc2 b{{0.f, 0.f}, {0.f, 0.f}, {0.f, 0.f}, {0.f, 0.f}, {0.f, 0.f}, {0.f, 0.f}, 0.f, 1.f, 0.f, 1.f, -1.f, -1.f};
+        for (int base = 0; base < OBJ_TILE; base += kPass) {
+          float l[OBJ_R], r[OBJ_R];
+          stereo_candidate_pass(s0, s1, base + lane, myprog, n0, n1, cd, p.apply_gain, l, r);
+          __syncwarp();  // the previous pass has read the scratch row
+#pragma unroll
+          for (int k = 0; k < OBJ_R; ++k) {
+            my0[lane + 32 * k] = l[k];
+            my1[lane + 32 * k] = r[k];
+          }
+          __syncwarp();
+          const float4* q0 = reinterpret_cast<const float4*>(my0 + 4 * lane);
+          const float4* q1 = reinterpret_cast<const float4*>(my1 + 4 * lane);
+#pragma unroll
+          for (int j = 0; j < OBJ_R / 4; ++j) {
+            const float4 u = q0[32 * j], v = q1[32 * j];
+            lane_acc_pair(b, u.x, u.y, v.x, v.y);
+            lane_acc_pair(b, u.z, u.w, v.z, v.w);
+          }
+        }
+        a.sr = b.sr[0] + b.sr[1];
+        a.srt = b.srt[0] + b.srt[1];
+        a.srt2 = b.srt2[0] + b.srt2[1];
+        a.srt3 = b.srt3[0] + b.srt3[1];
+        a.slr = b.slr[0] + b.slr[1];
+        a.sll = b.sll[0] + b.sll[1];
+        a.d_pos = b.d_pos;
+        a.s_pos = b.s_pos;
+        a.d_neg = b.d_neg;
+        a.s_neg = b.s_neg;
+      } else {
+        for (int base = 0; base < nvalid; base += kPass) {
+          float l[OBJ_R], r[OBJ_R];
+          stereo_candidate_pass(s0, s1, base + lane, myprog, n0, n1, cd, p.apply_gain, l, r);
+#pragma unroll
+          for (int k = 0; k < OBJ_R; ++k) {
+            const int i = base + lane + 32 * k;
+            if (i < nvalid) lane_acc_frame(a, l[k], r[k]);
+          }
+        }
+      }
+      a.sr = warp_sum(a.sr);
+      a.srt = warp_sum(a.srt);
+      a.srt2 = warp_sum(a.srt2);
+      a.srt3 = warp_sum(a.srt3);
+      a.slr = warp_sum(a.slr);
+      a.sll = warp_sum(a.sll);
+      warp_best_ratio(a.d_pos, a.s_pos);
+      warp_best_ratio(a.d_neg, a.s_neg);
+      if (lane == 0) {
+        double* q = acc + (size_t)ci * OBJ_SLOTS;
+        q[0] += (double)a.sr;
+        q[1] += (double)a.srt;
+        q[2] += (double)a.srt2;
+        q[3] += (double)a.srt3;
+        q[4] += (double)a.slr;
+        q[5] += (double)a.sll;
+        if ((double)a.d_pos * q[7] > q[6] * (double)a.s_pos) { q[6] = a.d_pos; q[7] = a.s_pos; }
+        if ((double)a.d_neg * q[9] > q[8] * (double)a.s_neg) { q[8] = a.d_neg; q[9] = a.s_neg; }
+        q[10] += (double)nvalid;
+      }
+    }
+  }
+  __syncthreads();
+  double* out = p.chunk_partials + ((size_t)blockIdx.x * p.n_cand + cand0) * OBJ_SLOTS;
+  for (int i = tid; i < ncand * OBJ_SLOTS; i += VND_OBJ_STEREO_NT) out[i] = acc[i];
+}
+
+// ------------------------------------------------------------------------------------------------
 // Haas candidates: float64 throughout (optimization.py:183-203 builds LR-mode HaasEffects whose
 // output is float64).  One CTA per (clip, candidate); 8 doubles per pair:
 //   [sum r, sum r*th, sum r*th^2, sum r*th^3, max|th|, sum L*R, sum L*L, frames]
@@ -552,36 +717,84 @@ struct HaasPairSrc {
   }
 };
 
+// candidate c = blockIdx.x: HaasEffect.decorrelate with the settings record cands[c] (any delayed channel, LR or MS, any
+// width, mono or stereo) on one float32 channel-planar clip, element (t, ch) = x[ch * chan_stride + t].  Today's score
+// of such a candidate is the objective of its float64 output z (frames + delay frames) as a delay-0 item, so frame m of
+// z is built with haas_frame, as haas_kernel builds it, and fed with the striding of the delay-0 stretch.
+struct HaasEffectSrc {
+  using T = float;
+  const float* x;
+  long long frames, chan_stride;
+  const vnd_haas_clip* cands;  // 16-byte aligned
+  double* partials;            // (n_cand, HAAS_SLOTS)
+};
+
+template <typename Src>
+struct haas_effect_src { static constexpr bool value = false; };
+template <>
+struct haas_effect_src<HaasEffectSrc> { static constexpr bool value = true; };
+
 template <typename Src>
 __global__ void __launch_bounds__(256) haas_objective_kernel(const Src src) {
   using TIn = typename Src::T;
-  const HaasItem<TIn> it = src.item();
-  const long long frames = it.frames;
-  const int d = it.d;
-  const TIn* __restrict__ x0 = it.x0;
-  const TIn* __restrict__ x1 = it.x1;
-  const long long total = frames + d;
   HaasAcc acc;
-  // Three stretches (decorrelation.py:220-222: channel 0 delayed by d, both padded to frames + d): only channel 1 for
-  // m < d, both channels for d <= m < frames, only the delayed channel 0 behind the end of channel 1.
-  const long long head = d < frames ? d : frames;
-  for (long long m = threadIdx.x; m < head; m += blockDim.x) {
-    const TIn r = x1[m];
-    acc.add(0.0, (double)r, 0.0f, (float)r);
-  }
-  if (d < frames) {
-    const TIn* __restrict__ p0 = x0 + threadIdx.x;      // x0[m - d]
-    const TIn* __restrict__ p1 = x1 + d + threadIdx.x;  // x1[m]
-    const long long n = frames - d;
-    for (long long k = threadIdx.x; k < n; k += blockDim.x, p0 += blockDim.x, p1 += blockDim.x) {
-      const TIn l = *p0, r = *p1;
-      acc.add((double)l, (double)r, (float)l, (float)r);
+  long long total;
+  double* out;
+  if constexpr (haas_effect_src<Src>::value) {
+    const int4* rec = reinterpret_cast<const int4*>(src.cands + blockIdx.x);
+    const int4 w0 = __ldg(rec), w1 = __ldg(rec + 1);
+    const int delay = w0.x, dch = w0.y, mode_ms = w0.z, mono = w0.w, use_width = w1.x;
+    const double width = __hiloint2double(w1.w, w1.z);
+    const long long L = src.frames;
+    const float* __restrict__ x0 = src.x;
+    const float* __restrict__ x1 = src.x + src.chan_stride;
+    const int sh0 = dch == 0 ? delay : 0, sh1 = dch == 1 ? delay : 0;
+    total = L + delay;
+    out = src.partials + (size_t)blockIdx.x * HAAS_SLOTS;
+    for (long long m = threadIdx.x; m < total; m += blockDim.x) {
+      const long long q0 = m - sh0, q1 = m - sh1;
+      const bool v0 = q0 >= 0 && q0 < L, v1 = q1 >= 0 && q1 < L;
+      float a0 = 0.0f, b0 = 0.0f, a1 = 0.0f, b1 = 0.0f;
+      if (v0) {
+        a0 = x0[q0];
+        b0 = x1[q0];
+      }
+      if (v1) {
+        a1 = x0[q1];
+        b1 = x1[q1];
+      }
+      const double2 z = haas_frame(a0, b0, v0, a1, b1, v1, mode_ms, mono, use_width, width);
+      acc.add(z.x, z.y, (float)z.x, (float)z.y);
     }
-  }  // (d >= frames: the frames between the two channels are silence and add nothing to any sum)
-  const long long tail0 = frames > d ? frames : d;
-  for (long long m = tail0 + threadIdx.x; m < total; m += blockDim.x) {
-    const TIn l = x0[m - d];
-    acc.add((double)l, 0.0, (float)l, 0.0f);
+  } else {
+    const HaasItem<TIn> it = src.item();
+    const long long frames = it.frames;
+    const int d = it.d;
+    const TIn* __restrict__ x0 = it.x0;
+    const TIn* __restrict__ x1 = it.x1;
+    total = frames + d;
+    out = it.out;
+    // Three stretches (decorrelation.py:220-222: channel 0 delayed by d, both padded to frames + d): only channel 1 for
+    // m < d, both channels for d <= m < frames, only the delayed channel 0 behind the end of channel 1.
+    const long long head = d < frames ? d : frames;
+    for (long long m = threadIdx.x; m < head; m += blockDim.x) {
+      const TIn r = x1[m];
+      acc.add(0.0, (double)r, 0.0f, (float)r);
+    }
+    if (d < frames) {
+      const TIn* __restrict__ p0 = x0 + threadIdx.x;      // x0[m - d]
+      const TIn* __restrict__ p1 = x1 + d + threadIdx.x;  // x1[m]
+      const long long n = frames - d;
+      for (long long k = threadIdx.x; k < n; k += blockDim.x, p0 += blockDim.x, p1 += blockDim.x) {
+        const TIn l = *p0, r = *p1;
+        acc.add((double)l, (double)r, (float)l, (float)r);
+      }
+    }  // (d >= frames: the frames between the two channels are silence and add nothing to any sum)
+    const long long tail0 = frames > d ? frames : d;
+    for (long long m = tail0 + threadIdx.x; m < total; m += blockDim.x) {
+      const TIn l = x0[m - d];
+      acc.add((double)l, 0.0, (float)l, 0.0f);
+    }
   }
   double v[7] = {acc.v0, acc.v1, acc.v2, acc.v3, __longlong_as_double(acc.vmax), acc.v5, acc.v6};
   __shared__ double red[8][7];
@@ -604,9 +817,9 @@ __global__ void __launch_bounds__(256) haas_objective_kernel(const Src src) {
     const int k = threadIdx.x;
     double r = red[0][k];
     for (int w = 1; w < 8; ++w) r = (k == 4) ? fmax(r, red[w][k]) : r + red[w][k];
-    it.out[k] = r;
+    out[k] = r;
   }
-  if (threadIdx.x == 7) it.out[7] = (double)total;
+  if (threadIdx.x == 7) out[7] = (double)total;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -942,6 +1155,74 @@ int haas_objective_pairs_launch(const float* x, long long chan_stride, const lon
   if (n_pairs == 0) return VND_OK;
   haas_objective_kernel<<<(unsigned)n_pairs, 256, 0, st>>>(HaasPairSrc{x, chan_stride, offs, pair_clip, pair_delay, partials});
   return after_launch("haas_objective_kernel");
+}
+
+int haas_effect_objective_launch(const float* x, long long frames, long long chan_stride, const vnd_haas_clip* cands, int n_cand, double* partials,
+                                 cudaStream_t st) {
+  if (n_cand == 0) return VND_OK;
+  haas_objective_kernel<<<(unsigned)n_cand, 256, 0, st>>>(HaasEffectSrc{x, frames, chan_stride, cands, partials});
+  return after_launch("haas_objective_kernel");
+}
+
+// ------------------------------------------------------------------------------------------------
+// velvet-noise stereo candidates (vnd_vn_stereo_objective_dev)
+// ------------------------------------------------------------------------------------------------
+// The chunks of today's score of one candidate: vn_objective_launch on its output with the one-tap identity program
+// (halo 1, padded to 4; 5 program words), one clip, one candidate.
+static int stereo_chunk_plan(long long frames, ObjPlan* pl) { return plan_objective(frames, 1, 1, 4, 5, pl); }
+
+int vn_stereo_objective_workspace_bytes(long long frames, int n_cand, size_t* bytes) {
+  DeviceInfo di;
+  int rc = device_info(&di);
+  if (rc) return rc;
+  const long long chunks = max_chunks(ceil_div<long long>(frames, OBJ_TILE), 1, di.sm_count);  // plan_objective's cap for one clip
+  *bytes = (size_t)chunks * n_cand * OBJ_SLOTS * 8 + 256;
+  return VND_OK;
+}
+
+int vn_stereo_objective_launch(const float* x, long long frames, long long chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,
+                               int n_cand, double* partials, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  if (n_cand == 0) return VND_OK;
+  if (!g_obj_disable_tmem) return VND_EUNSUPPORTED;  // today's score then comes from the tensor-memory kernel, whose tiles differ
+  DeviceInfo di;
+  int rc = device_info(&di);
+  if (rc) return rc;
+  ObjPlan chunks;
+  if ((rc = stereo_chunk_plan(frames, &chunks))) return rc;
+  int halo = taps->halo > 0 ? taps->halo : 0;
+  if (halo > frames) halo = (int)frames;
+  halo = (halo + 3) & ~3;
+  const int mpw = taps->max_channel_words > 0 ? taps->max_channel_words : 1;
+  constexpr int kWarps = VND_OBJ_STEREO_NT / 32;
+  const size_t fixed = (size_t)2 * ((OBJ_TILE + halo + 3) & ~3) * 4 + (size_t)kWarps * 2 * 32 * OBJ_R * 4 + (size_t)kWarps * 2 * mpw * 4 + 64;
+  if (fixed + (size_t)OBJ_SLOTS * 8 > (size_t)kMaxDynSmem) return VND_EUNSUPPORTED;  // the caller scores candidate by candidate
+  int cpg = (int)((kMaxDynSmem - fixed) / (OBJ_SLOTS * 8));
+  if (cpg > n_cand) cpg = n_cand;
+  if (cpg > 1024) cpg = 1024;
+  // groups small enough for about four CTAs per SM, never fewer candidates than warps
+  while ((long long)chunks.n_chunks * ceil_div(n_cand, cpg) < (long long)di.sm_count * 4 && cpg > kWarps) cpg = (cpg + 1) / 2;
+  const int groups = ceil_div(n_cand, cpg);
+  VND_REQUIRE(groups <= 65535, VND_EUNSUPPORTED, "too many candidate groups for one launch");
+  const size_t need = (size_t)chunks.n_chunks * n_cand * OBJ_SLOTS * 8;
+  VND_REQUIRE(workspace && workspace_bytes >= need, VND_ENOMEM, "objective workspace too small: need %zu bytes, have %zu", need, workspace_bytes);
+  VnStereoObjParams p{};
+  p.x = x;
+  p.frames = frames;
+  p.chan_stride = chan_stride;
+  p.words = taps->words;
+  p.offsets = taps->offsets;
+  p.cands = cands;
+  p.n_cand = n_cand;
+  p.apply_gain = taps->apply_gain;
+  p.halo = halo;
+  p.cand_per_group = cpg;
+  p.tiles_per_chunk = chunks.tiles_per_chunk;
+  p.chunk_partials = reinterpret_cast<double*>(workspace);
+  const size_t smem = fixed + (size_t)cpg * OBJ_SLOTS * 8;
+  VND_CUDA_OK(cudaFuncSetAttribute(vn_stereo_objective_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  vn_stereo_objective_kernel<<<dim3((unsigned)chunks.n_chunks, (unsigned)groups), VND_OBJ_STEREO_NT, smem, st>>>(p, mpw);
+  if ((rc = after_launch("vn_stereo_objective_kernel"))) return rc;
+  return obj_combine_launch(p.chunk_partials, partials, 1, chunks.n_chunks, n_cand, st);
 }
 
 }  // namespace vnd

@@ -5,8 +5,11 @@
 ``VelvetNoise(filtered_channels=(0,), mode='LR', normalizer=None, log_distribution_strength=k)``
 (optimization.py:260-272) and ``HaasEffect(delay_time_seconds=t, mode='LR')`` (:183-190) — and
 scores ALL candidates of a family in one kernel launch: the clip is read once per tile and every
-candidate is evaluated from shared memory.  Any other decorrelator is run and its output scored by
-the same kernels (one candidate).  The kernels return the sums the objective is made of; the scalar
+candidate is evaluated from shared memory.  Two wider families also score in one launch each, every score
+equal to that candidate's own decorrelate-then-score result: velvet-noise candidates with two outputs and no
+normaliser (any filtered channels, LR or MS, any width; ``vn_stereo_objective_partials``) and any ``HaasEffect``
+(``haas_effect_objective_partials``); a mixed list is split into its families.  Any other decorrelator is run and
+its output scored by the same kernels (one candidate).  The kernels return the sums the objective is made of; the scalar
 combination below follows the reference's dtype chain (float32 for velvet-noise candidates, float64
 for Haas candidates; SURVEY.md Appendix A.5).
 
@@ -32,14 +35,15 @@ import numpy as np
 
 from . import _native as N
 from . import runtime as R
-from .decorrelation import Decorrelator, HaasEffect, VelvetNoise, _is_mode
+from .decorrelation import Decorrelator, HaasEffect, VelvetNoise, _batch_program, _is_mode
 from .taps import IDENTITY_ENVELOPE, TapProgram, candidate_program, kappa_family_program
-from .utils.dsp import EPSILON, LayoutMode
+from .utils.dsp import EPSILON, LayoutMode, to_float32
 
 __all__ = [
     "symmetry_aware_objective", "grid_scan", "get_local_minima", "optimize_local_minima", "optimize_haas_delay",
     "optimize_velvet_noise", "optimize_velvet_noise_batch", "optimize_haas_delay_batch", "vn_objective_partials", "haas_objective_partials",
     "haas_objective_pair_partials", "vn_objective_run_partials", "vn_scores_from_partials", "haas_scores_from_partials",
+    "vn_stereo_objective_partials", "haas_effect_objective_partials",
 ]
 
 _F32_HALF_PI = np.float32(np.pi / 2)
@@ -229,6 +233,134 @@ def vn_objective_run_partials(x, frame_offsets, program: TapProgram, runs):
     return out
 
 
+def _planar_input(x):
+    """A cast and checked input (``to_float32``: numpy array or CUDA tensor) as a float32 channel-planar ``(2, frames)``
+    clip on the same side: a mono signal in both channels, a wider one cut to its first two."""
+    if R.is_torch_tensor(x):
+        import torch
+
+        if not x.is_cuda:
+            raise N.VndError(N.VND_EUNSUPPORTED, "objective", "CPU torch tensors are not supported (no CPU fallback); pass a CUDA tensor or a numpy array")
+        return (torch.stack((x, x)) if x.dim() == 1 else x[:, :2].t()).contiguous()
+    return np.ascontiguousarray(np.stack((x, x)) if x.ndim == 1 else x[:, :2].T)
+
+
+def _cast_input(input_signal):
+    """The input as ``decorrelate`` casts it."""
+    return to_float32(input_signal if R.is_torch_tensor(input_signal) else np.asarray(input_signal))
+
+
+def _vn_stereo_partials(x, xp, decorrelators):
+    """``vn_stereo_objective_partials`` on an input already cast and checked, ``xp`` its ``_planar_input``."""
+    lib = N.lib()
+    frames = x.shape[0]
+    progs = [d.tap_program(frames) for d in decorrelators]
+    if len({p.apply_gain for p in progs}) > 1:
+        raise ValueError("the candidates of one call must agree on whether the segment envelope is the identity (1.0,)")
+    prog = _batch_program(progs)
+    cands = np.zeros(len(decorrelators), dtype=N.VN_STEREO_CAND_DTYPE)
+    widths = [float(d.width) if d.width is not None else 0.0 for d in decorrelators]
+    cands["ms_encode"] = [_is_mode(d.mode, LayoutMode.MS) for d in decorrelators]
+    cands["use_width"] = [d.width is not None for d in decorrelators]
+    cands["w_mid"] = [np.float32(1.0 - w) for w in widths]  # the float32 roundings of vnd_vn_decorrelate_dev
+    cands["w_side"] = [np.float32(w) for w in widths]
+    n = len(decorrelators)
+    if R.is_torch_tensor(xp):
+        import torch
+
+        dev = xp.device
+        out = torch.empty((n, N.OBJ_SLOTS), dtype=torch.float64, device=dev)
+        nbytes = C.c_size_t()
+        N.check(lib.vnd_vn_stereo_objective_workspace(frames, n, C.byref(nbytes)), "vnd_vn_stereo_objective_workspace")
+        with torch.cuda.device(dev):
+            work = torch.empty(nbytes.value, dtype=torch.uint8, device=dev)
+            dc = torch.from_numpy(cands.view(np.uint8)).to(dev)
+            ps = R.device_program(prog, dev)
+            N.check(lib.vnd_vn_stereo_objective_dev(xp.data_ptr(), frames, xp.stride(0), C.byref(ps), dc.data_ptr(), n, out.data_ptr(), work.data_ptr(),
+                                                    nbytes.value, R.torch_stream_ptr(xp)), "vnd_vn_stereo_objective_dev")
+        return out
+    out = np.empty((n, N.OBJ_SLOTS), dtype=np.float64)
+    ps = prog.host_struct()
+    N.check(lib.vnd_vn_stereo_objective_host(R.HostContext.get().handle, xp.ctypes.data, frames, xp.shape[1], C.byref(ps), cands.ctypes.data, n,
+                                             out.ctypes.data), "vnd_vn_stereo_objective_host")
+    return out
+
+
+def _haas_effect_partials(x, xp, haas_effects):
+    """``haas_effect_objective_partials`` on an input already cast and checked, ``xp`` its ``_planar_input``."""
+    lib = N.lib()
+    n = len(haas_effects)
+    frames = x.shape[0]
+    table = np.zeros(n, dtype=N.HAAS_CLIP_DTYPE)
+    table["delay"] = [h.delay_len_samples for h in haas_effects]
+    table["delayed_channel"] = [h.delayed_channel % 2 for h in haas_effects]
+    table["mode_ms"] = [_is_mode(h.mode, LayoutMode.MS) for h in haas_effects]
+    table["mono"] = x.ndim == 1
+    table["use_width"] = [h.width is not None for h in haas_effects]
+    table["width"] = [float(h.width) if h.width is not None else 0.0 for h in haas_effects]
+    if R.is_torch_tensor(xp):
+        import torch
+
+        dev = xp.device
+        out = torch.empty((n, N.HAAS_SLOTS), dtype=torch.float64, device=dev)
+        with torch.cuda.device(dev):
+            dc = torch.from_numpy(table.view(np.uint8)).to(dev)
+            N.check(lib.vnd_haas_effect_objective_dev(xp.data_ptr(), frames, xp.stride(0), dc.data_ptr(), n, out.data_ptr(), R.torch_stream_ptr(xp)),
+                    "vnd_haas_effect_objective_dev")
+        return out
+    out = np.empty((n, N.HAAS_SLOTS), dtype=np.float64)
+    N.check(lib.vnd_haas_effect_objective_host(R.HostContext.get().handle, xp.ctypes.data, frames, xp.shape[1], table.ctypes.data, n, out.ctypes.data),
+            "vnd_haas_effect_objective_host")
+    return out
+
+
+def vn_stereo_objective_partials(clip, decorrelators: Sequence[VelvetNoise]):
+    """Partial sums of the objective of ``VelvetNoise`` candidates with two outputs and ``normalizer=None`` - any
+    ``filtered_channels``, mode LR or MS, any ``width`` - on one clip: one objective launch and one combine launch for
+    all of them, with each candidate's output computed in registers and never stored.
+
+    ``clip``: the input signal as ``decorrelate`` takes it (numpy array or CUDA tensor, mono or ``(frames, >= 2)``, any
+    dtype; cast with ``to_float32``).  The candidates may differ in taps, mode, filtered channels and width; they must
+    agree on whether the segment envelope is the identity ``(1.0,)``.  Each candidate's input checks run first and raise
+    what its ``decorrelate`` raises.  Returns float64 ``(n_candidates, 12)`` (the layout of ``vn_objective_partials``):
+    numpy for numpy input, a CUDA tensor enqueued on torch's current stream for a CUDA tensor (nothing is downloaded).
+
+    Bit contract: row ``j`` equals, bit for bit, the partials the objective computes from
+    ``decorrelators[j].decorrelate(clip)`` (``vn_objective_partials`` of that output with the one-tap identity program),
+    so ``vn_scores_from_partials`` gives the scores ``symmetry_aware_objective`` returns for each candidate alone.
+    A filter whose halo does not fit the kernel's shared memory raises ``VndError`` with ``VND_EUNSUPPORTED``."""
+    decorrelators = list(decorrelators)
+    for d in decorrelators:
+        if not _is_vn_stereo_candidate(d):
+            raise ValueError("candidates must be VelvetNoise with num_outs=2, normalizer=None, mode LR or MS and filtered_channels in (0, 1)")
+    x = _cast_input(clip)
+    for d in decorrelators:
+        d._check_input(x)
+    return _vn_stereo_partials(x, _planar_input(x), decorrelators)
+
+
+def haas_effect_objective_partials(clip, haas_effects: Sequence[HaasEffect]):
+    """Partial sums of the objective of ``HaasEffect`` candidates - delayed channel 0, 1, -1 or -2, mode LR or MS, any
+    ``width`` - on one clip: one launch, one CTA per candidate, the clip read in place and no candidate's output stored.
+
+    ``clip``: the input signal as ``HaasEffect.decorrelate`` takes it (numpy array or CUDA tensor, mono or
+    ``(frames, 2)``, any dtype; cast with ``to_float32``).  Each candidate's input checks run first and raise what its
+    ``decorrelate`` raises.  Returns float64 ``(n_candidates, 8)`` (the layout of ``haas_objective_partials``): numpy for
+    numpy input, a CUDA tensor enqueued on torch's current stream for a CUDA tensor.
+
+    Bit contract: row ``j`` equals, bit for bit, ``haas_objective_partials(z, [0])[0, 0]`` for the float64 output ``z`` of
+    ``haas_effects[j].decorrelate(clip)``, so ``haas_scores_from_partials`` gives the scores ``symmetry_aware_objective``
+    returns for each candidate alone."""
+    haas_effects = list(haas_effects)
+    for h in haas_effects:
+        if not _is_haas_effect_candidate(h):
+            raise ValueError("candidates must be HaasEffect with a delay in [0, 2**31)")
+    x = _cast_input(clip)
+    for h in haas_effects:
+        h._check(x)
+    return _haas_effect_partials(x, _planar_input(x), haas_effects)
+
+
 # ------------------------------------------------------------------------------------------------
 # scalar combination (optimization.py:71-105 and the helpers :11-43)
 # ------------------------------------------------------------------------------------------------
@@ -372,6 +504,20 @@ def _is_haas_candidate(d) -> bool:
     return isinstance(d, HaasEffect) and d.width is None and _is_mode(d.mode, LayoutMode.LR) and d.delayed_channel == 0
 
 
+def _is_vn_stereo_candidate(d) -> bool:
+    """A candidate ``vn_stereo_objective_partials`` scores (the reference's velvet-noise family is one of them)."""
+    return (
+        isinstance(d, VelvetNoise) and d.num_outs == 2 and d.normalizer is None and (_is_mode(d.mode, LayoutMode.LR) or _is_mode(d.mode, LayoutMode.MS))
+        and set(d.filtered_channels) <= {0, 1} and len(set(d.filtered_channels)) == len(tuple(d.filtered_channels))
+    )
+
+
+def _is_haas_effect_candidate(d) -> bool:
+    """A candidate ``haas_effect_objective_partials`` scores: any HaasEffect whose delay a settings record holds (the
+    per-candidate path reports any other delay itself)."""
+    return isinstance(d, HaasEffect) and 0 <= d.delay_len_samples < 2**31
+
+
 def _as_stereo_f32(input_signal):
     x = np.asarray(input_signal).astype(np.float32, copy=False)
     if x.ndim == 1:
@@ -428,7 +574,54 @@ def _scan(input_signal, decorrelators, kw) -> np.ndarray:
         x = _as_stereo_f32(input_signal)
         delays = [d.delay_len_samples for d in decorrelators]
         return haas_scores_from_partials(haas_objective_partials(x, delays), **kw)[0]
-    return np.array([_score_signal(d.decorrelate(input_signal), kw) for d in decorrelators])
+    return _scan_families(input_signal, decorrelators, kw)
+
+
+def _scan_families(input_signal, decorrelators, kw) -> np.ndarray:
+    """Scores of any candidate list: the velvet-noise stereo candidates in one launch per envelope kind
+    (``_vn_stereo_partials``), the Haas effects in one launch (``_haas_effect_partials``), every other candidate run and
+    scored on its own (``_score_signal``); each score is the one that candidate alone gets, in list order.  Every
+    candidate's input check runs before any device work, so the first exception is the one the candidate-by-candidate
+    loop raises."""
+    vn = [i for i, d in enumerate(decorrelators) if _is_vn_stereo_candidate(d)]
+    haas = [i for i, d in enumerate(decorrelators) if _is_haas_effect_candidate(d)]
+    cpu_tensor = R.is_torch_tensor(input_signal) and not input_signal.is_cuda  # decorrelate raises its own error for it
+    if (not vn and not haas) or cpu_tensor:
+        return np.array([_score_signal(d.decorrelate(input_signal), kw) for d in decorrelators])
+    grouped = set(vn) | set(haas)
+    others = [i for i in range(len(decorrelators)) if i not in grouped]
+    x = _cast_input(input_signal)
+    for i, d in enumerate(decorrelators):
+        if i not in grouped:
+            continue
+        try:
+            d._check_input(x) if isinstance(d, VelvetNoise) else d._check(x)
+        except Exception:
+            for j in others:  # the loop would have run these first: any exception of theirs comes first
+                if j < i:
+                    decorrelators[j].decorrelate(input_signal)
+            raise
+    xp = _planar_input(x)
+    scores: list = [None] * len(decorrelators)
+    by_gain: dict = {}
+    for i in vn:
+        by_gain.setdefault(decorrelators[i].tap_program(x.shape[0]).apply_gain, []).append(i)
+    for idx in by_gain.values():
+        try:
+            s = vn_scores_from_partials(_vn_stereo_partials(x, xp, [decorrelators[i] for i in idx]), **kw)
+        except N.VndError as e:
+            if e.status != N.VND_EUNSUPPORTED:
+                raise
+            others.extend(idx)  # a halo beyond the kernel's shared memory: candidate by candidate
+            continue
+        for i, v in zip(idx, s):
+            scores[i] = v
+    if haas:
+        for i, v in zip(haas, haas_scores_from_partials(_haas_effect_partials(x, xp, [decorrelators[i] for i in haas]), **kw)):
+            scores[i] = v
+    for i in sorted(others):
+        scores[i] = _score_signal(decorrelators[i].decorrelate(input_signal), kw)
+    return np.array(scores)
 
 
 def grid_scan(input_signal, decorrelators: list[Decorrelator], **kwargs) -> np.ndarray:
