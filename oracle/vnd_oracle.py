@@ -363,6 +363,101 @@ def objective(
     return -obj
 
 
+# --------------------------------------------------------------------------------------
+# float64 references of the objective kernels' partial sums (include/vnd_b200.h layouts)
+# --------------------------------------------------------------------------------------
+
+
+def _folded_theta(d: np.ndarray, s: np.ndarray) -> np.ndarray:
+    """float64 ``arctan2(d, s)`` folded into [-pi/2, pi/2] (utils/dsp.py:399-412)."""
+    th = np.arctan2(d, s)
+    return np.where(th < -np.pi / 2, th + np.pi, np.where(th > np.pi / 2, th - np.pi, th))
+
+
+def _sums(terms) -> tuple[np.ndarray, np.ndarray]:
+    """Correctly rounded sums (``math.fsum``) of each term array and of its magnitudes; ``np.sum`` where a term is not
+    finite (the sum is then inf or nan either way)."""
+    sums, mags = [], []
+    for t in terms:
+        if np.all(np.isfinite(t)):
+            sums.append(math.fsum(t.tolist()))
+            mags.append(math.fsum(np.abs(t).tolist()))
+        else:
+            sums.append(float(np.sum(t)))
+            mags.append(float(np.sum(np.abs(t))))
+    return np.array(sums), np.array(mags)
+
+
+def _best_ratio(ad: np.ndarray, as_: np.ndarray) -> tuple[float, float, int]:
+    """The frame with the largest ``ad / as`` as the kernels' tracker defines it: a frame replaces the record
+    (initially 0 / 1) when ``ad * rs > rd * as``, decided on float64 products of float32 operands (exact), so ties keep
+    the earliest frame.  Returns (|d|, |s|, frame index or -1)."""
+    a = ad.astype(np.float64)
+    b = as_.astype(np.float64)
+    live = a > 0.0  # nothing else ever beats the initial record (a nan compares false)
+    if not np.any(live):
+        return 0.0, 1.0, -1
+    with np.errstate(divide="ignore", invalid="ignore"):
+        q = np.where(b > 0.0, a / b, np.inf)
+    q = np.where(live, q, -1.0)
+    qmax = np.nanmax(q)
+    # float64 division rounds monotonically, so every frame of the largest exact ratio has q == qmax
+    bd, bs, at = 0.0, 1.0, -1
+    for i in np.flatnonzero(q == qmax):
+        if a[i] * bs > bd * b[i]:
+            bd, bs, at = float(a[i]), float(b[i]), int(i)
+    return bd, bs, at
+
+
+def objective_partials(y: np.ndarray) -> dict:
+    """float64 reference of the 12 velvet-noise partials (``vn_objective_partials``) of a float32 stereo signal ``y``
+    (frames, 2), e.g. ``vn_decorrelate(x, taps, ms_mode=..., width=..., normalizer=None)``.
+
+    d = L - R and s = L + R are the float32 values the reference computes; theta is the float64 folded ``arctan2`` of
+    them, and the radius the float64 root of the reference's float32 ``L*L + R*R`` (utils/dsp.py:413: each square and
+    the sum rounded to float32, so its underflow and overflow are the reference's).  The six sums are correctly rounded
+    (``math.fsum``); ``mag`` holds the sums of their terms' magnitudes, for tolerances.  Slots 6-9 are |d|, |s| of the
+    largest-|d|/|s| frame with s >= 0 and with s < 0 (``_best_ratio``; 0 / 1 when there is none); ``at`` their frame
+    indices."""
+    y = np.asarray(y, dtype=np.float32)
+    l, r = y[:, 0], y[:, 1]
+    with np.errstate(over="ignore", invalid="ignore"):
+        d, s = l - r, l + r
+        th = _folded_theta(d.astype(np.float64), s.astype(np.float64))
+        rad = np.sqrt((l * l + r * r).astype(np.float64))
+        l64, r64 = l.astype(np.float64), r.astype(np.float64)
+        terms = [rad, rad * th, rad * th * th, rad * th * th * th, l64 * r64, l64 * l64]
+        sums, mag = _sums(terms)
+    pos = s >= 0.0
+    ad, as_ = np.abs(d), np.abs(s)
+    dp, sp, ip = _best_ratio(np.where(pos, ad, 0.0), np.where(pos, as_, 1.0))
+    neg = s < 0.0
+    dn, sn, i_n = _best_ratio(np.where(neg, ad, 0.0), np.where(neg, as_, 1.0))
+    p = np.zeros(12)
+    p[:6] = sums
+    p[6:10] = dp, sp, dn, sn
+    p[10] = len(y)
+    return {"p": p, "mag": mag, "at": (ip, i_n), "frames": len(y), "theta": th, "d": d, "s": s}
+
+
+def haas_partials(y: np.ndarray) -> dict:
+    """float64 reference of the 8 Haas partials (``haas_objective_partials``) of a float64 stereo signal ``y``
+    (frames, 2), e.g. ``haas(x, ...)``: the sums of r, r*theta^n (n = 1..3), L*R and L*L correctly rounded, max|theta|,
+    and the frame count.  d, s, theta and r are float64, as the kernel computes them; ``mag`` as in
+    ``objective_partials``."""
+    y = np.asarray(y, dtype=np.float64)
+    l, r = y[:, 0], y[:, 1]
+    th = _folded_theta(l - r, l + r)
+    rad = np.sqrt(l * l + r * r)
+    sums, mag = _sums([rad, rad * th, rad * th * th, rad * th * th * th, l * r, l * l])
+    p = np.zeros(8)
+    p[:4] = sums[:4]
+    p[4] = float(np.max(np.abs(th))) if len(th) else 0.0
+    p[5:7] = sums[4:]
+    p[7] = len(y)
+    return {"p": p, "mag": np.concatenate([mag[:4], [0.0], mag[4:]]), "frames": len(y), "theta": th}
+
+
 def local_minima(scores: np.ndarray) -> list[int]:
     """Strict interior minima, else [argmin].  optimization.py:120-128."""
     g = len(scores)

@@ -216,12 +216,12 @@ __device__ __forceinline__ void run_candidate_v4(const float* __restrict__ px, c
 }
 
 // Shared memory: float x0[4][span4] (copy c = channel 0 shifted by c samples) | float x1[TILE] |
-//                double acc[cand_per_group][OBJ_SLOTS] | int prog[warps][max_prog_words] | int dec[warps][max_prog_words]
+//                double acc[cand_per_group][OBJ_CHUNK_SLOTS] | int prog[warps][max_prog_words] | int dec[warps][max_prog_words]
 #ifndef VND_OBJ_MINB
 #define VND_OBJ_MINB 1  // CTAs per SM the register and shared-memory budgets are planned for (measured: 16 frames per lane in one CTA beats 8 in two)
 #endif
 // Work-item sources of vn_objective_kernel.  A CTA scores the tiles [tile_first, tile_first + n_tiles) of one clip (the
-// loop stops at the clip's end) on the candidates [cand0, cand0 + ncand) of the program, and writes ncand x OBJ_SLOTS
+// loop stops at the clip's end) on the candidates [cand0, cand0 + ncand) of the program, and writes ncand x OBJ_CHUNK_SLOTS
 // chunk partials to out.  Tiles are counted from frame 0 of the clip and staging reads nothing past the clip's last
 // frame, so a (clip, candidate) pair gives the same bits whichever source hands it out.  Each field is asked for
 // where the kernel needs it.
@@ -236,7 +236,7 @@ struct ObjGridSrc {
   __device__ __forceinline__ long long tile_first() const { return (long long)blockIdx.x * p.tiles_per_chunk; }
   __device__ __forceinline__ int n_tiles() const { return p.tiles_per_chunk; }
   __device__ __forceinline__ double* out(int cand0) const {
-    return p.chunk_partials + (((size_t)blockIdx.y * p.n_chunks + blockIdx.x) * p.n_cand + cand0) * OBJ_SLOTS;
+    return p.chunk_partials + (((size_t)blockIdx.y * p.n_chunks + blockIdx.x) * p.n_cand + cand0) * OBJ_CHUNK_SLOTS;
   }
 };
 
@@ -251,7 +251,7 @@ struct ObjRunSrc {
   __device__ __forceinline__ long long frames() const { return items[blockIdx.x].frames; }
   __device__ __forceinline__ long long tile_first() const { return items[blockIdx.x].tile_first; }
   __device__ __forceinline__ int n_tiles() const { return items[blockIdx.x].n_tiles; }
-  __device__ __forceinline__ double* out(int) const { return p.chunk_partials + (size_t)items[blockIdx.x].part * OBJ_SLOTS; }
+  __device__ __forceinline__ double* out(int) const { return p.chunk_partials + (size_t)items[blockIdx.x].part * OBJ_CHUNK_SLOTS; }
 };
 
 template <typename Src>
@@ -263,7 +263,7 @@ __global__ void __launch_bounds__(OBJ_NT, VND_OBJ_MINB) vn_objective_kernel(cons
   float* s0 = reinterpret_cast<float*>(smem_raw);
   float* s1 = s0 + 4 * span4;
   double* acc = reinterpret_cast<double*>(s1 + OBJ_TILE);
-  int* progs = reinterpret_cast<int*>(acc + (size_t)p.cand_per_group * OBJ_SLOTS);
+  int* progs = reinterpret_cast<int*>(acc + (size_t)p.cand_per_group * OBJ_CHUNK_SLOTS);
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   constexpr int kWarps = OBJ_NT / 32;
@@ -274,10 +274,7 @@ __global__ void __launch_bounds__(OBJ_NT, VND_OBJ_MINB) vn_objective_kernel(cons
   int* myprog = progs + warp * max_prog_words;
   int* mydec = progs + (kWarps + warp) * max_prog_words;
 
-  for (int i = tid; i < ncand * OBJ_SLOTS; i += OBJ_NT) {
-    const int slot = i % OBJ_SLOTS;
-    acc[i] = (slot == 7 || slot == 9) ? 1.0 : 0.0;  // ratio trackers start at 0 / 1
-  }
+  for (int i = tid; i < ncand * OBJ_CHUNK_SLOTS; i += OBJ_NT) acc[i] = obj_acc_init(i % OBJ_CHUNK_SLOTS);
 
   const long long tile_first = src.tile_first();
   for (int ti = 0; ti < src.n_tiles(); ++ti) {
@@ -353,40 +350,32 @@ __global__ void __launch_bounds__(OBJ_NT, VND_OBJ_MINB) vn_objective_kernel(cons
       a.sll = warp_sum(a.sll);
       warp_best_ratio(a.d_pos, a.s_pos);
       warp_best_ratio(a.d_neg, a.s_neg);
-      if (lane == 0) {
-        double* q = acc + (size_t)ci * OBJ_SLOTS;
-        q[0] += (double)a.sr;
-        q[1] += (double)a.srt;
-        q[2] += (double)a.srt2;
-        q[3] += (double)a.srt3;
-        q[4] += (double)a.slr;
-        q[5] += (double)a.sll;
-        if ((double)a.d_pos * q[7] > q[6] * (double)a.s_pos) { q[6] = a.d_pos; q[7] = a.s_pos; }
-        if ((double)a.d_neg * q[9] > q[8] * (double)a.s_neg) { q[8] = a.d_neg; q[9] = a.s_neg; }
-        q[10] += (double)nvalid;
-      }
+      if (lane == 0) obj_acc_tile(acc + (size_t)ci * OBJ_CHUNK_SLOTS, a, nvalid);
     }
   }
   __syncthreads();
   double* out = src.out(cand0);
-  for (int i = tid; i < ncand * OBJ_SLOTS; i += OBJ_NT) out[i] = acc[i];
+  for (int i = tid; i < ncand * OBJ_CHUNK_SLOTS; i += OBJ_NT) out[i] = acc[i];
 }
 
-// Fixed-order combine of the chunk partials: sums added chunk by chunk, ratio trackers by exact
-// cross multiplication (earlier chunk wins ties, like np.max keeps the value either way).  Chunk ch of the row is
-// q[ch * stride].
+// Fixed-order combine of the chunk partials (OBJ_CHUNK_SLOTS doubles each): the double-double sums added chunk by
+// chunk, high then low part, and rounded once to double at the end; ratio trackers by exact cross multiplication
+// (earlier chunk wins ties, like np.max keeps the value either way).  Chunk ch of the row is q[ch * stride]; the row
+// written to o has OBJ_SLOTS doubles.
 __device__ __forceinline__ void obj_combine_row(const double* __restrict__ q, size_t stride, int n_chunks, double* __restrict__ o) {
-  double r[OBJ_SLOTS];
-  for (int k = 0; k < OBJ_SLOTS; ++k) r[k] = 0.0;
-  r[7] = 1.0;
-  r[9] = 1.0;
+  double r[OBJ_CHUNK_SLOTS];
+  for (int k = 0; k < OBJ_CHUNK_SLOTS; ++k) r[k] = obj_acc_init(k);
   for (int ch = 0; ch < n_chunks; ++ch, q += stride) {
-    for (int k = 0; k < 6; ++k) r[k] += q[k];
+    for (int k = 0; k < 6; ++k) {
+      dd_add(r[k], r[12 + k], q[k]);
+      dd_add(r[k], r[12 + k], q[12 + k]);
+    }
     if (q[6] * r[7] > r[6] * q[7]) { r[6] = q[6]; r[7] = q[7]; }
     if (q[8] * r[9] > r[8] * q[9]) { r[8] = q[8]; r[9] = q[9]; }
     r[10] += q[10];
   }
-  for (int k = 0; k < OBJ_SLOTS; ++k) o[k] = r[k];
+  for (int k = 0; k < 6; ++k) o[k] = r[k] + r[12 + k];
+  for (int k = 6; k < OBJ_SLOTS; ++k) o[k] = r[k];
 }
 
 __global__ void obj_combine_kernel(const double* __restrict__ chunk_partials, double* __restrict__ partials, int n_clips,
@@ -394,7 +383,7 @@ __global__ void obj_combine_kernel(const double* __restrict__ chunk_partials, do
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= (long long)n_clips * n_cand) return;
   const int clip = (int)(idx / n_cand), cand = (int)(idx % n_cand);
-  obj_combine_row(chunk_partials + ((size_t)clip * n_chunks * n_cand + cand) * OBJ_SLOTS, (size_t)n_cand * OBJ_SLOTS, n_chunks,
+  obj_combine_row(chunk_partials + ((size_t)clip * n_chunks * n_cand + cand) * OBJ_CHUNK_SLOTS, (size_t)n_cand * OBJ_CHUNK_SLOTS, n_chunks,
                   partials + (size_t)idx * OBJ_SLOTS);
 }
 
@@ -409,7 +398,7 @@ __global__ void obj_combine_runs_kernel(const double* __restrict__ chunk_partial
                                         const ObjRunCombine* __restrict__ runs) {
   const ObjRunCombine r = runs[blockIdx.x];
   for (int j = threadIdx.x; j < r.count; j += blockDim.x)
-    obj_combine_row(chunk_partials + (size_t)(r.part + j) * OBJ_SLOTS, (size_t)r.count * OBJ_SLOTS, r.n_chunks,
+    obj_combine_row(chunk_partials + (size_t)(r.part + j) * OBJ_CHUNK_SLOTS, (size_t)r.count * OBJ_CHUNK_SLOTS, r.n_chunks,
                     partials + (size_t)(r.out + j) * OBJ_SLOTS);
 }
 
@@ -428,12 +417,12 @@ int obj_combine_launch(const double* chunk_partials, double* partials, int n_cli
 // program's two adds (0 + (0 + y0), which turns -0 into +0), the right value as it is, whole tiles with lane l owning
 // the four consecutive frames 128 j + 4 l + e and lane_acc_pair, the last partial tile with frames base + lane + 32 r
 // and lane_acc_frame, and the chunks of the one-candidate plan (plan_objective for the identity program) combined by
-// obj_combine_kernel.  The per-tile float32 lane sums and the float64 chunk sums therefore see the same values in the
-// same order.
+// obj_combine_kernel.  The per-tile float32 lane sums and the double-double chunk sums therefore see the same values in
+// the same order.
 //
 // The output is computed in the conflict-free layout (lane owns frames base + lane + 32 r, plain LDS per tap, as
 // vn_stereo_kernel reads) and passed through a per-warp scratch row into the four-consecutive-frames layout.
-// Shared memory: float x0[span] | float x1[span] | float scratch[warps][2][32 OBJ_R] | double acc[cand_per_group][OBJ_SLOTS]
+// Shared memory: float x0[span] | float x1[span] | float scratch[warps][2][32 OBJ_R] | double acc[cand_per_group][OBJ_CHUNK_SLOTS]
 //                | int prog[warps][2 max_prog_words]
 // ------------------------------------------------------------------------------------------------
 #ifndef VND_OBJ_STEREO_NT
@@ -446,7 +435,7 @@ struct VnStereoObjParams {
   const int* offsets;  // candidate j: channels 2 j and 2 j + 1
   const vnd_vn_stereo_cand* cands;
   int n_cand, apply_gain, halo, cand_per_group, tiles_per_chunk;
-  double* chunk_partials;  // [chunk][cand][OBJ_SLOTS]
+  double* chunk_partials;  // [chunk][cand][OBJ_CHUNK_SLOTS]
 };
 
 // One pass of one candidate: its output (l, r) at frames i0 + 32 rr of the staged tile.
@@ -476,7 +465,7 @@ __global__ void __launch_bounds__(VND_OBJ_STEREO_NT, 1) vn_stereo_objective_kern
   float* s1 = s0 + span_al;
   float* scratch = s1 + span_al;
   double* acc = reinterpret_cast<double*>(scratch + kWarps * 2 * kPass);
-  int* progs = reinterpret_cast<int*>(acc + (size_t)p.cand_per_group * OBJ_SLOTS);
+  int* progs = reinterpret_cast<int*>(acc + (size_t)p.cand_per_group * OBJ_CHUNK_SLOTS);
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int cand0 = blockIdx.y * p.cand_per_group;
@@ -487,10 +476,7 @@ __global__ void __launch_bounds__(VND_OBJ_STEREO_NT, 1) vn_stereo_objective_kern
   float* my1 = my0 + kPass;
   int* myprog = progs + warp * 2 * max_prog_words;
 
-  for (int i = tid; i < ncand * OBJ_SLOTS; i += VND_OBJ_STEREO_NT) {
-    const int slot = i % OBJ_SLOTS;
-    acc[i] = (slot == 7 || slot == 9) ? 1.0 : 0.0;  // ratio trackers start at 0 / 1
-  }
+  for (int i = tid; i < ncand * OBJ_CHUNK_SLOTS; i += VND_OBJ_STEREO_NT) acc[i] = obj_acc_init(i % OBJ_CHUNK_SLOTS);
 
   for (int ti = 0; ti < p.tiles_per_chunk; ++ti) {
     const long long t0 = ((long long)blockIdx.x * p.tiles_per_chunk + ti) * OBJ_TILE;
@@ -564,23 +550,12 @@ __global__ void __launch_bounds__(VND_OBJ_STEREO_NT, 1) vn_stereo_objective_kern
       a.sll = warp_sum(a.sll);
       warp_best_ratio(a.d_pos, a.s_pos);
       warp_best_ratio(a.d_neg, a.s_neg);
-      if (lane == 0) {
-        double* q = acc + (size_t)ci * OBJ_SLOTS;
-        q[0] += (double)a.sr;
-        q[1] += (double)a.srt;
-        q[2] += (double)a.srt2;
-        q[3] += (double)a.srt3;
-        q[4] += (double)a.slr;
-        q[5] += (double)a.sll;
-        if ((double)a.d_pos * q[7] > q[6] * (double)a.s_pos) { q[6] = a.d_pos; q[7] = a.s_pos; }
-        if ((double)a.d_neg * q[9] > q[8] * (double)a.s_neg) { q[8] = a.d_neg; q[9] = a.s_neg; }
-        q[10] += (double)nvalid;
-      }
+      if (lane == 0) obj_acc_tile(acc + (size_t)ci * OBJ_CHUNK_SLOTS, a, nvalid);
     }
   }
   __syncthreads();
-  double* out = p.chunk_partials + ((size_t)blockIdx.x * p.n_cand + cand0) * OBJ_SLOTS;
-  for (int i = tid; i < ncand * OBJ_SLOTS; i += VND_OBJ_STEREO_NT) out[i] = acc[i];
+  double* out = p.chunk_partials + ((size_t)blockIdx.x * p.n_cand + cand0) * OBJ_CHUNK_SLOTS;
+  for (int i = tid; i < ncand * OBJ_CHUNK_SLOTS; i += VND_OBJ_STEREO_NT) out[i] = acc[i];
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -858,10 +833,10 @@ static int obj_group_budget(int halo, int max_prog_words, size_t* fixed_out, int
   // VND_OBJ_MINB CTAs share the SM's 228 KB (1 KB of each is reserved by the system); a single CTA may take it all
   size_t budget = (size_t)(233472 / VND_OBJ_MINB - 1024);
   if (budget > (size_t)kMaxDynSmem) budget = (size_t)kMaxDynSmem;
-  if (fixed + OBJ_SLOTS * 8 * 16 > budget) budget = (size_t)kMaxDynSmem;  // long filters: one CTA per SM
-  if (fixed + OBJ_SLOTS * 8 * 16 > budget) return VND_EUNSUPPORTED;
+  if (fixed + OBJ_CHUNK_SLOTS * 8 * 16 > budget) budget = (size_t)kMaxDynSmem;  // long filters: one CTA per SM
+  if (fixed + OBJ_CHUNK_SLOTS * 8 * 16 > budget) return VND_EUNSUPPORTED;
   *fixed_out = fixed;
-  *cpg_out = (int)((budget - fixed) / (OBJ_SLOTS * 8));
+  *cpg_out = (int)((budget - fixed) / (OBJ_CHUNK_SLOTS * 8));
   return VND_OK;
 }
 
@@ -904,7 +879,7 @@ static int plan_objective(long long frames, int n_clips, int n_cand, int halo, i
   pl->n_groups = ceil_div(n_cand, cpg);
   pl->tiles_per_chunk = tpc;
   pl->n_chunks = (int)n_chunks;
-  pl->smem = fixed + (size_t)cpg * OBJ_SLOTS * 8;
+  pl->smem = fixed + (size_t)cpg * OBJ_CHUNK_SLOTS * 8;
   return VND_OK;
 }
 
@@ -916,7 +891,7 @@ int objective_workspace_bytes(long long frames, int n_clips, int n_cand, size_t*
   if (rc) return rc;
   const long long tiles = ceil_div<long long>(frames, OBJ_TILE);
   const long long chunks = max_chunks(tiles, n_clips, di.sm_count);
-  *bytes = (size_t)n_clips * chunks * n_cand * OBJ_SLOTS * 8 + 256;
+  *bytes = (size_t)n_clips * chunks * n_cand * OBJ_CHUNK_SLOTS * 8 + 256;
   const size_t tm_bytes = objective_tmem_workspace_bytes(frames, n_clips, n_cand, di.sm_count);  // the tensor-memory kernel tiles finer
   if (tm_bytes > *bytes) *bytes = tm_bytes;
   return VND_OK;
@@ -939,7 +914,7 @@ int vn_objective_launch(const float* clips, long long frames, int n_clips, long 
   int rc = plan_objective(frames, n_clips, cand->channels, halo, mpw, &pl);
   if (rc == VND_EUNSUPPORTED) set_error("objective kernel: filter halo %d does not fit in shared memory", halo);
   if (rc) return rc;
-  const size_t need = (size_t)n_clips * pl.n_chunks * cand->channels * OBJ_SLOTS * 8;
+  const size_t need = (size_t)n_clips * pl.n_chunks * cand->channels * OBJ_CHUNK_SLOTS * 8;
   VND_REQUIRE(workspace && workspace_bytes >= need, VND_ENOMEM, "objective workspace too small: need %zu bytes, have %zu", need,
               workspace_bytes);
   VND_REQUIRE(n_clips <= 65535 && pl.n_groups <= 65535, VND_EUNSUPPORTED, "too many clips/candidate groups for one launch");
@@ -999,7 +974,7 @@ int objective_runs_workspace_bytes(const long long* offs, const int* run_clip, c
   int rc = device_info(&di);
   if (rc) return rc;
   const long long rows = runs_partial_rows_bound(offs, run_clip, run_count, n_runs, di.sm_count);
-  *bytes = runs_table_bytes(rows, n_runs) + (size_t)rows * OBJ_SLOTS * 8 + 256;
+  *bytes = runs_table_bytes(rows, n_runs) + (size_t)rows * OBJ_CHUNK_SLOTS * 8 + 256;
   return VND_OK;
 }
 
@@ -1085,7 +1060,7 @@ static int plan_runs(const long long* offs, const int* run_clip, const int* run_
       }
     }
   pl->cand_per_group = cpg;
-  pl->smem = fixed + (size_t)cpg * OBJ_SLOTS * 8;
+  pl->smem = fixed + (size_t)cpg * OBJ_CHUNK_SLOTS * 8;
   pl->partial_rows = rows;
   return VND_OK;
 }
@@ -1110,7 +1085,7 @@ int vn_objective_runs_launch(const float* x, long long chan_stride, const long l
   if (rc) return rc;
   VND_REQUIRE(pl.items.size() <= 0x7fffffffu, VND_EUNSUPPORTED, "too many work items for one launch");
   const size_t table = runs_table_bytes((long long)pl.items.size(), (long long)pl.comb.size());
-  const size_t need = table + (size_t)pl.partial_rows * OBJ_SLOTS * 8;
+  const size_t need = table + (size_t)pl.partial_rows * OBJ_CHUNK_SLOTS * 8;
   VND_REQUIRE(workspace && workspace_bytes >= need, VND_ENOMEM, "objective workspace too small: need %zu bytes, have %zu", need, workspace_bytes);
   // the tables, one copy: work items, then the combine table
   std::vector<unsigned char> host(table);
@@ -1176,7 +1151,7 @@ int vn_stereo_objective_workspace_bytes(long long frames, int n_cand, size_t* by
   int rc = device_info(&di);
   if (rc) return rc;
   const long long chunks = max_chunks(ceil_div<long long>(frames, OBJ_TILE), 1, di.sm_count);  // plan_objective's cap for one clip
-  *bytes = (size_t)chunks * n_cand * OBJ_SLOTS * 8 + 256;
+  *bytes = (size_t)chunks * n_cand * OBJ_CHUNK_SLOTS * 8 + 256;
   return VND_OK;
 }
 
@@ -1195,15 +1170,15 @@ int vn_stereo_objective_launch(const float* x, long long frames, long long chan_
   const int mpw = taps->max_channel_words > 0 ? taps->max_channel_words : 1;
   constexpr int kWarps = VND_OBJ_STEREO_NT / 32;
   const size_t fixed = (size_t)2 * ((OBJ_TILE + halo + 3) & ~3) * 4 + (size_t)kWarps * 2 * 32 * OBJ_R * 4 + (size_t)kWarps * 2 * mpw * 4 + 64;
-  if (fixed + (size_t)OBJ_SLOTS * 8 > (size_t)kMaxDynSmem) return VND_EUNSUPPORTED;  // the caller scores candidate by candidate
-  int cpg = (int)((kMaxDynSmem - fixed) / (OBJ_SLOTS * 8));
+  if (fixed + (size_t)OBJ_CHUNK_SLOTS * 8 > (size_t)kMaxDynSmem) return VND_EUNSUPPORTED;  // the caller scores candidate by candidate
+  int cpg = (int)((kMaxDynSmem - fixed) / (OBJ_CHUNK_SLOTS * 8));
   if (cpg > n_cand) cpg = n_cand;
   if (cpg > 1024) cpg = 1024;
   // groups small enough for about four CTAs per SM, never fewer candidates than warps
   while ((long long)chunks.n_chunks * ceil_div(n_cand, cpg) < (long long)di.sm_count * 4 && cpg > kWarps) cpg = (cpg + 1) / 2;
   const int groups = ceil_div(n_cand, cpg);
   VND_REQUIRE(groups <= 65535, VND_EUNSUPPORTED, "too many candidate groups for one launch");
-  const size_t need = (size_t)chunks.n_chunks * n_cand * OBJ_SLOTS * 8;
+  const size_t need = (size_t)chunks.n_chunks * n_cand * OBJ_CHUNK_SLOTS * 8;
   VND_REQUIRE(workspace && workspace_bytes >= need, VND_ENOMEM, "objective workspace too small: need %zu bytes, have %zu", need, workspace_bytes);
   VnStereoObjParams p{};
   p.x = x;
@@ -1218,7 +1193,7 @@ int vn_stereo_objective_launch(const float* x, long long frames, long long chan_
   p.cand_per_group = cpg;
   p.tiles_per_chunk = chunks.tiles_per_chunk;
   p.chunk_partials = reinterpret_cast<double*>(workspace);
-  const size_t smem = fixed + (size_t)cpg * OBJ_SLOTS * 8;
+  const size_t smem = fixed + (size_t)cpg * OBJ_CHUNK_SLOTS * 8;
   VND_CUDA_OK(cudaFuncSetAttribute(vn_stereo_objective_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   vn_stereo_objective_kernel<<<dim3((unsigned)chunks.n_chunks, (unsigned)groups), VND_OBJ_STEREO_NT, smem, st>>>(p, mpw);
   if ((rc = after_launch("vn_stereo_objective_kernel"))) return rc;

@@ -9,6 +9,9 @@
 namespace vnd {
 
 constexpr int OBJ_SLOTS = 12;  // doubles per (clip, candidate) partial, see vnd_b200.h
+// doubles per candidate in a CTA's accumulators and per chunk partial: the 12 slots, then the low parts of the
+// double-double sums of slots 0-5
+constexpr int OBJ_CHUNK_SLOTS = 18;
 #ifndef VND_OBJ_NT
 #define VND_OBJ_NT 640  // 20 warps: measured best of 512 / 640 / 768 / 896 / 1024 threads (16 frames per lane)
 #endif
@@ -30,7 +33,7 @@ struct ObjParams {
   int cand_per_group;
   int tiles_per_chunk;
   int n_chunks;
-  double* chunk_partials;  // [clip][chunk][cand][OBJ_SLOTS]
+  double* chunk_partials;  // [clip][chunk][cand][OBJ_CHUNK_SLOTS]
 };
 
 // One CTA of the run-list objective (vnd_vn_objective_runs_dev): a chunk of one clip's tiles on one group of one run's
@@ -38,7 +41,7 @@ struct ObjParams {
 struct ObjRunItem {
   long long base;    // packed column of the clip's frame 0
   long long frames;  // the clip's length
-  long long part;    // first chunk-partial row (OBJ_SLOTS doubles) of the item
+  long long part;    // first chunk-partial row (OBJ_CHUNK_SLOTS doubles) of the item
   int tile_first, n_tiles, cand0, ncand;
 };
 
@@ -126,8 +129,9 @@ __device__ __forceinline__ void lane_acc_frame(LaneAcc& a, float l, float r_) {
 //
 // Instruction diet (ncu, round 2: ~93 of the ~116 instructions a frame-evaluation costs are these moments, not the
 // taps): the radius uses sqrt.approx (2 ulp; it only enters amplitude-weighted sums, whose weights make 1e-7 relative
-// irrelevant), min/max uses rcp.approx on a denominator clamped to FLT_MIN instead of div.approx's denormal scaling
-// (frames below 1e-38 carry no weight), and the exact max|theta| tracker is entered through ONE test per pair on a
+// irrelevant; it flushes subnormal squares, whose frames take the rare path below), min/max uses rcp.approx on a
+// denominator clamped to FLT_MIN instead of div.approx's denormal scaling (frames below 1e-38 carry no weight), and the
+// exact max|theta| tracker is entered through ONE test per pair on a
 // key that is monotone in |d|/|s| (key = t or 2 - t with t = min/max): a frame can only beat the record if its key is
 // within the key's rounding error (< 1e-6) of the record's.
 struct LaneAcc2 {
@@ -142,9 +146,14 @@ __device__ __forceinline__ float obj_rcp(float x) {
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
-__device__ __forceinline__ float obj_sqrt(float x) {
+__device__ __forceinline__ float obj_sqrt(float x) {  // flushes a subnormal x to 0
   float y;
   asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+__device__ __forceinline__ float obj_sqrt_keep(float x) {  // a subnormal x keeps its root (a few more instructions)
+  float y;
+  asm("sqrt.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
 
@@ -169,6 +178,15 @@ __device__ __forceinline__ void track_exact(LaneAcc2& a, float ad, float as, flo
       a.k_neg = key - kKeyMargin;
     }
   }
+}
+
+// the r-weighted terms of a radius into chain c of the sums, as lane_acc_pair adds them
+__device__ __forceinline__ void obj_add_radius(LaneAcc2& a, int c, float rad, float th) {
+  const float rt = rad * th;
+  a.sr[c] += rad;
+  a.srt[c] += rt;
+  a.srt2[c] = fmaf(rt, th, a.srt2[c]);
+  a.srt3[c] = fmaf(rt * th, th, a.srt3[c]);
 }
 
 __device__ __forceinline__ void lane_acc_pair(LaneAcc2& a, float l0, float l1, float r0, float r1) {
@@ -218,14 +236,47 @@ __device__ __forceinline__ void lane_acc_pair(LaneAcc2& a, float l0, float l1, f
   obj_fma2(v0, v1, l0, l1, a.sll[0], a.sll[1]);
   a.sll[0] = v0;
   a.sll[1] = v1;
-  // max|theta| candidates: one test per pair; frames below FLT_MIN (their key is meaningless) always take the exact path
+  // max|theta| candidates: one test per pair.  Frames whose root came out 0 always take the rare path: their key is
+  // meaningless when max(|d|, |s|) < FLT_MIN (then l*l + r*r is 0), and a subnormal l*l + r*r (|l|, |r| below ~1e-19)
+  // was flushed by sqrt.approx.ftz: its radius is taken again there with subnormals kept and added to the sums right
+  // behind the 0 that stood for it, which gives the bits the kept radius would have given in place.
   const float k0 = steep0 ? 2.0f - t0 : t0, k1 = steep1 ? 2.0f - t1 : t1;
   const bool pos0 = s0 >= 0.0f, pos1 = s1 >= 0.0f;
-  const bool hit0 = k0 >= (pos0 ? a.k_pos : a.k_neg) || mx0 < kTiny, hit1 = k1 >= (pos1 ? a.k_pos : a.k_neg) || mx1 < kTiny;
+  const bool hit0 = k0 >= (pos0 ? a.k_pos : a.k_neg) || rad0 == 0.0f, hit1 = k1 >= (pos1 ? a.k_pos : a.k_neg) || rad1 == 0.0f;
   if (hit0 || hit1) {
+    if (rad0 == 0.0f) obj_add_radius(a, 0, obj_sqrt_keep(q0), th0);
+    if (rad1 == 0.0f) obj_add_radius(a, 1, obj_sqrt_keep(q1), th1);
     if (hit0) track_exact(a, ad0, as0, k0, pos0);
-    if (k1 >= (pos1 ? a.k_pos : a.k_neg) || mx1 < kTiny) track_exact(a, ad1, as1, k1, pos1);  // against the record frame 0 may just have set
+    if (k1 >= (pos1 ? a.k_pos : a.k_neg) || rad1 == 0.0f) track_exact(a, ad1, as1, k1, pos1);  // against the record frame 0 may just have set
   }
+}
+
+// (hi, lo) += v with hi + lo exact (TwoSum, then renormalised so that |lo| <= ulp(hi) / 2).  Every operation is exact
+// while the addends are float32 values (or such sums) spanning fewer than about 70 binades, so the pair holds the exact
+// sum and hi + lo rounds it once, whatever the order of the additions (DESIGN.md section 6).
+__device__ __forceinline__ void dd_add(double& hi, double& lo, double v) {
+  const double s = hi + v, vb = s - hi;
+  const double e = (hi - (s - vb)) + (v - vb);
+  const double t = lo + e;
+  hi = s + t;
+  const double tb = hi - s;
+  lo = (s - (hi - tb)) + (t - tb);
+}
+
+// A candidate's accumulators (OBJ_CHUNK_SLOTS doubles) as a CTA starts: sums zero, ratio trackers at 0 / 1.
+__device__ __forceinline__ double obj_acc_init(int slot) { return (slot == 7 || slot == 9) ? 1.0 : 0.0; }
+
+// One tile's warp-reduced lane sums into a candidate's accumulators q (lane 0 of the warp).
+__device__ __forceinline__ void obj_acc_tile(double* q, const LaneAcc& a, int nvalid) {
+  dd_add(q[0], q[12], (double)a.sr);
+  dd_add(q[1], q[13], (double)a.srt);
+  dd_add(q[2], q[14], (double)a.srt2);
+  dd_add(q[3], q[15], (double)a.srt3);
+  dd_add(q[4], q[16], (double)a.slr);
+  dd_add(q[5], q[17], (double)a.sll);
+  if ((double)a.d_pos * q[7] > q[6] * (double)a.s_pos) { q[6] = a.d_pos; q[7] = a.s_pos; }
+  if ((double)a.d_neg * q[9] > q[8] * (double)a.s_neg) { q[8] = a.d_neg; q[9] = a.s_neg; }
+  q[10] += (double)nvalid;
 }
 
 __device__ __forceinline__ float warp_sum(float v) {

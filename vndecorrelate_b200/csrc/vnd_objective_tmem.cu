@@ -67,7 +67,8 @@ struct OtParams {
   int mpw;   // words of the longest candidate program
 };
 
-// Shared memory: [0, 16) TMEM base | float in[nblk][100] | float x1[32][100] | double acc[cand_per_group][12] | int scratch[warps][ot_warp_words]
+// Shared memory: [0, 16) TMEM base | float in[nblk][100] | float x1[32][100] | double acc[cand_per_group][OBJ_CHUNK_SLOTS] |
+//                int scratch[warps][ot_warp_words]
 extern __shared__ __align__(128) unsigned char ot_smem[];
 
 // Decode candidate `prog` (SEGMENTED block: S, (n_neg, n_pos, gain) x S, taps) for the warp: operation words per group
@@ -118,7 +119,7 @@ __global__ void __launch_bounds__(T::NT, 1) vn_objective_tmem_kernel(const OtPar
   const int in_words = (P.nblk * OT_PITCH + 3) & ~3;
   float* s_x1 = s_in + in_words;
   double* acc = reinterpret_cast<double*>(s_x1 + OT_ROWS * OT_PITCH);
-  int* scratch = reinterpret_cast<int*>(acc + (size_t)p.cand_per_group * OBJ_SLOTS);
+  int* scratch = reinterpret_cast<int*>(acc + (size_t)p.cand_per_group * OBJ_CHUNK_SLOTS);
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int chunk = blockIdx.x, clip = blockIdx.y, group = blockIdx.z;
@@ -132,10 +133,7 @@ __global__ void __launch_bounds__(T::NT, 1) vn_objective_tmem_kernel(const OtPar
   int4* mysegs = reinterpret_cast<int4*>(myops + OT_G * opstride);
 
   if (warp == 0) tmem_alloc_all(tm_slot);
-  for (int i = tid; i < ncand * OBJ_SLOTS; i += OT_NT) {
-    const int slot = i % OBJ_SLOTS;
-    acc[i] = (slot == 7 || slot == 9) ? 1.0 : 0.0;  // ratio trackers start at 0 / 1
-  }
+  for (int i = tid; i < ncand * OBJ_CHUNK_SLOTS; i += OT_NT) acc[i] = obj_acc_init(i % OBJ_CHUNK_SLOTS);
   tmem_fence_before();
   __syncthreads();
   tmem_fence_after();
@@ -256,24 +254,13 @@ __global__ void __launch_bounds__(T::NT, 1) vn_objective_tmem_kernel(const OtPar
       a.sll = warp_sum(a.sll);
       warp_best_ratio(a.d_pos, a.s_pos);
       warp_best_ratio(a.d_neg, a.s_neg);
-      if (lane == 0) {
-        double* qd = acc + (size_t)ci * OBJ_SLOTS;
-        qd[0] += (double)a.sr;
-        qd[1] += (double)a.srt;
-        qd[2] += (double)a.srt2;
-        qd[3] += (double)a.srt3;
-        qd[4] += (double)a.slr;
-        qd[5] += (double)a.sll;
-        if ((double)a.d_pos * qd[7] > qd[6] * (double)a.s_pos) { qd[6] = a.d_pos; qd[7] = a.s_pos; }
-        if ((double)a.d_neg * qd[9] > qd[8] * (double)a.s_neg) { qd[8] = a.d_neg; qd[9] = a.s_neg; }
-        qd[10] += (double)(remain < OT_TILE ? remain : OT_TILE);
-      }
+      if (lane == 0) obj_acc_tile(acc + (size_t)ci * OBJ_CHUNK_SLOTS, a, (int)(remain < OT_TILE ? remain : OT_TILE));
     }
   }
   tmem_fence_before();
   __syncthreads();
-  double* out = p.chunk_partials + (((size_t)clip * p.n_chunks + chunk) * p.n_cand + cand0) * OBJ_SLOTS;
-  for (int i = tid; i < ncand * OBJ_SLOTS; i += OT_NT) out[i] = acc[i];
+  double* out = p.chunk_partials + (((size_t)clip * p.n_chunks + chunk) * p.n_cand + cand0) * OBJ_CHUNK_SLOTS;
+  for (int i = tid; i < ncand * OBJ_CHUNK_SLOTS; i += OT_NT) out[i] = acc[i];
   if (warp == 0) tmem_dealloc_all(*tm_slot);
 }
 
@@ -298,7 +285,7 @@ static int ot_variant() {
 
 size_t objective_tmem_workspace_bytes(long long frames, int n_clips, int n_cand, int sm_count) {
   const long long tiles = ceil_div<long long>(frames, OtNarrow::TILE);  // the finer tiling of the two shapes
-  return (size_t)n_clips * ot_max_chunks(tiles, n_clips, sm_count) * n_cand * OBJ_SLOTS * 8 + 256;
+  return (size_t)n_clips * ot_max_chunks(tiles, n_clips, sm_count) * n_cand * OBJ_CHUNK_SLOTS * 8 + 256;
 }
 
 // VND_EUNSUPPORTED (no error text) when the program family does not qualify; the caller then runs vn_objective_kernel.
@@ -318,8 +305,8 @@ static int ot_launch(const float* clips, long long frames, int n_clips, long lon
   const size_t in_words = ((size_t)nblk * OT_PITCH + 3) & ~(size_t)3;
   const size_t fixed = 16 + (in_words + (size_t)OT_ROWS * OT_PITCH) * 4 + (size_t)OT_WARPS * ot_warp_words(mpw) * 4;
   const size_t budget = (size_t)kMaxDynSmem;
-  if (fixed + OBJ_SLOTS * 8 * 16 > budget) return VND_EUNSUPPORTED;
-  int cpg = (int)((budget - fixed) / (OBJ_SLOTS * 8));
+  if (fixed + OBJ_CHUNK_SLOTS * 8 * 16 > budget) return VND_EUNSUPPORTED;
+  int cpg = (int)((budget - fixed) / (OBJ_CHUNK_SLOTS * 8));
   if (cpg > cand->channels) cpg = cand->channels;
   if (cpg > 1024) cpg = 1024;
   const long long tiles = ceil_div<long long>(frames, OT_TILE);
@@ -345,7 +332,7 @@ static int ot_launch(const float* clips, long long frames, int n_clips, long lon
     if (v > 0 && ceil_div<long long>(tiles, v) <= cap) tpc = v;
   }
   n_chunks = ceil_div<long long>(tiles, tpc);
-  const size_t need = (size_t)n_clips * n_chunks * cand->channels * OBJ_SLOTS * 8;
+  const size_t need = (size_t)n_clips * n_chunks * cand->channels * OBJ_CHUNK_SLOTS * 8;
   VND_REQUIRE(workspace && workspace_bytes >= need, VND_ENOMEM, "objective workspace too small: need %zu bytes, have %zu", need, workspace_bytes);
   OtParams P{};
   P.o.clips = clips;
@@ -363,7 +350,7 @@ static int ot_launch(const float* clips, long long frames, int n_clips, long lon
   P.o.chunk_partials = reinterpret_cast<double*>(workspace);
   P.nblk = nblk;
   P.mpw = mpw;
-  const size_t smem = fixed + (size_t)cpg * OBJ_SLOTS * 8;
+  const size_t smem = fixed + (size_t)cpg * OBJ_CHUNK_SLOTS * 8;
   VND_CUDA_OK(cudaFuncSetAttribute(vn_objective_tmem_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   dim3 grid((unsigned)n_chunks, (unsigned)n_clips, (unsigned)groups);
   vn_objective_tmem_kernel<T><<<grid, OT_NT, smem, st>>>(P);
