@@ -334,9 +334,9 @@ int vnd_haas_objective_pairs_dev(const float* x, int64_t rows, int64_t chan_stri
  * A filter whose halo (clamped to the longest clip of the runs) does not fit in shared memory returns VND_EUNSUPPORTED
  * before any launch.  n_runs == 0 launches nothing.
  * Bit contract: the 12 partials of (run r, candidate j) equal, bit for bit, row j of what vnd_vn_objective_batch_dev
- * returns for clip run_clip[r] alone (planar) with the one channel run_cand[r] + j as its program (shared-memory kernel,
- * VND_OBJ_TMEM unset): tiles are counted from frame 0 of each clip, staging reads nothing past the clip's last frame,
- * and the chunk partials are added in tile order. */
+ * returns for clip run_clip[r] alone (planar) with the one channel run_cand[r] + j as its program: tiles are counted
+ * from frame 0 of each clip, staging reads nothing past the clip's last frame, and the chunk partials are added in tile
+ * order. */
 int vnd_vn_objective_runs_workspace(const int64_t* frame_offsets, int32_t n_clips, const int32_t* run_clip, const int32_t* run_count,
                                     int32_t n_runs, size_t* bytes);
 int vnd_vn_objective_runs_dev(const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets, int32_t n_clips,
@@ -362,11 +362,11 @@ typedef struct vnd_vn_stereo_cand {
  *   cands    : n_cand settings records (device);
  *   partials : n_cand * 12 float64 on the device, the slots of vnd_vn_objective_batch_dev.
  * Bit contract: candidate j's 12 partials equal, bit for bit, those of vnd_vn_objective_batch_dev on the float32 output
- * of vnd_vn_decorrelate_dev for that candidate (planar, with the one-tap identity program; shared-memory kernel).  The
+ * of vnd_vn_decorrelate_dev for that candidate (planar, with the one-tap identity program).  The
  * output is never stored: the kernel builds it in registers with the same tap loop and epilogue and feeds the moments
  * with the same frame-to-lane mapping, tiles and chunks.  Checked before any launch: the program (SEGMENTED, 2 n_cand
  * channels), the sizes and the pointers.  VND_EUNSUPPORTED (no launch) when the program's halo does not fit shared
- * memory or VND_OBJ_TMEM selects the tensor-memory objective: the caller then scores candidate by candidate.
+ * memory: the caller then scores candidate by candidate.
  * Workspace: vnd_vn_stereo_objective_workspace bytes, 256-byte aligned. */
 int vnd_vn_stereo_objective_workspace(int64_t frames, int32_t n_cand, size_t* bytes);
 int vnd_vn_stereo_objective_dev(const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,

@@ -483,41 +483,6 @@ def test_more_randomised_families_against_the_oracle(api, family):
             assert G.same_bits(np.ascontiguousarray(got_t.cpu().numpy()), want), (family, i, p, "tensor path")
 
 
-@pytest.mark.parametrize("shape", list(range(1, 16)))
-def test_tmem_kernel_variants_are_bit_exact(api, shape):
-    """Every measured variant of the tensor-memory kernel (shapes, software pipelining, paired first / far segments,
-    alternating far phases, far-first, two taps per round trip; vnd_fir_tmem.cu: fir_tmem_launch) must produce the default kernel's - the oracle's -
-    bits: the reference's operations in the reference's order, however the work is scheduled.  Three programs: the
-    BASELINE shape of filter, uniform impulses (most taps outside the TMEM window, no paired loop) and a two-segment
-    envelope with a negative gain."""
-    import torch
-
-    from vndecorrelate_b200 import _native as N
-
-    lib = N.lib()
-    lib.vnd_debug_set_tm_shape.argtypes = [C.c_int]
-    lib.vnd_debug_set_tm_shape.restype = C.c_int
-    Cn = 5
-    filtered = (0, 1, 2, 3)
-    prev = lib.vnd_debug_set_tm_shape(shape)
-    try:
-        for kappa, envelope, frames in ((1.0, (0.85, 0.55, 0.35, 0.2), 190001), (0.0, (0.85, 0.55, 0.35, 0.2), 170003), (1.0, (0.9, -0.5), 160000)):
-            vn = api.VelvetNoise(sample_rate_hz=48000, duration_seconds=0.03, num_impulses=30, num_outs=Cn, filtered_channels=filtered, mode="LR",
-                                 normalizer=None, log_distribution_strength=kappa, segment_envelope=envelope, seed=11)
-            g = torch.Generator(device="cuda").manual_seed(7 + shape)
-            slab = torch.randn((Cn, frames), generator=g, device="cuda") * 0.1
-            y = vn.convolve(slab.t())
-            taps = O.class_taps(sample_rate_hz=48000, duration_seconds=0.03, num_impulses=30, num_outs=Cn, filtered_channels=filtered,
-                                num_segments=len(envelope), log_distribution_strength=kappa, seed=11)
-            want = O.fir_class_order(np.ascontiguousarray(slab.cpu().numpy().T), taps, envelope, Cn)
-            got = np.ascontiguousarray(y.cpu().numpy())
-            if not G.same_bits(got, want):
-                bad = np.argwhere(got.view(np.uint32) != want.view(np.uint32))
-                raise AssertionError(f"shape {shape}, strength {kappa}: {len(bad)} samples differ; first at (frame, channel) {bad[0]}")
-    finally:
-        lib.vnd_debug_set_tm_shape(prev)
-
-
 def test_many_channels_every_sample(api):
     """600 channels x 65 000 frames (more runs than four waves of persistent CTAs, one tap table sliced over all of them):
     EVERY output sample of every channel against the oracle, not just windows of the first and the last channel as in
@@ -847,39 +812,6 @@ def test_cfg5_full_shape_one_clip(api):
     assert abs(float(kappa[0]) - ref["kappa"]) <= 1e-4, (float(kappa[0]), ref["kappa"])
     single = OPT.optimize_velvet_noise(input_signal=clip, **kw)  # the one-clip entry point is the same computation
     assert float(single) == float(kappa[0])
-
-
-@pytest.mark.parametrize("variant", ["1", "2"])
-def test_objective_tensor_memory_variants(api, monkeypatch, variant):
-    """The opt-in tensor-memory objective kernels (VND_OBJ_TMEM=1: 16 frames per lane x 20 warps, 2: 32 x 12) against the
-    default shared-memory kernel and the oracle: same argmin, scores within the float32 evaluation noise, the exact
-    max|theta| tracker identical (slots 6-9 of the partial sums), on whole tiles, a ragged last tile and a clip shorter
-    than the filter."""
-    from vndecorrelate_b200 import optimization as OPT
-    from vndecorrelate_b200 import taps as T
-
-    kw = dict(angle_limit=np.pi / 4, lambda_mean=5.0, lambda_skew=2.0, lambda_correlation=15.0, lambda_penalty=1e3)
-    for frames, grid in ((50000, 24), (3072 * 3, 7), (1000, 5)):
-        clips = np.stack([O.coloured_clip(i, frames).T for i in range(2)])
-        ks = np.linspace(0.0, 1.0, grid)
-        prog = T.kappa_family_program(ks, sample_rate_hz=48000, duration_seconds=0.03, num_impulses=30, envelope=(0.85, 0.55, 0.35, 0.2), seed=1,
-                                      frames=frames)
-        if prog is None:
-            prog = T.candidate_program([T.generate_tap_table(sample_rate_hz=48000, duration_seconds=0.03, num_impulses=30, num_outs=2, num_segments=4,
-                                                             log_distribution_strength=float(k), filtered_channels=(0,), seed=1) for k in ks],
-                                       (0.85, 0.55, 0.35, 0.2), frames)
-        monkeypatch.delenv("VND_OBJ_TMEM", raising=False)
-        base = OPT.vn_objective_partials(clips, prog)
-        monkeypatch.setenv("VND_OBJ_TMEM", variant)
-        got = OPT.vn_objective_partials(clips, prog)
-        monkeypatch.delenv("VND_OBJ_TMEM")
-        assert np.array_equal(got[..., 6:11], base[..., 6:11])  # tracked frames and frame counts: exact
-        assert np.allclose(got[..., :6], base[..., :6], rtol=2e-6, atol=1e-9)
-        s_got, s_base = OPT.vn_scores_from_partials(got, **kw), OPT.vn_scores_from_partials(base, **kw)
-        assert np.max(np.abs(s_got.astype(np.float64) - s_base.astype(np.float64))) <= 2e-4
-        ref = np.stack([O.vn_grid_scores(np.ascontiguousarray(c.T), ks, sample_rate_hz=48000, duration_seconds=0.03, num_impulses=30, seed=1) for c in clips])
-        assert np.max(np.abs(s_got.astype(np.float64) - ref.astype(np.float64))) <= 5e-4
-        assert [int(np.argmin(r)) for r in s_got] == [int(np.argmin(r)) for r in ref]
 
 
 def test_empty_clip_is_an_error_not_a_crash(api):

@@ -412,17 +412,15 @@ def test_probe_sensitivity(name):
 
 # ------------------------------------------------------------------ GPU: velvet-noise objective, every kernel
 
-VARIANTS = [None, "1", "2"]  # shared-memory kernel, tensor-memory 16 x 20 warps, tensor-memory 32 x 12 warps
-
-
 @pytest.fixture
-def variant_env(monkeypatch):
-    def use(variant, tpc=None):
-        for k, v in (("VND_OBJ_TMEM", variant), ("VND_OBJ_TPC", tpc)):
-            if v is None:
-                monkeypatch.delenv(k, raising=False)
-            else:
-                monkeypatch.setenv(k, v)
+def tpc_env(monkeypatch):
+    """Sets VND_OBJ_TPC (the tiles per chunk of the objective's chunk plan; None: the planned chunks)."""
+
+    def use(tpc=None):
+        if tpc is None:
+            monkeypatch.delenv("VND_OBJ_TPC", raising=False)
+        else:
+            monkeypatch.setenv("VND_OBJ_TPC", tpc)
 
     use(None)
     return use
@@ -433,10 +431,8 @@ def _lengths(halo):
 
 
 @gpu
-@pytest.mark.parametrize("variant", VARIANTS)
 @pytest.mark.parametrize("fam_name", ["std", "long", "identity_env", "seg150"])
-def test_vn_partials_against_reference(variant_env, variant, fam_name):
-    variant_env(variant)
+def test_vn_partials_against_reference(tpc_env, fam_name):
     fam = family(fam_name)
     for frames in _lengths(fam.max_tap + 1):
         x = O.coloured_clip(frames % 7, frames) if frames > 1 else dense_clip(1)
@@ -446,19 +442,16 @@ def test_vn_partials_against_reference(variant_env, variant, fam_name):
 
 
 @gpu
-def test_vn_partials_thirty_seconds(variant_env):
+def test_vn_partials_thirty_seconds(tpc_env):
     fam = family("std")
     x = O.coloured_clip(3, 30 * FS)
-    refs = [O.objective_partials(fam.output(x, j)) for j in range(len(fam.kappas))]
-    for variant in VARIANTS:
-        variant_env(variant)
-        got = opt.vn_objective_partials(x, fam.program(len(x)))[0]
-        for j, ref in enumerate(refs):
-            check_vn(got[j], ref, f"30 s variant={variant} cand={j}")
+    got = opt.vn_objective_partials(x, fam.program(len(x)))[0]
+    for j in range(len(fam.kappas)):
+        check_vn(got[j], O.objective_partials(fam.output(x, j)), f"30 s cand={j}")
 
 
 @gpu
-def test_filter_beyond_shared_memory_is_refused(variant_env):
+def test_filter_beyond_shared_memory_is_refused(tpc_env):
     """A 1000-segment envelope's program does not fit the shared-memory budget of any objective kernel: an error, not a
     result."""
     fam = VnFamily([0.5], duration=0.03, num_impulses=1000 // 4, envelope=tuple(np.linspace(1.0, 0.1, 1000)))
@@ -469,7 +462,7 @@ def test_filter_beyond_shared_memory_is_refused(variant_env):
 
 @gpu
 @pytest.mark.parametrize("n_cand", [15, 16, 17, 40])
-def test_candidate_groups_and_chunk_plans(variant_env, n_cand):
+def test_candidate_groups_and_chunk_plans(tpc_env, n_cand):
     """Groups shrink to 16 candidates on a short clip; every chunk size must give the reference."""
     fam = VnFamily(np.linspace(0.0, 1.0, n_cand))
     frames = 3 * TILE + 5
@@ -478,7 +471,7 @@ def test_candidate_groups_and_chunk_plans(variant_env, n_cand):
     refs = [O.objective_partials(fam.output(x, j)) for j in range(n_cand)]
     first = None
     for tpc in ("1", "2", "3", None):
-        variant_env(None, tpc)
+        tpc_env(tpc)
         got = opt.vn_objective_partials(np.stack([x.T, x.T[::-1]]), prog)
         for j in range(n_cand):
             check_vn(got[0, j], refs[j], f"tpc={tpc} cand={j}")
@@ -487,16 +480,14 @@ def test_candidate_groups_and_chunk_plans(variant_env, n_cand):
 
 
 @gpu
-@pytest.mark.parametrize("variant", VARIANTS)
-def test_vn_probes(variant_env, variant):
-    variant_env(variant)
+def test_vn_probes(tpc_env):
     for name, (x, fam, sums, _) in probes().items():
         got = opt.vn_objective_partials(x, probe_program(name, len(x)))[0, 0]
-        check_vn(got, probe_ref(name), f"{name} variant={variant}", sums=True)
+        check_vn(got, probe_ref(name), name, sums=True)
 
 
 @gpu
-def test_run_list_probes_and_ragged_batches(variant_env):
+def test_run_list_probes_and_ragged_batches(tpc_env):
     """Every probe and 1-frame and ordinary clips packed in one buffer, loud neighbours around each, with runs of count
     0: one run-list call, every row against the reference."""
     loud = dense_clip(TILE + 3, seed=9, scale=3e4)
@@ -537,15 +528,13 @@ def test_run_list_probes_and_ragged_batches(variant_env):
 
 
 @gpu
-def test_loud_overflow_scores_are_non_finite_where_the_reference_is(variant_env):
+def test_loud_overflow_scores_are_non_finite_where_the_reference_is(tpc_env):
     x = loud_overflow_clip()
     fam = family("std")
     with np.errstate(all="ignore"):
         want = [O.objective(fam.output(x, j), **KW) for j in range(len(fam.kappas))]
-        for variant in VARIANTS:
-            variant_env(variant)
-            got = opt.vn_scores_from_partials(opt.vn_objective_partials(x, fam.program(len(x))), **KW)[0]
-            assert [bool(np.isfinite(g)) for g in got] == [bool(np.isfinite(w)) for w in want], variant
+        got = opt.vn_scores_from_partials(opt.vn_objective_partials(x, fam.program(len(x))), **KW)[0]
+        assert [bool(np.isfinite(g)) for g in got] == [bool(np.isfinite(w)) for w in want]
         ok = dense_clip(len(x))
         got = opt.vn_scores_from_partials(opt.vn_objective_partials(ok, fam.program(len(ok))), **KW)[0]
         assert np.all(np.isfinite(got))
@@ -555,7 +544,7 @@ def test_loud_overflow_scores_are_non_finite_where_the_reference_is(variant_env)
 
 
 @gpu
-def test_vn_stereo_partials_against_reference(variant_env):
+def test_vn_stereo_partials_against_reference(tpc_env):
     cases = [("LR", (0,), None), ("MS", (0, 1), None), ("MS", (0, 1), 0.3), ("LR", (0, 1), 1.0), ("MS", (), 0.7), ("LR", (), None)]
     for frames in (1, 7, 1000, TILE, TILE + 1, 3 * TILE + 5):
         x = O.coloured_clip(frames % 5, frames) if frames > 1 else dense_clip(1)
@@ -655,7 +644,7 @@ HDR_FAMILY = np.linspace(0.0, 1.0, 16)
 
 
 @gpu
-def test_sums_do_not_depend_on_the_chunk_plan(variant_env):
+def test_sums_do_not_depend_on_the_chunk_plan(tpc_env):
     import torch
 
     fam = VnFamily(HDR_FAMILY)
@@ -665,9 +654,9 @@ def test_sums_do_not_depend_on_the_chunk_plan(variant_env):
         x = hdr_clip(seed, frames, fade)
         alone = opt.vn_objective_partials(x, prog)[0]
         for tpc in ("1", "2", "3", "7"):
-            variant_env(None, tpc)
+            tpc_env(tpc)
             assert np.array_equal(opt.vn_objective_partials(x, prog)[0], alone), (seed, tpc)
-        variant_env(None)
+        tpc_env(None)
         xt = torch.from_numpy(np.ascontiguousarray(x.T)).cuda()
         for others in (1, 3, 64):
             g = torch.Generator(device="cuda").manual_seed(others)

@@ -1,6 +1,5 @@
 #!/usr/bin/env bash
-# Round 2, call 5: full gpu suite; cfg3 A/B (this tree's tensor-memory FIR file vs round 1's inside this tree); ncu of
-# both objective kernels on a small sweep.
+# Round 2, call 5: full gpu suite; cfg3 A/B (this tree's tensor-memory FIR file vs round 1's inside this tree).
 cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
 echo "== gpu tests"; timeout 900 python -m pytest tests -x -q -m gpu 2>&1 | tail -6
@@ -11,8 +10,3 @@ echo -n "cfg3 this tree:            "; b A=1
 echo -n "cfg3 round-1 kernel file:  "; b VND_B200_LIB=$PWD/vndecorrelate_b200/_lib/libvnd_b200_r1tm.so
 echo -n "cfg3 this tree:            "; b A=1
 echo -n "cfg3 round-1 kernel file:  "; b VND_B200_LIB=$PWD/vndecorrelate_b200/_lib/libvnd_b200_r1tm.so
-for mode in 1 0; do
-  cmd="python tools/bench_objective.py --clips 2 --reps 1"
-  VND_OBJ_TMEM=$mode timeout 600 ncu --set full --clock-control none --import-source on -k regex:vn_objective -s 1 -c 1 -f -o gpurun_out/r02_obj_tmem$mode env VND_OBJ_TMEM=$mode $cmd > gpurun_out/r02_obj_tmem${mode}_ncu.log 2>&1
-  echo "ncu objective tmem=$mode rc=$?"; tail -2 gpurun_out/r02_obj_tmem${mode}_ncu.log
-done

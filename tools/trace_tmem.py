@@ -32,7 +32,7 @@ os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
 np.save(os.path.join(ROOT, "gpurun_out", "tm_trace.npy"), buf)
 t = buf.astype(np.int64)
 t0 = t[0, 8, 0]
-names_c = ["start", "waits done", "near done", "far done", "staged", "stage free", "pair done / gate open", "full2 ok"]
+names_c = ["start", "waits done", "near done", "far done", "staged", "stage free"]
 names_h = ["fill start", "fill end", "store done", "-", "in_full ok"]
 for q in range(4):
     print(f"== quarter {q}")
@@ -40,7 +40,7 @@ for q in range(4):
         line = f"tile {ti}: "
         for g in range(3):
             w = q + 4 * g
-            line += f"| g{g} " + " ".join(f"{names_c[e][:5]}={t[w, ti, e] - t0:6d}" for e in {"5": (0, 1, 6, 7, 2, 3, 5, 4), "6": (0, 1, 2, 6, 3, 5, 4), "7": (0, 1, 2, 6, 3, 5, 4), "8": (0, 6, 1, 2, 3, 5, 4), "9": (0, 6, 1, 2, 3, 5, 4), "10": (0, 6, 1, 2, 3, 5, 4), "11": (0, 6, 1, 2, 3, 5, 4), "12": (0, 6, 1, 2, 3, 5, 4)}.get(os.environ.get("VND_TM_SHAPE", "0"), (0, 1, 2, 3, 5, 4)))
+            line += f"| g{g} " + " ".join(f"{names_c[e][:5]}={t[w, ti, e] - t0:6d}" for e in (0, 1, 2, 3, 5, 4))
         h = 12 + q
         line += " | helper " + " ".join(f"{names_h[e][:7]}={t[h, ti, e] - t0:6d}" for e in (4, 0, 1, 2))
         print(line)

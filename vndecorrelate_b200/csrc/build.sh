@@ -12,5 +12,5 @@ NVCC="${NVCC:-/usr/local/cuda/bin/nvcc}"
   ${VND_PTXAS_V:+-Xptxas -v} \
   -o "$out/libvnd_b200.so" \
   ${VND_EXTRA_DEFS:-} \
-  "$here/vnd_abi.cu" "$here/vnd_fir.cu" "$here/vnd_fir_window.cu" "$here/vnd_fir_tmem.cu" "$here/vnd_fir_ring.cu" "$here/vnd_post.cu" "$here/vnd_objective.cu" "$here/vnd_objective_tmem.cu" "$here/vnd_dsp.cu" "$here/vnd_batch.cu"
+  "$here/vnd_abi.cu" "$here/vnd_fir.cu" "$here/vnd_fir_window.cu" "$here/vnd_fir_tmem.cu" "$here/vnd_fir_ring.cu" "$here/vnd_post.cu" "$here/vnd_objective.cu" "$here/vnd_dsp.cu" "$here/vnd_batch.cu"
 echo "built $out/libvnd_b200.so"

@@ -715,31 +715,23 @@ static int launch_tile_nt(const FirParams& p, size_t smem, int nt, cudaStream_t 
 }
 
 // Long filters (halo beyond 4096 samples, e.g. 300 impulses over 0.3 s @ 96 kHz: BASELINE config 4): tile + halo
-// fills the SM's shared memory, so ONE CTA of 32 warps runs per SM.  R outputs per lane and pass; the tile is a whole
+// fills the SM's shared memory, so ONE CTA of 32 warps runs per SM.  kLongR outputs per lane and pass; the tile is a whole
 // number of passes for all 32 warps (round 1 ran 28 672 outputs = 3.5 passes of R = 8: half of the warps idled
 // through the fourth pass), and a larger R spreads the tap-index load and the loop overhead of a tap over more outputs.
-// Measured on 64 channels x 57.6 M frames (Gsamples/s, shared-memory pipe busy): round 1 (R = 8, 3.5 passes, scalar adds)
-// 25.1 / 81 %; R = 8 25.3 / 81 %; R = 12 26.0 / 84 %; R = 16 (one pass of 16 384 outputs) 27.5 / 89 %.
-// VND_LONG_R picks R in {8, 12, 16} (default 16).
-static int long_filter_r() {
-  static const int r = [] {
-    const char* e = getenv("VND_LONG_R");
-    const int v = e ? atoi(e) : 16;
-    return (v == 8 || v == 12 || v == 16) ? v : 16;
-  }();
-  return r;
-}
-static int plan_long_tile(int halo, int max_prog_words, int r, size_t* smem) {
+// Measured on 64 channels x 57.6 M frames (B200, Gsamples/s, shared-memory pipe busy): round 1 (R = 8, 3.5 passes, scalar
+// adds) 25.1 / 81 %; R = 8 25.3 / 81 %; R = 12 26.0 / 84 %; R = 16 (one pass of 16 384 outputs) 27.5 / 89 %.  The other
+// values of R were removed; last present at commit 915ac5a.
+constexpr int kLongR = 16;
+static int plan_long_tile(int halo, int max_prog_words, size_t* smem) {
   const long long budget = (long long)kMaxDynSmem - 16 - 16 - (long long)max_prog_words * 4;
-  const long long per_pass = 32LL * 32 * r;
+  const long long per_pass = 32LL * 32 * kLongR;
   const long long tile = (budget / 4 - halo) / per_pass * per_pass;
   if (tile <= 0) return 0;
   *smem = 16 + (((size_t)(tile + halo) * 4 + 15) & ~(size_t)15) + (size_t)max_prog_words * 4;
   return (int)tile;
 }
-template <int R>
 static int launch_long_tile(const FirParams& p, size_t smem, cudaStream_t st) {
-  auto k = fir_tile_kernel<float, MODE_SEG, 1024, R>;
+  auto k = fir_tile_kernel<float, MODE_SEG, 1024, kLongR>;
   VND_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const long long blocks = (long long)p.tiles_per_channel * p.channels;
   VND_REQUIRE(blocks < 0x7fffffffLL, VND_EUNSUPPORTED, "grid too large (%lld CTAs)", blocks);
@@ -841,14 +833,11 @@ int sparse_fir_launch(const vnd_signal* x, const vnd_signal* y, const vnd_tap_pr
     }
   }
   if (!f64 && mode == MODE_SEG && p.halo > 4096 && p.frames >= 4LL * p.halo) {
-    const int r = long_filter_r();
-    const int tile = plan_long_tile(p.halo, max_prog_words, r, &smem);
+    const int tile = plan_long_tile(p.halo, max_prog_words, &smem);
     if (tile > 0) {
       p.tile = tile;
       p.tiles_per_channel = (int)ceil_div<long long>(p.frames, p.tile);
-      if (r == 8) return launch_long_tile<8>(p, smem, st);
-      if (r == 12) return launch_long_tile<12>(p, smem, st);
-      return launch_long_tile<16>(p, smem, st);
+      return launch_long_tile(p, smem, st);
     }
   }
   p.tile = plan_tile(p.halo, elem, max_prog_words, p.frames, &nt, &smem);

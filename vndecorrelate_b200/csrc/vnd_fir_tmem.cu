@@ -51,10 +51,6 @@
 #define VND_TM_RUN_MIN 48   // fewest (a run pays a prologue and a pipeline fill of about two tiles)
 #endif
 
-#ifndef VND_TM_DEFAULT_SHAPE
-#define VND_TM_DEFAULT_SHAPE 0  // TmShape used unless VND_TM_SHAPE says otherwise (fir_tmem_launch)
-#endif
-
 #ifdef VND_TM_TRACE
 // Debug builds only: clock64() of a few events per warp and tile of CTA 0 (tools/trace_tmem.py).
 __device__ unsigned long long g_tm_trace[16][64][8];
@@ -78,64 +74,38 @@ namespace {
 using namespace tm;  // tensor-memory primitives and the tap machinery (vnd_tmem.cuh)
 constexpr int kBarBytes = 384;
 
-// Shape of the kernel: G compute warps per lane quarter, each thread owning RG consecutive outputs of its
-// row (a row is R = G * RG outputs), NBUF tile buffers in shared memory, RC / RH registers per compute /
-// data-movement thread (setmaxnreg; 32 * (4 G RC + 4 RH) must not exceed what the launch allocates).
-//   <3, 32, 3, 144, 80>  round 1: 12 compute warps x 32 outputs, rows of 96, reach 416
-//   <2, 48, 3, 200, 104> 8 compute warps x 48 outputs, rows of 96: two warps per scheduler is where the
-//                        tensor-memory read path is efficient (tools/microbench/tmem_lat.cu: 8 warps 415 B/clk/SM,
-//                        12 warps 279), and every per-tap overhead is spread over 48 outputs instead of 32
-//   <2, 64, 2, 200, 104> 8 compute warps x 64 outputs, rows of 128: TMEM refill 4 instead of 5.33 words per output,
-//                        reach 384; two tile buffers (tile + halo is 74 KB)
-//   <3, 32, 3, 152, 56, false, true>  round 2: the trailing all-far segment advances together with the first segment
-//                        (pair_first in vnd_tmem.cuh); TMEM is handed over in two column stages
-//   <3, 32, 3, 144, 80, false, false, false, true>  round 2: the lane quarters take their shared-memory phase in two
-//                        alternating groups (kGate, see compute_main)
-template <int G, int RG, int NBUF, int RC, int RH, bool PIPE = false, bool PAIR = false, bool PARK = false, int GATE = 0, int FF = 0, bool DUAL = false, bool SYM = false>
-struct TmShape {
-  static constexpr bool kSym = SYM;            // no data-movement warps: every warp computes, refills its share of the TMEM rows, and
-                                               // elected lanes issue the tile loads and the stores (sym_main)
-  static constexpr bool kDual = DUAL;          // two tensor-memory taps per round trip (two landing buffers, one wait)
-  static constexpr bool kFarFirst = FF != 0;   // the trailing all-far segment first (sum parked in the staging row), under the TMEM refill:
-  static constexpr int kFarFirstMode = FF;     // 1: every warp, double-buffered loads; 2: only the last warp of each quarter (two warps
-                                               // per scheduler in the tensor-memory taps at a time), 3: every warp, plain loop
-  static constexpr int kGate = GATE;           // 2: quarters {0, 1} and {2, 3} alternate in the all-far (shared-memory) phase; 4: one quarter at a time
-  static constexpr bool kPipe = PIPE;          // tensor-memory taps software-pipelined over two operand buffers
-  static constexpr bool kPair = PAIR;          // first segment and trailing all-far segment in one paired loop
-  static constexpr bool kPark = PARK;          // ... with the far sum parked in the staging row instead of in registers
-  static constexpr int kUnitsA = 7;            // PAIR: the data-movement warp announces the first 7 x 32 TMEM columns separately
-  static constexpr int kG = G;                 // compute warps per lane quarter
-  static constexpr int kRG = RG;               // outputs per thread
-  static constexpr int kR = G * RG;            // outputs per row
-  static constexpr int kCW = 4 * G;            // compute warps (warp w: lane quarter w & 3, group w >> 2)
-  static constexpr int kHelpers = SYM ? 0 : 4; // one data-movement warp per quarter
-  static constexpr int kNW = kCW + kHelpers;
-  static constexpr int kNT = kNW * 32;
-  static constexpr int kTile = kRows * kR;
-  static constexpr int kPitch = kR + 4;        // row pitch in shared memory (words); an odd number of 16-byte chunks
-  static constexpr int kUnitsPerBlock = kR / 32;
-  static constexpr int kNBuf = NBUF;
-  static constexpr int kRegsCompute = RC, kRegsHelper = RH;
-  static constexpr int kLaunchRegs = (65536 / kNT) / 8 * 8;
-  // mbarrier slots (uint64 each)
-  static constexpr int B_IN_FULL = 0, B_IN_FREE = NBUF, B_ST_FULL = 2 * NBUF, B_ST_FREE = 2 * NBUF + 4, B_TM_FULL = 2 * NBUF + 8,
-                       B_TM_FREE = 2 * NBUF + 12, B_TM_FULL2 = 2 * NBUF + 16, B_FAR_DONE = 2 * NBUF + 20, B_COUNT = 2 * NBUF + 24;
-  static_assert(RG == 32 || RG == 48 || RG == 64, "outputs per thread: one x32, x32 + x16 or x64 tcgen05.ld");
-  static_assert(kR % 32 == 0 && ((kPitch / 4) & 1) == 1, "rows are whole 32-column units; the pitch is an odd number of chunks");
-  static_assert(32 * (kCW * RC + kHelpers * RH) <= kLaunchRegs * kNT, "register file");
-  static_assert(!SYM || (kUnits % G == 0 && !PIPE && !PAIR && GATE == 0 && FF == 0 && !DUAL), "symmetric variant: plain loops, equal fill shares");
-  static_assert(RC % 8 == 0 && RH % 8 == 0, "setmaxnreg takes multiples of 8");
-  static_assert(B_COUNT * 8 <= 256, "mbarriers");
-  static_assert(GATE == 0 || GATE == 2 || GATE == 4, "far-phase gate");
-  static_assert(!FF || (RG == 32 && !PAIR), "far-first is written for 32 outputs per thread");
-  static_assert(!PAIR || RG == 32, "the paired loop is written for 32 outputs per thread");
-  // Largest tap offset whose columns (up to offset + kR - 1) lie inside the first column stage
-  static constexpr int kStageAMax = 32 * kUnitsA - G * RG;
-  // Largest tap offset served from TMEM (every group of a row: group g alone could reach RG (G - 1 - g) samples
-  // further, but per-group tap mixes measured slower - 366 instead of 384 Gsamples/s on the same box - because the
-  // three warps of a quarter hand TMEM back together and the quarter waits for its slowest group).
-  static constexpr int kNearMax = kCols - kR;
-};
+// Shape of the kernel: kG compute warps per lane quarter, each thread owning kRG consecutive outputs of its row (a row is
+// kR = kG * kRG outputs), kNBuf tile buffers in shared memory, kRegsCompute / kRegsHelper registers per compute /
+// data-movement thread (setmaxnreg; 32 * (4 kG kRegsCompute + 4 kRegsHelper) must not exceed what the launch allocates).
+// Round 2 measured other shapes and schedules of this kernel on a B200, 148 channels x 28.8 M frames (Gsamples/s, all
+// bit-exact; profiles/r02_summary.md, DESIGN.md section 4) against 357-380 for this one: 2 warps x 48 outputs 325,
+// 2 x 64 with rows of 128 338, 2 x 32 298 (272 with software-pipelined tensor-memory taps), the trailing all-far
+// segment paired tap by tap with the first 278, quarters taking the far phase in turns 375 / 268, the all-far segment
+// first 219-344, two tensor-memory taps per round trip 300 / 278, a symmetric CTA without data-movement warps 355.
+// A tap's tcgen05.ld round trip bounds the tensor-memory phase, and every form of overlap inside a warp made the taps
+// slower.  Code removed; last present at commit 915ac5a.
+constexpr int kG = 3;                       // compute warps per lane quarter
+constexpr int kR = kG * kRG;                // outputs per row
+constexpr int kCW = 4 * kG;                 // compute warps (warp w: lane quarter w & 3, group w >> 2)
+constexpr int kHelpers = 4;                 // one data-movement warp per quarter
+constexpr int kNT = (kCW + kHelpers) * 32;
+constexpr int kTile = kRows * kR;
+constexpr int kPitch = kR + 4;              // row pitch in shared memory (words); an odd number of 16-byte chunks
+constexpr int kUnitsPerBlock = kR / 32;
+constexpr int kNBuf = 3;
+constexpr int kRegsCompute = 144, kRegsHelper = 80;
+constexpr int kLaunchRegs = (65536 / kNT) / 8 * 8;
+// mbarrier slots (uint64 each)
+constexpr int B_IN_FULL = 0, B_IN_FREE = kNBuf, B_ST_FULL = 2 * kNBuf, B_ST_FREE = 2 * kNBuf + 4, B_TM_FULL = 2 * kNBuf + 8,
+              B_TM_FREE = 2 * kNBuf + 12, B_COUNT = 2 * kNBuf + 16;
+static_assert(kR % 32 == 0 && ((kPitch / 4) & 1) == 1, "rows are whole 32-column units; the pitch is an odd number of chunks");
+static_assert(32 * (kCW * kRegsCompute + kHelpers * kRegsHelper) <= kLaunchRegs * kNT, "register file");
+static_assert(kRegsCompute % 8 == 0 && kRegsHelper % 8 == 0, "setmaxnreg takes multiples of 8");
+static_assert(B_COUNT * 8 <= 256, "mbarriers");
+// Largest tap offset served from TMEM (every group of a row: group g alone could reach kRG (kG - 1 - g) samples
+// further, but per-group tap mixes measured slower - 366 instead of 384 Gsamples/s on the same box - because the
+// three warps of a quarter hand TMEM back together and the quarter waits for its slowest group).
+constexpr int kNearMax = kCols - kR;
 
 struct TmParams {
   // TMA descriptors of x and y seen as (R samples, rows, channels).  The boxes are R + 4 wide: the four
@@ -153,40 +123,36 @@ struct TmParams {
   int tiles_per_channel;  // interior tiles
 };
 
-// Dynamic shared memory: [0,256) mbarriers | [256,260) TMEM base | [260,264) first all-far segment | [264,280) paired-loop plan |
-//   [384, ...) float in[NBUF][nblk][pitch] | float stage[128][pitch] | int program[] | int ops[G][] | int4 segtab[]
+// Dynamic shared memory: [0,256) mbarriers | [256,260) TMEM base | [260,264) first all-far segment |
+//   [384, ...) float in[kNBuf][nblk][pitch] | float stage[128][pitch] | int program[] | int ops[kG][] | int4 segtab[]
 // The role functions rebuild their pointers from this symbol so that every access stays in the
 // shared address space (LDS/STS, not generic loads).
 extern __shared__ __align__(128) unsigned char tm_smem[];
 
-template <class T>
 struct Smem {
   uint64_t* bars;
   int* s_near_end;  // first segment without a tap in the TMEM window
-  int* s_pair;      // [0] run takes the paired loop, [1] first segment that needs the second column stage, [2] word offset of the last segment's operations
   float* in_all;
   float* stage;
   int* sprog;
-  int* ops;  // [G][opstride]: decoded tap operations per thread group
+  int* ops;  // [kG][opstride]: decoded tap operations per thread group
   int4* segtab;  // per segment: taps of the negative and positive list, their leading tensor-memory taps, gain bits
   int bufw;
   int opstride;
   __device__ __forceinline__ explicit Smem(const TmParams& P) {
     bars = reinterpret_cast<uint64_t*>(tm_smem);
     s_near_end = reinterpret_cast<int*>(tm_smem + 260);
-    s_pair = reinterpret_cast<int*>(tm_smem + 264);
     in_all = reinterpret_cast<float*>(tm_smem + kBarBytes);
-    bufw = (P.nblk * T::kPitch + 31) & ~31;  // TMA tensor copies want 128-byte aligned shared-memory addresses
-    stage = in_all + T::kNBuf * bufw;
-    sprog = reinterpret_cast<int*>(stage + kRows * T::kPitch);
+    bufw = (P.nblk * kPitch + 31) & ~31;  // TMA tensor copies want 128-byte aligned shared-memory addresses
+    stage = in_all + kNBuf * bufw;
+    sprog = reinterpret_cast<int*>(stage + kRows * kPitch);
     opstride = P.opstride;
     ops = sprog + opstride;
-    segtab = reinterpret_cast<int4*>(ops + T::kG * opstride);  // opstride is a multiple of 4 words: 16-byte aligned
+    segtab = reinterpret_cast<int4*>(ops + kG * opstride);  // opstride is a multiple of 4 words: 16-byte aligned
   }
 };
-template <class T>
 constexpr size_t tm_tail_words(int opstride) {  // program + decoded lists + segment tables
-  return (size_t)(3 + T::kG) * opstride;
+  return (size_t)(3 + kG) * opstride;
 }
 
 struct RunInfo {
@@ -196,8 +162,7 @@ struct RunInfo {
 // Per-run prologue shared by both roles (every thread of the CTA takes part): decode the run, copy
 // the unfiltered channel through or load and decode the channel's program.  Returns false for a
 // copied run.
-template <class T>
-__device__ __forceinline__ bool begin_run(const TmParams& P, const Smem<T>& sm, int run, int tid, RunInfo& r) {
+__device__ __forceinline__ bool begin_run(const TmParams& P, const Smem& sm, int run, int tid, RunInfo& r) {
   const FirParams& p = P.f;
   r.c = run / P.runs_per_channel;
   r.first_tile = (run % P.runs_per_channel) * P.tiles_per_run;
@@ -208,13 +173,13 @@ __device__ __forceinline__ bool begin_run(const TmParams& P, const Smem<T>& sm, 
   if (r.nprog == 0) {  // unfiltered channel: copy through (decorrelation.py:399-400)
     const float* xc = reinterpret_cast<const float*>(p.x) + (long long)r.c * p.x_sc;
     float* yc = p.y + (long long)r.c * p.y_sc;
-    const long long t_begin = (long long)r.first_tile * T::kTile, t_end = t_begin + (long long)r.n_tiles * T::kTile;
-    for (long long t = t_begin + 4 * tid; t < t_end; t += 4 * T::kNT)
+    const long long t_begin = (long long)r.first_tile * kTile, t_end = t_begin + (long long)r.n_tiles * kTile;
+    for (long long t = t_begin + 4 * tid; t < t_end; t += 4 * kNT)
       *reinterpret_cast<float4*>(yc + t) = *reinterpret_cast<const float4*>(xc + t);
     return false;
   }
   __syncthreads();  // the pipeline of the previous run has drained: program, buffers and TMEM are free
-  for (int i = tid; i < r.nprog; i += T::kNT) sm.sprog[i] = p.words[w0 + i];
+  for (int i = tid; i < r.nprog; i += kNT) sm.sprog[i] = p.words[w0 + i];
   __syncthreads();
   const int S = sm.sprog[0];
   const int* taps = sm.sprog + 1 + 3 * S;
@@ -225,50 +190,29 @@ __device__ __forceinline__ bool begin_run(const TmParams& P, const Smem<T>& sm, 
     for (int s = 0; s < S; ++s) {
       const int n_neg = sm.sprog[1 + 3 * s], n = n_neg + sm.sprog[2 + 3 * s];
       for (int k = 0; k < n; ++k)
-        if (tq[k] <= T::kNearMax) ne = s + 1;
+        if (tq[k] <= kNearMax) ne = s + 1;
       int a = 0, b = 0;  // leading tensor-memory taps of the two lists
-      while (a < n_neg && tq[a] <= T::kNearMax) ++a;
-      while (n_neg + b < n && tq[n_neg + b] <= T::kNearMax) ++b;
+      while (a < n_neg && tq[a] <= kNearMax) ++a;
+      while (n_neg + b < n && tq[n_neg + b] <= kNearMax) ++b;
       sm.segtab[s] = make_int4(n_neg, n - n_neg, a | (b << 16), p.apply_gain ? sm.sprog[3 + 3 * s] : __float_as_int(1.0f));
       tq += n;
     }
     *sm.s_near_end = ne;
-    if constexpr (T::kPair || T::kFarFirst) {
-      // paired loop: exactly one trailing all-far segment and a first segment served from TMEM only
-      // (far-first only needs the former)
-      const int4 d0 = sm.segtab[0];
-      bool ok = S >= 2 && ne == S - 1 && (T::kFarFirst || ((d0.z & 0xffff) == d0.x && (d0.z >> 16) == d0.y && d0.x + d0.y > 0));
-      int sa = 0, off = 0;  // leading segments whose tensor-memory taps stay inside the first column stage
-      tq = taps;
-      bool in_a = true;
-      for (int s = 0; s < S; ++s) {
-        const int n = sm.sprog[1 + 3 * s] + sm.sprog[2 + 3 * s];
-        if (s == S - 1) off = (int)(tq - taps);
-        for (int k = 0; k < n; ++k)
-          if (tq[k] <= T::kNearMax && tq[k] > T::kStageAMax) in_a = false;
-        if (in_a && s < ne) sa = s + 1;
-        tq += n;
-      }
-      sm.s_pair[0] = ok ? 1 : 0;
-      sm.s_pair[1] = sa;
-      sm.s_pair[2] = off;
-      sm.s_pair[3] = 1;  // see compute_main: the first middle segment, as a run-time value
-    }
   }
-  // decode the taps for the thread groups (group g owns outputs RG g .. RG g + RG - 1 of a row)
-  for (int t = tid; t < T::kG * (ntaps + 2); t += T::kNT) {
+  // decode the taps for the thread groups (group g owns outputs kRG g .. kRG g + kRG - 1 of a row)
+  for (int t = tid; t < kG * (ntaps + 2); t += kNT) {
     const int g = t / (ntaps + 2), k = t - g * (ntaps + 2);
     int op = 0;  // two slack words behind each list
     if (k < ntaps) {
       const int i = taps[k];
-      if (i <= T::kNearMax) {
+      if (i <= kNearMax) {
         op = i;
       } else {
-        const int o = i + T::kRG * g, A = o & 3, oal = o - A;
-        const int blk = oal / T::kR, w = oal - blk * T::kR;
-        int kx = (T::kR - w) >> 2;
+        const int o = i + kRG * g, A = o & 3, oal = o - A;
+        const int blk = oal / kR, w = oal - blk * kR;
+        int kx = (kR - w) >> 2;
         if (kx > 31) kx = 31;
-        op = kOpFar | (A << 24) | (kx << 16) | (blk * T::kPitch + w);
+        op = kOpFar | (A << 24) | (kx << 16) | (blk * kPitch + w);
       }
     }
     sm.ops[g * sm.opstride + k] = op;
@@ -289,17 +233,16 @@ __device__ __forceinline__ void stagger(int q, int ns) {
 }
 
 // ---------------------------------------------------------------- data-movement warp of lane quarter q
-// One elected lane per warp: quarter 0 issues the tile loads (one TMA request per tile, NBUF - 1 tiles
+// One elected lane per warp: quarter 0 issues the tile loads (one TMA request per tile, kNBuf - 1 tiles
 // ahead), every quarter stores its own 32 staged rows (one request per tile).
-template <class T>
 __device__ __noinline__ void helper_main(const TmParams& P, uint32_t tbase, int tid) {
-  const Smem<T> sm(P);
+  const Smem sm(P);
   const int nblk = P.nblk, n_runs = P.n_runs, stagger_ns = P.stagger_ns;  // P lives behind a generic pointer here
   const int lane = tid & 31, q = (tid >> 5) & 3;
   const int m = 32 * q + lane;
   const uint32_t bars = smem_u32(sm.bars), in0 = smem_u32(sm.in_all), buf_bytes = (uint32_t)sm.bufw * 4u;
-  const uint32_t stage_q = smem_u32(sm.stage + 32 * q * T::kPitch);
-  const uint32_t tx_bytes = (uint32_t)nblk * (T::kPitch * 4u);  // the whole box counts, zero-filled columns included
+  const uint32_t stage_q = smem_u32(sm.stage + 32 * q * kPitch);
+  const uint32_t tx_bytes = (uint32_t)nblk * (kPitch * 4u);  // the whole box counts, zero-filled columns included
   const void* tmx = &P.tmx;
   const void* tmy = &P.tmy;
   const bool loader = q == 0 && lane == 0;
@@ -308,36 +251,36 @@ __device__ __noinline__ void helper_main(const TmParams& P, uint32_t tbase, int 
   unsigned tpar = 0;           // parity of the tile counter (TMEM and staging barriers)
   for (int run = blockIdx.x; run < n_runs; run += gridDim.x) {
     RunInfo r;
-    if (!begin_run<T>(P, sm, run, tid, r)) continue;
-    if constexpr (T::kGate == 0) stagger(q, stagger_ns);
+    if (!begin_run(P, sm, run, tid, r)) continue;
+    stagger(q, stagger_ns);
     int load_row = r.first_tile * kRows;  // first row (R samples) of the next tile to load
     int store_row = r.first_tile * kRows + 32 * q;
     int to_load = r.n_tiles;
 #define VND_ISSUE_LOAD()                                                                   \
   do {                                                                                     \
     if (loader) {                                                                          \
-      mbar_wait_u32(bars + 8u * (T::B_IN_FREE + lb), lpar); /* every warp is done with the tile that was there */ \
-      const uint32_t full = bars + 8u * (T::B_IN_FULL + lb);                               \
+      mbar_wait_u32(bars + 8u * (B_IN_FREE + lb), lpar); /* every warp is done with the tile that was there */ \
+      const uint32_t full = bars + 8u * (B_IN_FULL + lb);                                  \
       mbar_expect_tx_u32(full, tx_bytes);                                                  \
       fence_proxy_async();                                                                 \
       tma_load_3d(in0 + (uint32_t)lb * buf_bytes, tmx, 0, load_row, r.c, full);            \
     }                                                                                      \
     load_row += kRows;                                                                     \
     --to_load;                                                                             \
-    if (++lb == T::kNBuf) {                                                                \
+    if (++lb == kNBuf) {                                                                   \
       lb = 0;                                                                              \
       lpar ^= 1u;                                                                          \
     }                                                                                      \
   } while (0)
-    for (int d = 0; d < T::kNBuf - 1 && to_load > 0; ++d) VND_ISSUE_LOAD();
+    for (int d = 0; d < kNBuf - 1 && to_load > 0; ++d) VND_ISSUE_LOAD();
     for (int ti = 0; ti < r.n_tiles; ++ti) {
-      mbar_wait_u32(bars + 8u * (T::B_IN_FULL + fb), fpar);
+      mbar_wait_u32(bars + 8u * (B_IN_FULL + fb), fpar);
       VND_TRACE(ti, 4);
-      mbar_wait_u32(bars + 8u * (T::B_TM_FREE + q), tpar ^ 1u);  // the quarter is past its last TMEM tap of the previous tile
+      mbar_wait_u32(bars + 8u * (B_TM_FREE + q), tpar ^ 1u);  // the quarter is past its last TMEM tap of the previous tile
       tmem_fence_after();
       VND_TRACE(ti, 0);
       {  // fill row m: 32 columns per step; a block of R samples is R / 32 steps, then the pitch skips 4 words
-        const float4* src = reinterpret_cast<const float4*>(sm.in_all + fb * sm.bufw + m * T::kPitch);
+        const float4* src = reinterpret_cast<const float4*>(sm.in_all + fb * sm.bufw + m * kPitch);
         uint32_t tcol = tbase;
         int sub = 0;
 #pragma unroll 1
@@ -348,17 +291,9 @@ __device__ __noinline__ void helper_main(const TmParams& P, uint32_t tbase, int 
           tmem_st32(tcol, v);
           tcol += 32;
           src += 8;
-          if (++sub == T::kUnitsPerBlock) {
+          if (++sub == kUnitsPerBlock) {
             sub = 0;
             src += 1;
-          }
-          if constexpr (T::kPair) {
-            if (k32 == T::kUnitsA - 1) {  // the first column stage is complete: the quarter may start its first segments
-              tmem_wait_st();
-              tmem_fence_before();
-              __syncwarp();
-              if (lane == 0) mbar_arrive_u32(bars + 8u * (T::B_TM_FULL + q));
-            }
           }
         }
         tmem_wait_st();
@@ -367,20 +302,20 @@ __device__ __noinline__ void helper_main(const TmParams& P, uint32_t tbase, int 
       __syncwarp();
       VND_TRACE(ti, 1);
       if (lane == 0) {
-        mbar_arrive_u32(bars + 8u * ((T::kPair ? T::B_TM_FULL2 : T::B_TM_FULL) + q));
-        mbar_arrive_u32(bars + 8u * (T::B_IN_FREE + fb));
+        mbar_arrive_u32(bars + 8u * (B_TM_FULL + q));
+        mbar_arrive_u32(bars + 8u * (B_IN_FREE + fb));
       }
-      if (++fb == T::kNBuf) {
+      if (++fb == kNBuf) {
         fb = 0;
         fpar ^= 1u;
       }
       if (to_load > 0) VND_ISSUE_LOAD();
       if (ti > 0 && lane == 0) {  // the previous tile's 32 rows of this quarter
-        mbar_wait_u32(bars + 8u * (T::B_ST_FULL + q), tpar ^ 1u);
+        mbar_wait_u32(bars + 8u * (B_ST_FULL + q), tpar ^ 1u);
         tma_store_3d(tmy, 0, store_row, r.c, stage_q);
         bulk_commit();
         bulk_wait_read0();
-        mbar_arrive_u32(bars + 8u * (T::B_ST_FREE + q));
+        mbar_arrive_u32(bars + 8u * (B_ST_FREE + q));
       }
       if (ti > 0) store_row += kRows;
       __syncwarp();
@@ -389,321 +324,69 @@ __device__ __noinline__ void helper_main(const TmParams& P, uint32_t tbase, int 
     }
 #undef VND_ISSUE_LOAD
     if (lane == 0) {
-      mbar_wait_u32(bars + 8u * (T::B_ST_FULL + q), tpar ^ 1u);
+      mbar_wait_u32(bars + 8u * (B_ST_FULL + q), tpar ^ 1u);
       tma_store_3d(tmy, 0, store_row, r.c, stage_q);
       bulk_commit();
       bulk_wait_read0();
-      mbar_arrive_u32(bars + 8u * (T::B_ST_FREE + q));
+      mbar_arrive_u32(bars + 8u * (B_ST_FREE + q));
     }
     __syncwarp();
   }
 }
 
 // ---------------------------------------------------------------- compute warp (q, g)
-template <class T>
 __device__ __noinline__ void compute_main(const TmParams& P, uint32_t tbase, int tid) {
-  constexpr int RG = T::kRG;
-  const Smem<T> sm(P);
+  const Smem sm(P);
   const int n_runs = P.n_runs, stagger_ns = P.stagger_ns;  // P lives behind a generic pointer here
   const int lane = tid & 31, warp = tid >> 5;
   const int q = warp & 3, g = warp >> 2;
   const int m = 32 * q + lane;
   uint64_t* bars = sm.bars;
-  const uint32_t tcol0 = tbase + (uint32_t)(RG * g);  // column of this thread's first output
+  const uint32_t tcol0 = tbase + (uint32_t)(kRG * g);  // column of this thread's first output
   const int4* segtab = sm.segtab;
   int b = 0;           // ring slot of the current tile
   unsigned fpar = 0;   // in_full parity of slot b
   unsigned tpar = 0;   // parity of the tile counter (TMEM and staging barriers)
-  bool first_tile = true;  // kGate: no far phase of the other group precedes the very first tile
   for (int run = blockIdx.x; run < n_runs; run += gridDim.x) {
     RunInfo r;
-    if (!begin_run<T>(P, sm, run, tid, r)) continue;
-    if constexpr (T::kGate == 0) stagger(q, stagger_ns);
+    if (!begin_run(P, sm, run, tid, r)) continue;
+    stagger(q, stagger_ns);
     const int S = sm.sprog[0];
     const int near_end = *sm.s_near_end;
-    const bool pair_ok = (T::kPair || T::kFarFirst) && sm.s_pair[0] != 0 && (T::kFarFirstMode != 2 || g == T::kG - 1);
-    const int stage_a = T::kPair ? sm.s_pair[1] : 0;
-    const int* ops_far = sm.ops + g * sm.opstride + ((T::kPair || T::kFarFirst) ? sm.s_pair[2] : 0);
-    // Always 1, but read from shared memory: with a constant, run_segments loses its `s == 0` branch, the segment's
-    // multiply and the add into the running output land in one basic block, and ptxas contracts the two packed
-    // operations into FFMA2 (one rounding instead of two) although both carry .rn and the build says -fmad=false.
-    // tests/test_host_logic.py checks the SASS of the FIR kernels for such contractions.
-    const int seg1 = T::kPair ? sm.s_pair[3] : 1;
     for (int ti = 0; ti < r.n_tiles; ++ti) {
-      const uint32_t row = smem_u32(sm.in_all + b * sm.bufw + m * T::kPitch);
+      const uint32_t row = smem_u32(sm.in_all + b * sm.bufw + m * kPitch);
       const int* ops = sm.ops + g * sm.opstride;
       VND_TRACE(ti, 0);
-      mbar_wait(&bars[T::B_IN_FULL + b], fpar);
-      bool staged_wait = false;
-      // kGate: the phase that loads the shared-memory pipe (the all-far segments, next to the TMEM refill) is taken in turns.
-      // Left alone, the four quarters fall into step (tools/trace_tmem.py): the pipe saturates while all of them are in that
-      // phase and idles during the tensor-memory phase.  kGate == 2: quarters {0, 1} and {2, 3} alternate - group 1 enters
-      // the far phase of its n-th tile when group 0 has finished that of its n-th tile, group 0 that of tile n + 1 when
-      // group 1 has finished tile n.  kGate == 4: a ring, one quarter at a time.
-      auto gate_enter = [&]() {
-        if constexpr (T::kGate == 2) {
-          if (q < 2) {
-            if (!first_tile) mbar_wait(&bars[T::B_FAR_DONE + 1], tpar ^ 1u);
-          } else {
-            mbar_wait(&bars[T::B_FAR_DONE + 0], tpar);
-          }
-        } else if constexpr (T::kGate == 4) {
-          if (q == 0) {
-            if (!first_tile) mbar_wait(&bars[T::B_FAR_DONE + 3], tpar ^ 1u);
-          } else {
-            mbar_wait(&bars[T::B_FAR_DONE + q - 1], tpar);
-          }
-        }
-      };
-      auto gate_leave = [&]() {
-        if constexpr (T::kGate != 0) {
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&bars[T::B_FAR_DONE + (T::kGate == 2 ? (q >> 1) : q)]);
-          first_tile = false;
-        }
-      };
-      if constexpr (T::kFarFirst) {
-        if (pair_ok) {
-          // The trailing all-far segment first: it only needs the staged tile, so it runs while the data-movement warp
-          // still refills the quarter's TMEM rows; its scaled sum waits in the thread's slot of the staging row.
-          float far[RG];
-          gate_enter();
-          if constexpr (T::kFarFirstMode == 1) {
-            far_first(segtab, S, ops_far, row, far);
-          } else {  // the plain far loop on a zeroed accumulator: 0 + acc * gain (the running output is never -0, so
-                    // adding +0 instead of -0 later cannot change it)
+      mbar_wait(&bars[B_IN_FULL + b], fpar);
+      float yv[kRG];
 #pragma unroll
-            for (int rr = 0; rr < RG; ++rr) far[rr] = 0.0f;
-            const int* of = ops_far;
-            run_segments<true, false>(segtab, S - 1, S, of, tcol0, row, far);
-          }
-          gate_leave();
-          mbar_wait(&bars[T::B_ST_FREE + q], tpar ^ 1u);  // the previous tile's store has read the staging rows
-          staged_wait = true;
-          float4* park = reinterpret_cast<float4*>(sm.stage + m * T::kPitch + RG * g);
-#pragma unroll
-          for (int jj = 0; jj < RG / 4; ++jj) park[jj] = make_float4(far[4 * jj], far[4 * jj + 1], far[4 * jj + 2], far[4 * jj + 3]);
-          VND_TRACE(ti, 6);
-        }
-      }
-      float yv[RG];  // (zeroed only here: live zeros across the far-first loop cost 32 registers)
-#pragma unroll
-      for (int rr = 0; rr < RG; ++rr) yv[rr] = 0.0f;
-      mbar_wait(&bars[T::B_TM_FULL + q], tpar);
+      for (int rr = 0; rr < kRG; ++rr) yv[rr] = 0.0f;
+      mbar_wait(&bars[B_TM_FULL + q], tpar);
       tmem_fence_after();
       VND_TRACE(ti, 1);
-      if constexpr (T::kFarFirst) {
-        if (pair_ok) {
-          run_segments<false, false>(segtab, 0, near_end, ops, tcol0, row, yv);
-          VND_TRACE(ti, 2);
-          tmem_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&bars[T::B_TM_FREE + q]);  // the helper may fill TMEM for the next tile
-          const float4* park = reinterpret_cast<const float4*>(sm.stage + m * T::kPitch + RG * g);
-#pragma unroll
-          for (int jj = 0; jj < RG / 4; ++jj) {
-            const float4 v = park[jj];
-            add2(yv[4 * jj], yv[4 * jj + 1], v.x, v.y);
-            add2(yv[4 * jj + 2], yv[4 * jj + 3], v.z, v.w);
-          }
-        }
-      }
-      if constexpr (T::kPair) {
-        if (pair_ok) {
-          // Segment 0 and the trailing all-far segment together (vnd_tmem.cuh: pair_first), then the middle segments; the
-          // far sum is added last, as in the reference.
-          if (stage_a < 1) {
-            mbar_wait(&bars[T::B_TM_FULL2 + q], tpar);
-            tmem_fence_after();
-          }
-          float far[RG];
-          pair_first(segtab, S, ops, ops_far, tcol0, row, yv, far);
-          VND_TRACE(ti, 6);
-          float4* park = reinterpret_cast<float4*>(sm.stage + m * T::kPitch + RG * g);
-          if constexpr (T::kPark) {
-            mbar_wait(&bars[T::B_ST_FREE + q], tpar ^ 1u);  // the previous tile's store has read the staging rows
-            staged_wait = true;
-#pragma unroll
-            for (int jj = 0; jj < RG / 4; ++jj) park[jj] = make_float4(far[4 * jj], far[4 * jj + 1], far[4 * jj + 2], far[4 * jj + 3]);
-          }
-          const int* ops1 = ops + segtab[0].x + segtab[0].y;
-          const int s_mid = stage_a < 1 ? 1 : (stage_a < near_end ? stage_a : near_end);
-          run_segments<false, false>(segtab, seg1, s_mid, ops1, tcol0, row, yv);
-          if (stage_a >= 1) {
-            mbar_wait(&bars[T::B_TM_FULL2 + q], tpar);
-            tmem_fence_after();
-          }
-          VND_TRACE(ti, 7);
-          run_segments<false, false>(segtab, s_mid, near_end, ops1, tcol0, row, yv);
-          VND_TRACE(ti, 2);
-          tmem_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&bars[T::B_TM_FREE + q]);  // the helper may fill TMEM for the next tile
-          if constexpr (T::kPark) {
-#pragma unroll
-            for (int jj = 0; jj < RG / 4; ++jj) {
-              const float4 v = park[jj];
-              far[4 * jj] = v.x;
-              far[4 * jj + 1] = v.y;
-              far[4 * jj + 2] = v.z;
-              far[4 * jj + 3] = v.w;
-            }
-          }
-#pragma unroll
-          for (int j = 0; j < RG / 2; ++j) add2(yv[2 * j], yv[2 * j + 1], far[2 * j], far[2 * j + 1]);
-        } else {
-          mbar_wait(&bars[T::B_TM_FULL2 + q], tpar);
-          tmem_fence_after();
-        }
-      }
-      if (!(T::kPair || T::kFarFirst) || !pair_ok) {
-        run_segments<false, T::kPipe, RG, T::kDual>(segtab, 0, near_end, ops, tcol0, row, yv);
-        VND_TRACE(ti, 2);
-        tmem_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&bars[T::B_TM_FREE + q]);  // the helper may fill TMEM for the next tile
-        gate_enter();
-        VND_TRACE(ti, 6);
-        run_segments<true, false>(segtab, near_end, S, ops, tcol0, row, yv);
-        gate_leave();
-      }
-      VND_TRACE(ti, 3);
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bars[T::B_IN_FREE + b]);  // this warp is done with the tile buffer
-      if (!staged_wait) mbar_wait(&bars[T::B_ST_FREE + q], tpar ^ 1u);
-      VND_TRACE(ti, 5);  // the previous tile's stores have read the staging rows
-      {
-        float4* dst = reinterpret_cast<float4*>(sm.stage + m * T::kPitch + RG * g);
-#pragma unroll
-        for (int jj = 0; jj < RG / 4; ++jj) dst[jj] = make_float4(yv[4 * jj], yv[4 * jj + 1], yv[4 * jj + 2], yv[4 * jj + 3]);
-      }
-      fence_proxy_async();
-      __syncwarp();
-      VND_TRACE(ti, 4);
-      if (lane == 0) mbar_arrive(&bars[T::B_ST_FULL + q]);
-      tpar ^= 1u;
-      if (++b == T::kNBuf) {
-        b = 0;
-        fpar ^= 1u;
-      }
-    }
-  }
-}
-
-// ---------------------------------------------------------------- symmetric variant: warp (q, g) does everything
-// No data-movement warps (TmShape::kSym): G = 4 warps per quarter x 32 outputs, rows of 128, 16 x 128 registers.  Each
-// warp fills its share of the quarter's TMEM rows (group g: the 128 columns that are row m + g's samples) at the top of
-// a tile, then runs the tile like compute_main; lane 0 of warp 0 issues the tile loads (two buffers), lane 0 of the
-// first warp of each quarter the quarter's output store.
-template <class T>
-__device__ __noinline__ void sym_main(const TmParams& P, uint32_t tbase, int tid) {
-  constexpr int RG = T::kRG;
-  constexpr int kShare = kUnits / T::kG;  // 32-column units of a row that one warp fills
-  static_assert(kShare * 32 == T::kR, "a warp's fill share is one block of the row");
-  const Smem<T> sm(P);
-  const int nblk = P.nblk, n_runs = P.n_runs;
-  const int lane = tid & 31, warp = tid >> 5;
-  const int q = warp & 3, g = warp >> 2;
-  const int m = 32 * q + lane;
-  uint64_t* bars = sm.bars;
-  const uint32_t bars32 = smem_u32(sm.bars), in0 = smem_u32(sm.in_all), buf_bytes = (uint32_t)sm.bufw * 4u;
-  const uint32_t stage_q = smem_u32(sm.stage + 32 * q * T::kPitch);
-  const uint32_t tx_bytes = (uint32_t)nblk * (T::kPitch * 4u);
-  const void* tmx = &P.tmx;
-  const void* tmy = &P.tmy;
-  const bool loader = tid == 0, storer = g == 0 && lane == 0;
-  const uint32_t tcol0 = tbase + (uint32_t)(RG * g);
-  const int4* segtab = sm.segtab;
-  int b = 0, lb = 0;            // ring slots of the current tile and of the next load
-  unsigned fpar = 0, lpar = 1;  // in_full parity of slot b; in_free parity that releases slot lb
-  unsigned tpar = 0;            // parity of the tile counter
-  for (int run = blockIdx.x; run < n_runs; run += gridDim.x) {
-    RunInfo r;
-    if (!begin_run<T>(P, sm, run, tid, r)) continue;
-    const int S = sm.sprog[0];
-    const int near_end = *sm.s_near_end;
-    int load_row = r.first_tile * kRows, to_load = r.n_tiles;
-    int store_row = r.first_tile * kRows + 32 * q;
-    auto issue_load = [&]() {  // loader lane only
-      mbar_wait_u32(bars32 + 8u * (T::B_IN_FREE + lb), lpar);  // every warp is done with the tile that was there
-      const uint32_t full = bars32 + 8u * (T::B_IN_FULL + lb);
-      mbar_expect_tx_u32(full, tx_bytes);
-      fence_proxy_async();
-      tma_load_3d(in0 + (uint32_t)lb * buf_bytes, tmx, 0, load_row, r.c, full);
-      load_row += kRows;
-      --to_load;
-      if (++lb == T::kNBuf) {
-        lb = 0;
-        lpar ^= 1u;
-      }
-    };
-    if (loader)
-      for (int d = 0; d < T::kNBuf && to_load > 0; ++d) issue_load();
-    __syncwarp();
-    for (int ti = 0; ti < r.n_tiles; ++ti) {
-      const uint32_t row = smem_u32(sm.in_all + b * sm.bufw + m * T::kPitch);
-      const int* ops = sm.ops + g * sm.opstride;
-      VND_TRACE(ti, 0);
-      mbar_wait(&bars[T::B_IN_FULL + b], fpar);
-      mbar_wait(&bars[T::B_TM_FREE + q], tpar ^ 1u);  // every warp of the quarter is past its last TMEM tap of the previous tile
-      tmem_fence_after();
-      {  // this warp's share of the rows: row m + g's samples are columns [R g, R g + R) of TMEM row m
-        const float4* src = reinterpret_cast<const float4*>(sm.in_all + b * sm.bufw + (m + g) * T::kPitch);
-        uint32_t tcol = tbase + (uint32_t)(T::kR * g);
-#pragma unroll 1
-        for (int u = 0; u < kShare; ++u) {
-          float4 v[8];
-#pragma unroll
-          for (int jj = 0; jj < 8; ++jj) v[jj] = src[jj];
-          tmem_st32(tcol, v);
-          tcol += 32;
-          src += 8;
-        }
-        tmem_wait_st();
-      }
-      tmem_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bars[T::B_TM_FULL + q]);
-      VND_TRACE(ti, 6);
-      float yv[RG];
-#pragma unroll
-      for (int rr = 0; rr < RG; ++rr) yv[rr] = 0.0f;
-      mbar_wait(&bars[T::B_TM_FULL + q], tpar);
-      tmem_fence_after();
-      VND_TRACE(ti, 1);
-      run_segments<false, false>(segtab, 0, near_end, ops, tcol0, row, yv);
+      run_segments<false>(segtab, 0, near_end, ops, tcol0, row, yv);
       VND_TRACE(ti, 2);
       tmem_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(&bars[T::B_TM_FREE + q]);
-      run_segments<true, false>(segtab, near_end, S, ops, tcol0, row, yv);
+      if (lane == 0) mbar_arrive(&bars[B_TM_FREE + q]);  // the helper may fill TMEM for the next tile
+      VND_TRACE(ti, 6);
+      run_segments<true>(segtab, near_end, S, ops, tcol0, row, yv);
       VND_TRACE(ti, 3);
       __syncwarp();
-      if (lane == 0) mbar_arrive(&bars[T::B_IN_FREE + b]);  // this warp is done with the tile buffer
-      mbar_wait(&bars[T::B_ST_FREE + q], tpar ^ 1u);       // the previous tile's store has read the staging rows
-      VND_TRACE(ti, 5);
+      if (lane == 0) mbar_arrive(&bars[B_IN_FREE + b]);  // this warp is done with the tile buffer
+      mbar_wait(&bars[B_ST_FREE + q], tpar ^ 1u);
+      VND_TRACE(ti, 5);  // the previous tile's stores have read the staging rows
       {
-        float4* dst = reinterpret_cast<float4*>(sm.stage + m * T::kPitch + RG * g);
+        float4* dst = reinterpret_cast<float4*>(sm.stage + m * kPitch + kRG * g);
 #pragma unroll
-        for (int jj = 0; jj < RG / 4; ++jj) dst[jj] = make_float4(yv[4 * jj], yv[4 * jj + 1], yv[4 * jj + 2], yv[4 * jj + 3]);
+        for (int jj = 0; jj < kRG / 4; ++jj) dst[jj] = make_float4(yv[4 * jj], yv[4 * jj + 1], yv[4 * jj + 2], yv[4 * jj + 3]);
       }
       fence_proxy_async();
       __syncwarp();
-      if (lane == 0) mbar_arrive(&bars[T::B_ST_FULL + q]);
       VND_TRACE(ti, 4);
-      if (storer) {  // the quarter's 32 staged rows, once its G warps have staged them
-        mbar_wait_u32(bars32 + 8u * (T::B_ST_FULL + q), tpar);
-        tma_store_3d(tmy, 0, store_row, r.c, stage_q);
-        bulk_commit();
-        bulk_wait_read0();
-        mbar_arrive_u32(bars32 + 8u * (T::B_ST_FREE + q));
-      }
-      store_row += kRows;
-      if (loader && to_load > 0) issue_load();
-      __syncwarp();
-      VND_TRACE(ti, 7);
+      if (lane == 0) mbar_arrive(&bars[B_ST_FULL + q]);
       tpar ^= 1u;
-      if (++b == T::kNBuf) {
+      if (++b == kNBuf) {
         b = 0;
         fpar ^= 1u;
       }
@@ -711,26 +394,23 @@ __device__ __noinline__ void sym_main(const TmParams& P, uint32_t tbase, int tid
   }
 }
 
-template <class T>
-__global__ void __launch_bounds__(T::kNT, 1) fir_tmem_kernel(const __grid_constant__ TmParams P) {
-  const Smem<T> sm(P);
+__global__ void __launch_bounds__(kNT, 1) fir_tmem_kernel(const __grid_constant__ TmParams P) {
+  const Smem sm(P);
   uint32_t* tm_slot = reinterpret_cast<uint32_t*>(tm_smem + 256);
 
   const int tid = threadIdx.x;
   const int warp = tid >> 5;
   if (tid == 0) {
-    for (int b = 0; b < T::kNBuf; ++b) {
-      mbar_init(&sm.bars[T::B_IN_FULL + b], 1);
-      mbar_init(&sm.bars[T::B_IN_FREE + b], T::kCW + T::kHelpers);
+    for (int b = 0; b < kNBuf; ++b) {
+      mbar_init(&sm.bars[B_IN_FULL + b], 1);
+      mbar_init(&sm.bars[B_IN_FREE + b], kCW + kHelpers);
     }
     for (int k = 0; k < 4; ++k) {
-      mbar_init(&sm.bars[T::B_ST_FULL + k], T::kG);
-      mbar_init(&sm.bars[T::B_ST_FREE + k], 1);
-      mbar_init(&sm.bars[T::B_TM_FULL + k], T::kSym ? T::kG : 1);
-      mbar_init(&sm.bars[T::B_TM_FREE + k], T::kG);
-      mbar_init(&sm.bars[T::B_TM_FULL2 + k], 1);
+      mbar_init(&sm.bars[B_ST_FULL + k], kG);
+      mbar_init(&sm.bars[B_ST_FREE + k], 1);
+      mbar_init(&sm.bars[B_TM_FULL + k], 1);
+      mbar_init(&sm.bars[B_TM_FREE + k], kG);
     }
-    for (int k = 0; k < 4; ++k) mbar_init(&sm.bars[T::B_FAR_DONE + k], T::kGate == 2 ? 2 * T::kG : T::kG);
     mbar_fence_init();
   }
   if (warp == 0) tmem_alloc_all(tm_slot);
@@ -738,14 +418,12 @@ __global__ void __launch_bounds__(T::kNT, 1) fir_tmem_kernel(const __grid_consta
   __syncthreads();
   tmem_fence_after();
   const uint32_t tbase = *tm_slot + ((uint32_t)(32 * (warp & 3)) << 16);
-  if constexpr (T::kSym) {
-    sym_main<T>(P, tbase, tid);
-  } else if (warp >= T::kCW) {
-    set_max_regs_dec<T::kRegsHelper>();
-    helper_main<T>(P, tbase, tid);
+  if (warp >= kCW) {
+    set_max_regs_dec<kRegsHelper>();
+    helper_main(P, tbase, tid);
   } else {
-    set_max_regs_inc<T::kRegsCompute>();
-    compute_main<T>(P, tbase, tid);
+    set_max_regs_inc<kRegsCompute>();
+    compute_main(P, tbase, tid);
   }
   tmem_fence_before();
   __syncthreads();
@@ -759,19 +437,6 @@ static const int g_stagger_ns = [] {
   const char* e = getenv("VND_TM_STAGGER_NS");
   return e ? atoi(e) : 2000;
 }();
-// VND_TM_SHAPE picks the kernel variant (see TmShape and fir_tmem_launch): 0 = 3 x 32 (default), 1 = 2 x 48, 2 = 2 x 64, 3 = 2 x 32,
-// 4 = 3 pipelined, 5-14 = scheduling variants of the default shape, 15 = symmetric 4 x 32.
-static int g_tm_shape = [] {
-  const char* e = getenv("VND_TM_SHAPE");
-  return e ? atoi(e) : VND_TM_DEFAULT_SHAPE;
-}();
-// Debug / test aid (not part of the ABI in include/vnd_b200.h): select the kernel variant at run time so that the
-// parity tests can exercise every measured variant in one process; returns the previous selection.  Not thread-safe.
-extern "C" int vnd_debug_set_tm_shape(int shape) {
-  const int prev = g_tm_shape;
-  g_tm_shape = shape;
-  return prev;
-}
 
 // cuTensorMapEncodeTiled through the runtime (no link against libcuda).
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
@@ -824,9 +489,7 @@ static void plan_runs(long long tiles, int channels, int sm_count, int* tiles_pe
 // Runs the interior tiles of every channel and reports the frames covered per channel in
 // *frames_done (a multiple of the tile).  VND_EUNSUPPORTED (no error text) when the request does
 // not qualify; the caller then uses the other kernels for everything.
-template <class T>
-static int fir_tmem_launch_t(const FirParams& f, int max_prog_words, cudaStream_t st, long long* frames_done) {
-  constexpr int kR = T::kR, kPitch = T::kPitch, kTile = T::kTile;
+int fir_tmem_launch(const FirParams& f, int max_prog_words, cudaStream_t st, long long* frames_done) {
   *frames_done = 0;
   if (!f.bulk_ok || f.x_st != 1 || f.y_st != 1) return VND_EUNSUPPORTED;
   if ((reinterpret_cast<uintptr_t>(f.y) % 16) != 0 || (f.y_sc % 4) != 0) return VND_EUNSUPPORTED;
@@ -835,7 +498,7 @@ static int fir_tmem_launch_t(const FirParams& f, int max_prog_words, cudaStream_
   if (nblk < fill_blocks) nblk = fill_blocks;
   const int opstride = (max_prog_words + 4 + 3) & ~3;  // a multiple of 4 words: the segment tables behind the lists stay 16-byte aligned
   const size_t bufw = ((size_t)nblk * kPitch + 31) & ~(size_t)31;
-  const size_t smem = kBarBytes + T::kNBuf * bufw * 4 + (size_t)kRows * kPitch * 4 + tm_tail_words<T>(opstride) * 4;
+  const size_t smem = kBarBytes + kNBuf * bufw * 4 + (size_t)kRows * kPitch * 4 + tm_tail_words(opstride) * 4;
   if (smem > (size_t)kMaxDynSmem || nblk > 256) return VND_EUNSUPPORTED;  // a TMA box has at most 256 rows
   if (f.channels > 1 && (f.x_sc % 4 != 0 || f.x_sc < f.frames || f.y_sc < f.frames)) return VND_EUNSUPPORTED;
   const long long span = (long long)nblk * kR;  // samples a tile's bulk loads touch
@@ -856,86 +519,35 @@ static int fir_tmem_launch_t(const FirParams& f, int max_prog_words, cudaStream_
   P.tiles_per_channel = (int)tiles;
   plan_runs(tiles, f.channels, di.sm_count, &P.tiles_per_run, &P.runs_per_channel);
   P.n_runs = P.runs_per_channel * f.channels;
-  VND_CUDA_OK(cudaFuncSetAttribute(fir_tmem_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  VND_CUDA_OK(cudaFuncSetAttribute(fir_tmem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int grid = di.sm_count;
   if (grid > P.n_runs) grid = P.n_runs;
-  fir_tmem_kernel<T><<<(unsigned)grid, T::kNT, smem, st>>>(P);
+  fir_tmem_kernel<<<(unsigned)grid, kNT, smem, st>>>(P);
   rc = after_launch("fir_tmem_kernel");
   if (rc) return rc;
   *frames_done = tiles * kTile;
   return VND_OK;
 }
 
-// Shapes measured in round 2 (148 channels x 28.8 M frames, Gsamples/s, all bit-exact; profiles/r02_summary.md):
-//   0: 3 x 32 outputs, rows of 96 (default)                       357
-//   1: 2 x 48 outputs, rows of 96                                 325
-//   2: 2 x 64 outputs, rows of 128, two tile buffers              338
-//   3: 2 x 32 outputs, rows of 64 (TMEM refill 8 words/output)    298
-//   4: shape 3 with software-pipelined tensor-memory taps         272 (235 before the loop exits kept ptxas from
-//      interleaving the adds of the landed and of the in-flight buffer)
-// Two compute warps per scheduler do not make the tensor-memory path faster in the kernel (they do in
-// tools/microbench/tmem_lat.cu), and a second tcgen05.ld in flight per warp slows the taps down even with the
-// intended instruction order, so the round-1 shape stays.
-// Scheduling variants of the default shape (third session of round 2, same measurement, default 378-380; the timelines
-// behind the verdicts are in profiles/r02_summary.md):
-//   5: trailing all-far segment paired tap by tap with the first segment (pair_first), far sum parked           278
-//      (full-width steps spilled scalars into the hot loops: 203 at 144 registers, 277 at 152)
-//   6: quarters {0,1} / {2,3} alternate in the far phase (kGate 2)                                                 375
-//   7: one quarter at a time in the far phase (kGate 4, a ring)                                                    268
-//   8: all-far segment first with double-buffered loads, sum parked (kFarFirstMode 1)                              321
-//   9 / 10: 8 with kGate 2 / 4                                                                                      306 / 219
-//   11: all-far segment first on the last warp of each quarter only (two warps per scheduler in TMEM taps)        307
-//   12: all-far segment first on every warp, plain loop                                                            344
-//   15: symmetric CTA, 4 warps per quarter x 32 outputs, rows of 128, no data-movement warps (sym_main)          355
-//   13 / 14: two tensor-memory taps per round trip (both loads issued, one wait, then both sets of adds; kDual),   300 / 278
-//      152 / 56 and 144 / 80 registers (16 / 128 bytes of spilled scalars)
-// With four warps per scheduler (15) a tensor-memory tap takes 300 clk per warp, with three 240, with two of the three (11)
-// still 240 while the third is elsewhere: ~75-80 clk of the quarter's TMEM read path per x32 load however many warps ask,
-// i.e. ~54 B/clk per scheduler - the tensor-memory phase (22 taps x 3 warps x 4 KB) is bound by that path.
-// The per-warp chain of a tap (~240 clk from tensor memory, ~400 clk from shared memory) does not shorten when fewer
-// warps contend (far phase 3.2 k clk per tile with one quarter in it, 3.5 k with two, 3.8 k with four), so taking turns
-// buys nothing, and every form of overlap inside a warp has made the taps slower.
-int fir_tmem_launch(const FirParams& f, int max_prog_words, cudaStream_t st, long long* frames_done) {
-  switch (g_tm_shape) {
-    case 1: return fir_tmem_launch_t<TmShape<2, 48, 3, 200, 104>>(f, max_prog_words, st, frames_done);
-    case 2: return fir_tmem_launch_t<TmShape<2, 64, 2, 216, 72>>(f, max_prog_words, st, frames_done);
-    case 3: return fir_tmem_launch_t<TmShape<2, 32, 3, 200, 104>>(f, max_prog_words, st, frames_done);
-    case 4: return fir_tmem_launch_t<TmShape<2, 32, 3, 200, 104, true>>(f, max_prog_words, st, frames_done);
-    case 5: return fir_tmem_launch_t<TmShape<3, 32, 3, 144, 80, false, true, true>>(f, max_prog_words, st, frames_done);
-    case 6: return fir_tmem_launch_t<TmShape<3, 32, 3, 144, 80, false, false, false, 2>>(f, max_prog_words, st, frames_done);
-    case 7: return fir_tmem_launch_t<TmShape<3, 32, 3, 144, 80, false, false, false, 4>>(f, max_prog_words, st, frames_done);
-    case 8: return fir_tmem_launch_t<TmShape<3, 32, 3, 144, 80, false, false, false, 0, 1>>(f, max_prog_words, st, frames_done);
-    case 9: return fir_tmem_launch_t<TmShape<3, 32, 3, 144, 80, false, false, false, 2, 1>>(f, max_prog_words, st, frames_done);
-    case 10: return fir_tmem_launch_t<TmShape<3, 32, 3, 144, 80, false, false, false, 4, 1>>(f, max_prog_words, st, frames_done);
-    case 11: return fir_tmem_launch_t<TmShape<3, 32, 3, 144, 80, false, false, false, 0, 2>>(f, max_prog_words, st, frames_done);
-    case 12: return fir_tmem_launch_t<TmShape<3, 32, 3, 144, 80, false, false, false, 0, 3>>(f, max_prog_words, st, frames_done);
-    case 13: return fir_tmem_launch_t<TmShape<3, 32, 3, 152, 56, false, false, false, 0, 0, true>>(f, max_prog_words, st, frames_done);
-    case 14: return fir_tmem_launch_t<TmShape<3, 32, 3, 144, 80, false, false, false, 0, 0, true>>(f, max_prog_words, st, frames_done);
-    case 15: return fir_tmem_launch_t<TmShape<4, 32, 2, 128, 0, false, false, false, 0, 0, false, true>>(f, max_prog_words, st, frames_done);
-    default: return fir_tmem_launch_t<TmShape<3, 32, 3, 144, 80>>(f, max_prog_words, st, frames_done);
-  }
-}
-
-// Debug / test aid (not part of the ABI in include/vnd_b200.h): the run plan of the default shape for a slab -
+// Debug / test aid (not part of the ABI in include/vnd_b200.h): the run plan of the kernel for a slab -
 // out[0] = tiles per run, out[1] = runs per channel, out[2] = frames per tile; bench.py uses it to place a parity
 // window across a run boundary.  Returns VND_EUNSUPPORTED when the slab would not take the tensor-memory kernel.
 extern "C" int vnd_debug_fir_plan(long long frames, int channels, int halo, int* out) {
-  using T = TmShape<3, 32, 3, 144, 80>;
-  if (!out || g_tm_shape != 0) return VND_EUNSUPPORTED;
+  if (!out) return VND_EUNSUPPORTED;
   halo = (halo + 3) & ~3;
-  int nblk = kRows + (halo + 4 + T::kR - 1) / T::kR;
-  const int fill_blocks = kRows + (kCols + T::kR - 1) / T::kR;
+  int nblk = kRows + (halo + 4 + kR - 1) / kR;
+  const int fill_blocks = kRows + (kCols + kR - 1) / kR;
   if (nblk < fill_blocks) nblk = fill_blocks;
-  const long long span = (long long)nblk * T::kR;
-  if (nblk > 256 || frames < span + 3LL * T::kTile) return VND_EUNSUPPORTED;
+  const long long span = (long long)nblk * kR;
+  if (nblk > 256 || frames < span + 3LL * kTile) return VND_EUNSUPPORTED;
   DeviceInfo di;
   if (device_info(&di)) return VND_ECUDA;
-  const long long tiles = (frames - span) / T::kTile + 1;
+  const long long tiles = (frames - span) / kTile + 1;
   int tpr = 0, rpc = 0;
   plan_runs(tiles, channels, di.sm_count, &tpr, &rpc);
   out[0] = tpr;
   out[1] = rpc;
-  out[2] = T::kTile;
+  out[2] = kTile;
   return VND_OK;
 }
 

@@ -1,8 +1,7 @@
-// Tensor-memory gather primitives shared by the sparse-FIR kernel (vnd_fir_tmem.cu) and the batched objective kernel
-// (vnd_objective_tmem.cu): tcgen05 allocation / load / store wrappers, packed fp32 arithmetic, and the tap machinery
-// that applies one decay segment after the other to a thread's RG consecutive outputs in the reference's order
-// (src/vndecorrelate/decorrelation.py:402-414) - taps inside the TMEM window as one tcgen05.ld each, the others as
-// 16-byte shared-memory loads from the staged tile.
+// Tensor-memory gather primitives of the sparse-FIR kernel (vnd_fir_tmem.cu): tcgen05 allocation / load / store
+// wrappers, packed fp32 arithmetic, and the tap machinery that applies one decay segment after the other to a thread's
+// kRG consecutive outputs in the reference's order (src/vndecorrelate/decorrelation.py:402-414) - taps inside the TMEM
+// window as one tcgen05.ld each, the others as 16-byte shared-memory loads from the staged tile.
 #pragma once
 
 #include "vnd_common.cuh"
@@ -19,6 +18,7 @@ namespace tm {
 constexpr int kRows = 128;             // TMEM lanes = rows of a tile
 constexpr int kCols = 512;             // TMEM columns
 constexpr int kUnits = kCols / 32;     // 32-column units of a TMEM row
+constexpr int kRG = 32;                // consecutive outputs per compute thread: a tensor-memory tap is one x32 tcgen05.ld
 
 // ---- tensor-memory primitives -------------------------------------------------------------------
 __device__ __forceinline__ void tmem_alloc_all(uint32_t* slot) {
@@ -38,45 +38,18 @@ __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.
 #define VND_IO16(v, i) VND_IO4(v, i), VND_IO4(v, i + 4), VND_IO4(v, i + 8), VND_IO4(v, i + 12)
 #define VND_I4(v, i) "f"(v[i].x), "f"(v[i].y), "f"(v[i].z), "f"(v[i].w)
 
-// N consecutive columns of this thread's TMEM lane, starting at column (taddr & 0xffff), into v[O .. O + N).
-template <int N, int O, int RG>
-__device__ __forceinline__ void tmem_ld(float (&v)[RG], uint32_t taddr) {
-  static_assert(N == 16 || N == 32 || N == 64, "tcgen05.ld.32x32b.x16 / .x32 / .x64");
-  static_assert(O + N <= RG, "destination range");
-  if constexpr (N == 16) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                 : VND_O16(v, O)
-                 : "r"(taddr));
-  } else if constexpr (N == 32) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-        "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-        : VND_O16(v, O), VND_O16(v, O + 16)
-        : "r"(taddr));
-  } else {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x64.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-        "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31,"
-        "%32,%33,%34,%35,%36,%37,%38,%39,%40,%41,%42,%43,%44,%45,%46,%47,"
-        "%48,%49,%50,%51,%52,%53,%54,%55,%56,%57,%58,%59,%60,%61,%62,%63}, [%64];"
-        : VND_O16(v, O), VND_O16(v, O + 16), VND_O16(v, O + 32), VND_O16(v, O + 48)
-        : "r"(taddr));
-  }
+// 32 consecutive columns of this thread's TMEM lane, starting at column (taddr & 0xffff).
+__device__ __forceinline__ void tmem_ld32(float (&v)[kRG], uint32_t taddr) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
+      "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+      : VND_O16(v, 0), VND_O16(v, 16)
+      : "r"(taddr));
 }
 // The loaded registers are only defined after the wait; naming them as in/out operands keeps the
 // compiler from moving their consumers above it.
-template <int RG>
-__device__ __forceinline__ void tmem_wait_ld(float (&v)[RG]) {
-  static_assert(RG == 16 || RG == 32 || RG == 48 || RG == 64, "outputs per thread");
-  if constexpr (RG == 16) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;" : VND_IO16(v, 0)::"memory");
-  } else if constexpr (RG == 32) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;" : VND_IO16(v, 0), VND_IO16(v, 16)::"memory");
-  } else if constexpr (RG == 48) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;" : VND_IO16(v, 0), VND_IO16(v, 16), VND_IO16(v, 32)::"memory");
-  } else {
-    asm volatile("tcgen05.wait::ld.sync.aligned;" : VND_IO16(v, 0), VND_IO16(v, 16), VND_IO16(v, 32), VND_IO16(v, 48)::"memory");
-  }
+__device__ __forceinline__ void tmem_wait_ld(float (&v)[kRG]) {
+  asm volatile("tcgen05.wait::ld.sync.aligned;" : VND_IO16(v, 0), VND_IO16(v, 16)::"memory");
 }
 // 32 consecutive columns written from eight float4.
 __device__ __forceinline__ void tmem_st32(uint32_t taddr, const float4 (&v)[8]) {
@@ -157,39 +130,12 @@ VND_PACKED_OP(add2, "add")
 VND_PACKED_OP(sub2, "sub")
 VND_PACKED_OP(mul2, "mul")
 
-// A tap served from tensor memory: the thread's RG columns starting at the tap's column, then RG / 2
+// A tap served from tensor memory: the thread's kRG columns starting at the tap's column (tmem_ld32), then kRG / 2
 // packed adds (or subtracts).
-template <int RG>
-__device__ __forceinline__ void near_issue(float (&t)[RG], uint32_t tcol) {
-  if constexpr (RG == 16) {
-    tmem_ld<16, 0>(t, tcol);
-  } else if constexpr (RG == 32) {
-#if defined(VND_TM_PROBE) && VND_TM_PROBE == 1  // timing probe (results wrong by construction): half of the tensor-memory bytes per tap
-    tmem_ld<16, 0>(t, tcol);
-    tmem_ld<16, 16>(t, tcol);
-#elif defined(VND_TM_PROBE) && VND_TM_PROBE == 3  // ... a quarter
-    tmem_ld<16, 0>(t, tcol);
+template <bool SUB>
+__device__ __forceinline__ void near_add(const float (&t)[kRG], float (&acc)[kRG]) {
 #pragma unroll
-    for (int j = 16; j < 32; ++j) t[j] = 0.0f;
-#else
-    tmem_ld<32, 0>(t, tcol);
-#endif
-  } else if constexpr (RG == 48) {
-    tmem_ld<32, 0>(t, tcol);
-    tmem_ld<16, 32>(t, tcol + 32);
-  } else {
-    tmem_ld<64, 0>(t, tcol);
-  }
-}
-template <bool SUB, int RG>
-__device__ __forceinline__ void near_add(const float (&t)[RG], float (&acc)[RG]) {
-#if defined(VND_TM_PROBE) && VND_TM_PROBE == 2  // timing probe (results wrong by construction): a quarter of the adds per tap
-  constexpr int kAdds = RG / 8;
-#else
-  constexpr int kAdds = RG / 2;
-#endif
-#pragma unroll
-  for (int j = 0; j < kAdds; ++j) {
+  for (int j = 0; j < kRG / 2; ++j) {
     if constexpr (SUB) sub2(acc[2 * j], acc[2 * j + 1], t[2 * j], t[2 * j + 1]);
     else add2(acc[2 * j], acc[2 * j + 1], t[2 * j], t[2 * j + 1]);
   }
@@ -199,7 +145,7 @@ __device__ __forceinline__ void near_add(const float (&t)[RG], float (&acc)[RG])
 // operation word (build_ops) carries the word offset of the aligned 16-byte chunk that holds the
 // thread's first operand, the operand's position A inside it and kx, the number of chunks before the
 // run crosses into the next block, where the pitch inserts a 4-word gap (kx >= chunks of the tap: no crossing).
-// The RG operands lie in RG / 4 (A == 0) or RG / 4 + 1 chunks.
+// The kRG operands lie in kRG / 4 (A == 0) or kRG / 4 + 1 chunks.
 // The chunks are read with explicit 16-byte loads: left to the compiler, the partly used first and last
 // chunk become 4- and 8-byte loads, which cost as many shared-memory wavefronts each as the full chunk
 // (lanes are a pitch apart: a 4-way conflict for LDS.32, 2-way for LDS.64) and up to twice together.
@@ -208,17 +154,13 @@ __device__ __forceinline__ float4 lds128(uint32_t addr) {
   asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
   return v;
 }
-template <int A, bool SUB, int RG>
-__device__ __forceinline__ void far_tap_a(uint32_t row, int op, float (&acc)[RG]) {
-  constexpr int NC = RG / 4 + ((A == 0) ? 0 : 1);
+template <int A, bool SUB>
+__device__ __forceinline__ void far_tap_a(uint32_t row, int op, float (&acc)[kRG]) {
+  constexpr int NC = kRG / 4 + ((A == 0) ? 0 : 1);
   const uint32_t p = row + 4u * (uint32_t)(op & 0xffff);  // `row`: shared-memory address of the thread's row
   const int kx = (op >> 16) & 31;
   float4 c[NC];
-#if defined(VND_TM_PROBE) && (VND_TM_PROBE == 5 || VND_TM_PROBE == 7)  // timing probe (results wrong by construction): no block crossing
-  if (true) {
-#else
   if (kx >= NC) {
-#endif
 #pragma unroll
     for (int k = 0; k < NC; ++k) c[k] = lds128(p + 16u * k);
   } else {
@@ -235,60 +177,13 @@ __device__ __forceinline__ void far_tap_a(uint32_t row, int op, float (&acc)[RG]
   }
   if constexpr (A % 2 == 0) {  // operands arrive as aligned register pairs
 #pragma unroll
-    for (int j = 0; j < RG / 2; ++j) {
+    for (int j = 0; j < kRG / 2; ++j) {
       if constexpr (SUB) sub2(acc[2 * j], acc[2 * j + 1], t[2 * j + A], t[2 * j + 1 + A]);
       else add2(acc[2 * j], acc[2 * j + 1], t[2 * j + A], t[2 * j + 1 + A]);
     }
   } else {  // odd shift: the pairs of the loaded data straddle the accumulator pairs -> scalar adds
 #pragma unroll
-    for (int r = 0; r < RG; ++r) acc[r] = SUB ? fsub(acc[r], t[r + A]) : fadd(acc[r], t[r + A]);
-  }
-}
-
-// The same tap in two steps, for the paired loop below: the nine (eight when A == 0) 16-byte loads first, the adds once
-// something else has been issued behind them.
-__device__ __forceinline__ void far_load9(uint32_t row, int op, float4 (&c)[9]) {
-  const uint32_t p = row + 4u * (uint32_t)(op & 0xffff);
-  const int kx = (op >> 16) & 31;
-  if (kx >= 9) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) c[k] = lds128(p + 16u * k);
-  } else {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) c[k] = lds128(p + 16u * k + (k < kx ? 0u : 16u));
-  }
-  if ((op >> 24) & 3) c[8] = lds128(p + 128u + (8 < kx ? 0u : 16u));  // the ninth chunk only exists for an unaligned tap
-  else c[8] = c[7];
-}
-template <int A, bool SUB, int RG>
-__device__ __forceinline__ void far_add9(const float4 (&c)[9], float (&acc)[RG]) {
-  static_assert(RG == 32, "nine chunks hold 32 operands");
-  float t[36];
-#pragma unroll
-  for (int k = 0; k < 9; ++k) {
-    t[4 * k] = c[k].x;
-    t[4 * k + 1] = c[k].y;
-    t[4 * k + 2] = c[k].z;
-    t[4 * k + 3] = c[k].w;
-  }
-  if constexpr (A % 2 == 0) {
-#pragma unroll
-    for (int j = 0; j < RG / 2; ++j) {
-      if constexpr (SUB) sub2(acc[2 * j], acc[2 * j + 1], t[2 * j + A], t[2 * j + 1 + A]);
-      else add2(acc[2 * j], acc[2 * j + 1], t[2 * j + A], t[2 * j + 1 + A]);
-    }
-  } else {
-#pragma unroll
-    for (int r = 0; r < RG; ++r) acc[r] = SUB ? fsub(acc[r], t[r + A]) : fadd(acc[r], t[r + A]);
-  }
-}
-template <bool SUB, int RG>
-__device__ __forceinline__ void far_add9_any(const float4 (&c)[9], int op, float (&acc)[RG]) {
-  switch ((op >> 24) & 3) {
-    case 0: far_add9<0, SUB>(c, acc); break;
-    case 1: far_add9<1, SUB>(c, acc); break;
-    case 2: far_add9<2, SUB>(c, acc); break;
-    default: far_add9<3, SUB>(c, acc); break;
+    for (int r = 0; r < kRG; ++r) acc[r] = SUB ? fsub(acc[r], t[r + A]) : fadd(acc[r], t[r + A]);
   }
 }
 
@@ -297,12 +192,8 @@ __device__ __forceinline__ void far_add9_any(const float4 (&c)[9], int op, float
 //   far tap:  kOpFar | A << 24 | kx << 16 | word offset of the first chunk relative to the thread's row
 constexpr int kOpFar = (int)0x80000000u;
 
-template <bool SUB, int RG>
-__device__ __forceinline__ void far_tap(uint32_t row, int op, float (&acc)[RG]) {
-#if defined(VND_TM_PROBE) && (VND_TM_PROBE == 6 || VND_TM_PROBE == 7)  // timing probe (results wrong by construction): every far tap as an aligned one
-  far_tap_a<0, SUB>(row, op, acc);
-  return;
-#endif
+template <bool SUB>
+__device__ __forceinline__ void far_tap(uint32_t row, int op, float (&acc)[kRG]) {
   switch ((op >> 24) & 3) {
     case 0: far_tap_a<0, SUB>(row, op, acc); break;
     case 1: far_tap_a<1, SUB>(row, op, acc); break;
@@ -312,11 +203,11 @@ __device__ __forceinline__ void far_tap(uint32_t row, int op, float (&acc)[RG]) 
 }
 
 // One tap: from tensor memory (op >= 0) or from shared memory.
-template <bool SUB, bool ALLFAR, int RG>
-__device__ __forceinline__ void one_tap(int op, uint32_t tcol0, uint32_t row, float (&acc)[RG]) {
+template <bool SUB, bool ALLFAR>
+__device__ __forceinline__ void one_tap(int op, uint32_t tcol0, uint32_t row, float (&acc)[kRG]) {
   if (!ALLFAR && op >= 0) {
-    float t[RG];
-    near_issue(t, tcol0 + (uint32_t)op);
+    float t[kRG];
+    tmem_ld32(t, tcol0 + (uint32_t)op);
     tmem_wait_ld(t);
     near_add<SUB>(t, acc);
   } else {
@@ -331,74 +222,17 @@ __device__ __forceinline__ void one_tap(int op, uint32_t tcol0, uint32_t row, fl
 // The loops are unrolled by two with the operation words in alternating registers, so that each word
 // is loaded a whole tap before it is needed and never copied (a single loop-carried register made
 // ptxas copy the loaded word at once and stall on the shared-memory latency at every tap).
-template <bool SUB, bool ALLFAR, bool PIPE, int RG, bool DUAL = false>
-__device__ __forceinline__ void tap_list(const int* __restrict__ ops, int n, int nn, uint32_t tcol0, uint32_t row, float (&acc)[RG]) {
+template <bool SUB, bool ALLFAR>
+__device__ __forceinline__ void tap_list(const int* __restrict__ ops, int n, int nn, uint32_t tcol0, uint32_t row, float (&acc)[kRG]) {
   if (n <= 0) return;
   int k = 0;
   int op_a = ops[0];
-  if constexpr (!ALLFAR && PIPE) {
-    // Two operand buffers with fixed roles: the load of tap k + 1 is issued right after the wait for tap k, so its
-    // latency runs under the adds of tap k.  tcgen05.wait::ld waits for every outstanding load of the thread, hence
-    // exactly one load is in flight at each wait.
-    if (nn > 0) {
-      // One tap per half, with the loop exit BETWEEN the halves: the branch keeps ptxas from hoisting the adds of the
-      // buffer whose load was just issued above the adds of the buffer that has landed (it interleaves them when both
-      // sit in one basic block, and the warp then stalls on the fresh load with most of its adds still to issue).
-      float ta[RG], tb[RG];
-      near_issue(ta, tcol0 + (uint32_t)op_a);
-      for (;;) {
-        {
-          const int op_n = ops[k + 1];  // slack words follow the lists
-          tmem_wait_ld(ta);
-          if (k + 1 < nn) near_issue(tb, tcol0 + (uint32_t)op_n);
-          near_add<SUB>(ta, acc);
-          if (++k >= nn) break;
-        }
-        {
-          const int op_n = ops[k + 1];
-          tmem_wait_ld(tb);
-          if (k + 1 < nn) near_issue(ta, tcol0 + (uint32_t)op_n);
-          near_add<SUB>(tb, acc);
-          if (++k >= nn) break;
-        }
-      }
-      if (k >= n) return;
-      op_a = ops[k];
-    }
-  } else if constexpr (!ALLFAR && DUAL) {
-    // Two taps per tensor-memory round trip: both loads are issued, ONE wait covers them (tcgen05.wait::ld waits for every
-    // outstanding load of the thread anyway), then both sets of adds.  Needs a second landing buffer (64 registers).
-    for (; k + 1 < nn; k += 2) {
-      const int op_b = ops[k + 1];
-      float ta[RG], tb[RG];
-      near_issue(ta, tcol0 + (uint32_t)op_a);
-      near_issue(tb, tcol0 + (uint32_t)op_b);
-      op_a = ops[k + 2];  // two words of slack follow the lists
-      tmem_wait_ld(ta);
-      tmem_wait_ld(tb);
-      near_add<SUB>(ta, acc);
-      near_add<SUB>(tb, acc);
-    }
-    if (k < nn) {
-      float t[RG];
-      near_issue(t, tcol0 + (uint32_t)op_a);
-      tmem_wait_ld(t);
-      near_add<SUB>(t, acc);
-      ++k;
-      op_a = ops[k];
-    }
-    if (k >= n) return;
-  } else if constexpr (!ALLFAR) {
+  if constexpr (!ALLFAR) {
     for (; k < nn; k += 2) {  // near prefix
-#if defined(VND_TM_PROBE) && VND_TM_PROBE == 4  // timing probe (results wrong by construction): tap columns without the operation words
-      const int op_b = 8 * k + 8;
-      op_a = 8 * k;
-#else
       const int op_b = ops[k + 1];  // two words of slack follow the lists, so the prefetches stay in bounds
-#endif
       {
-        float t[RG];
-        near_issue(t, tcol0 + (uint32_t)op_a);
+        float t[kRG];
+        tmem_ld32(t, tcol0 + (uint32_t)op_a);
         tmem_wait_ld(t);
         near_add<SUB>(t, acc);
       }
@@ -409,8 +243,8 @@ __device__ __forceinline__ void tap_list(const int* __restrict__ ops, int n, int
         break;
       }
       {
-        float t[RG];
-        near_issue(t, tcol0 + (uint32_t)op_b);
+        float t[kRG];
+        tmem_ld32(t, tcol0 + (uint32_t)op_b);
         tmem_wait_ld(t);
         near_add<SUB>(t, acc);
       }
@@ -430,201 +264,36 @@ __device__ __forceinline__ void tap_list(const int* __restrict__ ops, int n, int
 // Segments [s0, s1) of the program added into the running output, in the reference's order
 // (decorrelation.py:402-414): acc = 0; acc -= x[n + i] over the negative list; acc += x[n + i] over
 // the positive list; acc *= gain; y += acc.
-template <bool ALLFAR, bool PIPE, int RG, bool DUAL = false>
+template <bool ALLFAR>
 __device__ __forceinline__ void run_segments(const int4* __restrict__ segtab, int s0, int s1, const int*& ops, uint32_t tcol0, uint32_t row,
-                                             float (&yv)[RG]) {
+                                             float (&yv)[kRG]) {
   for (int s = s0; s < s1; ++s) {
     const int4 d = segtab[s];  // x = negative taps, y = positive taps, z = leading tensor-memory taps of both lists, w = gain bits
     const int n_neg = d.x, n_pos = d.y;
-    float acc[RG];
+    float acc[kRG];
 #pragma unroll
-    for (int r = 0; r < RG; ++r) acc[r] = 0.0f;
+    for (int r = 0; r < kRG; ++r) acc[r] = 0.0f;
     const int nn = ALLFAR ? 0 : d.z;  // leading tensor-memory taps: neg list in the low half, pos list in the high half
-    tap_list<true, ALLFAR, PIPE, RG, DUAL>(ops, n_neg, nn & 0xffff, tcol0, row, acc);
-    tap_list<false, ALLFAR, PIPE, RG, DUAL>(ops + n_neg, n_pos, nn >> 16, tcol0, row, acc);
+    tap_list<true, ALLFAR>(ops, n_neg, nn & 0xffff, tcol0, row, acc);
+    tap_list<false, ALLFAR>(ops + n_neg, n_pos, nn >> 16, tcol0, row, acc);
     ops += n_neg + n_pos;
     {  // 1.0f when the program carries no gains (x * 1 == x bit for bit)
       const float gain = __int_as_float(d.w);
 #pragma unroll
-      for (int j = 0; j < RG / 2; ++j) mul2(acc[2 * j], acc[2 * j + 1], gain, gain);
+      for (int j = 0; j < kRG / 2; ++j) mul2(acc[2 * j], acc[2 * j + 1], gain, gain);
     }
     if (s == 0) {  // the reference adds into zeros (a -0 partial sum becomes +0)
 #pragma unroll
-      for (int j = 0; j < RG / 2; ++j) {
+      for (int j = 0; j < kRG / 2; ++j) {
         yv[2 * j] = acc[2 * j];
         yv[2 * j + 1] = acc[2 * j + 1];
         add2(yv[2 * j], yv[2 * j + 1], 0.0f, 0.0f);
       }
     } else {
 #pragma unroll
-      for (int j = 0; j < RG / 2; ++j) add2(yv[2 * j], yv[2 * j + 1], acc[2 * j], acc[2 * j + 1]);
+      for (int j = 0; j < kRG / 2; ++j) add2(yv[2 * j], yv[2 * j + 1], acc[2 * j], acc[2 * j + 1]);
     }
   }
-}
-
-// ---- paired first step (TmShape::kPair) ------------------------------------------------------------
-// The decay segments are independent sums (decorrelation.py:402-414: `acc` restarts per segment); only the running
-// output adds them in order.  So the trailing all-far segment need not wait for the tensor-memory segments: here it
-// advances together with the FIRST segment, one tap of each per step - the nine shared-memory loads of the far tap
-// are issued, a tensor-memory tap runs behind them, then the far tap's adds - while the running output is not live
-// yet (its registers hold the second accumulator).  The far sum is scaled, kept, and added last, so every output
-// sees the reference's operations in the reference's order.
-// One half of a paired step: outputs [16 H, 16 H + 16) of the thread.  The far tap's operands for that half lie in
-// chunks 4 H .. 4 H + 4 of its nine (the fifth only for an unaligned tap); the tensor-memory tap reads 16 columns.
-// Halves keep the loop at ~100 live registers (two 32-float accumulators, 16 + 20 landing registers): the full-width
-// version (36 + 32 landing registers) spilled scalars into the hot loops and ran at 277 instead of 378 Gsamples/s.
-template <int H, bool SUBF, int A>
-__device__ __forceinline__ void far_add_half(const float4 (&c)[5], float (&far)[32]) {
-  float t[20];
-#pragma unroll
-  for (int k = 0; k < 5; ++k) {
-    t[4 * k] = c[k].x;
-    t[4 * k + 1] = c[k].y;
-    t[4 * k + 2] = c[k].z;
-    t[4 * k + 3] = c[k].w;
-  }
-  if constexpr (A % 2 == 0) {
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      if constexpr (SUBF) sub2(far[16 * H + 2 * j], far[16 * H + 2 * j + 1], t[2 * j + A], t[2 * j + 1 + A]);
-      else add2(far[16 * H + 2 * j], far[16 * H + 2 * j + 1], t[2 * j + A], t[2 * j + 1 + A]);
-    }
-  } else {
-#pragma unroll
-    for (int r = 0; r < 16; ++r) far[16 * H + r] = SUBF ? fsub(far[16 * H + r], t[r + A]) : fadd(far[16 * H + r], t[r + A]);
-  }
-}
-template <int H>
-__device__ __forceinline__ void pair_half(int opn, int opf, bool subn, bool subf, uint32_t tcol0, uint32_t row, float (&acc)[32], float (&far)[32]) {
-  const uint32_t p = row + 4u * (uint32_t)(opf & 0xffff);
-  const int kx = (opf >> 16) & 31, A = (opf >> 24) & 3;
-  float4 c[5];
-#pragma unroll
-  for (int k = 0; k < 4; ++k) c[k] = lds128(p + 16u * (4 * H + k) + ((4 * H + k) < kx ? 0u : 16u));
-  if (A) c[4] = lds128(p + 16u * (4 * H + 4) + ((4 * H + 4) < kx ? 0u : 16u));
-  else c[4] = c[3];
-  {
-    float t[16];
-    tmem_ld<16, 0>(t, tcol0 + (uint32_t)opn + 16u * H);
-    tmem_wait_ld(t);
-    if (subn) {
-#pragma unroll
-      for (int j = 0; j < 8; ++j) sub2(acc[16 * H + 2 * j], acc[16 * H + 2 * j + 1], t[2 * j], t[2 * j + 1]);
-    } else {
-#pragma unroll
-      for (int j = 0; j < 8; ++j) add2(acc[16 * H + 2 * j], acc[16 * H + 2 * j + 1], t[2 * j], t[2 * j + 1]);
-    }
-  }
-  if (subf) {
-    switch (A) {
-      case 0: far_add_half<H, true, 0>(c, far); break;
-      case 1: far_add_half<H, true, 1>(c, far); break;
-      case 2: far_add_half<H, true, 2>(c, far); break;
-      default: far_add_half<H, true, 3>(c, far); break;
-    }
-  } else {
-    switch (A) {
-      case 0: far_add_half<H, false, 0>(c, far); break;
-      case 1: far_add_half<H, false, 1>(c, far); break;
-      case 2: far_add_half<H, false, 2>(c, far); break;
-      default: far_add_half<H, false, 3>(c, far); break;
-    }
-  }
-}
-template <int RG>
-__device__ __forceinline__ void pair_step(int opn, int opf, bool subn, bool subf, uint32_t tcol0, uint32_t row, float (&acc)[RG], float (&far)[RG]) {
-  static_assert(RG == 32, "two halves of 16 outputs");
-  pair_half<0>(opn, opf, subn, subf, tcol0, row, acc, far);
-  pair_half<1>(opn, opf, subn, subf, tcol0, row, acc, far);
-}
-
-// Segment 0 (every tap inside the TMEM window) into yv, segment S - 1 (no tap inside it) scaled into far.
-// ops: decoded operations of segment 0 (those of the later segments follow), opsF: those of segment S - 1.
-template <int RG>
-__device__ __forceinline__ void pair_first(const int4* __restrict__ segtab, int S, const int* __restrict__ ops, const int* __restrict__ opsF,
-                                           uint32_t tcol0, uint32_t row, float (&yv)[RG], float (&far)[RG]) {
-  const int4 d0 = segtab[0], dF = segtab[S - 1];
-  const int nneg0 = d0.x, n0 = d0.x + d0.y, nnegF = dF.x, nF = dF.x + dF.y;
-  const int np = n0 < nF ? n0 : nF;
-  float acc[RG];
-#pragma unroll
-  for (int r = 0; r < RG; ++r) {
-    acc[r] = 0.0f;
-    far[r] = 0.0f;
-  }
-  int k = 0;
-  if (np > 0) {  // unrolled by two with the operation words in alternating registers (see tap_list)
-    int na = ops[0], fa = opsF[0];
-    for (;;) {
-      const int nb = ops[k + 1], fb = opsF[k + 1];  // slack words follow the lists
-      pair_step(na, fa, k < nneg0, k < nnegF, tcol0, row, acc, far);
-      if (++k >= np) break;
-      na = ops[k + 1];
-      fa = opsF[k + 1];
-      pair_step(nb, fb, k < nneg0, k < nnegF, tcol0, row, acc, far);
-      if (++k >= np) break;
-    }
-  }
-  for (int j = k; j < n0; ++j) {  // the first segment has more taps than the far one
-    float t[RG];
-    near_issue(t, tcol0 + (uint32_t)ops[j]);
-    tmem_wait_ld(t);
-    if (j < nneg0) near_add<true>(t, acc);
-    else near_add<false>(t, acc);
-  }
-  {
-    const float g0 = __int_as_float(d0.w);
-#pragma unroll
-    for (int j = 0; j < RG / 2; ++j) {
-      mul2(acc[2 * j], acc[2 * j + 1], g0, g0);
-      yv[2 * j] = acc[2 * j];
-      yv[2 * j + 1] = acc[2 * j + 1];
-      add2(yv[2 * j], yv[2 * j + 1], 0.0f, 0.0f);  // the reference adds into zeros
-    }
-  }
-  for (int j = k; j < nF; ++j) {  // ... or fewer
-    if (j < nnegF) far_tap<true>(row, opsF[j], far);
-    else far_tap<false>(row, opsF[j], far);
-  }
-  {
-    const float gF = __int_as_float(dF.w);
-#pragma unroll
-    for (int j = 0; j < RG / 2; ++j) mul2(far[2 * j], far[2 * j + 1], gF, gF);
-  }
-}
-
-// ---- far-first (TmShape::kFarFirst) ------------------------------------------------------------------
-// The trailing all-far segment alone, before anything else of the tile: the running output is not live yet, so two
-// landing buffers fit and the nine loads of tap k + 1 are in flight under the adds of tap k.  Scaled sum into far.
-template <int RG>
-__device__ __forceinline__ void far_first(const int4* __restrict__ segtab, int S, const int* __restrict__ opsF, uint32_t row, float (&far)[RG]) {
-  const int4 dF = segtab[S - 1];
-  const int nneg = dF.x, n = dF.x + dF.y;
-#pragma unroll
-  for (int r = 0; r < RG; ++r) far[r] = 0.0f;
-  if (n > 0) {
-    float4 ca[9], cb[9];
-    int oa = opsF[0];
-    far_load9(row, oa, ca);
-    int k = 0;
-    for (;;) {
-      // (the prefetch behind the last tap reads the zero slack word that follows the list: nine loads from the start
-      // of the thread's row, unused - cheaper than a conditional load, whose two definitions cost registers)
-      const int ob = opsF[k + 1];
-      far_load9(row, ob, cb);
-      if (k < nneg) far_add9_any<true>(ca, oa, far);
-      else far_add9_any<false>(ca, oa, far);
-      if (++k >= n) break;
-      oa = opsF[k + 1];
-      far_load9(row, oa, ca);
-      if (k < nneg) far_add9_any<true>(cb, ob, far);
-      else far_add9_any<false>(cb, ob, far);
-      if (++k >= n) break;
-    }
-  }
-  const float gF = __int_as_float(dF.w);
-#pragma unroll
-  for (int j = 0; j < RG / 2; ++j) mul2(far[2 * j], far[2 * j + 1], gF, gF);
 }
 
 }  // namespace tm
