@@ -399,7 +399,9 @@ int vnd_ctx_host_alloc(vnd_ctx* ctx, size_t bytes, void** ptr);
 int vnd_host_free(void* ptr);
 
 /* Host-buffer versions of the calls above (all pointers, including taps->words/offsets, are HOST
- * pointers).  Each call uploads, runs and downloads; on return the result is in `y`/`out`.
+ * pointers).  Each call takes the context's lock, runs the argument checks of its _dev twin and then those that read
+ * its host tables (offsets, indices, records), all before any copy, then uploads the inputs, runs the _dev call on
+ * them and downloads; on return the result is in `y`/`out`.
  * vnd_sparse_fir_host overlaps the three for float32 slabs of 8 MB and more: planar (channels, frames) slabs are
  * cut into channel groups, C-order (frames, channels) slabs - the reference's layout - into runs of frames
  * uploaded with the filter's halo (wide ones are transposed to planar on the device around the kernel), and
@@ -407,20 +409,17 @@ int vnd_host_free(void* ptr);
 int vnd_sparse_fir_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal* y, const vnd_tap_program* taps);
 int vnd_vn_decorrelate_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal* out,
                             const vnd_tap_program* taps, const vnd_epilogue* ep);
-/* vnd_vn_decorrelate_batch_dev with host buffers (offsets, program indices and tap program on the host too).  Checks
- * that the offsets start at 0, never decrease and end at rows, and that every program index is in range, before any
- * copy.  Inputs of 8 MB and more flow through the overlapped pipeline in chunks of whole clips (about
- * VND_PIPE_CHUNK_MB each); filters whose halo does not fit the batched kernel run clip by clip through
- * vnd_vn_decorrelate_host. */
+/* vnd_vn_decorrelate_batch_dev with host buffers (offsets, program indices and tap program on the host too).  Inputs
+ * of 8 MB and more flow through the overlapped pipeline in chunks of whole clips (about VND_PIPE_CHUNK_MB each);
+ * filters whose halo does not fit the batched kernel run clip by clip through vnd_vn_decorrelate_host. */
 int vnd_vn_decorrelate_batch_host(vnd_ctx* ctx, const void* x, int32_t x_dtype, int64_t rows, const int64_t* frame_offsets,
                                   int32_t n_clips, const int32_t* program_of_clip, const vnd_tap_program* taps, const vnd_epilogue* ep,
                                   void* out, int32_t out_dtype);
 int vnd_haas_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal* out, int32_t delay,
                   int32_t delayed_channel, int32_t mode_ms, int32_t mono, int32_t use_width, double width);
-/* vnd_haas_batch_dev with host buffers (x, offsets, settings and out on the host).  Checks, before any copy, that the
- * offsets start at 0, never decrease and end at rows, and that every clip's delay is >= 0 and its delayed_channel 0 or 1;
- * derives the out offsets itself (out holds rows + sum of the delays rows).  Inputs of 8 MB and more flow through the
- * overlapped pipeline in chunks of whole clips (about VND_PIPE_CHUNK_MB each). */
+/* vnd_haas_batch_dev with host buffers (x, offsets, settings and out on the host).  Derives the out offsets itself (out
+ * holds rows + sum of the delays rows).  Inputs of 8 MB and more flow through the overlapped pipeline in chunks of whole
+ * clips (about VND_PIPE_CHUNK_MB each). */
 int vnd_haas_batch_host(vnd_ctx* ctx, const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_clips,
                         const vnd_haas_clip* clips, double* out);
 int vnd_stereo_op_host(vnd_ctx* ctx, const vnd_signal* a, const vnd_signal* dry, int32_t op, double width);
@@ -435,22 +434,19 @@ int vnd_vn_objective_batch_host(vnd_ctx* ctx, const float* clips, int64_t frames
 int vnd_haas_objective_batch_host(vnd_ctx* ctx, const void* clips, int32_t clip_dtype, int64_t frames, int32_t n_clips,
                                   int64_t clip_stride, int64_t chan_stride, const int32_t* delays,
                                   int32_t n_cand, double* partials);
-/* vnd_haas_objective_pairs_dev with host buffers.  Checks, before any copy, that the offsets start at 0, never decrease
- * and end at rows, that every pair_clip is in [0, n_clips), that every delay is >= 0, and that no pair puts delay 0 on
- * an empty clip (an empty signal has no objective: optimization.py:41-43).  Then one upload, one launch, one download. */
+/* vnd_haas_objective_pairs_dev with host buffers.  No pair may put delay 0 on an empty clip (an empty signal has no
+ * objective: optimization.py:41-43). */
 int vnd_haas_objective_pairs_host(vnd_ctx* ctx, const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets,
                                   int32_t n_clips, const int32_t* pair_clip, const int32_t* pair_delay, int32_t n_pairs, double* partials);
 
-/* vnd_vn_stereo_objective_dev and vnd_haas_effect_objective_dev with host buffers (x, program, records and partials):
- * the same checks before any copy - for the Haas records also every delay >= 0 and every delayed_channel 0 or 1 -,
- * then one upload, one launch of each kernel, one download. */
+/* vnd_vn_stereo_objective_dev and vnd_haas_effect_objective_dev with host buffers (x, program, records and partials). */
 int vnd_vn_stereo_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps,
                                  const vnd_vn_stereo_cand* cands, int32_t n_cand, double* partials);
 int vnd_haas_effect_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, int64_t chan_stride, const vnd_haas_clip* cands, int32_t n_cand,
                                    double* partials);
 
-/* vnd_vn_objective_runs_dev with host buffers (x, program, tables and partials): the same checks before any copy, then
- * one upload, one launch of each kernel, one download.  Rows no run names come back as zeros. */
+/* vnd_vn_objective_runs_dev with host buffers (x, program, tables and partials).  Rows no run names come back as
+ * zeros. */
 int vnd_vn_objective_runs_host(vnd_ctx* ctx, const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets, int32_t n_clips,
                                const vnd_tap_program* cand, const int32_t* run_clip, const int32_t* run_cand, const int32_t* run_count,
                                const int32_t* run_out, int32_t n_runs, double* partials, int64_t n_partial_rows);

@@ -834,6 +834,32 @@ def test_empty_clip_is_an_error_not_a_crash(api):
     ps = prog.host_struct()
     rc = N.lib().vnd_vn_objective_batch_host(R.HostContext.get().handle, dummy.ctypes.data, 0, 1, 0, 0, C_.byref(ps), out.ctypes.data)
     assert rc == N.VND_EINVAL and b"empty" in N.lib().vnd_last_error()
+    # the objective kernel reads SEGMENTED headers: the host call rejects any other order before a copy, as the _dev call does
+    clip = np.zeros((1, 2, 64), dtype=np.float32)
+    ps.order = N.ORDER_ASCENDING
+    rc = N.lib().vnd_vn_objective_batch_host(R.HostContext.get().handle, clip.ctypes.data, 64, 1, 128, 64, C_.byref(ps), out.ctypes.data)
+    assert rc == N.VND_EINVAL and b"SEGMENTED" in N.lib().vnd_last_error()
+
+
+def test_host_calls_reject_what_their_dev_calls_reject(api):
+    """A _host call runs the checks of its _dev twin before any copy, also where its own path would not reach them."""
+    import ctypes as C_
+
+    from vndecorrelate_b200 import _native as N
+    from vndecorrelate_b200 import runtime as R
+
+    lib, ctx = N.lib(), R.HostContext.get().handle
+    # a float64 y of a wide frame-interleaved slab: the host path runs the kernel on float32 planar copies
+    vn = api.VelvetNoise(sample_rate_hz=48000, num_outs=4, filtered_channels=(0, 1, 2, 3), mode="LR", normalizer=None, seed=1)
+    prog = vn.tap_program(256)
+    ps = prog.host_struct()
+    x, y = np.zeros((256, 4), np.float32), np.zeros((256, 4), np.float64)
+    xs, ys = N.SignalStruct(x.ctypes.data, 256, 4, N.VND_F32, 4, 1), N.SignalStruct(y.ctypes.data, 256, 4, N.VND_F64, 4, 1)
+    assert lib.vnd_sparse_fir_host(ctx, C_.byref(xs), C_.byref(ys), C_.byref(ps)) == N.VND_EINVAL
+    assert b"y must be float32" in lib.vnd_last_error()
+    # an unknown clip dtype, also with nothing to score
+    assert lib.vnd_haas_objective_batch_host(ctx, None, 7, 0, 0, 0, 0, None, 0, None) == N.VND_EINVAL
+    assert b"unknown clip dtype" in lib.vnd_last_error()
 
 
 def test_batch_optimiser_equals_clip_by_clip(api):

@@ -137,7 +137,7 @@ extern "C" int vnd_device_count(int* count) {
 // ================================================================================================
 // device entry points
 // ================================================================================================
-extern "C" int vnd_sparse_fir_dev(const vnd_signal* x, const vnd_signal* y, const vnd_tap_program* taps, void* stream) {
+static int check_sparse_fir(const vnd_signal* x, const vnd_signal* y, const vnd_tap_program* taps) {
   int rc;
   if ((rc = check_signal(x, "x")) || (rc = check_signal(y, "y")) || (rc = check_taps(taps))) return rc;
   VND_REQUIRE(y->dtype == VND_F32, VND_EINVAL, "y must be float32 (the reference's output buffers are float32)");
@@ -145,6 +145,12 @@ extern "C" int vnd_sparse_fir_dev(const vnd_signal* x, const vnd_signal* y, cons
   VND_REQUIRE(y->channels == taps->channels, VND_EINVAL, "y has %d channels but the tap program has %d", y->channels, taps->channels);
   VND_REQUIRE(x->channels >= taps->channels || x->stride_c == 0, VND_EINVAL, "x has %d channels, fewer than the %d outputs",
               x->channels, taps->channels);
+  return VND_OK;
+}
+
+extern "C" int vnd_sparse_fir_dev(const vnd_signal* x, const vnd_signal* y, const vnd_tap_program* taps, void* stream) {
+  int rc;
+  if ((rc = check_sparse_fir(x, y, taps))) return rc;
   return sparse_fir_launch(x, y, taps, taps->max_channel_words, (cudaStream_t)stream);
 }
 
@@ -157,23 +163,30 @@ extern "C" int vnd_vn_decorrelate_workspace(int64_t frames, int32_t channels, co
   return VND_OK;
 }
 
-extern "C" int vnd_vn_decorrelate_dev(const vnd_signal* x, const vnd_signal* out, const vnd_tap_program* taps,
-                                      const vnd_epilogue* ep, void* workspace, size_t workspace_bytes, void* stream) {
+static int check_vn_decorrelate(const vnd_signal* x, const vnd_signal* out, const vnd_tap_program* taps, const vnd_epilogue* ep) {
   int rc;
   if ((rc = check_signal(x, "x")) || (rc = check_signal(out, "out")) || (rc = check_taps(taps))) return rc;
   VND_REQUIRE(ep != nullptr, VND_EINVAL, "epilogue is null");
   VND_REQUIRE(x->dtype == VND_F32, VND_EINVAL, "x must be float32 (decorrelate casts first, decorrelation.py:426)");
   VND_REQUIRE(taps->order == VND_ORDER_SEGMENTED, VND_EINVAL, "decorrelate needs a SEGMENTED tap program");
   const int C = taps->channels;
-  const long long L = x->frames;
   VND_REQUIRE(ep->haas_delay >= 0, VND_EINVAL, "negative Haas delay");
   VND_REQUIRE(out->channels == C, VND_EINVAL, "out has %d channels but the tap program has %d", out->channels, C);
-  VND_REQUIRE(out->frames == L + ep->haas_delay, VND_EINVAL, "out must have frames + haas_delay = %lld frames, has %lld",
-              L + ep->haas_delay, (long long)out->frames);
+  VND_REQUIRE(out->frames == x->frames + ep->haas_delay, VND_EINVAL, "out must have frames + haas_delay = %lld frames, has %lld",
+              (long long)x->frames + ep->haas_delay, (long long)out->frames);
   VND_REQUIRE(x->channels >= C || x->stride_c == 0, VND_EINVAL, "x has fewer channels than the program");
   if (ep->ms_encode || ep->use_width || ep->haas_delay > 0)
     VND_REQUIRE(C == 2, VND_EINVAL, "M/S encode, width and the Haas delay need exactly 2 channels (utils/dsp.py:297-302)");
   if (ep->haas_delay > 0) VND_REQUIRE(ep->haas_channel == 0 || ep->haas_channel == 1, VND_EINVAL, "haas_channel must be 0 or 1");
+  return VND_OK;
+}
+
+extern "C" int vnd_vn_decorrelate_dev(const vnd_signal* x, const vnd_signal* out, const vnd_tap_program* taps,
+                                      const vnd_epilogue* ep, void* workspace, size_t workspace_bytes, void* stream) {
+  int rc;
+  if ((rc = check_vn_decorrelate(x, out, taps, ep))) return rc;
+  const int C = taps->channels;
+  const long long L = x->frames;
   cudaStream_t st = (cudaStream_t)stream;
   const int delay = ep->haas_delay, dch = ep->haas_channel;
 
@@ -278,14 +291,20 @@ extern "C" int vnd_colsumsq_seq_f32_dev(const vnd_signal* a, float* sums, void* 
   return seq_sumsq_launch(a, nullptr, sums, (cudaStream_t)stream);
 }
 
-extern "C" int vnd_haas_dev(const vnd_signal* x, const vnd_signal* out, int32_t delay, int32_t delayed_channel, int32_t mode_ms,
-                            int32_t mono, int32_t use_width, double width, void* stream) {
+static int check_haas(const vnd_signal* x, const vnd_signal* out, int32_t delay, int32_t delayed_channel) {
   int rc;
   if ((rc = check_signal(x, "x")) || (rc = check_signal(out, "out"))) return rc;
   VND_REQUIRE(x->dtype == VND_F32 && out->dtype == VND_F64, VND_EINVAL, "Haas takes float32 in and float64 out (decorrelation.py:194,206)");
   VND_REQUIRE(delay >= 0, VND_EINVAL, "negative delay");
   VND_REQUIRE(delayed_channel == 0 || delayed_channel == 1, VND_EINVAL, "delayed_channel must be 0 or 1");
   VND_REQUIRE(out->channels == 2 && out->frames == x->frames + delay, VND_EINVAL, "out must be (frames + delay, 2)");
+  return VND_OK;
+}
+
+extern "C" int vnd_haas_dev(const vnd_signal* x, const vnd_signal* out, int32_t delay, int32_t delayed_channel, int32_t mode_ms,
+                            int32_t mono, int32_t use_width, double width, void* stream) {
+  int rc;
+  if ((rc = check_haas(x, out, delay, delayed_channel))) return rc;
   return haas_launch(x, out, delay, delayed_channel, mode_ms, mono, use_width, width, (cudaStream_t)stream);
 }
 
@@ -415,18 +434,24 @@ extern "C" int vnd_fir_block_step_dev(const void* x, int32_t dtype, int64_t rows
   return fir_block_step_launch(b, out_rows, dtype, program_of_signal, taps, out, (cudaStream_t)stream);
 }
 
-extern "C" int vnd_stereo_op_dev(const vnd_signal* a, const vnd_signal* dry, int32_t op, double width, void* workspace,
-                                 size_t workspace_bytes, void* stream) {
+static int check_stereo_op(const vnd_signal* a, const vnd_signal* dry, int32_t op) {
   int rc;
   if ((rc = check_signal(a, "a"))) return rc;
   VND_REQUIRE(op >= 0 && op <= 4, VND_EINVAL, "unknown stereo op %d", op);
   VND_REQUIRE(a->channels == 2, VND_EINVAL, "stereo helpers need a (frames, 2) signal (utils/dsp.py:297-302)");
-  cudaStream_t st = (cudaStream_t)stream;
   if (op == 3 || op == 4) {
     if ((rc = check_signal(dry, "dry"))) return rc;
     VND_REQUIRE(dry->channels == 2 && dry->frames == a->frames && dry->dtype == a->dtype, VND_EINVAL,
                 "dry must match a in shape and dtype");
   }
+  return VND_OK;
+}
+
+extern "C" int vnd_stereo_op_dev(const vnd_signal* a, const vnd_signal* dry, int32_t op, double width, void* workspace,
+                                 size_t workspace_bytes, void* stream) {
+  int rc;
+  if ((rc = check_stereo_op(a, dry, op))) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
   if (op == 4) {
     const size_t esz = a->dtype == VND_F64 ? 8 : 4;
     VND_REQUIRE(workspace != nullptr && workspace_bytes >= 64, VND_ENOMEM, "rms workspace needs at least 64 bytes");
@@ -446,16 +471,33 @@ extern "C" int vnd_objective_workspace(int64_t frames, int32_t n_clips, int32_t 
   return objective_workspace_bytes(frames, n_clips, n_cand, bytes);
 }
 
-extern "C" int vnd_vn_objective_batch_dev(const float* clips, int64_t frames, int32_t n_clips, int64_t clip_stride, int64_t chan_stride,
-                                          const vnd_tap_program* cand, double* partials, void* workspace, size_t workspace_bytes,
-                                          void* stream) {
+static int check_vn_objective_batch(const float* clips, int64_t frames, int32_t n_clips, const vnd_tap_program* cand, const double* partials) {
   int rc;
   if ((rc = check_taps(cand))) return rc;
   VND_REQUIRE(cand->order == VND_ORDER_SEGMENTED, VND_EINVAL, "objective candidates need SEGMENTED tap programs");
   VND_REQUIRE(frames >= 0 && n_clips >= 0, VND_EINVAL, "negative extent");
-  VND_REQUIRE((clips != nullptr && partials != nullptr) || n_clips == 0 || cand->channels == 0, VND_EINVAL, "null buffer");
+  if (n_clips == 0 || cand->channels == 0) return VND_OK;
+  VND_REQUIRE(clips != nullptr && partials != nullptr, VND_EINVAL, "null buffer");
+  // the reference takes max(|theta|) of the frames: an empty signal is a ValueError there (optimization.py:41-43)
+  VND_REQUIRE(frames > 0, VND_EINVAL, "objective of an empty signal (zero-size array to reduction operation maximum which has no identity)");
+  return VND_OK;
+}
+
+extern "C" int vnd_vn_objective_batch_dev(const float* clips, int64_t frames, int32_t n_clips, int64_t clip_stride, int64_t chan_stride,
+                                          const vnd_tap_program* cand, double* partials, void* workspace, size_t workspace_bytes,
+                                          void* stream) {
+  int rc;
+  if ((rc = check_vn_objective_batch(clips, frames, n_clips, cand, partials))) return rc;
   return vn_objective_launch(clips, frames, n_clips, clip_stride, chan_stride, cand, partials, workspace, workspace_bytes,
                              (cudaStream_t)stream);
+}
+
+static int check_haas_objective_batch(const void* clips, int32_t clip_dtype, int64_t frames, int32_t n_clips, const int32_t* delays,
+                                      int32_t n_cand, const double* partials) {
+  VND_REQUIRE(frames >= 0 && n_clips >= 0 && n_cand >= 0, VND_EINVAL, "negative extent");
+  VND_REQUIRE((clips != nullptr && partials != nullptr && delays != nullptr) || n_clips == 0 || n_cand == 0, VND_EINVAL, "null buffer");
+  VND_REQUIRE(clip_dtype == VND_F32 || clip_dtype == VND_F64, VND_EINVAL, "unknown clip dtype %d", clip_dtype);
+  return VND_OK;
 }
 
 extern "C" int vnd_haas_objective_batch_dev(const void* clips, int32_t clip_dtype, int64_t frames, int32_t n_clips, int64_t clip_stride,
@@ -463,9 +505,8 @@ extern "C" int vnd_haas_objective_batch_dev(const void* clips, int32_t clip_dtyp
                                             size_t workspace_bytes, void* stream) {
   (void)workspace;
   (void)workspace_bytes;
-  VND_REQUIRE(frames >= 0 && n_clips >= 0 && n_cand >= 0, VND_EINVAL, "negative extent");
-  VND_REQUIRE((clips != nullptr && partials != nullptr && delays != nullptr) || n_clips == 0 || n_cand == 0, VND_EINVAL, "null buffer");
-  VND_REQUIRE(clip_dtype == VND_F32 || clip_dtype == VND_F64, VND_EINVAL, "unknown clip dtype %d", clip_dtype);
+  int rc;
+  if ((rc = check_haas_objective_batch(clips, clip_dtype, frames, n_clips, delays, n_cand, partials))) return rc;
   return haas_objective_launch(clips, clip_dtype, frames, n_clips, clip_stride, chan_stride, delays, n_cand, partials, (cudaStream_t)stream);
 }
 
@@ -492,26 +533,25 @@ extern "C" int vnd_haas_objective_pairs_dev(const float* x, int64_t rows, int64_
                                      (cudaStream_t)stream);
 }
 
-// The clip of the one-clip family objectives: float32 channel-planar, at least one frame.
-static int check_family_clip(const float* x, int64_t frames, int64_t chan_stride, int32_t n_cand, const double* partials) {
+// The clip and the candidate records of the one-clip family objectives: a float32 channel-planar clip of at least one frame.
+static int check_family_clip(const float* x, int64_t frames, int64_t chan_stride, const void* cands, int32_t n_cand, const double* partials) {
   VND_REQUIRE(n_cand >= 0, VND_EINVAL, "negative n_cand %d", n_cand);
   // the reference takes max(|theta|) of the frames: an empty signal is a ValueError there (optimization.py:41-43)
   VND_REQUIRE(frames > 0, VND_EINVAL, "objective of an empty signal (zero-size array to reduction operation maximum which has no identity)");
   VND_REQUIRE(chan_stride >= frames, VND_EINVAL, "chan_stride %lld is shorter than frames = %lld: the two channels overlap", (long long)chan_stride,
               (long long)frames);
   VND_REQUIRE((x != nullptr && partials != nullptr) || n_cand == 0, VND_EINVAL, "x or partials is null");
+  VND_REQUIRE(cands != nullptr || n_cand == 0, VND_EINVAL, "cands is null");
   return VND_OK;
 }
 
 static int check_vn_stereo(const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,
                            int32_t n_cand, const double* partials) {
   int rc;
-  if ((rc = check_family_clip(x, frames, chan_stride, n_cand, partials))) return rc;
-  if ((rc = check_taps(taps))) return rc;
+  if ((rc = check_family_clip(x, frames, chan_stride, cands, n_cand, partials)) || (rc = check_taps(taps))) return rc;
   VND_REQUIRE(taps->order == VND_ORDER_SEGMENTED, VND_EINVAL, "objective candidates need SEGMENTED tap programs");
   VND_REQUIRE((long long)taps->channels == 2LL * n_cand, VND_EINVAL, "the tap program has %d channels, %d candidates need %lld", taps->channels,
               n_cand, 2LL * n_cand);
-  VND_REQUIRE(cands != nullptr || n_cand == 0, VND_EINVAL, "cands is null");
   return VND_OK;
 }
 
@@ -532,23 +572,29 @@ extern "C" int vnd_vn_stereo_objective_dev(const float* x, int64_t frames, int64
 extern "C" int vnd_haas_effect_objective_dev(const float* x, int64_t frames, int64_t chan_stride, const vnd_haas_clip* cands, int32_t n_cand,
                                              double* partials, void* stream) {
   int rc;
-  if ((rc = check_family_clip(x, frames, chan_stride, n_cand, partials))) return rc;
-  VND_REQUIRE(cands != nullptr || n_cand == 0, VND_EINVAL, "cands is null");
+  if ((rc = check_family_clip(x, frames, chan_stride, cands, n_cand, partials))) return rc;
   VND_REQUIRE(reinterpret_cast<uintptr_t>(cands) % 16 == 0, VND_EINVAL, "cands must be 16-byte aligned");
   return haas_effect_objective_launch(x, frames, chan_stride, cands, n_cand, partials, (cudaStream_t)stream);
 }
 
-// Host tables of the run-list objective: offsets (n_clips + 1, from 0, non-decreasing, ending at rows) and every run's
-// clip.  Runs of at least one candidate need a clip with frames.
+// Host frame offsets of n clips (n + 1 values): from 0, never decreasing, ending at rows.
+static int check_offsets(const int64_t* offs, int32_t n, int64_t rows) {
+  VND_REQUIRE(offs[0] == 0, VND_EINVAL, "frame_offsets[0] is %lld, not 0", (long long)offs[0]);
+  for (int i = 0; i < n; ++i)
+    VND_REQUIRE(offs[i + 1] >= offs[i], VND_EINVAL, "frame_offsets decrease at clip %d (%lld -> %lld)", i, (long long)offs[i],
+                (long long)offs[i + 1]);
+  VND_REQUIRE(offs[n] == rows, VND_EINVAL, "frame_offsets end at %lld, not at rows = %lld", (long long)offs[n], (long long)rows);
+  return VND_OK;
+}
+
+// Host tables of the run-list objective: offsets (check_offsets) and every run's clip.  Runs of at least one candidate
+// need a clip with frames.
 static int check_run_clips(int64_t rows, const int64_t* offs, int32_t n_clips, const int32_t* run_clip, const int32_t* run_count, int32_t n_runs) {
   VND_REQUIRE(rows >= 0 && n_clips >= 0 && n_runs >= 0, VND_EINVAL, "negative extent (rows %lld, n_clips %d, n_runs %d)", (long long)rows,
               n_clips, n_runs);
   VND_REQUIRE(offs != nullptr, VND_EINVAL, "frame_offsets is null");
-  VND_REQUIRE(offs[0] == 0, VND_EINVAL, "frame_offsets[0] is %lld, not 0", (long long)offs[0]);
-  for (int i = 0; i < n_clips; ++i)
-    VND_REQUIRE(offs[i + 1] >= offs[i], VND_EINVAL, "frame_offsets decrease at clip %d (%lld -> %lld)", i, (long long)offs[i],
-                (long long)offs[i + 1]);
-  VND_REQUIRE(offs[n_clips] == rows, VND_EINVAL, "frame_offsets end at %lld, not at rows = %lld", (long long)offs[n_clips], (long long)rows);
+  int rc;
+  if ((rc = check_offsets(offs, n_clips, rows))) return rc;
   if (n_runs == 0) return VND_OK;
   VND_REQUIRE(run_clip != nullptr && run_count != nullptr, VND_EINVAL, "run_clip or run_count is null");
   for (int r = 0; r < n_runs; ++r) {
@@ -630,11 +676,17 @@ extern "C" int vnd_dsp_workspace(int64_t elems, size_t* bytes) {
   return VND_OK;
 }
 
-extern "C" int vnd_rms_normalize_dev(const vnd_signal* x, int32_t x_ndim, const vnd_signal* y, int32_t y_ndim, int32_t stereo_mode, double epsilon,
-                                     void* workspace, size_t workspace_bytes, void* stream) {
+static int check_rms_normalize(const vnd_signal* x, int32_t x_ndim, const vnd_signal* y, int32_t y_ndim) {
   int rc;
   if ((rc = check_flat(x, x_ndim, "input_signal")) || (rc = check_flat(y, y_ndim, "output_signal"))) return rc;
   VND_REQUIRE(x->dtype == y->dtype, VND_EINVAL, "input and output must have the same dtype");
+  return VND_OK;
+}
+
+extern "C" int vnd_rms_normalize_dev(const vnd_signal* x, int32_t x_ndim, const vnd_signal* y, int32_t y_ndim, int32_t stereo_mode, double epsilon,
+                                     void* workspace, size_t workspace_bytes, void* stream) {
+  int rc;
+  if ((rc = check_rms_normalize(x, x_ndim, y, y_ndim))) return rc;
   const long long nx = x->frames * (long long)(x_ndim == 1 ? 1 : x->channels), ny = y->frames * (long long)(y_ndim == 1 ? 1 : y->channels);
   VND_REQUIRE(workspace != nullptr && workspace_bytes >= dsp_workspace_bytes(nx > ny ? nx : ny), VND_ENOMEM, "dsp workspace too small");
   return rms_normalize_launch(x, y, x_ndim, y_ndim, stereo_mode, epsilon, workspace, (cudaStream_t)stream);
@@ -648,11 +700,17 @@ extern "C" int vnd_peak_normalize_dev(const vnd_signal* y, int32_t ndim, int32_t
   return peak_normalize_launch(y, ndim, stereo_mode, epsilon, workspace, (cudaStream_t)stream);
 }
 
-extern "C" int vnd_polar_dev(const void* left, const void* right, int64_t n, int32_t dtype, int32_t mode_ms, int32_t semicircular, int32_t normalize,
-                             void* radii, void* thetas, void* weights, void* workspace, size_t workspace_bytes, void* stream) {
+static int check_polar(const void* left, const void* right, int64_t n, int32_t dtype, const void* radii, const void* thetas) {
   VND_REQUIRE(n >= 0, VND_EINVAL, "negative length");
   VND_REQUIRE(dtype == VND_F32 || dtype == VND_F64, VND_EINVAL, "unknown dtype %d", dtype);
   VND_REQUIRE(n == 0 || (left && right && radii && thetas), VND_EINVAL, "null buffer");
+  return VND_OK;
+}
+
+extern "C" int vnd_polar_dev(const void* left, const void* right, int64_t n, int32_t dtype, int32_t mode_ms, int32_t semicircular, int32_t normalize,
+                             void* radii, void* thetas, void* weights, void* workspace, size_t workspace_bytes, void* stream) {
+  int rc;
+  if ((rc = check_polar(left, right, n, dtype, radii, thetas))) return rc;
   VND_REQUIRE(workspace != nullptr && workspace_bytes >= dsp_workspace_bytes(n), VND_ENOMEM, "dsp workspace too small");
   return polar_launch(left, right, n, dtype, mode_ms, semicircular, normalize, radii, thetas, weights, workspace, (cudaStream_t)stream);
 }
@@ -714,14 +772,21 @@ Dense dense_extent(const vnd_signal* s) {
 
 size_t esize(int dtype) { return dtype == VND_F64 ? 8 : 4; }
 
+// Arena slot `slot`, holding a copy of `bytes` host bytes from `src` once stream `st` gets there.
+int upload(vnd_ctx* ctx, int slot, const void* src, size_t bytes, cudaStream_t st, void** dev) {
+  int rc;
+  if ((rc = arena(ctx, slot, bytes, dev))) return rc;
+  if (bytes) VND_CUDA_OK(cudaMemcpyAsync(*dev, src, bytes, cudaMemcpyHostToDevice, st));
+  return VND_OK;
+}
+
 int upload_program(vnd_ctx* ctx, const vnd_tap_program* host, vnd_tap_program* dev, cudaStream_t st) {
   *dev = *host;
   void *w = nullptr, *o = nullptr;
   int rc;
-  if ((rc = arena(ctx, S_WORDS, (size_t)host->n_words * 4, &w))) return rc;
-  if ((rc = arena(ctx, S_OFFS, ((size_t)host->channels + 1) * 4, &o))) return rc;
-  if (host->n_words) VND_CUDA_OK(cudaMemcpyAsync(w, host->words, (size_t)host->n_words * 4, cudaMemcpyHostToDevice, st));
-  if (host->channels) VND_CUDA_OK(cudaMemcpyAsync(o, host->offsets, ((size_t)host->channels + 1) * 4, cudaMemcpyHostToDevice, st));
+  if ((rc = upload(ctx, S_WORDS, host->words, (size_t)host->n_words * 4, st, &w)) ||
+      (rc = upload(ctx, S_OFFS, host->offsets, host->channels ? ((size_t)host->channels + 1) * 4 : 0, st, &o)))
+    return rc;
   dev->words = reinterpret_cast<const int32_t*>(w);
   dev->offsets = reinterpret_cast<const int32_t*>(o);
   return VND_OK;
@@ -838,15 +903,15 @@ extern "C" int vnd_rms_normalize_host(vnd_ctx* ctx, const vnd_signal* x, int32_t
                                       double epsilon) {
   VND_ENTER(ctx);
   int rc;
-  if ((rc = check_flat(x, x_ndim, "input_signal")) || (rc = check_flat(y, y_ndim, "output_signal"))) return rc;
+  if ((rc = check_rms_normalize(x, x_ndim, y, y_ndim))) return rc;
   const size_t es = esize(x->dtype);
   const size_t nx = (size_t)x->frames * (x_ndim == 1 ? 1 : x->channels), ny = (size_t)y->frames * (y_ndim == 1 ? 1 : y->channels);
   cudaStream_t st = ctx->streams[0];
   void *dx = nullptr, *dy = nullptr, *work = nullptr;
   const size_t wbytes = dsp_workspace_bytes((long long)(nx > ny ? nx : ny));
-  if ((rc = arena(ctx, S_IN, nx * es, &dx)) || (rc = arena(ctx, S_OUT, ny * es, &dy)) || (rc = arena(ctx, S_WORK, wbytes, &work))) return rc;
-  if (nx) VND_CUDA_OK(cudaMemcpyAsync(dx, x->data, nx * es, cudaMemcpyHostToDevice, st));
-  if (ny) VND_CUDA_OK(cudaMemcpyAsync(dy, y->data, ny * es, cudaMemcpyHostToDevice, st));
+  if ((rc = upload(ctx, S_IN, x->data, nx * es, st, &dx)) || (rc = upload(ctx, S_OUT, y->data, ny * es, st, &dy)) ||
+      (rc = arena(ctx, S_WORK, wbytes, &work)))
+    return rc;
   vnd_signal xd = *x, yd = *y;
   xd.data = dx;
   yd.data = dy;
@@ -864,8 +929,7 @@ extern "C" int vnd_peak_normalize_host(vnd_ctx* ctx, const vnd_signal* y, int32_
   cudaStream_t st = ctx->streams[0];
   void *dy = nullptr, *work = nullptr;
   const size_t wbytes = dsp_workspace_bytes(0);
-  if ((rc = arena(ctx, S_IN, ny * es, &dy)) || (rc = arena(ctx, S_WORK, wbytes, &work))) return rc;
-  if (ny) VND_CUDA_OK(cudaMemcpyAsync(dy, y->data, ny * es, cudaMemcpyHostToDevice, st));
+  if ((rc = upload(ctx, S_IN, y->data, ny * es, st, &dy)) || (rc = arena(ctx, S_WORK, wbytes, &work))) return rc;
   vnd_signal yd = *y;
   yd.data = dy;
   if ((rc = vnd_peak_normalize_dev(&yd, ndim, stereo_mode, epsilon, work, wbytes, st))) return rc;
@@ -878,10 +942,8 @@ extern "C" int vnd_polar_host(vnd_ctx* ctx, const void* left, const void* right,
                               int32_t normalize, void* radii, void* thetas, void* weights) {
   VND_ENTER(ctx);
   int rc;
-  VND_REQUIRE(n >= 0, VND_EINVAL, "negative length");
-  VND_REQUIRE(dtype == VND_F32 || dtype == VND_F64, VND_EINVAL, "unknown dtype %d", dtype);
+  if ((rc = check_polar(left, right, n, dtype, radii, thetas))) return rc;
   if (n == 0) return VND_OK;
-  VND_REQUIRE(left && right && radii && thetas, VND_EINVAL, "null buffer");
   const size_t bytes = (size_t)n * esize(dtype);
   cudaStream_t st = ctx->streams[0];
   void *din = nullptr, *dout = nullptr, *work = nullptr;
@@ -1101,6 +1163,25 @@ size_t pipe_chunk_bytes() {  // bytes uploaded per pipeline stage (VND_PIPE_CHUN
 }
 constexpr size_t kPipeMinBytes = 8u << 20;  // below this one blocking copy each way is as fast
 
+// Does an upload of `in_bytes` go through run_pipeline?  VND_NO_PIPELINE forces the one-shot path, the reference
+// the pipelined one is tested against.
+bool pipelined(size_t in_bytes) { return in_bytes >= kPipeMinBytes && getenv("VND_NO_PIPELINE") == nullptr; }
+
+// Chunks of whole clips of a packed (rows, 2) float32 batch of about pipe_chunk_bytes() each (at least four chunks when
+// there are four clips): first[k] .. first[k + 1] are the clips of chunk k.
+std::vector<int> clip_chunks(const int64_t* offs, int32_t n_clips, int64_t rows) {
+  size_t target = pipe_chunk_bytes();
+  if (target > (size_t)rows * 8 / 4) target = (size_t)rows * 8 / 4;
+  std::vector<int> first{0};
+  while (first.back() < n_clips) {
+    const int a = first.back();
+    int b = a + 1;
+    while (b < n_clips && (size_t)(offs[b + 1] - offs[a]) * 8 <= target) ++b;
+    first.push_back(b);
+  }
+  return first;
+}
+
 // Planar (channels, frames) float32 host slabs: chunks are groups of whole channels.
 int fir_pipeline_planar(vnd_ctx* ctx, const float* x, float* y, long long frames, int channels, const vnd_tap_program* dprog,
                         int channels_per_chunk) {
@@ -1181,15 +1262,14 @@ int fir_pipeline_interleaved(vnd_ctx* ctx, const float* x, int x_channels, float
 extern "C" int vnd_sparse_fir_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal* y, const vnd_tap_program* taps) {
   VND_ENTER(ctx);
   int rc;
-  if ((rc = check_signal(x, "x")) || (rc = check_signal(y, "y")) || (rc = check_taps(taps))) return rc;
+  if ((rc = check_sparse_fir(x, y, taps))) return rc;
   const Dense dx = dense_extent(x), dy = dense_extent(y);
   VND_REQUIRE(dx.ok && dy.ok, VND_EUNSUPPORTED, "host signals must be contiguous C-order (frames, channels) or planar (channels, frames)");
   cudaStream_t st = ctx->streams[0];
   vnd_tap_program dprog;
   if ((rc = upload_program(ctx, taps, &dprog, st))) return rc;
   // Large float32 slabs: upload, kernels and download overlapped chunk by chunk (run_pipeline)
-  if (x->dtype == VND_F32 && y->dtype == VND_F32 && x->frames == y->frames && dx.elems * 4 >= kPipeMinBytes && x->stride_c != 0 &&
-      taps->channels == y->channels && x->channels >= y->channels && getenv("VND_NO_PIPELINE") == nullptr) {
+  if (x->dtype == VND_F32 && x->stride_c != 0 && pipelined(dx.elems * 4)) {
     const long long L = x->frames;
     const int C = y->channels;
     const bool x_planar = x->stride_t == 1 && (x->stride_c == L || x->channels == 1), y_planar = y->stride_t == 1 && (y->stride_c == L || C == 1);
@@ -1201,9 +1281,7 @@ extern "C" int vnd_sparse_fir_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_
       return fir_pipeline_interleaved(ctx, (const float*)x->data, x->channels, (float*)y->data, L, C, &dprog);
   }
   void *din = nullptr, *dout = nullptr;
-  if ((rc = arena(ctx, S_IN, dx.elems * esize(x->dtype), &din))) return rc;
-  if ((rc = arena(ctx, S_OUT, dy.elems * 4, &dout))) return rc;
-  if (dx.elems) VND_CUDA_OK(cudaMemcpyAsync(din, x->data, dx.elems * esize(x->dtype), cudaMemcpyHostToDevice, st));
+  if ((rc = upload(ctx, S_IN, x->data, dx.elems * esize(x->dtype), st, &din)) || (rc = arena(ctx, S_OUT, dy.elems * 4, &dout))) return rc;
   vnd_signal xd = *x, yd = *y;
   xd.data = din;
   yd.data = dout;
@@ -1228,12 +1306,12 @@ extern "C" int vnd_sparse_fir_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_
   return VND_OK;
 }
 
-extern "C" int vnd_vn_decorrelate_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal* out, const vnd_tap_program* taps,
-                                       const vnd_epilogue* ep) {
-  VND_ENTER(ctx);
+namespace {
+
+// vnd_vn_decorrelate_host once the context is entered (its lock held, its device current).
+int vn_decorrelate_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal* out, const vnd_tap_program* taps, const vnd_epilogue* ep) {
   int rc;
-  if ((rc = check_signal(x, "x")) || (rc = check_signal(out, "out")) || (rc = check_taps(taps))) return rc;
-  VND_REQUIRE(ep != nullptr, VND_EINVAL, "epilogue is null");
+  if ((rc = check_vn_decorrelate(x, out, taps, ep))) return rc;
   const Dense dx = dense_extent(x), dy = dense_extent(out);
   VND_REQUIRE(dx.ok && dy.ok, VND_EUNSUPPORTED, "host signals must be contiguous C-order (frames, channels) or planar (channels, frames)");
   cudaStream_t st = ctx->streams[0];
@@ -1242,10 +1320,9 @@ extern "C" int vnd_vn_decorrelate_host(vnd_ctx* ctx, const vnd_signal* x, const 
   void *din = nullptr, *dout = nullptr, *work = nullptr;
   size_t wbytes = 0;
   if ((rc = vnd_vn_decorrelate_workspace(x->frames, taps->channels, ep, &wbytes))) return rc;
-  if ((rc = arena(ctx, S_IN, dx.elems * esize(x->dtype), &din))) return rc;
-  if ((rc = arena(ctx, S_OUT, dy.elems * esize(out->dtype), &dout))) return rc;
-  if ((rc = arena(ctx, S_WORK, wbytes, &work))) return rc;
-  if (dx.elems) VND_CUDA_OK(cudaMemcpyAsync(din, x->data, dx.elems * esize(x->dtype), cudaMemcpyHostToDevice, st));
+  if ((rc = upload(ctx, S_IN, x->data, dx.elems * esize(x->dtype), st, &din)) ||
+      (rc = arena(ctx, S_OUT, dy.elems * esize(out->dtype), &dout)) || (rc = arena(ctx, S_WORK, wbytes, &work)))
+    return rc;
   vnd_signal xd = *x, od = *out;
   xd.data = din;
   od.data = dout;
@@ -1254,8 +1331,6 @@ extern "C" int vnd_vn_decorrelate_host(vnd_ctx* ctx, const vnd_signal* x, const 
   VND_CUDA_OK(cudaStreamSynchronize(st));
   return VND_OK;
 }
-
-namespace {
 
 // 1 + the largest tap index of channel c of a host SEGMENTED program (0 for an empty block or no taps)
 int channel_halo(const vnd_tap_program* t, int c) {
@@ -1269,7 +1344,7 @@ int channel_halo(const vnd_tap_program* t, int c) {
   return halo;
 }
 
-// Clip by clip through vnd_vn_decorrelate_host: for filters whose halo does not fit the batched kernel.  Correct, but
+// Clip by clip through vn_decorrelate_host: for filters whose halo does not fit the batched kernel.  Correct, but
 // one upload / launch sequence / download per clip.
 int batch_host_per_clip(vnd_ctx* ctx, const float* x, const int64_t* offs, int32_t n, const int32_t* prog_of, const vnd_tap_program* taps,
                         const vnd_epilogue* ep, void* out, int32_t out_dtype) {
@@ -1287,7 +1362,7 @@ int batch_host_per_clip(vnd_ctx* ctx, const float* x, const int64_t* offs, int32
     vnd_signal xs{const_cast<float*>(x) + 2 * offs[i], L, 2, VND_F32, 2, 1};
     vnd_signal os{reinterpret_cast<char*>(out) + (size_t)(offs[i] + (long long)i * ep->haas_delay) * 2 * es, L + ep->haas_delay, 2, out_dtype,
                   2, 1};
-    const int rc = vnd_vn_decorrelate_host(ctx, &xs, &os, &sub, ep);
+    const int rc = vn_decorrelate_host(ctx, &xs, &os, &sub, ep);
     if (rc) return rc;
   }
   return VND_OK;
@@ -1295,19 +1370,21 @@ int batch_host_per_clip(vnd_ctx* ctx, const float* x, const int64_t* offs, int32
 
 }  // namespace
 
+extern "C" int vnd_vn_decorrelate_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal* out, const vnd_tap_program* taps,
+                                       const vnd_epilogue* ep) {
+  VND_ENTER(ctx);
+  return vn_decorrelate_host(ctx, x, out, taps, ep);
+}
+
 extern "C" int vnd_vn_decorrelate_batch_host(vnd_ctx* ctx, const void* x, int32_t x_dtype, int64_t rows, const int64_t* frame_offsets,
                                              int32_t n_clips, const int32_t* program_of_clip, const vnd_tap_program* taps,
                                              const vnd_epilogue* ep, void* out, int32_t out_dtype) {
-  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  VND_ENTER(ctx);
   int rc;
   if ((rc = check_batch(x, x_dtype, rows, frame_offsets, n_clips, program_of_clip, taps, ep, out, out_dtype))) return rc;
   if (n_clips == 0) return VND_OK;
   const int64_t* offs = frame_offsets;
-  VND_REQUIRE(offs[0] == 0, VND_EINVAL, "frame_offsets[0] is %lld, not 0", (long long)offs[0]);
-  for (int i = 0; i < n_clips; ++i)
-    VND_REQUIRE(offs[i + 1] >= offs[i], VND_EINVAL, "frame_offsets decrease at clip %d (%lld -> %lld)", i, (long long)offs[i],
-                (long long)offs[i + 1]);
-  VND_REQUIRE(offs[n_clips] == rows, VND_EINVAL, "frame_offsets end at %lld, not at rows = %lld", (long long)offs[n_clips], (long long)rows);
+  if ((rc = check_offsets(offs, n_clips, rows))) return rc;
   const int n_prog = taps->channels / 2;
   for (int i = 0; i < n_clips; ++i)
     VND_REQUIRE(program_of_clip[i] >= 0 && program_of_clip[i] < n_prog, VND_EINVAL, "program_of_clip[%d] = %d is outside [0, %d)", i,
@@ -1315,76 +1392,56 @@ extern "C" int vnd_vn_decorrelate_batch_host(vnd_ctx* ctx, const void* x, int32_
   const float* xf = reinterpret_cast<const float*>(x);
   if (!batch_fits(taps, rows)) return batch_host_per_clip(ctx, xf, offs, n_clips, program_of_clip, taps, ep, out, out_dtype);
 
-  VND_ENTER(ctx);
   cudaStream_t st = ctx->streams[0];
   vnd_tap_program dprog;
   if ((rc = upload_program(ctx, taps, &dprog, st))) return rc;
   const int delay = ep->haas_delay;
   const size_t es = esize(out_dtype);
-  const size_t in_bytes = (size_t)rows * 8;
-
-  if (in_bytes >= kPipeMinBytes && getenv("VND_NO_PIPELINE") == nullptr) {
-    // chunks of whole clips of about pipe_chunk_bytes() (at least four chunks when there are four clips), each with its
-    // own offsets rebased to its first row: first[k] .. first[k + 1] are the clips of chunk k
-    size_t target = pipe_chunk_bytes();
-    if (target > in_bytes / 4) target = in_bytes / 4;
-    std::vector<int> first{0};
-    while (first.back() < n_clips) {
-      const int a = first.back();
-      int b = a + 1;
-      while (b < n_clips && (size_t)(offs[b + 1] - offs[a]) * 8 <= target) ++b;
-      first.push_back(b);
-    }
-    const int nchunks = (int)first.size() - 1;
-    std::vector<long long> meta;  // rebased offsets of every chunk (n_k + 1 each), then the program indices
-    meta.reserve((size_t)n_clips + nchunks + n_clips / 2 + 1);
-    long long max_rows = 0, max_out_rows = 0;
-    int max_clips = 0;
-    for (int k = 0; k < nchunks; ++k) {
-      const int a = first[k], b = first[k + 1];
-      for (int i = a; i <= b; ++i) meta.push_back(offs[i] - offs[a]);
-      const long long r = offs[b] - offs[a];
-      max_rows = r > max_rows ? r : max_rows;
-      max_out_rows = r + (long long)(b - a) * delay > max_out_rows ? r + (long long)(b - a) * delay : max_out_rows;
-      max_clips = b - a > max_clips ? b - a : max_clips;
-    }
-    const size_t off_bytes = meta.size() * 8;
-    void* dmeta = nullptr;
-    if ((rc = arena(ctx, S_AUX, off_bytes + (size_t)n_clips * 4, &dmeta))) return rc;
-    VND_CUDA_OK(cudaMemcpyAsync(dmeta, meta.data(), off_bytes, cudaMemcpyHostToDevice, st));
-    VND_CUDA_OK(cudaMemcpyAsync((char*)dmeta + off_bytes, program_of_clip, (size_t)n_clips * 4, cudaMemcpyHostToDevice, st));
-    VND_CUDA_OK(cudaStreamSynchronize(st));  // the program and the offsets are on the device before the other streams read them
-    const long long* doffs = reinterpret_cast<const long long*>(dmeta);
-    const int32_t* dprog_of = reinterpret_cast<const int32_t*>((char*)dmeta + off_bytes);
-    auto chunk_of = [&](int k) {
-      const int a = first[k], b = first[k + 1];
-      const long long r = offs[b] - offs[a];
-      return PipeChunk{reinterpret_cast<const char*>(xf + 2 * offs[a]), (size_t)r * 8,
-                       reinterpret_cast<char*>(out) + (size_t)(offs[a] + (long long)a * delay) * 2 * es, (size_t)(r + (long long)(b - a) * delay) * 2 * es};
-    };
-    auto compute = [&](int k, void* din, void* dout, void* sa, void*, cudaStream_t cs) {
-      const int a = first[k], b = first[k + 1];
-      return vn_batch_launch(reinterpret_cast<const float*>(din), offs[b] - offs[a], doffs + a + k, b - a, dprog_of + a, &dprog, ep, dout,
-                             out_dtype, sa, cs);
-    };
-    return run_pipeline(ctx, nchunks, (size_t)max_rows * 8, (size_t)max_out_rows * 2 * es, vn_batch_workspace_bytes(max_rows, max_clips, ep->rms_normalize),
-                        chunk_of, compute);
+  // chunks of whole clips (clip_chunks, or the whole batch as one), each with its own offsets rebased to its first row
+  const bool pipe = pipelined((size_t)rows * 8);
+  const std::vector<int> first = pipe ? clip_chunks(offs, n_clips, rows) : std::vector<int>{0, n_clips};
+  const int nchunks = (int)first.size() - 1;
+  std::vector<long long> meta;  // rebased offsets of every chunk (n_k + 1 each)
+  meta.reserve((size_t)n_clips + nchunks);
+  long long max_rows = 0, max_out_rows = 0;
+  int max_clips = 0;
+  for (int k = 0; k < nchunks; ++k) {
+    const int a = first[k], b = first[k + 1];
+    for (int i = a; i <= b; ++i) meta.push_back(offs[i] - offs[a]);
+    const long long r = offs[b] - offs[a];
+    max_rows = r > max_rows ? r : max_rows;
+    max_out_rows = r + (long long)(b - a) * delay > max_out_rows ? r + (long long)(b - a) * delay : max_out_rows;
+    max_clips = b - a > max_clips ? b - a : max_clips;
   }
-
-  const size_t out_bytes = (size_t)(rows + (long long)n_clips * delay) * 2 * es;
-  const size_t wbytes = vn_batch_workspace_bytes(rows, n_clips, ep->rms_normalize);
-  const size_t off_bytes = ((size_t)n_clips + 1) * 8;
-  void *din = nullptr, *dout = nullptr, *work = nullptr, *dmeta = nullptr;
-  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) || (rc = arena(ctx, S_WORK, wbytes, &work)) ||
-      (rc = arena(ctx, S_AUX, off_bytes + (size_t)n_clips * 4, &dmeta)))
-    return rc;
-  if (in_bytes) VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
-  VND_CUDA_OK(cudaMemcpyAsync(dmeta, offs, off_bytes, cudaMemcpyHostToDevice, st));
+  const size_t off_bytes = meta.size() * 8;
+  void* dmeta = nullptr;
+  if ((rc = arena(ctx, S_AUX, off_bytes + (size_t)n_clips * 4, &dmeta))) return rc;
+  VND_CUDA_OK(cudaMemcpyAsync(dmeta, meta.data(), off_bytes, cudaMemcpyHostToDevice, st));
   VND_CUDA_OK(cudaMemcpyAsync((char*)dmeta + off_bytes, program_of_clip, (size_t)n_clips * 4, cudaMemcpyHostToDevice, st));
-  if ((rc = vnd_vn_decorrelate_batch_dev(din, VND_F32, rows, reinterpret_cast<const int64_t*>(dmeta), n_clips,
-                                         reinterpret_cast<const int32_t*>((char*)dmeta + off_bytes), &dprog, ep, dout, out_dtype, work, wbytes, st)))
+  const int64_t* doffs = reinterpret_cast<const int64_t*>(dmeta);
+  const int32_t* dprog_of = reinterpret_cast<const int32_t*>((char*)dmeta + off_bytes);
+  const size_t wbytes = vn_batch_workspace_bytes(max_rows, max_clips, ep->rms_normalize);
+  auto chunk_of = [&](int k) {
+    const int a = first[k], b = first[k + 1];
+    const long long r = offs[b] - offs[a];
+    return PipeChunk{reinterpret_cast<const char*>(xf + 2 * offs[a]), (size_t)r * 8,
+                     reinterpret_cast<char*>(out) + (size_t)(offs[a] + (long long)a * delay) * 2 * es, (size_t)(r + (long long)(b - a) * delay) * 2 * es};
+  };
+  auto compute = [&](int k, void* din, void* dout, void* work, void*, cudaStream_t cs) {
+    const int a = first[k], b = first[k + 1];
+    return vnd_vn_decorrelate_batch_dev(din, VND_F32, offs[b] - offs[a], doffs + a + k, b - a, dprog_of + a, &dprog, ep, dout, out_dtype, work,
+                                        wbytes, cs);
+  };
+  if (pipe) {
+    VND_CUDA_OK(cudaStreamSynchronize(st));  // the program and the offsets are on the device before the other streams read them
+    return run_pipeline(ctx, nchunks, (size_t)max_rows * 8, (size_t)max_out_rows * 2 * es, wbytes, chunk_of, compute);
+  }
+  const PipeChunk c = chunk_of(0);
+  void *din = nullptr, *dout = nullptr, *work = nullptr;
+  if ((rc = upload(ctx, S_IN, c.src, c.src_bytes, st, &din)) || (rc = arena(ctx, S_OUT, c.dst_bytes, &dout)) ||
+      (rc = arena(ctx, S_WORK, wbytes, &work)) || (rc = compute(0, din, dout, work, nullptr, st)))
     return rc;
-  if (out_bytes) VND_CUDA_OK(cudaMemcpyAsync(out, dout, out_bytes, cudaMemcpyDeviceToHost, st));
+  if (c.dst_bytes) VND_CUDA_OK(cudaMemcpyAsync(c.dst, dout, c.dst_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
   return VND_OK;
 }
@@ -1393,14 +1450,13 @@ extern "C" int vnd_haas_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal
                              int32_t mode_ms, int32_t mono, int32_t use_width, double width) {
   VND_ENTER(ctx);
   int rc;
-  if ((rc = check_signal(x, "x")) || (rc = check_signal(out, "out"))) return rc;
+  if ((rc = check_haas(x, out, delay, delayed_channel))) return rc;
   const Dense dx = dense_extent(x), dy = dense_extent(out);
   VND_REQUIRE(dx.ok && dy.ok, VND_EUNSUPPORTED, "host signals must be contiguous");
   cudaStream_t st = ctx->streams[0];
   void *din = nullptr, *dout = nullptr;
-  if ((rc = arena(ctx, S_IN, dx.elems * esize(x->dtype), &din))) return rc;
-  if ((rc = arena(ctx, S_OUT, dy.elems * esize(out->dtype), &dout))) return rc;
-  if (dx.elems) VND_CUDA_OK(cudaMemcpyAsync(din, x->data, dx.elems * esize(x->dtype), cudaMemcpyHostToDevice, st));
+  if ((rc = upload(ctx, S_IN, x->data, dx.elems * esize(x->dtype), st, &din)) || (rc = arena(ctx, S_OUT, dy.elems * esize(out->dtype), &dout)))
+    return rc;
   vnd_signal xd = *x, od = *out;
   xd.data = din;
   od.data = dout;
@@ -1412,95 +1468,66 @@ extern "C" int vnd_haas_host(vnd_ctx* ctx, const vnd_signal* x, const vnd_signal
 
 extern "C" int vnd_haas_batch_host(vnd_ctx* ctx, const float* x, int64_t rows, const int64_t* frame_offsets, int32_t n_clips,
                                    const vnd_haas_clip* clips, double* out) {
-  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  VND_ENTER(ctx);
   int rc;
   if ((rc = check_haas_batch(x, rows, frame_offsets, n_clips, clips))) return rc;
   if (n_clips == 0) return VND_OK;
   const int64_t* offs = frame_offsets;
-  VND_REQUIRE(offs[0] == 0, VND_EINVAL, "frame_offsets[0] is %lld, not 0", (long long)offs[0]);
-  for (int i = 0; i < n_clips; ++i)
-    VND_REQUIRE(offs[i + 1] >= offs[i], VND_EINVAL, "frame_offsets decrease at clip %d (%lld -> %lld)", i, (long long)offs[i],
-                (long long)offs[i + 1]);
-  VND_REQUIRE(offs[n_clips] == rows, VND_EINVAL, "frame_offsets end at %lld, not at rows = %lld", (long long)offs[n_clips], (long long)rows);
+  if ((rc = check_offsets(offs, n_clips, rows))) return rc;
   // out offsets of every clip and one more (the total)
-  std::vector<long long> oo((size_t)n_clips + 1);
-  long long shift = 0;
+  std::vector<long long> oo((size_t)n_clips + 1, 0);
   for (int i = 0; i < n_clips; ++i) {
     VND_REQUIRE(clips[i].delay >= 0, VND_EINVAL, "clip %d has a negative delay (%d)", i, clips[i].delay);
     VND_REQUIRE(clips[i].delayed_channel == 0 || clips[i].delayed_channel == 1, VND_EINVAL, "clip %d: delayed_channel must be 0 or 1, is %d", i,
                 clips[i].delayed_channel);
-    oo[i] = offs[i] + shift;
-    shift += clips[i].delay;
+    oo[i + 1] = oo[i] + (offs[i + 1] - offs[i]) + clips[i].delay;
   }
-  oo[n_clips] = rows + shift;
-  const long long out_rows = oo[n_clips];
-  VND_REQUIRE(out != nullptr || out_rows == 0, VND_EINVAL, "out is null");
+  VND_REQUIRE(out != nullptr || oo[n_clips] == 0, VND_EINVAL, "out is null");
 
-  VND_ENTER(ctx);
   cudaStream_t st = ctx->streams[0];
-  const size_t in_bytes = (size_t)rows * 8, clip_bytes = (size_t)n_clips * sizeof(vnd_haas_clip);
-
-  if (in_bytes >= kPipeMinBytes && getenv("VND_NO_PIPELINE") == nullptr) {
-    // chunks of whole clips of about pipe_chunk_bytes() (at least four chunks when there are four clips), each with its
-    // own offsets rebased to its first row: first[k] .. first[k + 1] are the clips of chunk k, meta[at[k]..] their frame
-    // offsets (n_k + 1) and then their out offsets (n_k)
-    size_t target = pipe_chunk_bytes();
-    if (target > in_bytes / 4) target = in_bytes / 4;
-    std::vector<int> first{0};
-    while (first.back() < n_clips) {
-      const int a = first.back();
-      int b = a + 1;
-      while (b < n_clips && (size_t)(offs[b + 1] - offs[a]) * 8 <= target) ++b;
-      first.push_back(b);
-    }
-    const int nchunks = (int)first.size() - 1;
-    std::vector<long long> meta;
-    std::vector<size_t> at;
-    meta.reserve(2 * (size_t)n_clips + nchunks);
-    long long max_rows = 0, max_out_rows = 0;
-    for (int k = 0; k < nchunks; ++k) {
-      const int a = first[k], b = first[k + 1];
-      at.push_back(meta.size());
-      for (int i = a; i <= b; ++i) meta.push_back(offs[i] - offs[a]);
-      for (int i = a; i < b; ++i) meta.push_back(oo[i] - oo[a]);
-      max_rows = offs[b] - offs[a] > max_rows ? offs[b] - offs[a] : max_rows;
-      max_out_rows = oo[b] - oo[a] > max_out_rows ? oo[b] - oo[a] : max_out_rows;
-    }
-    void* dmeta = nullptr;
-    if ((rc = arena(ctx, S_AUX, clip_bytes + meta.size() * 8, &dmeta))) return rc;
-    VND_CUDA_OK(cudaMemcpyAsync(dmeta, clips, clip_bytes, cudaMemcpyHostToDevice, st));
-    VND_CUDA_OK(cudaMemcpyAsync((char*)dmeta + clip_bytes, meta.data(), meta.size() * 8, cudaMemcpyHostToDevice, st));
+  const size_t clip_bytes = (size_t)n_clips * sizeof(vnd_haas_clip);
+  // chunks of whole clips (clip_chunks, or the whole batch as one), each with its own offsets rebased to its first row:
+  // chunk k's frame offsets (n_k + 1) and then its out offsets (n_k) start at meta[2 first[k] + k]
+  const bool pipe = pipelined((size_t)rows * 8);
+  const std::vector<int> first = pipe ? clip_chunks(offs, n_clips, rows) : std::vector<int>{0, n_clips};
+  const int nchunks = (int)first.size() - 1;
+  std::vector<long long> meta;
+  meta.reserve(2 * (size_t)n_clips + nchunks);
+  long long max_rows = 0, max_out_rows = 0;
+  for (int k = 0; k < nchunks; ++k) {
+    const int a = first[k], b = first[k + 1];
+    for (int i = a; i <= b; ++i) meta.push_back(offs[i] - offs[a]);
+    for (int i = a; i < b; ++i) meta.push_back(oo[i] - oo[a]);
+    max_rows = offs[b] - offs[a] > max_rows ? offs[b] - offs[a] : max_rows;
+    max_out_rows = oo[b] - oo[a] > max_out_rows ? oo[b] - oo[a] : max_out_rows;
+  }
+  void* dmeta = nullptr;
+  if ((rc = arena(ctx, S_AUX, clip_bytes + meta.size() * 8, &dmeta))) return rc;
+  VND_CUDA_OK(cudaMemcpyAsync(dmeta, clips, clip_bytes, cudaMemcpyHostToDevice, st));
+  VND_CUDA_OK(cudaMemcpyAsync((char*)dmeta + clip_bytes, meta.data(), meta.size() * 8, cudaMemcpyHostToDevice, st));
+  const vnd_haas_clip* dclips = reinterpret_cast<const vnd_haas_clip*>(dmeta);
+  const int64_t* dtab = reinterpret_cast<const int64_t*>((char*)dmeta + clip_bytes);
+  auto chunk_of = [&](int k) {
+    const int a = first[k], b = first[k + 1];
+    return PipeChunk{reinterpret_cast<const char*>(x + 2 * offs[a]), (size_t)(offs[b] - offs[a]) * 8, reinterpret_cast<char*>(out + 2 * oo[a]),
+                     (size_t)(oo[b] - oo[a]) * 16};
+  };
+  auto compute = [&](int k, void* din, void* dout, void*, void*, cudaStream_t cs) {
+    const int a = first[k], b = first[k + 1];
+    const int64_t* tab = dtab + 2 * a + k;
+    return vnd_haas_batch_dev(reinterpret_cast<const float*>(din), offs[b] - offs[a], tab, b - a, dclips + a, tab + (b - a + 1), oo[b] - oo[a],
+                              reinterpret_cast<double*>(dout), cs);
+  };
+  if (pipe) {
     VND_CUDA_OK(cudaStreamSynchronize(st));  // the tables are on the device before the other streams read them
-    const vnd_haas_clip* dclips = reinterpret_cast<const vnd_haas_clip*>(dmeta);
-    const long long* dtab = reinterpret_cast<const long long*>((char*)dmeta + clip_bytes);
-    auto chunk_of = [&](int k) {
-      const int a = first[k], b = first[k + 1];
-      return PipeChunk{reinterpret_cast<const char*>(x + 2 * offs[a]), (size_t)(offs[b] - offs[a]) * 8, reinterpret_cast<char*>(out + 2 * oo[a]),
-                       (size_t)(oo[b] - oo[a]) * 16};
-    };
-    auto compute = [&](int k, void* din, void* dout, void*, void*, cudaStream_t cs) {
-      const int a = first[k], b = first[k + 1];
-      return haas_batch_launch(reinterpret_cast<const float*>(din), dtab + at[k], b - a, dclips + a, dtab + at[k] + (b - a + 1), oo[b] - oo[a],
-                               reinterpret_cast<double*>(dout), cs);
-    };
     return run_pipeline(ctx, nchunks, (size_t)max_rows * 8, (size_t)max_out_rows * 16, 0, chunk_of, compute);
   }
-
-  const size_t out_bytes = (size_t)out_rows * 16;
-  void *din = nullptr, *dout = nullptr, *dmeta = nullptr;
-  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) ||
-      (rc = arena(ctx, S_AUX, clip_bytes + (2 * (size_t)n_clips + 1) * 8, &dmeta)))
+  const PipeChunk c = chunk_of(0);
+  void *din = nullptr, *dout = nullptr;
+  if ((rc = upload(ctx, S_IN, c.src, c.src_bytes, st, &din)) || (rc = arena(ctx, S_OUT, c.dst_bytes, &dout)) ||
+      (rc = compute(0, din, dout, nullptr, nullptr, st)))
     return rc;
-  if (in_bytes) VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
-  char* dm = reinterpret_cast<char*>(dmeta);
-  VND_CUDA_OK(cudaMemcpyAsync(dm, clips, clip_bytes, cudaMemcpyHostToDevice, st));
-  VND_CUDA_OK(cudaMemcpyAsync(dm + clip_bytes, offs, ((size_t)n_clips + 1) * 8, cudaMemcpyHostToDevice, st));
-  VND_CUDA_OK(cudaMemcpyAsync(dm + clip_bytes + ((size_t)n_clips + 1) * 8, oo.data(), (size_t)n_clips * 8, cudaMemcpyHostToDevice, st));
-  if ((rc = vnd_haas_batch_dev(reinterpret_cast<const float*>(din), rows, reinterpret_cast<const int64_t*>(dm + clip_bytes), n_clips,
-                               reinterpret_cast<const vnd_haas_clip*>(dm), reinterpret_cast<const int64_t*>(dm + clip_bytes + ((size_t)n_clips + 1) * 8),
-                               out_rows, reinterpret_cast<double*>(dout), st)))
-    return rc;
-  if (out_bytes) VND_CUDA_OK(cudaMemcpyAsync(out, dout, out_bytes, cudaMemcpyDeviceToHost, st));
+  if (c.dst_bytes) VND_CUDA_OK(cudaMemcpyAsync(c.dst, dout, c.dst_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
   return VND_OK;
 }
@@ -1508,27 +1535,20 @@ extern "C" int vnd_haas_batch_host(vnd_ctx* ctx, const float* x, int64_t rows, c
 extern "C" int vnd_stereo_op_host(vnd_ctx* ctx, const vnd_signal* a, const vnd_signal* dry, int32_t op, double width) {
   VND_ENTER(ctx);
   int rc;
-  if ((rc = check_signal(a, "a"))) return rc;
-  const Dense da = dense_extent(a);
-  VND_REQUIRE(da.ok, VND_EUNSUPPORTED, "host signals must be contiguous");
+  if ((rc = check_stereo_op(a, dry, op))) return rc;
+  const bool with_dry = op == 3 || op == 4;
+  const Dense da = dense_extent(a), dd = with_dry ? dense_extent(dry) : Dense{0, true};
+  VND_REQUIRE(da.ok && dd.ok, VND_EUNSUPPORTED, "host signals must be contiguous");
   cudaStream_t st = ctx->streams[0];
   void *dA = nullptr, *dD = nullptr, *work = nullptr;
-  if ((rc = arena(ctx, S_IN, da.elems * esize(a->dtype), &dA))) return rc;
   const size_t wbytes = 64 + colsumsq_workspace_bytes(a->frames);
-  if ((rc = arena(ctx, S_WORK, wbytes, &work))) return rc;
-  if (da.elems) VND_CUDA_OK(cudaMemcpyAsync(dA, a->data, da.elems * esize(a->dtype), cudaMemcpyHostToDevice, st));
-  vnd_signal ad = *a, dd{};
+  if ((rc = upload(ctx, S_IN, a->data, da.elems * esize(a->dtype), st, &dA)) || (rc = arena(ctx, S_WORK, wbytes, &work)) ||
+      (with_dry && (rc = upload(ctx, S_OUT, dry->data, dd.elems * esize(dry->dtype), st, &dD))))
+    return rc;
+  vnd_signal ad = *a, drd = with_dry ? *dry : vnd_signal{};
   ad.data = dA;
-  if (op == 3 || op == 4) {
-    if ((rc = check_signal(dry, "dry"))) return rc;
-    const Dense d2 = dense_extent(dry);
-    VND_REQUIRE(d2.ok, VND_EUNSUPPORTED, "host signals must be contiguous");
-    if ((rc = arena(ctx, S_OUT, d2.elems * esize(dry->dtype), &dD))) return rc;
-    if (d2.elems) VND_CUDA_OK(cudaMemcpyAsync(dD, dry->data, d2.elems * esize(dry->dtype), cudaMemcpyHostToDevice, st));
-    dd = *dry;
-    dd.data = dD;
-  }
-  if ((rc = vnd_stereo_op_dev(&ad, (op == 3 || op == 4) ? &dd : nullptr, op, width, work, wbytes, st))) return rc;
+  drd.data = dD;
+  if ((rc = vnd_stereo_op_dev(&ad, with_dry ? &drd : nullptr, op, width, work, wbytes, st))) return rc;
   if (da.elems) VND_CUDA_OK(cudaMemcpyAsync(a->data, dA, da.elems * esize(a->dtype), cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
   return VND_OK;
@@ -1538,11 +1558,8 @@ extern "C" int vnd_vn_objective_batch_host(vnd_ctx* ctx, const float* clips, int
                                            int64_t chan_stride, const vnd_tap_program* cand, double* partials) {
   VND_ENTER(ctx);
   int rc;
-  if ((rc = check_taps(cand))) return rc;
-  VND_REQUIRE(frames >= 0 && n_clips >= 0, VND_EINVAL, "negative extent");
+  if ((rc = check_vn_objective_batch(clips, frames, n_clips, cand, partials))) return rc;
   if (n_clips == 0 || cand->channels == 0) return VND_OK;
-  VND_REQUIRE(frames > 0, VND_EINVAL, "objective of an empty signal (zero-size array to reduction operation maximum which has no identity)");
-  VND_REQUIRE(clips != nullptr && partials != nullptr, VND_EINVAL, "null buffer");
   VND_REQUIRE(chan_stride >= frames && clip_stride >= chan_stride + frames, VND_EUNSUPPORTED, "clips must be planar: clip, channel, frame");
   cudaStream_t st = ctx->streams[0];
   vnd_tap_program dprog;
@@ -1550,13 +1567,11 @@ extern "C" int vnd_vn_objective_batch_host(vnd_ctx* ctx, const float* clips, int
   const size_t in_bytes = ((size_t)(n_clips - 1) * clip_stride + chan_stride + frames) * 4;
   const size_t out_bytes = (size_t)n_clips * cand->channels * 12 * 8;
   size_t wbytes = 0;
-  if ((rc = objective_workspace_bytes(frames, n_clips, cand->channels, &wbytes))) return rc;
+  if ((rc = vnd_objective_workspace(frames, n_clips, cand->channels, &wbytes))) return rc;
   void *din = nullptr, *dout = nullptr, *work = nullptr;
-  if ((rc = arena(ctx, S_IN, in_bytes, &din))) return rc;
-  if ((rc = arena(ctx, S_OUT, out_bytes, &dout))) return rc;
-  if ((rc = arena(ctx, S_WORK, wbytes, &work))) return rc;
-  VND_CUDA_OK(cudaMemcpyAsync(din, clips, in_bytes, cudaMemcpyHostToDevice, st));
-  if ((rc = vn_objective_launch((const float*)din, frames, n_clips, clip_stride, chan_stride, &dprog, (double*)dout, work, wbytes, st)))
+  if ((rc = upload(ctx, S_IN, clips, in_bytes, st, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) || (rc = arena(ctx, S_WORK, wbytes, &work)))
+    return rc;
+  if ((rc = vnd_vn_objective_batch_dev((const float*)din, frames, n_clips, clip_stride, chan_stride, &dprog, (double*)dout, work, wbytes, st)))
     return rc;
   VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
@@ -1567,21 +1582,18 @@ extern "C" int vnd_haas_objective_batch_host(vnd_ctx* ctx, const void* clips, in
                                              int64_t chan_stride, const int32_t* delays, int32_t n_cand, double* partials) {
   VND_ENTER(ctx);
   int rc;
-  VND_REQUIRE(frames >= 0 && n_clips >= 0 && n_cand >= 0, VND_EINVAL, "negative extent");
+  if ((rc = check_haas_objective_batch(clips, clip_dtype, frames, n_clips, delays, n_cand, partials))) return rc;
   if (n_clips == 0 || n_cand == 0) return VND_OK;
-  VND_REQUIRE(clips != nullptr && partials != nullptr && delays != nullptr, VND_EINVAL, "null buffer");
-  VND_REQUIRE(clip_dtype == VND_F32 || clip_dtype == VND_F64, VND_EINVAL, "unknown clip dtype %d", clip_dtype);
   VND_REQUIRE(chan_stride >= frames && clip_stride >= chan_stride + frames, VND_EUNSUPPORTED, "clips must be planar: clip, channel, frame");
   cudaStream_t st = ctx->streams[0];
   const size_t in_bytes = ((size_t)(n_clips - 1) * clip_stride + chan_stride + frames) * esize(clip_dtype);
   const size_t out_bytes = (size_t)n_clips * n_cand * 8 * 8;
   void *din = nullptr, *dout = nullptr, *dd = nullptr;
-  if ((rc = arena(ctx, S_IN, in_bytes, &din))) return rc;
-  if ((rc = arena(ctx, S_OUT, out_bytes, &dout))) return rc;
-  if ((rc = arena(ctx, S_AUX, (size_t)n_cand * 4, &dd))) return rc;
-  VND_CUDA_OK(cudaMemcpyAsync(din, clips, in_bytes, cudaMemcpyHostToDevice, st));
-  VND_CUDA_OK(cudaMemcpyAsync(dd, delays, (size_t)n_cand * 4, cudaMemcpyHostToDevice, st));
-  if ((rc = haas_objective_launch(din, clip_dtype, frames, n_clips, clip_stride, chan_stride, (const int*)dd, n_cand, (double*)dout, st)))
+  if ((rc = upload(ctx, S_IN, clips, in_bytes, st, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) ||
+      (rc = upload(ctx, S_AUX, delays, (size_t)n_cand * 4, st, &dd)))
+    return rc;
+  if ((rc = vnd_haas_objective_batch_dev(din, clip_dtype, frames, n_clips, clip_stride, chan_stride, (const int32_t*)dd, n_cand, (double*)dout,
+                                         nullptr, 0, st)))
     return rc;
   VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
@@ -1591,16 +1603,12 @@ extern "C" int vnd_haas_objective_batch_host(vnd_ctx* ctx, const void* clips, in
 extern "C" int vnd_haas_objective_pairs_host(vnd_ctx* ctx, const float* x, int64_t rows, int64_t chan_stride, const int64_t* frame_offsets,
                                              int32_t n_clips, const int32_t* pair_clip, const int32_t* pair_delay, int32_t n_pairs,
                                              double* partials) {
-  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  VND_ENTER(ctx);
   int rc;
   if ((rc = check_haas_pairs(x, rows, chan_stride, frame_offsets, n_clips, pair_clip, pair_delay, n_pairs, partials))) return rc;
   if (n_pairs == 0) return VND_OK;
   const int64_t* offs = frame_offsets;
-  VND_REQUIRE(offs[0] == 0, VND_EINVAL, "frame_offsets[0] is %lld, not 0", (long long)offs[0]);
-  for (int i = 0; i < n_clips; ++i)
-    VND_REQUIRE(offs[i + 1] >= offs[i], VND_EINVAL, "frame_offsets decrease at clip %d (%lld -> %lld)", i, (long long)offs[i],
-                (long long)offs[i + 1]);
-  VND_REQUIRE(offs[n_clips] == rows, VND_EINVAL, "frame_offsets end at %lld, not at rows = %lld", (long long)offs[n_clips], (long long)rows);
+  if ((rc = check_offsets(offs, n_clips, rows))) return rc;
   for (int p = 0; p < n_pairs; ++p) {
     const int c = pair_clip[p], d = pair_delay[p];
     VND_REQUIRE(c >= 0 && c < n_clips, VND_EINVAL, "pair_clip[%d] = %d is outside [0, %d)", p, c, n_clips);
@@ -1610,23 +1618,21 @@ extern "C" int vnd_haas_objective_pairs_host(vnd_ctx* ctx, const float* x, int64
                 "pair %d: objective of an empty signal (clip %d has no frames and delay 0: zero-size array to reduction operation maximum "
                 "which has no identity)", p, c);
   }
-  VND_ENTER(ctx);
   cudaStream_t st = ctx->streams[0];
   const size_t in_bytes = rows > 0 ? ((size_t)chan_stride + rows) * 4 : 0;
   const size_t out_bytes = (size_t)n_pairs * 8 * 8;
   const size_t off_bytes = ((size_t)n_clips + 1) * 8, idx_bytes = (size_t)n_pairs * 4;
   void *din = nullptr, *dout = nullptr, *dmeta = nullptr;
-  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) ||
+  if ((rc = upload(ctx, S_IN, x, in_bytes, st, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) ||
       (rc = arena(ctx, S_AUX, off_bytes + 2 * idx_bytes, &dmeta)))
     return rc;
   char* meta = reinterpret_cast<char*>(dmeta);
-  if (in_bytes) VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
   VND_CUDA_OK(cudaMemcpyAsync(meta, offs, off_bytes, cudaMemcpyHostToDevice, st));
   VND_CUDA_OK(cudaMemcpyAsync(meta + off_bytes, pair_clip, idx_bytes, cudaMemcpyHostToDevice, st));
   VND_CUDA_OK(cudaMemcpyAsync(meta + off_bytes + idx_bytes, pair_delay, idx_bytes, cudaMemcpyHostToDevice, st));
-  if ((rc = haas_objective_pairs_launch((const float*)din, chan_stride, reinterpret_cast<const long long*>(meta),
-                                        reinterpret_cast<const int*>(meta + off_bytes), reinterpret_cast<const int*>(meta + off_bytes + idx_bytes),
-                                        n_pairs, (double*)dout, st)))
+  if ((rc = vnd_haas_objective_pairs_dev((const float*)din, rows, chan_stride, reinterpret_cast<const int64_t*>(meta), n_clips,
+                                         reinterpret_cast<const int32_t*>(meta + off_bytes), reinterpret_cast<const int32_t*>(meta + off_bytes + idx_bytes),
+                                         n_pairs, (double*)dout, st)))
     return rc;
   VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
@@ -1635,26 +1641,23 @@ extern "C" int vnd_haas_objective_pairs_host(vnd_ctx* ctx, const float* x, int64
 
 extern "C" int vnd_vn_stereo_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps,
                                             const vnd_vn_stereo_cand* cands, int32_t n_cand, double* partials) {
-  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  VND_ENTER(ctx);
   int rc;
   if ((rc = check_vn_stereo(x, frames, chan_stride, taps, cands, n_cand, partials))) return rc;
   if (n_cand == 0) return VND_OK;
-  VND_ENTER(ctx);
   cudaStream_t st = ctx->streams[0];
   size_t wbytes = 0;
-  if ((rc = vn_stereo_objective_workspace_bytes(frames, n_cand, &wbytes))) return rc;
+  if ((rc = vnd_vn_stereo_objective_workspace(frames, n_cand, &wbytes))) return rc;
   const size_t in_bytes = ((size_t)chan_stride + frames) * 4;
   const size_t out_bytes = (size_t)n_cand * 12 * 8, cand_bytes = (size_t)n_cand * sizeof(vnd_vn_stereo_cand);
   vnd_tap_program dprog;
   void *din = nullptr, *dout = nullptr, *work = nullptr, *dc = nullptr;
   if ((rc = upload_program(ctx, taps, &dprog, st))) return rc;
-  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) || (rc = arena(ctx, S_WORK, wbytes, &work)) ||
-      (rc = arena(ctx, S_AUX, cand_bytes, &dc)))
+  if ((rc = upload(ctx, S_IN, x, in_bytes, st, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) || (rc = arena(ctx, S_WORK, wbytes, &work)) ||
+      (rc = upload(ctx, S_AUX, cands, cand_bytes, st, &dc)))
     return rc;
-  VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
-  VND_CUDA_OK(cudaMemcpyAsync(dc, cands, cand_bytes, cudaMemcpyHostToDevice, st));
-  if ((rc = vn_stereo_objective_launch((const float*)din, frames, chan_stride, &dprog, (const vnd_vn_stereo_cand*)dc, n_cand, (double*)dout, work,
-                                       wbytes, st)))
+  if ((rc = vnd_vn_stereo_objective_dev((const float*)din, frames, chan_stride, &dprog, (const vnd_vn_stereo_cand*)dc, n_cand, (double*)dout, work,
+                                        wbytes, st)))
     return rc;
   VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
@@ -1663,25 +1666,23 @@ extern "C" int vnd_vn_stereo_objective_host(vnd_ctx* ctx, const float* x, int64_
 
 extern "C" int vnd_haas_effect_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, int64_t chan_stride, const vnd_haas_clip* cands,
                                               int32_t n_cand, double* partials) {
-  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  VND_ENTER(ctx);
   int rc;
-  if ((rc = check_family_clip(x, frames, chan_stride, n_cand, partials))) return rc;
-  VND_REQUIRE(cands != nullptr || n_cand == 0, VND_EINVAL, "cands is null");
+  if ((rc = check_family_clip(x, frames, chan_stride, cands, n_cand, partials))) return rc;
   for (int i = 0; i < n_cand; ++i) {
     VND_REQUIRE(cands[i].delay >= 0, VND_EINVAL, "candidate %d: negative delay %d", i, cands[i].delay);
     VND_REQUIRE(cands[i].delayed_channel == 0 || cands[i].delayed_channel == 1, VND_EINVAL, "candidate %d: delayed_channel %d is not 0 or 1", i,
                 cands[i].delayed_channel);
   }
   if (n_cand == 0) return VND_OK;
-  VND_ENTER(ctx);
   cudaStream_t st = ctx->streams[0];
   const size_t in_bytes = ((size_t)chan_stride + frames) * 4;
   const size_t out_bytes = (size_t)n_cand * 8 * 8, cand_bytes = (size_t)n_cand * sizeof(vnd_haas_clip);
   void *din = nullptr, *dout = nullptr, *dc = nullptr;
-  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) || (rc = arena(ctx, S_AUX, cand_bytes, &dc))) return rc;
-  VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
-  VND_CUDA_OK(cudaMemcpyAsync(dc, cands, cand_bytes, cudaMemcpyHostToDevice, st));
-  if ((rc = haas_effect_objective_launch((const float*)din, frames, chan_stride, (const vnd_haas_clip*)dc, n_cand, (double*)dout, st))) return rc;
+  if ((rc = upload(ctx, S_IN, x, in_bytes, st, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) ||
+      (rc = upload(ctx, S_AUX, cands, cand_bytes, st, &dc)))
+    return rc;
+  if ((rc = vnd_haas_effect_objective_dev((const float*)din, frames, chan_stride, (const vnd_haas_clip*)dc, n_cand, (double*)dout, st))) return rc;
   VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
   return VND_OK;
@@ -1691,28 +1692,25 @@ extern "C" int vnd_vn_objective_runs_host(vnd_ctx* ctx, const float* x, int64_t 
                                           int32_t n_clips, const vnd_tap_program* cand, const int32_t* run_clip, const int32_t* run_cand,
                                           const int32_t* run_count, const int32_t* run_out, int32_t n_runs, double* partials,
                                           int64_t n_partial_rows) {
-  VND_REQUIRE(ctx != nullptr, VND_EINVAL, "context is null");
+  VND_ENTER(ctx);
   int rc;
   if ((rc = check_runs(x, rows, chan_stride, frame_offsets, n_clips, cand, run_clip, run_cand, run_count, run_out, n_runs, partials,
                        n_partial_rows)))
     return rc;
   if (n_partial_rows == 0) return VND_OK;
-  VND_ENTER(ctx);
   cudaStream_t st = ctx->streams[0];
   size_t wbytes = 0;
-  if (n_runs > 0 &&
-      (rc = objective_runs_workspace_bytes(reinterpret_cast<const long long*>(frame_offsets), run_clip, run_count, n_runs, &wbytes)))
-    return rc;
+  if ((rc = vnd_vn_objective_runs_workspace(frame_offsets, n_clips, run_clip, run_count, n_runs, &wbytes))) return rc;
   const size_t in_bytes = rows > 0 ? ((size_t)chan_stride + rows) * 4 : 0;
   const size_t out_bytes = (size_t)n_partial_rows * 12 * 8;
   vnd_tap_program dprog;
   void *din = nullptr, *dout = nullptr, *work = nullptr;
   if ((rc = upload_program(ctx, cand, &dprog, st))) return rc;
-  if ((rc = arena(ctx, S_IN, in_bytes, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) || (rc = arena(ctx, S_WORK, wbytes, &work))) return rc;
-  if (in_bytes) VND_CUDA_OK(cudaMemcpyAsync(din, x, in_bytes, cudaMemcpyHostToDevice, st));
+  if ((rc = upload(ctx, S_IN, x, in_bytes, st, &din)) || (rc = arena(ctx, S_OUT, out_bytes, &dout)) || (rc = arena(ctx, S_WORK, wbytes, &work)))
+    return rc;
   VND_CUDA_OK(cudaMemsetAsync(dout, 0, out_bytes, st));  // rows no run names come back as zeros
-  if (n_runs > 0 && (rc = vn_objective_runs_launch((const float*)din, chan_stride, reinterpret_cast<const long long*>(frame_offsets), run_clip,
-                                                   run_cand, run_count, run_out, n_runs, &dprog, (double*)dout, work, wbytes, st)))
+  if ((rc = vnd_vn_objective_runs_dev((const float*)din, rows, chan_stride, frame_offsets, n_clips, &dprog, run_clip, run_cand, run_count, run_out,
+                                      n_runs, (double*)dout, n_partial_rows, work, wbytes, st)))
     return rc;
   VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
