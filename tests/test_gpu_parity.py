@@ -16,6 +16,7 @@ import pytest
 
 from oracle import vnd_oracle as O
 from tests import _golden as G
+from tests.test_fir_kernels import DIRECT, RING, TILE, TMEM, WIN, predict_route, routed
 
 pytestmark = pytest.mark.gpu
 
@@ -337,7 +338,10 @@ def test_planar_slab_tile_edges(api, frames):
                          mode="LR", normalizer=None, seed=1)
     g = torch.Generator(device="cuda").manual_seed(1234)
     slab = torch.randn((C, frames), generator=g, device="cuda") * 0.1
-    y = vn.convolve(slab.t())  # (frames, C) view of a planar slab
+    prog = vn.tap_program(frames)
+    aligned = frames % 4 == 0  # the channel stride of the slab: bulk copies need a multiple of 16 bytes
+    route = predict_route(frames, prog.halo, prog.max_channel_words, bulk=aligned, y_ok=aligned)
+    y = routed(lambda: vn.convolve(slab.t()), route, f"{frames} frames")  # (frames, C) view of a planar slab
     assert y.shape == (frames, C) and y.stride(0) == 1 or frames == 1
     taps = O.class_taps(sample_rate_hz=48000, num_outs=C, filtered_channels=tuple(range(C)), seed=1)
     want = O.fir_class_order(np.ascontiguousarray(slab.cpu().numpy().T), taps, O.DEFAULT_ENVELOPE, C)
@@ -356,49 +360,52 @@ def test_planar_slab_filter_shapes(api, kappa, envelope):
     slab = torch.randn((C, frames), device="cuda") * 0.1
     slab[2, 100:5000] = 0.0  # runs of exact zeros (signed-zero handling of the negated accumulation)
     slab[2, 5000:5100] = -0.0
-    y = vn.convolve(slab.t())
+    # the same slab through a view that starts 4 bytes into a buffer: TMA-ineligible input and output
+    buf = torch.empty(C * frames + 1, device="cuda")
+    view = buf[1:].view(C, frames)
+    view.copy_(slab)
+    y = routed(lambda: vn.convolve(slab.t()), {WIN}, "aligned slab")
+    y2 = vn.convolve(view.t())
     taps = O.class_taps(sample_rate_hz=48000, num_outs=C, filtered_channels=(0, 1, 2, 3), num_segments=len(envelope),
                         log_distribution_strength=kappa, seed=3)
     want = O.fir_class_order(np.ascontiguousarray(slab.cpu().numpy().T), taps, envelope, C)
     assert G.same_bits(np.ascontiguousarray(y.cpu().numpy()), want)
-    # same slab through a view that starts 4 bytes into a buffer: TMA-ineligible input and output
-    buf = torch.empty(C * frames + 1, device="cuda")
-    view = buf[1:].view(C, frames)
-    view.copy_(slab)
-    y2 = vn.convolve(view.t())
     assert torch.equal(y2, y)
 
 
 @pytest.mark.parametrize(
-    "frames,kappa,envelope,duration",
+    "frames,kappa,envelope,duration,route",
     [
-        (-1, 1.0, (0.85, 0.55, 0.35, 0.2), 0.03),  # one frame short of the shortest slab the kernel takes (window kernel instead)
-        (0, 1.0, (0.85, 0.55, 0.35, 0.2), 0.03),  # the shortest slab it takes: 4 interior tiles, tail of exactly the halo blocks
-        (1, 1.0, (0.85, 0.55, 0.35, 0.2), 0.03),
-        (200003, 0.0, (0.85, 0.55, 0.35, 0.2), 0.03),  # uniform impulses: most taps beyond the TMEM window
-        (150000, 0.4, (1.0,), 0.03),  # identity envelope (no gain multiply), one segment
-        (131072 + 9000, 1.0, (0.9, -0.5), 0.03),
-        (300001, 1.0, (0.85, 0.55, 0.35, 0.2), 0.06),  # 2 880-sample halo: more staged blocks per tile
-        (180000, 1.0, (0.85, 0.55, 0.35, 0.2), 0.004),  # every tap inside the TMEM window
+        # four frames short of the shortest slab the kernel takes (frames stay a multiple of four, so that the channel stride
+        # of the slab allows the bulk copies): the window kernel instead
+        (-4, 1.0, (0.85, 0.55, 0.35, 0.2), 0.03, {WIN}),
+        (0, 1.0, (0.85, 0.55, 0.35, 0.2), 0.03, {TMEM, TILE("float", 0, 256)}),  # the shortest slab it takes: 4 interior tiles
+        (4, 1.0, (0.85, 0.55, 0.35, 0.2), 0.03, {TMEM, TILE("float", 0, 256)}),
+        (200004, 0.0, (0.85, 0.55, 0.35, 0.2), 0.03, {TMEM, TILE("float", 0, 256)}),  # uniform impulses: most taps far
+        (150000, 0.4, (1.0,), 0.03, {TMEM, TILE("float", 0, 256)}),  # identity envelope (no gain multiply), one segment
+        (131072 + 9000, 1.0, (0.9, -0.5), 0.03, {TMEM, WIN}),
+        (300000, 1.0, (0.85, 0.55, 0.35, 0.2), 0.048, {TMEM, WIN}),  # 2 009-sample halo: the largest it takes
+        (300000, 1.0, (0.85, 0.55, 0.35, 0.2), 0.0485, {WIN}),  # 2 030-sample halo: past it
+        (180000, 1.0, (0.85, 0.55, 0.35, 0.2), 0.004, {TMEM, WIN}),  # every tap inside the TMEM window
     ],
 )
-def test_planar_slab_tmem_kernel(api, frames, kappa, envelope, duration):
-    """Long planar slabs take the tensor-memory kernel for the interior tiles and the tile kernel
-    for the tail of each channel; the whole output must equal the oracle bit for bit."""
+def test_planar_slab_tmem_kernel(api, frames, kappa, envelope, duration, route):
+    """Long planar slabs take the tensor-memory kernel for the interior tiles and the window or tile kernel
+    for the tail of each channel; the kernels launched are asserted and the whole output must equal the oracle bit for bit."""
     import torch
 
     C = 5
     filtered = (0, 1, 2, 3)  # channel 4 is copied through
     vn = api.VelvetNoise(sample_rate_hz=48000, duration_seconds=duration, num_impulses=30, num_outs=C, filtered_channels=filtered,
                          mode="LR", normalizer=None, log_distribution_strength=kappa, segment_envelope=envelope, seed=5)
-    if frames <= 1:  # relative to the kernel's minimum: (128 + halo blocks) x 96 samples staged per tile + 3 more tiles of 12288
-        halo = vn.tap_program(1 << 20).halo
-        frames += (128 + -(-(halo + 4) // 96)) * 96 + 3 * 12288
+    if frames <= 4:  # relative to the kernel's minimum: (128 + halo blocks) x 96 samples staged per tile + 3 more tiles of 12288
+        halo = (vn.tap_program(1 << 20).halo + 3) & ~3
+        frames += max(128 + -(-(halo + 4) // 96), 134) * 96 + 3 * 12288
     g = torch.Generator(device="cuda").manual_seed(99)
     slab = torch.randn((C, frames), generator=g, device="cuda") * 0.1
     slab[1, 20000:26000] = 0.0
     slab[1, 26000:26100] = -0.0
-    y = vn.convolve(slab.t())
+    y = routed(lambda: vn.convolve(slab.t()), route, f"{frames} frames")
     taps = O.class_taps(sample_rate_hz=48000, duration_seconds=duration, num_impulses=30, num_outs=C, filtered_channels=filtered,
                         num_segments=len(envelope), log_distribution_strength=kappa, seed=5)
     want = O.fir_class_order(np.ascontiguousarray(slab.cpu().numpy().T), taps, envelope, C)
@@ -546,20 +553,26 @@ def test_cfg4_long_filter_large_halo(api):
     assert G.same_bits(np.ascontiguousarray(y.cpu().numpy()), want)
 
 
+_RING_TAIL = {RING, TILE("float", 0, 1024)}
+_ENV5 = (0.9, -0.5, 0.25, 0.3, 0.1)
+
+
 @pytest.mark.parametrize(
-    "fs,duration,n_imp,envelope,frames,filtered",
+    "fs,duration,n_imp,envelope,frames,filtered,route",
     [
-        (96000, 0.3, 300, (0.85, 0.55, 0.35, 0.2), 700003, (0, 1, 2)),      # BASELINE config 4's filter, several runs per channel, channel 3 copied
-        (96000, 0.2, 120, (1.0,), 400000, (0, 1, 2, 3)),                    # identity envelope (no gain multiply), four ring slots less one
-        (48000, 0.25, 64, (0.9, -0.5, 0.25), 9216 * 30, (0, 1)),             # frames a whole number of steps (9216 outputs): the tail is whole chunks
-        (96000, 0.3, 300, (0.85, 0.55, 0.35, 0.2), 9216 * 12 + 5, (0, 1, 2, 3)),   # the shortest slab the ring kernel takes (eight steps + four chunks of halo)
-        (96000, 0.3, 300, (0.85, 0.55, 0.35, 0.2), 9216 * 12 - 1, (0, 1, 2, 3)),   # one frame short of it: tile kernels only
+        # BASELINE config 4's filter (28 420-sample halo), several runs per channel, channel 3 copied
+        (96000, 0.3, 300, (0.85, 0.55, 0.35, 0.2), 700004, (0, 1, 2), _RING_TAIL),
+        (96000, 0.35, 120, (1.0,), 400000, (0, 1, 2, 3), _RING_TAIL),        # identity envelope (no gain multiply), 32 534-sample halo
+        (96000, 0.36, 100, (0.9, -0.5, 0.25), 9216 * 30, (0, 1), _RING_TAIL),  # three segments (one single-stream pass), whole steps
+        (96000, 0.34, 100, _ENV5, 125776, (0, 1, 2, 3), _RING_TAIL),          # five segments; the shortest slab it takes: 4 x halo
+        (96000, 0.34, 100, _ENV5, 125772, (0, 1, 2, 3), {TILE("float", 0, 1024)}),  # four frames short of it: the tile kernel only
     ],
 )
-def test_ring_kernel_long_filters(api, fs, duration, n_imp, envelope, frames, filtered):
+def test_ring_kernel_long_filters(api, fs, duration, n_imp, envelope, frames, filtered, route):
     """Long filters on long planar slabs: the interior of every channel goes through the ring-buffer kernel
-    (vnd_fir_ring.cu: persistent CTAs, every sample fetched once), the tail through the tile kernels; every output sample
-    must equal the oracle's."""
+    (vnd_fir_ring.cu: persistent CTAs, every sample fetched once), the tail through the tile kernels; the kernels launched
+    are asserted and every output sample must equal the oracle's.  Frames are multiples of four, so that the channel
+    stride of the slab allows the bulk copies."""
     import torch
 
     Cn = 4
@@ -569,7 +582,7 @@ def test_ring_kernel_long_filters(api, fs, duration, n_imp, envelope, frames, fi
     slab = torch.randn((Cn, frames), generator=g, device="cuda") * 0.1
     slab[0, 1000:9000] = 0.0
     slab[0, 9000:9100] = -0.0
-    y = vn.convolve(slab.t())
+    y = routed(lambda: vn.convolve(slab.t()), route, f"{frames} frames")
     taps = O.class_taps(sample_rate_hz=fs, duration_seconds=duration, num_impulses=n_imp, num_outs=Cn, num_segments=len(envelope),
                         filtered_channels=filtered, seed=9)
     want = O.fir_class_order(np.ascontiguousarray(slab.cpu().numpy().T), taps, envelope, Cn)
@@ -584,7 +597,8 @@ def test_filter_longer_than_shared_memory_uses_direct_kernel(api):
     x = (rng.standard_normal((300000, 2)) * 0.1).astype(np.float32)
     vn = api.VelvetNoise(sample_rate_hz=96000, duration_seconds=2.5, num_impulses=40, seed=3)  # 240 000-sample halo
     taps = O.class_taps(sample_rate_hz=96000, duration_seconds=2.5, num_impulses=40, seed=3)
-    assert G.same_bits(vn.convolve(x), O.fir_class_order(x, taps, O.DEFAULT_ENVELOPE, 2))
+    y = routed(lambda: vn.convolve(x), {DIRECT("float", 0)})
+    assert G.same_bits(y, O.fir_class_order(x, taps, O.DEFAULT_ENVELOPE, 2))
     assert G.same_bits(vn.decorrelate(x), O.vn_decorrelate(x, taps))
 
 

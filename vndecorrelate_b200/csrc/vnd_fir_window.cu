@@ -354,7 +354,12 @@ static int launch_window(const FirParams& f, int max_prog_words, int store_bulk_
   constexpr int TILE = NW * BLK;
   if (f.frames < TILE) return VND_EUNSUPPORTED;
   const size_t smem = 32 + (size_t)2 * (TILE + f.halo) * 4 + (size_t)NW * BLK * 4 + (size_t)(max_prog_words + 4) * 4;
-  if (smem > (size_t)kMaxDynSmem) return VND_EUNSUPPORTED;
+  auto k = fir_window_kernel<R, W, NW, MINB>;
+  // the kernel's static shared memory (s_win_shared, 128-byte aligned) comes out of the same 227 KB as the dynamic part:
+  // without it, halos whose dynamic part fits but whose sum does not made cudaFuncSetAttribute fail instead of declining
+  cudaFuncAttributes fa;
+  VND_CUDA_OK(cudaFuncGetAttributes(&fa, k));
+  if (smem + fa.sharedSizeBytes > (size_t)kMaxDynSmem) return VND_EUNSUPPORTED;
   DeviceInfo di;
   int rc = device_info(&di);
   if (rc) return rc;
@@ -366,7 +371,6 @@ static int launch_window(const FirParams& f, int max_prog_words, int store_bulk_
   P.tiles_per_run = (int)(tiles < VND_WIN_RUN ? tiles : VND_WIN_RUN);
   P.runs_per_channel = (int)ceil_div<long long>(tiles, P.tiles_per_run);
   P.n_runs = (long long)P.runs_per_channel * f.channels;
-  auto k = fir_window_kernel<R, W, NW, MINB>;
   VND_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
   VND_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, NW * 32, smem));
