@@ -372,6 +372,25 @@ int vnd_vn_stereo_objective_workspace(int64_t frames, int32_t n_cand, size_t* by
 int vnd_vn_stereo_objective_dev(const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,
                                 int32_t n_cand, double* partials, void* workspace, size_t workspace_bytes, void* stream);
 
+/* The objective of many VelvetNoise candidates with two outputs and the default normaliser rms_normalize (DUAL_MONO) -
+ * any filtered channels, LR or MS, any width - on one clip, in three launches on `stream` for any number of candidates:
+ * vn_rms_sums_kernel (the sums of squares of x and of every candidate's un-normalised output, then its gains),
+ * vn_stereo_objective_kernel on the scaled outputs, and the combine.  No host synchronisation between them.
+ *   x, taps, cands, partials: as vnd_vn_stereo_objective_dev (the candidates' records hold no normaliser flag: the
+ *              normaliser is what this call adds);
+ *   gains    : 2 n_cand float32 on the device, written: candidate j's channel-0 and channel-1 gains at 2 j, 2 j + 1.
+ * Bit contract: gains[2 j + c] is the gain vnd_vn_decorrelate_dev with rms_normalize = 1 applies to channel c of
+ * candidate j's output when its input is C-order (frames, 2) or mono (x's sums of squares are strict left-to-right
+ * float32 running sums, numpy's order for such an input), and candidate j's 12 partials equal, bit for bit, those of
+ * vnd_vn_objective_batch_dev on that scaled output (planar, with the one-tap identity program).  Checked before any
+ * launch: the program (SEGMENTED, 2 n_cand channels), the sizes and the pointers, gains included.  VND_EUNSUPPORTED (no
+ * launch) when the program's halo does not fit either kernel's shared memory.
+ * Workspace: vnd_vn_stereo_rms_objective_workspace bytes, 256-byte aligned. */
+int vnd_vn_stereo_rms_objective_workspace(int64_t frames, int32_t n_cand, size_t* bytes);
+int vnd_vn_stereo_rms_objective_dev(const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps,
+                                    const vnd_vn_stereo_cand* cands, int32_t n_cand, float* gains, double* partials, void* workspace,
+                                    size_t workspace_bytes, void* stream);
+
 /* The objective of many HaasEffect candidates - any delayed channel, LR or MS, any width - on one clip: one launch, one
  * CTA per candidate.
  *   x        : float32 channel-planar clip as above (a mono clip with its samples in both channels and mono = 1 in every
@@ -444,6 +463,11 @@ int vnd_vn_stereo_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, i
                                  const vnd_vn_stereo_cand* cands, int32_t n_cand, double* partials);
 int vnd_haas_effect_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, int64_t chan_stride, const vnd_haas_clip* cands, int32_t n_cand,
                                    double* partials);
+
+/* vnd_vn_stereo_rms_objective_dev with host buffers (x, program, records, gains and partials): the same checks, then
+ * staging, the device call and the download of partials and gains. */
+int vnd_vn_stereo_rms_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps,
+                                     const vnd_vn_stereo_cand* cands, int32_t n_cand, float* gains, double* partials);
 
 /* vnd_vn_objective_runs_dev with host buffers (x, program, tables and partials).  Rows no run names come back as
  * zeros. */

@@ -122,6 +122,9 @@ SIGNATURES = {
     "vnd_vn_stereo_objective_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, _P(TapProgramStruct), C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
                                               C.c_size_t, C.c_void_p]),
     "vnd_haas_effect_objective_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
+    "vnd_vn_stereo_rms_objective_workspace": (C.c_int, [C.c_int64, C.c_int32, _P(C.c_size_t)]),
+    "vnd_vn_stereo_rms_objective_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, _P(TapProgramStruct), C.c_void_p, C.c_int32, C.c_void_p,
+                                                  C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "vnd_ctx_create": (C.c_int, [C.c_int, _P(C.c_void_p)]),
     "vnd_ctx_destroy": (C.c_int, [C.c_void_p]),
     "vnd_host_alloc": (C.c_int, [C.c_size_t, _P(C.c_void_p)]),
@@ -142,6 +145,8 @@ SIGNATURES = {
                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64]),
     "vnd_vn_stereo_objective_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, _P(TapProgramStruct), C.c_void_p, C.c_int32, C.c_void_p]),
     "vnd_haas_effect_objective_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p]),
+    "vnd_vn_stereo_rms_objective_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, _P(TapProgramStruct), C.c_void_p, C.c_int32,
+                                                   C.c_void_p, C.c_void_p]),
     "vnd_sparse_fir_stream_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, _P(TapProgramStruct), C.c_int32]),
     "vnd_launch_count": (C.c_int64, []),
 }

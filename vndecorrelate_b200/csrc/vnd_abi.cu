@@ -49,6 +49,9 @@ int haas_effect_objective_launch(const float* x, long long frames, long long cha
 int vn_stereo_objective_workspace_bytes(long long frames, int n_cand, size_t* bytes);
 int vn_stereo_objective_launch(const float* x, long long frames, long long chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,
                                int n_cand, double* partials, void* workspace, size_t workspace_bytes, cudaStream_t st);
+int vn_stereo_rms_objective_launch(const float* x, long long frames, long long chan_stride, const vnd_tap_program* taps,
+                                   const vnd_vn_stereo_cand* cands, int n_cand, float* gains, double* partials, void* workspace,
+                                   size_t workspace_bytes, cudaStream_t st);
 size_t dsp_workspace_bytes(long long elems);
 int rms_normalize_launch(const vnd_signal* x, const vnd_signal* y, int x_ndim, int y_ndim, int stereo_mode, double eps, void* ws, cudaStream_t st);
 int peak_normalize_launch(const vnd_signal* y, int ndim, int stereo_mode, double eps, void* ws, cudaStream_t st);
@@ -567,6 +570,27 @@ extern "C" int vnd_vn_stereo_objective_dev(const float* x, int64_t frames, int64
   int rc;
   if ((rc = check_vn_stereo(x, frames, chan_stride, taps, cands, n_cand, partials))) return rc;
   return vn_stereo_objective_launch(x, frames, chan_stride, taps, cands, n_cand, partials, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+static int check_vn_stereo_rms(const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,
+                               int32_t n_cand, const float* gains, const double* partials) {
+  int rc;
+  if ((rc = check_vn_stereo(x, frames, chan_stride, taps, cands, n_cand, partials))) return rc;
+  VND_REQUIRE(gains != nullptr || n_cand == 0, VND_EINVAL, "gains is null");
+  return VND_OK;
+}
+
+extern "C" int vnd_vn_stereo_rms_objective_workspace(int64_t frames, int32_t n_cand, size_t* bytes) {
+  return vnd_vn_stereo_objective_workspace(frames, n_cand, bytes);
+}
+
+extern "C" int vnd_vn_stereo_rms_objective_dev(const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps,
+                                               const vnd_vn_stereo_cand* cands, int32_t n_cand, float* gains, double* partials, void* workspace,
+                                               size_t workspace_bytes, void* stream) {
+  int rc;
+  if ((rc = check_vn_stereo_rms(x, frames, chan_stride, taps, cands, n_cand, gains, partials))) return rc;
+  return vn_stereo_rms_objective_launch(x, frames, chan_stride, taps, cands, n_cand, gains, partials, workspace, workspace_bytes,
+                                        (cudaStream_t)stream);
 }
 
 extern "C" int vnd_haas_effect_objective_dev(const float* x, int64_t frames, int64_t chan_stride, const vnd_haas_clip* cands, int32_t n_cand,
@@ -1660,6 +1684,33 @@ extern "C" int vnd_vn_stereo_objective_host(vnd_ctx* ctx, const float* x, int64_
                                         wbytes, st)))
     return rc;
   VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
+  VND_CUDA_OK(cudaStreamSynchronize(st));
+  return VND_OK;
+}
+
+extern "C" int vnd_vn_stereo_rms_objective_host(vnd_ctx* ctx, const float* x, int64_t frames, int64_t chan_stride, const vnd_tap_program* taps,
+                                                const vnd_vn_stereo_cand* cands, int32_t n_cand, float* gains, double* partials) {
+  VND_ENTER(ctx);
+  int rc;
+  if ((rc = check_vn_stereo_rms(x, frames, chan_stride, taps, cands, n_cand, gains, partials))) return rc;
+  if (n_cand == 0) return VND_OK;
+  cudaStream_t st = ctx->streams[0];
+  size_t wbytes = 0;
+  if ((rc = vnd_vn_stereo_rms_objective_workspace(frames, n_cand, &wbytes))) return rc;
+  const size_t in_bytes = ((size_t)chan_stride + frames) * 4;
+  const size_t out_bytes = (size_t)n_cand * 12 * 8, gain_bytes = (size_t)n_cand * 2 * 4, cand_bytes = (size_t)n_cand * sizeof(vnd_vn_stereo_cand);
+  vnd_tap_program dprog;
+  void *din = nullptr, *dout = nullptr, *work = nullptr, *dc = nullptr;
+  if ((rc = upload_program(ctx, taps, &dprog, st))) return rc;
+  if ((rc = upload(ctx, S_IN, x, in_bytes, st, &din)) || (rc = arena(ctx, S_OUT, out_bytes + gain_bytes, &dout)) ||
+      (rc = arena(ctx, S_WORK, wbytes, &work)) || (rc = upload(ctx, S_AUX, cands, cand_bytes, st, &dc)))
+    return rc;
+  float* dgains = reinterpret_cast<float*>(reinterpret_cast<char*>(dout) + out_bytes);  // behind the partials
+  if ((rc = vnd_vn_stereo_rms_objective_dev((const float*)din, frames, chan_stride, &dprog, (const vnd_vn_stereo_cand*)dc, n_cand, dgains,
+                                            (double*)dout, work, wbytes, st)))
+    return rc;
+  VND_CUDA_OK(cudaMemcpyAsync(partials, dout, out_bytes, cudaMemcpyDeviceToHost, st));
+  VND_CUDA_OK(cudaMemcpyAsync(gains, dgains, gain_bytes, cudaMemcpyDeviceToHost, st));
   VND_CUDA_OK(cudaStreamSynchronize(st));
   return VND_OK;
 }

@@ -638,24 +638,41 @@ struct VnStereoObjParams {
   double* chunk_partials;  // [chunk][cand][OBJ_CHUNK_SLOTS]
 };
 
-// One pass of one candidate: its output (l, r) at frames i0 + 32 rr of the staged tile.
+// One pass of one candidate: its output (l, r) at frames i0 + 32 rr of the staged tile.  With kGain the output is scaled
+// by candidate c's rms_normalize gains g[2 c], g[2 c + 1] as place_kernel scales the stored output.  They are read here,
+// per pass, through a pointer without __restrict__: loads the compiler may hoist out of the pass loop hold two more
+// registers across it, and those spill.
+template <bool kGain>
 __device__ __forceinline__ void stereo_candidate_pass(const float* __restrict__ s0, const float* __restrict__ s1, int i0, const int* __restrict__ prog,
-                                                      int n0, int n1, const vnd_vn_stereo_cand& cd, int apply_gain, float (&l)[OBJ_R],
-                                                      float (&r)[OBJ_R]) {
+                                                      int n0, int n1, const vnd_vn_stereo_cand& cd, int apply_gain, const float* g,
+                                                      int c, float (&l)[OBJ_R], float (&r)[OBJ_R]) {
   if (n0 > 0) run_candidate<OBJ_R>(s0 + i0, prog, apply_gain, l);
   if (n1 > 0) run_candidate<OBJ_R>(s1 + i0, prog + n0, apply_gain, r);
+  float g0 = 1.0f, g1 = 1.0f;
+  if constexpr (kGain) {
+    g0 = g[2 * c];
+    g1 = g[2 * c + 1];
+  }
 #pragma unroll
   for (int k = 0; k < OBJ_R; ++k) {
     const float a = s0[i0 + 32 * k], b = s1[i0 + 32 * k];
     float u = n0 > 0 ? l[k] : a;  // unfiltered channel: copied through
     float v = n1 > 0 ? r[k] : b;
     ms_width_epilogue(a, b, u, v, cd.ms_encode, cd.use_width, cd.w_mid, cd.w_side);
+    if constexpr (kGain) {
+      u = fmul(u, g0);
+      v = fmul(v, g1);
+    }
     l[k] = fadd(0.0f, fadd(0.0f, u));  // the identity program's segment sum and running output
     r[k] = v;
   }
 }
 
-__global__ void __launch_bounds__(VND_OBJ_STEREO_NT, 1) vn_stereo_objective_kernel(const VnStereoObjParams p, int max_prog_words) {
+// kGain: candidate j's output is scaled by its rms_normalize gains gains[2 j], gains[2 j + 1].  The gains come as a
+// parameter of their own behind the others, so that the kernel without them reads its parameters at the same offsets.
+template <bool kGain>
+__global__ void __launch_bounds__(VND_OBJ_STEREO_NT, 1) vn_stereo_objective_kernel(const VnStereoObjParams p, int max_prog_words,
+                                                                                   const float* gains) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int kWarps = VND_OBJ_STEREO_NT / 32;
   constexpr int kPass = 32 * OBJ_R;
@@ -704,7 +721,7 @@ __global__ void __launch_bounds__(VND_OBJ_STEREO_NT, 1) vn_stereo_objective_kern
         LaneAcc2 b{{0.f, 0.f}, {0.f, 0.f}, {0.f, 0.f}, {0.f, 0.f}, {0.f, 0.f}, {0.f, 0.f}, 0.f, 1.f, 0.f, 1.f, -1.f, -1.f};
         for (int base = 0; base < OBJ_TILE; base += kPass) {
           float l[OBJ_R], r[OBJ_R];
-          stereo_candidate_pass(s0, s1, base + lane, myprog, n0, n1, cd, p.apply_gain, l, r);
+          stereo_candidate_pass<kGain>(s0, s1, base + lane, myprog, n0, n1, cd, p.apply_gain, gains, c, l, r);
           __syncwarp();  // the previous pass has read the scratch row
 #pragma unroll
           for (int k = 0; k < OBJ_R; ++k) {
@@ -734,7 +751,7 @@ __global__ void __launch_bounds__(VND_OBJ_STEREO_NT, 1) vn_stereo_objective_kern
       } else {
         for (int base = 0; base < nvalid; base += kPass) {
           float l[OBJ_R], r[OBJ_R];
-          stereo_candidate_pass(s0, s1, base + lane, myprog, n0, n1, cd, p.apply_gain, l, r);
+          stereo_candidate_pass<kGain>(s0, s1, base + lane, myprog, n0, n1, cd, p.apply_gain, gains, c, l, r);
 #pragma unroll
           for (int k = 0; k < OBJ_R; ++k) {
             const int i = base + lane + 32 * k;
@@ -756,6 +773,123 @@ __global__ void __launch_bounds__(VND_OBJ_STEREO_NT, 1) vn_stereo_objective_kern
   __syncthreads();
   double* out = p.chunk_partials + ((size_t)blockIdx.x * p.n_cand + cand0) * OBJ_CHUNK_SLOTS;
   for (int i = tid; i < ncand * OBJ_CHUNK_SLOTS; i += VND_OBJ_STEREO_NT) out[i] = acc[i];
+}
+
+// ------------------------------------------------------------------------------------------------
+// rms_normalize gains of velvet-noise stereo candidates (vnd_vn_stereo_rms_objective_dev).  decorrelate with the default
+// normaliser scales channel c of its output y by sqrt(mean(x_c^2)) / sqrt(mean(y_c^2) + eps), where each sum of squares
+// is numpy's strict left-to-right float32 running sum over the whole signal (SURVEY.md H1): a dependent chain of one
+// rounded add per frame that no reordering may shorten.  This kernel runs those chains for G candidates per CTA at the
+// cost of one: producer warps build each candidate's un-normalised output y with stereo_candidate_pass's arithmetic
+// (run_candidate, ms_width_epilogue; the identity-program adds belong to the objective, not to y) and write the rounded
+// squares of a sub-tile as rows [frame][2 G + 2] of a double-buffered array; one consumer warp walks the rows in frame
+// order, lane 2 j + c adding candidate j's channel c and lanes 2 G, 2 G + 1 the two channels of x.  Rows have a pitch of
+// 33 words, so the producers' writes (lane = frame) and the consumer's row reads (lane = column) are both conflict-free.
+// The sums and gains are those of rms_gain_kernel after seq_sumsq_kernel on decorrelate's C-order (frames, 2) output.
+// Shared memory: float x0[span] | float x1[span] | float sq[2][RMS_SUB][RMS_PITCH] | int prog[G][2 max_prog_words]
+// ------------------------------------------------------------------------------------------------
+constexpr int RMS_NT = 512;                 // 15 producer warps and the consumer warp
+constexpr int RMS_PROD = RMS_NT / 32 - 1;
+constexpr int RMS_MAX_G = 15;               // 2 G + 2 chains in the consumer warp
+constexpr int RMS_SUB = 256;                // frames per squares buffer
+constexpr int RMS_XTILE = 2048;             // frames per staged input tile (a multiple of RMS_SUB)
+constexpr int RMS_PITCH = 33;
+constexpr int RMS_R = 2;                    // frames per lane and unit: a unit is one candidate on 64 frames
+constexpr int RMS_UNITS = RMS_SUB / (32 * RMS_R);  // units per candidate and sub-tile
+
+struct VnRmsSumsParams {
+  const float* x;  // channel 0; channel 1 at x + chan_stride
+  long long frames, chan_stride;
+  const int* words;
+  const int* offsets;  // candidate j: channels 2 j and 2 j + 1
+  const vnd_vn_stereo_cand* cands;
+  int n_cand, apply_gain, halo, group;
+  float* gains;  // 2 n_cand
+};
+
+__global__ void __launch_bounds__(RMS_NT, 1) vn_rms_sums_kernel(const VnRmsSumsParams p, int max_prog_words) {
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  const int span = RMS_XTILE + p.halo;
+  const int span_al = (span + 3) & ~3;
+  float* s0 = reinterpret_cast<float*>(smem_raw);
+  float* s1 = s0 + span_al;
+  float* sq = s1 + span_al;
+  int* progs = reinterpret_cast<int*>(sq + 2 * RMS_SUB * RMS_PITCH);
+
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int cand0 = blockIdx.x * p.group;
+  const int ng = min(p.group, p.n_cand - cand0);
+  const float* __restrict__ x0 = p.x;
+  const float* __restrict__ x1 = p.x + p.chan_stride;
+  for (int j = 0; j < ng; ++j) {
+    const int w0 = p.offsets[2 * (cand0 + j)], n = p.offsets[2 * (cand0 + j) + 2] - w0;
+    for (int i = tid; i < n; i += RMS_NT) progs[j * 2 * max_prog_words + i] = p.words[w0 + i];
+  }
+  __syncthreads();
+
+  const long long nsub = ceil_div<long long>(p.frames, RMS_SUB);
+  float chain = 0.0f;  // consumer lane 2 j + c: candidate j, channel c; lanes 2 ng, 2 ng + 1: x
+  for (long long k = 0; k <= nsub; ++k) {
+    if (warp < RMS_PROD) {
+      if (k < nsub) {
+        const int base = (int)(k % (RMS_XTILE / RMS_SUB)) * RMS_SUB;
+        if (base == 0) {  // the previous __syncthreads ended every read of the old tile
+          const long long t0 = k * RMS_SUB, remain = p.frames - t0;
+          for (int i = tid; i < span; i += RMS_PROD * 32) {
+            s0[i] = i < remain ? x0[t0 + i] : 0.0f;
+            s1[i] = i < remain ? x1[t0 + i] : 0.0f;
+          }
+          asm volatile("bar.sync 1, %0;" ::"r"(RMS_PROD * 32) : "memory");
+        }
+        float* buf = sq + (k & 1) * (RMS_SUB * RMS_PITCH);
+        for (int i = tid; i < RMS_SUB; i += RMS_PROD * 32) {
+          const float a = s0[base + i], b = s1[base + i];
+          buf[i * RMS_PITCH + 2 * ng] = fmul(a, a);
+          buf[i * RMS_PITCH + 2 * ng + 1] = fmul(b, b);
+        }
+        for (int u = warp; u < ng * RMS_UNITS; u += RMS_PROD) {
+          const int j = u / RMS_UNITS, c = cand0 + j;
+          const int f0 = (u % RMS_UNITS) * 32 * RMS_R + lane;  // frames f0 + 32 k of the sub-tile
+          const int n0 = p.offsets[2 * c + 1] - p.offsets[2 * c];
+          const int n1 = p.offsets[2 * c + 2] - p.offsets[2 * c + 1];
+          const int* prog = progs + j * 2 * max_prog_words;
+          const vnd_vn_stereo_cand cd = p.cands[c];
+          float l[RMS_R], r[RMS_R];
+          if (n0 > 0) run_candidate<RMS_R>(s0 + base + f0, prog, p.apply_gain, l);
+          if (n1 > 0) run_candidate<RMS_R>(s1 + base + f0, prog + n0, p.apply_gain, r);
+#pragma unroll
+          for (int q = 0; q < RMS_R; ++q) {
+            const float a = s0[base + f0 + 32 * q], b = s1[base + f0 + 32 * q];
+            float y0 = n0 > 0 ? l[q] : a;  // unfiltered channel: copied through
+            float y1 = n1 > 0 ? r[q] : b;
+            ms_width_epilogue(a, b, y0, y1, cd.ms_encode, cd.use_width, cd.w_mid, cd.w_side);
+            float* row = buf + (f0 + 32 * q) * RMS_PITCH + 2 * j;
+            row[0] = fmul(y0, y0);
+            row[1] = fmul(y1, y1);
+          }
+        }
+      }
+    } else if (k > 0 && lane < 2 * ng + 2) {  // the consumer: sub-tile k - 1, rows past the last frame skipped
+      const float* q = sq + ((k - 1) & 1) * (RMS_SUB * RMS_PITCH) + lane;
+      const long long left = p.frames - (k - 1) * RMS_SUB;
+      const int n = (int)(left < RMS_SUB ? left : RMS_SUB);
+      int i = 0;
+#pragma unroll 2
+      for (; i + 8 <= n; i += 8) {
+        float v[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) v[e] = q[(i + e) * RMS_PITCH];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) chain = fadd(chain, v[e]);
+      }
+      for (; i < n; ++i) chain = fadd(chain, q[i * RMS_PITCH]);
+    }
+    __syncthreads();
+  }
+  if (warp == RMS_PROD) {
+    const float sx = __shfl_sync(0xffffffffu, chain, 2 * ng + (lane & 1));
+    if (lane < 2 * ng) p.gains[2 * (long long)cand0 + lane] = rms_gain_f32(sx, chain, p.frames);
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1338,9 +1472,17 @@ int vn_stereo_objective_workspace_bytes(long long frames, int n_cand, size_t* by
   return VND_OK;
 }
 
-int vn_stereo_objective_launch(const float* x, long long frames, long long chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,
-                               int n_cand, double* partials, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  if (n_cand == 0) return VND_OK;
+// One call's launch of vn_stereo_objective_kernel: its parameters, grid and shared memory.
+struct StereoObjLaunch {
+  VnStereoObjParams p;
+  int mpw, n_chunks, groups;
+  size_t smem;
+};
+
+// Plans a call without launching anything: VND_EUNSUPPORTED (no error text, the caller scores candidate by candidate)
+// when tile + halo does not fit the kernel's shared memory.
+static int plan_stereo_objective(const float* x, long long frames, long long chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,
+                                 int n_cand, void* workspace, size_t workspace_bytes, StereoObjLaunch* out) {
   DeviceInfo di;
   int rc = device_info(&di);
   if (rc) return rc;
@@ -1352,7 +1494,7 @@ int vn_stereo_objective_launch(const float* x, long long frames, long long chan_
   const int mpw = taps->max_channel_words > 0 ? taps->max_channel_words : 1;
   constexpr int kWarps = VND_OBJ_STEREO_NT / 32;
   const size_t fixed = (size_t)2 * ((OBJ_TILE + halo + 3) & ~3) * 4 + (size_t)kWarps * 2 * 32 * OBJ_R * 4 + (size_t)kWarps * 2 * mpw * 4 + 64;
-  if (fixed + (size_t)OBJ_CHUNK_SLOTS * 8 > (size_t)kMaxDynSmem) return VND_EUNSUPPORTED;  // the caller scores candidate by candidate
+  if (fixed + (size_t)OBJ_CHUNK_SLOTS * 8 > (size_t)kMaxDynSmem) return VND_EUNSUPPORTED;
   int cpg = (int)((kMaxDynSmem - fixed) / (OBJ_CHUNK_SLOTS * 8));
   if (cpg > n_cand) cpg = n_cand;
   if (cpg > 1024) cpg = 1024;
@@ -1375,11 +1517,57 @@ int vn_stereo_objective_launch(const float* x, long long frames, long long chan_
   p.cand_per_group = cpg;
   p.tiles_per_chunk = chunks.tiles_per_chunk;
   p.chunk_partials = reinterpret_cast<double*>(workspace);
-  const size_t smem = fixed + (size_t)cpg * OBJ_CHUNK_SLOTS * 8;
-  VND_CUDA_OK(cudaFuncSetAttribute(vn_stereo_objective_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  vn_stereo_objective_kernel<<<dim3((unsigned)chunks.n_chunks, (unsigned)groups), VND_OBJ_STEREO_NT, smem, st>>>(p, mpw);
-  if ((rc = after_launch("vn_stereo_objective_kernel"))) return rc;
-  return obj_combine_launch(p.chunk_partials, partials, 1, chunks.n_chunks, n_cand, st);
+  *out = {p, mpw, chunks.n_chunks, groups, fixed + (size_t)cpg * OBJ_CHUNK_SLOTS * 8};
+  return VND_OK;
+}
+
+template <bool kGain>
+static int stereo_objective_run(const StereoObjLaunch& l, const float* gains, double* partials, cudaStream_t st) {
+  VND_CUDA_OK(cudaFuncSetAttribute(vn_stereo_objective_kernel<kGain>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l.smem));
+  vn_stereo_objective_kernel<kGain><<<dim3((unsigned)l.n_chunks, (unsigned)l.groups), VND_OBJ_STEREO_NT, l.smem, st>>>(l.p, l.mpw, gains);
+  const int rc = after_launch("vn_stereo_objective_kernel");
+  if (rc) return rc;
+  return obj_combine_launch(l.p.chunk_partials, partials, 1, l.n_chunks, l.p.n_cand, st);
+}
+
+int vn_stereo_objective_launch(const float* x, long long frames, long long chan_stride, const vnd_tap_program* taps, const vnd_vn_stereo_cand* cands,
+                               int n_cand, double* partials, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  if (n_cand == 0) return VND_OK;
+  StereoObjLaunch l;
+  const int rc = plan_stereo_objective(x, frames, chan_stride, taps, cands, n_cand, workspace, workspace_bytes, &l);
+  if (rc) return rc;
+  return stereo_objective_run<false>(l, nullptr, partials, st);
+}
+
+// Shared memory of vn_rms_sums_kernel for a launch halo (a multiple of 4) and program block size.
+static size_t rms_sums_smem(int halo, int mpw) {
+  return (size_t)2 * ((RMS_XTILE + halo + 3) & ~3) * 4 + (size_t)2 * RMS_SUB * RMS_PITCH * 4 + (size_t)RMS_MAX_G * 2 * mpw * 4;
+}
+
+// vn_rms_sums_kernel -> vn_stereo_objective_kernel<true> -> obj_combine_kernel on one stream.  Everything that can refuse
+// the call is decided before the first launch.
+int vn_stereo_rms_objective_launch(const float* x, long long frames, long long chan_stride, const vnd_tap_program* taps,
+                                   const vnd_vn_stereo_cand* cands, int n_cand, float* gains, double* partials, void* workspace,
+                                   size_t workspace_bytes, cudaStream_t st) {
+  if (n_cand == 0) return VND_OK;
+  StereoObjLaunch l;
+  int rc = plan_stereo_objective(x, frames, chan_stride, taps, cands, n_cand, workspace, workspace_bytes, &l);
+  if (rc == VND_EUNSUPPORTED || (!rc && rms_sums_smem(l.p.halo, l.mpw) > (size_t)kMaxDynSmem)) {
+    set_error("rms objective kernels: filter halo %d does not fit in shared memory", taps->halo);
+    return VND_EUNSUPPORTED;
+  }
+  if (rc) return rc;
+  const size_t smem = rms_sums_smem(l.p.halo, l.mpw);
+  DeviceInfo di;
+  if ((rc = device_info(&di))) return rc;
+  // the fewest candidates per CTA that keep the launch within one wave: the producers, not the chain, bound a full group
+  int group = ceil_div(n_cand, di.sm_count);
+  if (group > RMS_MAX_G) group = RMS_MAX_G;
+  const VnRmsSumsParams sp{x, frames, chan_stride, taps->words, taps->offsets, cands, n_cand, taps->apply_gain, l.p.halo, group, gains};
+  VND_CUDA_OK(cudaFuncSetAttribute(vn_rms_sums_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  vn_rms_sums_kernel<<<(unsigned)ceil_div(n_cand, group), RMS_NT, smem, st>>>(sp, l.mpw);
+  if ((rc = after_launch("vn_rms_sums_kernel"))) return rc;
+  return stereo_objective_run<true>(l, gains, partials, st);
 }
 
 }  // namespace vnd

@@ -37,13 +37,13 @@ from . import _native as N
 from . import runtime as R
 from .decorrelation import Decorrelator, HaasEffect, VelvetNoise, _batch_program, _is_mode
 from .taps import IDENTITY_ENVELOPE, TapProgram, candidate_program, kappa_family_program
-from .utils.dsp import EPSILON, LayoutMode, to_float32
+from .utils.dsp import EPSILON, LayoutMode, rms_normalize, to_float32
 
 __all__ = [
     "symmetry_aware_objective", "grid_scan", "get_local_minima", "optimize_local_minima", "optimize_haas_delay",
     "optimize_velvet_noise", "optimize_velvet_noise_batch", "optimize_haas_delay_batch", "vn_objective_partials", "haas_objective_partials",
     "haas_objective_pair_partials", "vn_objective_run_partials", "vn_scores_from_partials", "haas_scores_from_partials",
-    "vn_stereo_objective_partials", "haas_effect_objective_partials",
+    "vn_stereo_objective_partials", "vn_stereo_rms_objective_partials", "haas_effect_objective_partials",
 ]
 
 _F32_HALF_PI = np.float32(np.pi / 2)
@@ -250,20 +250,25 @@ def _cast_input(input_signal):
     return to_float32(input_signal if R.is_torch_tensor(input_signal) else np.asarray(input_signal))
 
 
-def _vn_stereo_partials(x, xp, decorrelators):
-    """``vn_stereo_objective_partials`` on an input already cast and checked, ``xp`` its ``_planar_input``."""
-    lib = N.lib()
-    frames = x.shape[0]
+def _vn_stereo_records(frames: int, decorrelators):
+    """The program (candidate j: channels 2 j, 2 j + 1) and the settings records of a velvet-noise stereo call."""
     progs = [d.tap_program(frames) for d in decorrelators]
     if len({p.apply_gain for p in progs}) > 1:
         raise ValueError("the candidates of one call must agree on whether the segment envelope is the identity (1.0,)")
-    prog = _batch_program(progs)
     cands = np.zeros(len(decorrelators), dtype=N.VN_STEREO_CAND_DTYPE)
     widths = [float(d.width) if d.width is not None else 0.0 for d in decorrelators]
     cands["ms_encode"] = [_is_mode(d.mode, LayoutMode.MS) for d in decorrelators]
     cands["use_width"] = [d.width is not None for d in decorrelators]
     cands["w_mid"] = [np.float32(1.0 - w) for w in widths]  # the float32 roundings of vnd_vn_decorrelate_dev
     cands["w_side"] = [np.float32(w) for w in widths]
+    return _batch_program(progs), cands
+
+
+def _vn_stereo_partials(x, xp, decorrelators):
+    """``vn_stereo_objective_partials`` on an input already cast and checked, ``xp`` its ``_planar_input``."""
+    lib = N.lib()
+    frames = x.shape[0]
+    prog, cands = _vn_stereo_records(frames, decorrelators)
     n = len(decorrelators)
     if R.is_torch_tensor(xp):
         import torch
@@ -284,6 +289,48 @@ def _vn_stereo_partials(x, xp, decorrelators):
     N.check(lib.vnd_vn_stereo_objective_host(R.HostContext.get().handle, xp.ctypes.data, frames, xp.shape[1], C.byref(ps), cands.ctypes.data, n,
                                              out.ctypes.data), "vnd_vn_stereo_objective_host")
     return out
+
+
+def _vn_stereo_rms_partials(x, xp, decorrelators):
+    """``vn_stereo_rms_objective_partials`` on an input already cast and checked, ``xp`` its ``_planar_input``."""
+    frames = x.shape[0]
+    prog, cands = _vn_stereo_records(frames, decorrelators)
+    lib = N.lib()
+    n = len(decorrelators)
+    if R.is_torch_tensor(xp):
+        import torch
+
+        dev = xp.device
+        out = torch.empty((n, N.OBJ_SLOTS), dtype=torch.float64, device=dev)
+        gains = torch.empty((n, 2), dtype=torch.float32, device=dev)
+        nbytes = C.c_size_t()
+        N.check(lib.vnd_vn_stereo_rms_objective_workspace(frames, n, C.byref(nbytes)), "vnd_vn_stereo_rms_objective_workspace")
+        with torch.cuda.device(dev):
+            work = torch.empty(nbytes.value, dtype=torch.uint8, device=dev)
+            dc = torch.from_numpy(cands.view(np.uint8)).to(dev)
+            ps = R.device_program(prog, dev)
+            N.check(lib.vnd_vn_stereo_rms_objective_dev(xp.data_ptr(), frames, xp.stride(0), C.byref(ps), dc.data_ptr(), n, gains.data_ptr(),
+                                                        out.data_ptr(), work.data_ptr(), nbytes.value, R.torch_stream_ptr(xp)),
+                    "vnd_vn_stereo_rms_objective_dev")
+        return out, gains
+    out = np.empty((n, N.OBJ_SLOTS), dtype=np.float64)
+    gains = np.empty((n, 2), dtype=np.float32)
+    ps = prog.host_struct()
+    N.check(lib.vnd_vn_stereo_rms_objective_host(R.HostContext.get().handle, xp.ctypes.data, frames, xp.shape[1], C.byref(ps), cands.ctypes.data, n,
+                                                 gains.ctypes.data, out.ctypes.data), "vnd_vn_stereo_rms_objective_host")
+    return out, gains
+
+
+def _sums_follow_frames(x) -> bool:
+    """Whether ``decorrelate`` sums the squares of the cast input ``x`` frame by frame, as numpy's axis-0 reduction of a
+    C-order array does and as the rms family's kernel does.  A channel-planar 2-D input of more than one frame (a
+    Fortran-order array, a transposed tensor) is summed column by column in numpy's pairwise order instead; any other
+    numpy layout is copied to C order first."""
+    if x.ndim != 2 or x.shape[0] <= 1:
+        return True
+    if R.is_torch_tensor(x):
+        return not (x.stride(0) == 1 and x.stride(1) >= x.shape[0])
+    return bool(x.flags.c_contiguous) or not x.T.flags.c_contiguous
 
 
 def _haas_effect_partials(x, xp, haas_effects):
@@ -337,6 +384,37 @@ def vn_stereo_objective_partials(clip, decorrelators: Sequence[VelvetNoise]):
     for d in decorrelators:
         d._check_input(x)
     return _vn_stereo_partials(x, _planar_input(x), decorrelators)
+
+
+def vn_stereo_rms_objective_partials(clip, decorrelators: Sequence[VelvetNoise]):
+    """Partial sums of the objective, and the gains, of ``VelvetNoise`` candidates with two outputs and the default
+    normaliser ``rms_normalize`` - any ``filtered_channels``, mode LR or MS, any ``width`` - on one clip, in three
+    launches for all of them: the exact sums of squares of every candidate's output and its two gains, the objective
+    of the scaled outputs, and the combine.  No candidate's output is stored.
+
+    ``clip``: the input signal as ``decorrelate`` takes it (numpy array or CUDA tensor, mono or ``(frames, 2)``, any
+    dtype; cast with ``to_float32``), in a layout that ``decorrelate`` sums frame by frame: not channel-planar (a
+    Fortran-order array or a transposed tensor of more than one frame), whose sums numpy takes in pairwise order.  The
+    candidates must agree on whether the segment envelope is the identity ``(1.0,)``.  Each candidate's input checks run
+    first and raise what its ``decorrelate`` raises.  Returns ``(partials, gains)``: float64 ``(n_candidates, 12)`` (the
+    layout of ``vn_objective_partials``) and float32 ``(n_candidates, 2)``; numpy for numpy input, CUDA tensors enqueued
+    on torch's current stream for a CUDA tensor (nothing is downloaded).
+
+    Bit contract: ``gains[j]`` are the per-channel gains ``rms_normalize`` applies in ``decorrelators[j].decorrelate(clip)``
+    and row ``j`` of ``partials`` equals, bit for bit, the partials of that output (``vn_objective_partials`` with the
+    one-tap identity program), so ``vn_scores_from_partials`` gives the scores ``symmetry_aware_objective`` returns for
+    each candidate alone.  A filter whose halo does not fit the kernels' shared memory raises ``VndError`` with
+    ``VND_EUNSUPPORTED``."""
+    decorrelators = list(decorrelators)
+    for d in decorrelators:
+        if not _is_vn_rms_candidate(d):
+            raise ValueError("candidates must be VelvetNoise with num_outs=2, normalizer=rms_normalize, mode LR or MS and filtered_channels in (0, 1)")
+    x = _cast_input(clip)
+    for d in decorrelators:
+        d._check_input(x)
+    if not _sums_follow_frames(x):
+        raise ValueError("a channel-planar input is summed in numpy's pairwise order, which this call does not reproduce; pass it in C order")
+    return _vn_stereo_rms_partials(x, _planar_input(x), decorrelators)
 
 
 def haas_effect_objective_partials(clip, haas_effects: Sequence[HaasEffect]):
@@ -512,6 +590,16 @@ def _is_vn_stereo_candidate(d) -> bool:
     )
 
 
+def _is_vn_rms_candidate(d) -> bool:
+    """A candidate ``vn_stereo_rms_objective_partials`` scores: a ``_is_vn_stereo_candidate`` but with the default
+    normaliser (the identity check ``VelvetNoise._decorrelate`` makes)."""
+    return (
+        isinstance(d, VelvetNoise) and d.num_outs == 2 and d.normalizer is rms_normalize
+        and (_is_mode(d.mode, LayoutMode.LR) or _is_mode(d.mode, LayoutMode.MS))
+        and set(d.filtered_channels) <= {0, 1} and len(set(d.filtered_channels)) == len(tuple(d.filtered_channels))
+    )
+
+
 def _is_haas_effect_candidate(d) -> bool:
     """A candidate ``haas_effect_objective_partials`` scores: any HaasEffect whose delay a settings record holds (the
     per-candidate path reports any other delay itself)."""
@@ -577,20 +665,38 @@ def _scan(input_signal, decorrelators, kw) -> np.ndarray:
     return _scan_families(input_signal, decorrelators, kw)
 
 
+# Fewest rms-normalised velvet-noise candidates of one envelope kind that take the family route.  Below it the loop is
+# faster: the family's sums pass walks the whole clip once at about 13.5 ns a frame whatever the number of candidates
+# (measured; not profiled further), while the loop costs 2.7 ns a frame and candidate on a CUDA
+# tensor of 30 s, the cheapest case measured: about five candidates' worth (B200 at 1000 W; tools/bench_objective_rms.py,
+# profiles/r11_objective_rms.json).  Both scale with the clip's length, so the threshold is a candidate count.
+_RMS_FAMILY_MIN = 6
+
+
 def _scan_families(input_signal, decorrelators, kw) -> np.ndarray:
     """Scores of any candidate list: the velvet-noise stereo candidates in one launch per envelope kind
-    (``_vn_stereo_partials``), the Haas effects in one launch (``_haas_effect_partials``), every other candidate run and
-    scored on its own (``_score_signal``); each score is the one that candidate alone gets, in list order.  Every
-    candidate's input check runs before any device work, so the first exception is the one the candidate-by-candidate
-    loop raises."""
+    (``_vn_stereo_partials``), groups of at least ``_RMS_FAMILY_MIN`` rms-normalised ones in three launches per envelope
+    kind (``_vn_stereo_rms_partials``), the Haas effects in one launch (``_haas_effect_partials``), every other candidate
+    run and scored on its own (``_score_signal``); each score is the one that candidate alone gets, in list order.  Every
+    grouped candidate's input check runs before any device work, so the first exception is the one the
+    candidate-by-candidate loop raises."""
     vn = [i for i, d in enumerate(decorrelators) if _is_vn_stereo_candidate(d)]
+    rms = [i for i, d in enumerate(decorrelators) if _is_vn_rms_candidate(d)]
     haas = [i for i, d in enumerate(decorrelators) if _is_haas_effect_candidate(d)]
     cpu_tensor = R.is_torch_tensor(input_signal) and not input_signal.is_cuda  # decorrelate raises its own error for it
-    if (not vn and not haas) or cpu_tensor:
-        return np.array([_score_signal(d.decorrelate(input_signal), kw) for d in decorrelators])
-    grouped = set(vn) | set(haas)
-    others = [i for i in range(len(decorrelators)) if i not in grouped]
+    loop = lambda: np.array([_score_signal(d.decorrelate(input_signal), kw) for d in decorrelators])  # noqa: E731
+    if (not vn and not haas and len(rms) < _RMS_FAMILY_MIN) or cpu_tensor:
+        return loop()
     x = _cast_input(input_signal)
+    rms_groups: dict = {}
+    if len(rms) >= _RMS_FAMILY_MIN and _sums_follow_frames(x):
+        for i in rms:
+            rms_groups.setdefault(decorrelators[i].tap_program(x.shape[0]).apply_gain, []).append(i)
+        rms_groups = {g: idx for g, idx in rms_groups.items() if len(idx) >= _RMS_FAMILY_MIN}
+    if not vn and not haas and not rms_groups:
+        return loop()
+    grouped = set(vn) | set(haas) | {i for idx in rms_groups.values() for i in idx}
+    others = [i for i in range(len(decorrelators)) if i not in grouped]
     for i, d in enumerate(decorrelators):
         if i not in grouped:
             continue
@@ -606,13 +712,15 @@ def _scan_families(input_signal, decorrelators, kw) -> np.ndarray:
     by_gain: dict = {}
     for i in vn:
         by_gain.setdefault(decorrelators[i].tap_program(x.shape[0]).apply_gain, []).append(i)
-    for idx in by_gain.values():
+    families = [(idx, lambda c: _vn_stereo_partials(x, xp, c)) for idx in by_gain.values()]
+    families += [(idx, lambda c: _vn_stereo_rms_partials(x, xp, c)[0]) for idx in rms_groups.values()]
+    for idx, partials in families:
         try:
-            s = vn_scores_from_partials(_vn_stereo_partials(x, xp, [decorrelators[i] for i in idx]), **kw)
+            s = vn_scores_from_partials(partials([decorrelators[i] for i in idx]), **kw)
         except N.VndError as e:
             if e.status != N.VND_EUNSUPPORTED:
                 raise
-            others.extend(idx)  # a halo beyond the kernel's shared memory: candidate by candidate
+            others.extend(idx)  # a halo beyond the kernels' shared memory: candidate by candidate
             continue
         for i, v in zip(idx, s):
             scores[i] = v
